@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the B200 audio hot path (BASELINE.json metric:
 audio-seconds processed per second; HBM GB/s vs measured peak; CPU path timed beside it).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the fused pipeline (downmix -> resample -> STFT -> log-mel, PCM and
@@ -33,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [os.path.join(ROOT, "audio-flow-rs_b200"), os.path.join(ROOT, "oracle")]
+sys.dont_write_bytecode = True      # the bench writes nothing into the tree it runs from (which may be read-only)
 
 STREAMS_PER_GPU = 256
 SECONDS = 30.0
@@ -43,6 +44,7 @@ BYTES_PER_AUDIO_S = RATE * 1 * 4 + 16000 * 4 + 100 * N_MELS * 4          # 28800
 BYTES_PER_AUDIO_S_VAD = BYTES_PER_AUDIO_S + 100                          # + u8 VAD state per frame
 WORKLOAD = "cfg2: 256 x 30 s 48 kHz mono f32 streams per GPU -> 16 kHz PCM + 25/10 ms STFT + 80-bin log-mel"
 PRE_MS = float(os.environ.get("AF_BENCH_PRE_MS", "50"))   # untimed load in front of a timed window (0 under ncu: fixed launch counts)
+DUMP_STREAMS = 16     # --dump-outputs: whole streams of a fixed, seeded sample of the batch (16 x 2.88 MB; all 256 are 737 MB)
 
 
 def config_dict(world: int, variant: str = "auto") -> dict:
@@ -356,6 +358,19 @@ class Env:
         return ms_max, [round(v / steps, 4) for v in per_rank], launches, (sampler.summary() if sampler else None)
 
 
+def dump_outputs(out_dir: str, b, pcm, lm):
+    """What a caller of the timed cfg2 step holds after its last step: the 16 kHz PCM [k, n_out] and the log-mel
+    [k, T, N_MELS] of DUMP_STREAMS streams picked with a fixed seed (sorted batch rows), as float32 .npy files.  The inputs
+    are seeded too, so two builds of the library run with the same arguments can be compared output for output."""
+    import torch
+    rows = np.sort(np.random.default_rng(0).choice(STREAMS_PER_GPU, DUMP_STREAMS, replace=False))
+    n_out, T = int(b.n_out[0]), int(b.n_feat[0])          # every stream of the batch has the same length
+    idx = torch.as_tensor(rows, device=pcm.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pcm.npy"), pcm[idx, :n_out].cpu().numpy())
+    np.save(os.path.join(out_dir, "logmel.npy"), lm[idx, :T * N_MELS].reshape(len(rows), T, N_MELS).cpu().numpy())
+
+
 def measure_cfg2(env: Env, steps: int, warmup: int):
     """The contract line: cfg2 per GPU, VAD off, no collective; then the same with the VAD on and -- at N > 1 -- the
     gather of the VAD states inside the library."""
@@ -378,6 +393,8 @@ def measure_cfg2(env: Env, steps: int, warmup: int):
     ms, per_rank, launches, clocks = env.timed(step, steps, warmup, clocks=True)
     if args.pipe_stats:
         pipe_stats_print()
+    if args.dump_outputs and env.rank == 0:
+        dump_outputs(args.dump_outputs, b, pcm, lm)      # before the runs below reuse pcm / lm
     res = {"ms_per_step": ms / steps, "per_rank": per_rank, "launches": launches, "clocks": clocks, "x": x, "pipe": pipe,
            "lm": lm, "batch": b}
     if not args.quick:
@@ -683,7 +700,14 @@ def main():
                     help="print the fused kernel's per-role wait cycles (needs AF_GPU_LIB=.../libaudioflow_gpu_stats.so)")
     ap.add_argument("--workload", default="all", choices=["all", "cfg2", "cfg3", "cfg4", "cfg5"],
                     help="all = the contract line (cfg2) carrying the other configs as keys; cfgN = that config's object alone")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed cfg2 steps, write the PCM and log-mel of their last step (rank 0, a fixed sample of "
+                         f"{DUMP_STREAMS} streams) as DIR/pcm.npy and DIR/logmel.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload not in ("all", "cfg2")):
+        ap.error("--dump-outputs writes the outputs of the cfg2 line: not with --impl reference or --workload cfg3/cfg4/cfg5")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference_arm(args)
