@@ -71,6 +71,15 @@ class OutputsC(C.Structure):
                 ("vad_final", C.c_void_p)]
 
 
+class WireConfigC(C.Structure):
+    _fields_ = [("gate", C.c_uint32), ("pcm16", C.c_uint32), ("base64", C.c_uint32), ("mem", C.c_int32)]
+
+
+class WireTickC(C.Structure):
+    _fields_ = [("n_samples", C.c_uint32), ("n_chars", C.c_uint32), ("continued", C.c_uint32), ("started", C.c_uint16),
+                ("ended", C.c_uint16), ("in_speech", C.c_uint8), ("pad", C.c_uint8 * 3)]
+
+
 AF_MAX_GPUS = 16
 
 
@@ -159,6 +168,9 @@ def load_library():
         "af_session_reset": (C.c_int, [vp]),
         "af_session_enable_levels": (C.c_int, [vp, C.c_int]),
         "af_session_levels": (C.c_int, [vp, fp, fp, u8p]),
+        "af_session_enable_wire": (C.c_int, [vp, C.POINTER(WireConfigC)]),
+        "af_session_wire": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(vp), C.POINTER(C.c_uint64),
+                                      C.POINTER(WireTickC), C.POINTER(C.c_uint64)]),
         "af_ring_create": (C.c_int, [sz, C.POINTER(vp)]), "af_ring_destroy": (None, [vp]),
         "af_ring_capacity": (sz, [vp]), "af_ring_write": (sz, [vp, fp, sz]),
         "af_ring_read": (C.c_int, [vp, fp, sz, szp]), "af_ring_available": (sz, [vp]), "af_ring_clear": (None, [vp]),
@@ -650,6 +662,7 @@ class Session:
         max_frames = max_tick_samples // channels
         self.max_pcm = load_library().af_resample_max_output(sample_rate, 16000, max_frames + 128) + 8
         self.max_T = self.max_pcm // 160 + 4
+        self.wire_mem = None                            # where the wire rows live (enable_wire)
 
     def __del__(self):
         if getattr(self, "_h", None) and _lib is not None:
@@ -701,6 +714,41 @@ class Session:
         arr = (C.c_void_p * self.S)(*[r._h for r in rings])
         L = load_library()
         return self._tick(lambda o, a, b, c: L.af_session_push_rings(self._h, arr, n_samples, o, a, b, c))
+
+    def enable_wire(self, gate: bool, pcm16: bool = True, base64: bool = True, mem: int = AF_MEM_HOST):
+        """Per-tick wire payloads (WebSocketClient::send_audio, websocket.rs:244-254); gate: speech frames only.
+        gate=None switches the output off."""
+        L = load_library()
+        if gate is None:
+            _check(L.af_session_enable_wire(self._h, None))
+            self.wire_mem = None
+            return
+        cfg = WireConfigC(int(gate), int(pcm16), int(base64), mem)
+        _check(L.af_session_enable_wire(self._h, C.byref(cfg)))
+        self.wire_mem = mem
+
+    def wire(self) -> dict:
+        """The payloads of the last push: {"first_frame", "streams": [per stream {pcm16: int16[n], base64: bytes, started,
+        ended, in_speech, continued, n_samples, n_chars}]}.  With AF_MEM_DEVICE rows, pcm16 / base64 are None and the device
+        rows are reported as "pcm16_ptr", "pcm16_stride" (elements), "base64_ptr", "base64_stride" (bytes)."""
+        p, ps, b, bs, ff = C.c_void_p(), C.c_uint64(0), C.c_void_p(), C.c_uint64(0), C.c_uint64(0)
+        ticks = (WireTickC * self.S)()
+        _check(load_library().af_session_wire(self._h, C.byref(p), C.byref(ps), C.byref(b), C.byref(bs), ticks, C.byref(ff)))
+        host = self.wire_mem == AF_MEM_HOST
+        streams = []
+        for k, t in enumerate(ticks):
+            r = {"started": int(t.started), "ended": int(t.ended), "in_speech": bool(t.in_speech), "continued": int(t.continued),
+                 "n_samples": int(t.n_samples), "n_chars": int(t.n_chars), "pcm16": None, "base64": None}
+            if host and p.value:
+                r["pcm16"] = np.ctypeslib.as_array((C.c_int16 * t.n_samples).from_address(p.value + 2 * k * ps.value)).copy() \
+                    if t.n_samples else np.zeros(0, np.int16)
+            if host and b.value:
+                r["base64"] = C.string_at(b.value + k * bs.value, t.n_chars)
+            streams.append(r)
+        out = {"first_frame": int(ff.value), "streams": streams}
+        if not host:
+            out.update(pcm16_ptr=p.value, pcm16_stride=int(ps.value), base64_ptr=b.value, base64_stride=int(bs.value))
+        return out
 
 
 # ---------------------------------------------------------------------------------------------

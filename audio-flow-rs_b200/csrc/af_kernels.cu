@@ -1035,23 +1035,114 @@ __device__ __forceinline__ uint32_t b64_char(uint32_t v)      // standard alphab
 {
     return v < 26u ? 'A' + v : (v < 52u ? 'a' + (v - 26u) : (v < 62u ? '0' + (v - 52u) : (v == 62u ? '+' : '/')));
 }
+// the 4 characters of 3-byte group g of a stream of n_bytes little-endian PCM16 bytes: bytes 3g, 3g+1, 3g+2, where byte k
+// is the low (k even) or high half of sample k / 2; a and b are the PCM16 samples 3g / 2 and 3g / 2 + 1 (b = 0 past the end)
+__device__ __forceinline__ uint32_t b64_quad(uint32_t a, uint32_t b, uint64_t g, uint64_t n_bytes)
+{
+    const uint64_t k0 = 3 * g;
+    // 32 bits of the stream starting at sample k0 / 2 (little endian), shifted to byte k0
+    const uint32_t w = (a | (b << 16)) >> (8 * (uint32_t)(k0 & 1));
+    const uint32_t left = (uint32_t)(n_bytes - k0 < 3 ? n_bytes - k0 : 3);          // bytes of this group that exist
+    const uint32_t b0 = w & 0xffu, b1 = left > 1 ? (w >> 8) & 0xffu : 0u, b2 = left > 2 ? (w >> 16) & 0xffu : 0u;
+    const uint32_t t = (b0 << 16) | (b1 << 8) | b2;
+    const uint32_t c0 = b64_char(t >> 18), c1 = b64_char((t >> 12) & 63u);
+    const uint32_t c2 = left > 1 ? b64_char((t >> 6) & 63u) : '=', c3 = left > 2 ? b64_char(t & 63u) : '=';
+    return c0 | (c1 << 8) | (c2 << 16) | (c3 << 24);
+}
 __global__ void af_pcm16_base64_kernel(const float *__restrict__ in, uint64_t n, uint32_t *__restrict__ out4)
 {
     const uint64_t n_bytes = 2 * n, n_groups = (n_bytes + 2) / 3;
     for (uint64_t g = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; g < n_groups; g += (uint64_t)gridDim.x * blockDim.x) {
-        // bytes 3g, 3g+1, 3g+2 of the little-endian sample stream: byte k is the low (k even) or high half of sample k / 2
-        const uint64_t k0 = 3 * g, s0 = k0 >> 1;
+        const uint64_t s0 = (3 * g) >> 1;
         const uint32_t a = pcm16_of(in[s0]);
         const uint32_t b = s0 + 1 < n ? pcm16_of(in[s0 + 1]) : 0u;
-        // 32 bits of the stream starting at sample s0 (little endian), shifted to byte k0
-        const uint32_t w = (a | (b << 16)) >> (8 * (uint32_t)(k0 & 1));
-        const uint32_t left = (uint32_t)(n_bytes - k0 < 3 ? n_bytes - k0 : 3);          // bytes of this group that exist
-        const uint32_t b0 = w & 0xffu, b1 = left > 1 ? (w >> 8) & 0xffu : 0u, b2 = left > 2 ? (w >> 16) & 0xffu : 0u;
-        const uint32_t t = (b0 << 16) | (b1 << 8) | b2;
-        const uint32_t c0 = b64_char(t >> 18), c1 = b64_char((t >> 12) & 63u);
-        const uint32_t c2 = left > 1 ? b64_char((t >> 6) & 63u) : '=', c3 = left > 2 ? b64_char(t & 63u) : '=';
-        out4[g] = c0 | (c1 << 8) | (c2 << 16) | (c3 << 24);
+        out4[g] = b64_quad(a, b, g, n_bytes);
     }
+}
+
+// ---- session wire output (websocket.rs:244-254 per tick; gated: specs/0001-spec.md:466) ----
+// One CTA per stream (grid.x).  Gated, the CTA first lists the tick's kept frames -- the frames of af_vad_segments'
+// segments: Speech, or Ending right after Speech -- with ballots and a block scan per 128 frames (T reaches thousands
+// with a small custom hop), counting segment starts / closes on the way; payload sample i is then sample
+// kept[i / hop] * hop + i % hop of the tick's 16 kHz row.  Ungated, sample i is the tick's new sample i.  Then the PCM16
+// row (two samples per 32-bit store), the base64 row (one 3-byte group = 4 characters per 32-bit store) and the record.
+constexpr uint32_t WIRE_THREADS = 128;
+constexpr uint32_t VAD_SPEECH = 1, VAD_ENDING = 2;             // AF_VAD_SPEECH, AF_VAD_ENDING
+__device__ __forceinline__ float wire_sample(const WireJob &J, const float *row, const uint16_t *kept, uint32_t i)
+{
+    return J.gate ? row[(uint32_t)kept[i / J.hop] * J.hop + i % J.hop] : row[J.y_new + i];
+}
+__global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const WireJob J)
+{
+    extern __shared__ uint16_t s_kept[];                         // gated: the kept frames of the tick, in order
+    __shared__ uint32_t s_warp[WIRE_THREADS / 32];
+    __shared__ uint32_t s_break;                                 // first frame that is not Speech (T if none)
+    const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const float *row = J.y + (uint64_t)s * J.y_stride;
+    const uint8_t *st = J.states ? J.states + (uint64_t)s * J.st_stride : nullptr;
+    const uint32_t T = st ? J.T : 0u;
+    const uint32_t prev = J.prev[s];
+    if (t == 0) s_break = T;
+    __syncthreads();
+    uint32_t kept = 0, started = 0, ended = 0;
+    for (uint32_t base = 0; base < T; base += WIRE_THREADS) {   // (uniform trip count: every lane takes the ballots)
+        const uint32_t f = base + t;
+        const bool valid = f < T;
+        const uint32_t cur = valid ? st[f] : 0u, pre = valid ? (f ? st[f - 1] : prev) : 0u;
+        const bool sp = cur == VAD_SPEECH, psp = pre == VAD_SPEECH;
+        const bool keep = valid && (sp || (cur == VAD_ENDING && psp));
+        if (valid && !sp) atomicMin(&s_break, f);
+        const uint32_t bal = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        started += __syncthreads_count(valid && sp && !psp);    // (the barrier also publishes s_warp)
+        ended += __syncthreads_count(valid && psp && !sp);
+        uint32_t off = kept, all = 0;
+#pragma unroll
+        for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { off += w < warp ? s_warp[w] : 0u; all += s_warp[w]; }
+        if (J.gate && keep) s_kept[off + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)f;
+        kept += all;
+        __syncthreads();                                         // s_warp is rewritten by the next round
+    }
+    const uint32_t brk = s_break;
+    const uint32_t n = J.gate ? kept * J.hop : J.n_new;
+    if (J.pcm16) {
+        uint32_t *dst = reinterpret_cast<uint32_t *>(J.pcm16 + (uint64_t)s * J.pcm16_stride);
+        for (uint32_t j = t; 2 * j < n; j += WIRE_THREADS) {
+            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, 2 * j));
+            const uint32_t b = 2 * j + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, 2 * j + 1)) : 0u;
+            dst[j] = a | (b << 16);
+        }
+    }
+    const uint32_t n_bytes = 2 * n, n_groups = (n_bytes + 2) / 3;
+    if (J.b64) {
+        uint32_t *dst = reinterpret_cast<uint32_t *>(J.b64 + (uint64_t)s * J.b64_stride);
+        for (uint32_t g = t; g < n_groups; g += WIRE_THREADS) {
+            const uint32_t s0 = (3 * g) >> 1;
+            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, s0));
+            const uint32_t b = s0 + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, s0 + 1)) : 0u;
+            dst[g] = b64_quad(a, b, g, n_bytes);
+        }
+    }
+    if (t == 0) {
+        // the segment open when the tick began runs on through its Speech frames and the Ending frame closing it
+        uint32_t cont = 0;
+        if (J.gate && prev == VAD_SPEECH) cont = brk < T ? brk + (st[brk] == VAD_ENDING ? 1u : 0u) : T;
+        const uint32_t last = T ? st[T - 1] : prev;
+        WireTick r;
+        r.n_samples = n; r.n_chars = J.b64 ? 4 * n_groups : 0u; r.continued = cont * J.hop;
+        r.started = (uint16_t)started; r.ended = (uint16_t)ended; r.in_speech = last == VAD_SPEECH ? 1 : 0;
+        r.pad[0] = r.pad[1] = r.pad[2] = 0;
+        J.ticks[s] = r;
+        J.prev[s] = (uint8_t)last;
+    }
+}
+
+cudaError_t launch_session_wire(const WireJob &J, cudaStream_t st)
+{
+    if (J.n_streams == 0) return cudaSuccess;
+    const size_t smem = J.gate && J.states ? ((size_t)J.T * sizeof(uint16_t) + 3) & ~(size_t)3 : 0;
+    af_session_wire_kernel<<<J.n_streams, WIRE_THREADS, smem, st>>>(J);
+    return cudaGetLastError();
 }
 
 // the same over the rows of a batch: in [rows][in_stride] f32 -> out [rows][out_stride] i16, `width` samples per row

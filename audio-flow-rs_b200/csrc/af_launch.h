@@ -72,6 +72,25 @@ struct GateJob {             // VAD-gated compaction (all device pointers)
 };
 cudaError_t launch_vad_gate(const GateJob &job, cudaStream_t st);
 
+struct WireTick {            // af_wire_tick (static_assert'ed in af_runtime.cu)
+    uint32_t n_samples, n_chars, continued;
+    uint16_t started, ended;
+    uint8_t in_speech, pad[3];
+};
+
+struct WireJob {             // a session tick's wire payloads (all device pointers)
+    const float *y; uint64_t y_stride;               // 16 kHz rows: frame f of the tick starts at y[f * hop]
+    uint32_t y_new, n_new;                           // the tick's new samples are y[y_new, y_new + n_new)
+    const uint8_t *states; uint64_t st_stride;       // VadState of the tick's T frames (nullptr: no VAD, or T == 0)
+    uint32_t T, hop, gate;
+    uint8_t *prev;                                   // per stream: state of the latest completed frame, carried across ticks
+    int16_t *pcm16; uint64_t pcm16_stride;           // (or nullptr)
+    char *b64; uint64_t b64_stride;                  // (or nullptr; stride a multiple of 4)
+    WireTick *ticks;
+    uint32_t n_streams;
+};
+cudaError_t launch_session_wire(const WireJob &job, cudaStream_t st);
+
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st);

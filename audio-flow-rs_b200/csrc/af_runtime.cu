@@ -1372,7 +1372,36 @@ struct af_session {
     bool levels = false, levels_valid = false;
     float *d_peak = nullptr, *h_peak = nullptr;
     VadState *h_vad = nullptr;
+    // wire output (af_session_enable_wire): device rows written by the wire kernel, pinned host copies for AF_MEM_HOST
+    uint64_t max_new_y = 0;                                   // bound of the 16 kHz samples one tick produces
+    bool wire = false, wire_valid = false;
+    af_wire_config wire_cfg{};
+    uint8_t *d_wire_prev = nullptr;                           // per stream: state of the latest completed frame
+    int16_t *d_wire_pcm16 = nullptr, *h_wire_pcm16 = nullptr; uint64_t wire_pcm16_stride = 0;   // int16_t elements
+    char *d_wire_b64 = nullptr, *h_wire_b64 = nullptr; uint64_t wire_b64_stride = 0;            // bytes
+    uint64_t wire_cap = 0;                                    // payload samples a row holds
+    WireTick *d_wire_ticks = nullptr;
+    af_wire_tick *h_wire_ticks = nullptr;
+    uint64_t wire_first_frame = 0;
 };
+static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
+              offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
+
+namespace {
+void wire_free(af_session *s)
+{
+    if (s->d_wire_pcm16) cudaFree(s->d_wire_pcm16);
+    if (s->h_wire_pcm16) cudaFreeHost(s->h_wire_pcm16);
+    if (s->d_wire_b64) cudaFree(s->d_wire_b64);
+    if (s->h_wire_b64) cudaFreeHost(s->h_wire_b64);
+    if (s->d_wire_ticks) cudaFree(s->d_wire_ticks);
+    if (s->h_wire_ticks) cudaFreeHost(s->h_wire_ticks);
+    s->d_wire_pcm16 = s->h_wire_pcm16 = nullptr; s->d_wire_b64 = s->h_wire_b64 = nullptr;
+    s->d_wire_ticks = nullptr; s->h_wire_ticks = nullptr;
+    s->wire_pcm16_stride = s->wire_b64_stride = s->wire_cap = 0;
+    s->wire = s->wire_valid = false;
+}
+}  // namespace
 
 extern "C" {
 
@@ -1399,6 +1428,8 @@ AF_API void af_session_destroy(af_session *s)
     if (s->d_peak) cudaFree(s->d_peak);
     if (s->h_peak) cudaFreeHost(s->h_peak);
     if (s->h_vad) cudaFreeHost(s->h_vad);
+    wire_free(s);
+    if (s->d_wire_prev) cudaFree(s->d_wire_prev);
     delete s;
 }
 
@@ -1412,6 +1443,7 @@ AF_API int af_session_reset(af_session *s)
     s->in_base = -2 * RS_POLY;
     AF_CUDA(cudaMemset(s->in_buf[0], 0, s->S * s->in_stride * sizeof(float)));
     AF_CUDA(cudaMemset(s->d_vad, 0, s->S * sizeof(VadState)));
+    if (s->d_wire_prev) AF_CUDA(cudaMemset(s->d_wire_prev, 0, s->S));   // no segment open
     return AF_OK;
 }
 
@@ -1438,6 +1470,7 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
     if (cfg.vad_enable && cfg.vad_frame_len != 0) { s->frame_len = cfg.vad_frame_len; s->hop = cfg.vad_hop; }
     s->in_stride = round_up(2 * RS_POLY + RS_CHUNK + s->max_tick_frames + 8, 4);
     const uint64_t max_new_y = af_resample_max_output(sample_rate, OUT_RATE, s->max_tick_frames + RS_CHUNK) + 8;
+    s->max_new_y = max_new_y;
     s->y_stride = round_up(s->frame_len + s->hop + max_new_y + 8, 4);
     s->packed = s->framing && s->frame_len == WIN && s->hop == HOP;
     if (s->packed) s->y_stride = round_up(s->y_stride, HOP);           // rows a whole number of hops apart (HOP % 4 == 0)
@@ -1540,6 +1573,8 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
     const bool want_pcm = cfg.write_pcm && o->pcm && n_y_new;
     const bool want_lm = T && cfg.n_mels && o->logmel;
     const bool want_states = T && cfg.vad_enable && o->vad;
+    // the wire output needs the tick's states for its events and its gate, whatever the caller asked for
+    const bool need_states = want_states || (s->wire && T && cfg.vad_enable);
     if (want_pcm && o->pcm_stride < n_y_new) return fail(AF_ERR_CAPACITY, "pcm_stride %llu too small for %u samples", (unsigned long long)o->pcm_stride, n_y_new);
     if (want_lm && o->logmel_stride < (uint64_t)T * cfg.n_mels) return fail(AF_ERR_CAPACITY, "logmel_stride too small for %u frames", T);
     if (want_states && o->vad_stride < T) return fail(AF_ERR_CAPACITY, "vad_stride too small for %u frames", T);
@@ -1554,13 +1589,15 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
         } else { lm = o->logmel; lm_stride = o->logmel_stride; }
         if (lm_stride < (uint64_t)T * cfg.n_mels) return fail(AF_ERR_CAPACITY, "internal: log-mel staging too small for %u frames", T);
     }
-    if (want_states) {
-        if (mem == AF_MEM_HOST) {
+    if (need_states) {
+        if (mem == AF_MEM_HOST || !want_states) {
             if (!s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));
             states = s->d_states; st_stride = s->st_stride;
         } else { states = o->vad; st_stride = o->vad_stride; }
         if (st_stride < T) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", T);
     }
+    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)T * s->hop : n_y_new;   // bound of this tick's payloads
+    if (s->wire && wire_n > s->wire_cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
     const void *d_in = data;
     uint64_t d_in_stride_bytes = in_stride * bps;
     if (mem == AF_MEM_HOST && n_samples) {
@@ -1575,8 +1612,9 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
     }
 
     // From here on only CUDA failures can occur.  The bookkeeping is restored if one does (the ping-pong buffers keep
-    // the previous tick intact); the detector states on the device may already have advanced -- af_session_reset
-    // after an AF_ERR_CUDA.
+    // the previous tick intact); the detector states and the wire output's carried segment state on the device may
+    // already have advanced -- af_session_reset after an AF_ERR_CUDA.  The wire rows may hold part of the failed tick,
+    // so af_session_wire refuses them until the next push.
     struct Restore {
         af_session *s; bool armed = true;
         RsRecurrence rec; int in_cur, y_cur; uint32_t in_len, in_drop, y_len, y_drop; long long in_base; uint64_t frames_emitted;
@@ -1587,9 +1625,11 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
             if (!armed) return;
             s->rec = rec; s->in_cur = in_cur; s->y_cur = y_cur; s->in_len = in_len; s->in_drop = in_drop; s->y_len = y_len;
             s->y_drop = y_drop; s->in_base = in_base; s->frames_emitted = frames_emitted;
+            if (s->wire) s->wire_valid = false;
         }
     } restore(s);
 
+    const uint32_t y_new = s->y_len;                             // where the tick's new samples start in its 16 kHz rows
     // ---- 1. input: host ticks are staged; then carry history + residual and append the downmixed frames ----
     if (mem == AF_MEM_HOST && n_samples)
         AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)n_samples * bps, S, cudaMemcpyHostToDevice, st));
@@ -1682,10 +1722,33 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
         if (mem == AF_MEM_HOST) {
             if (lm) AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
                                               (size_t)T * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
-            if (states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, T, S, cudaMemcpyDeviceToHost, st));
+            if (want_states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, T, S, cudaMemcpyDeviceToHost, st));
             if (cfg.vad_enable && o->vad_final)
                 AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad, S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
         }
+    }
+    // ---- 5. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
+    if (s->wire) {
+        const af_wire_config &wc = s->wire_cfg;
+        WireJob wj{};
+        wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = y_new; wj.n_new = n_y_new;
+        wj.states = (T && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
+        wj.T = T; wj.hop = s->hop; wj.gate = wc.gate;
+        wj.prev = s->d_wire_prev;
+        wj.pcm16 = s->d_wire_pcm16; wj.pcm16_stride = s->wire_pcm16_stride;
+        wj.b64 = s->d_wire_b64; wj.b64_stride = s->wire_b64_stride;
+        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S;
+        AF_CUDA(launch_session_wire(wj, st));
+        count_launch();
+        if (wc.mem == AF_MEM_HOST && wire_n) {
+            if (wc.pcm16)
+                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_pcm16, s->wire_pcm16_stride * sizeof(int16_t), s->d_wire_pcm16,
+                                          s->wire_pcm16_stride * sizeof(int16_t), wire_n * sizeof(int16_t), S, cudaMemcpyDeviceToHost, st));
+            if (wc.base64)
+                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_b64, s->wire_b64_stride, s->d_wire_b64, s->wire_b64_stride,
+                                          af_pcm16_base64_len(wire_n), S, cudaMemcpyDeviceToHost, st));
+        }
+        AF_CUDA(cudaMemcpyAsync(s->h_wire_ticks, s->d_wire_ticks, S * sizeof(af_wire_tick), cudaMemcpyDeviceToHost, st));
     }
     if (s->levels) {
         AF_CUDA(cudaMemcpyAsync(s->h_peak, s->d_peak, S * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1694,8 +1757,9 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
     AF_CUDA(cudaStreamSynchronize(st));
     restore.armed = false;
     s->levels_valid = s->levels;
+    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->frames_emitted; }
 
-    // ---- 5. bookkeeping: the consumed chunks and the samples every future frame starts after are dropped by the next
+    // ---- 6. bookkeeping: the consumed chunks and the samples every future frame starts after are dropped by the next
     //         tick's ingest / resample kernels (in_drop, y_drop): no kernel and no second synchronisation here ----
     if (!s->rec.passthrough) {
         const uint32_t consumed = chunks * RS_CHUNK;              // keep [history 16 | new residual]
@@ -1751,6 +1815,67 @@ AF_API int af_session_levels(const af_session *s, float *level_db, float *peak, 
         if (level_db) level_db[k] = e <= 0.0f ? -INFINITY : 20.0f * log10f(e);
         if (is_speech) is_speech[k] = (vad && s->h_vad[k].state == 1) ? 1 : 0;          // is_speaking, vad.rs:197-199
     }
+    return AF_OK;
+}
+
+// ---- streaming wire output (websocket.rs:244-254 per tick): rows sized for the largest payload a tick can produce ----
+AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    AF_SCOPE(s->device);
+    if (!cfg) {
+        cudaDeviceSynchronize();                     // (a failed tick may still be writing the rows)
+        wire_free(s);
+        return AF_OK;
+    }
+    const af_pipeline_config &pc = s->pipe->cfg;
+    if (cfg->gate > 1) return fail(AF_ERR_INVALID, "gate must be 0 or 1");
+    if (cfg->gate && !pc.vad_enable) return fail(AF_ERR_INVALID, "the gated wire output needs the VAD (vad_enable)");
+    if (cfg->gate && s->hop > s->frame_len)
+        return fail(AF_ERR_INVALID, "the gated wire output needs vad_hop <= vad_frame_len (a completed frame's hop must have arrived)");
+    if (!cfg->pcm16 && !cfg->base64) return fail(AF_ERR_INVALID, "the wire output needs pcm16 or base64");
+    if (cfg->mem != AF_MEM_DEVICE && cfg->mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", cfg->mem);
+    cudaDeviceSynchronize();
+    wire_free(s);
+    const size_t S = s->S;
+    // ungated: the tick's new samples; gated: the hops of at most y_stride / hop + 2 frames
+    s->wire_cap = cfg->gate ? (s->y_stride / s->hop + 2) * s->hop : s->max_new_y;
+    if (cfg->pcm16) {
+        s->wire_pcm16_stride = round_up(s->wire_cap, 4);
+        AF_CUDA(cudaMalloc(&s->d_wire_pcm16, S * s->wire_pcm16_stride * sizeof(int16_t)));
+        if (cfg->mem == AF_MEM_HOST)
+            AF_CUDA(cudaHostAlloc((void **)&s->h_wire_pcm16, S * s->wire_pcm16_stride * sizeof(int16_t), cudaHostAllocDefault));
+    }
+    if (cfg->base64) {
+        s->wire_b64_stride = round_up(af_pcm16_base64_len(s->wire_cap), 4);
+        AF_CUDA(cudaMalloc(&s->d_wire_b64, S * s->wire_b64_stride));
+        if (cfg->mem == AF_MEM_HOST) AF_CUDA(cudaHostAlloc((void **)&s->h_wire_b64, S * s->wire_b64_stride, cudaHostAllocDefault));
+    }
+    AF_CUDA(cudaMalloc(&s->d_wire_ticks, S * sizeof(WireTick)));
+    AF_CUDA(cudaHostAlloc((void **)&s->h_wire_ticks, S * sizeof(af_wire_tick), cudaHostAllocDefault));
+    if (!s->d_wire_prev) {                           // the carried segment state survives a re-enable, as the detector's does
+        AF_CUDA(cudaMalloc(&s->d_wire_prev, S));
+        AF_CUDA(cudaMemset(s->d_wire_prev, 0, S));
+    }
+    if (pc.vad_enable && !s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));   // the scan's states for the kernel
+    s->wire_cfg = *cfg;
+    s->wire = true;
+    s->wire_valid = false;
+    return AF_OK;
+}
+
+AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t *pcm16_stride, const char **base64,
+                           uint64_t *base64_stride, af_wire_tick *ticks, uint64_t *first_frame)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    if (!s->wire_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire");
+    const bool host = s->wire_cfg.mem == AF_MEM_HOST;
+    if (pcm16) *pcm16 = host ? s->h_wire_pcm16 : s->d_wire_pcm16;
+    if (pcm16_stride) *pcm16_stride = s->wire_pcm16_stride;
+    if (base64) *base64 = host ? s->h_wire_b64 : s->d_wire_b64;
+    if (base64_stride) *base64_stride = s->wire_b64_stride;
+    if (ticks) memcpy(ticks, s->h_wire_ticks, s->S * sizeof(af_wire_tick));
+    if (first_frame) *first_frame = s->wire_first_frame;
     return AF_OK;
 }
 

@@ -136,6 +136,83 @@ private:
     af_ring *h_ = nullptr;
 };
 
+// af_session: n lockstep streams with their state on the GPU between ticks; outputs of a tick go to caller rows `out`
+// (af_outputs, may be null), the wire payloads and levels stay in the session until the next push.
+struct WirePayload {
+    std::vector<int16_t> pcm16;       // empty unless the PCM16 encoding is on (and the rows are host rows)
+    std::string base64;               // the "audio_base_64" field of send_audio (websocket.rs:244-254)
+    uint32_t continued = 0;
+    uint16_t started = 0, ended = 0;
+    bool in_speech = false;
+};
+struct TickCounts { std::vector<uint32_t> n_pcm, n_feat, n_vad; };
+
+class Session {
+public:
+    Session(af_pipeline *p, size_t n_streams, uint32_t sample_rate, uint16_t channels, uint16_t format, uint32_t max_tick_samples)
+        : n_(n_streams)
+    {
+        check(af_session_create(p, n_streams, sample_rate, channels, format, max_tick_samples, &h_));
+    }
+    Session(const Session &) = delete;
+    ~Session() { if (h_) af_session_destroy(h_); }
+
+    TickCounts push(const void *data, uint64_t in_stride, uint32_t n_samples, int mem, const af_outputs *out = nullptr)
+    {
+        TickCounts c{std::vector<uint32_t>(n_), std::vector<uint32_t>(n_), std::vector<uint32_t>(n_)};
+        check(af_session_push(h_, data, in_stride, n_samples, mem, out, c.n_pcm.data(), c.n_feat.data(), c.n_vad.data()));
+        return c;
+    }
+    TickCounts push_rings(std::vector<RingBuffer *> &rings, uint32_t n_samples, const af_outputs *out = nullptr)
+    {
+        std::vector<af_ring *> hs;
+        for (RingBuffer *r : rings) hs.push_back(r->handle());
+        TickCounts c{std::vector<uint32_t>(n_), std::vector<uint32_t>(n_), std::vector<uint32_t>(n_)};
+        check(af_session_push_rings(h_, hs.data(), n_samples, out, c.n_pcm.data(), c.n_feat.data(), c.n_vad.data()));
+        return c;
+    }
+    void reset() { check(af_session_reset(h_)); }
+
+    void enable_levels(bool on = true) { check(af_session_enable_levels(h_, on ? 1 : 0)); }
+    // AudioLevel{level, peak} / VolumeLevel{level, is_speech} of the last tick, per stream
+    void levels(std::vector<float> *level_db, std::vector<float> *peak, std::vector<uint8_t> *is_speech) const
+    {
+        level_db->resize(n_); peak->resize(n_); is_speech->resize(n_);
+        check(af_session_levels(h_, level_db->data(), peak->data(), is_speech->data()));
+    }
+
+    // gate: only the hops of the VAD's speech frames; mem AF_MEM_HOST (payloads copied out by wire()) or AF_MEM_DEVICE
+    void enable_wire(bool gate, bool pcm16 = true, bool base64 = true, int mem = AF_MEM_HOST)
+    {
+        const af_wire_config cfg{gate ? 1u : 0u, pcm16 ? 1u : 0u, base64 ? 1u : 0u, mem};
+        check(af_session_enable_wire(h_, &cfg));
+        wire_host_ = mem == AF_MEM_HOST;
+    }
+    void disable_wire() { check(af_session_enable_wire(h_, nullptr)); }
+    std::vector<WirePayload> wire(uint64_t *first_frame = nullptr) const
+    {
+        const int16_t *pcm = nullptr;
+        const char *b64 = nullptr;
+        uint64_t ps = 0, bs = 0;
+        std::vector<af_wire_tick> t(n_);
+        check(af_session_wire(h_, &pcm, &ps, &b64, &bs, t.data(), first_frame));
+        std::vector<WirePayload> out(n_);
+        for (size_t k = 0; k < n_; ++k) {
+            WirePayload &w = out[k];
+            if (wire_host_ && pcm) w.pcm16.assign(pcm + k * ps, pcm + k * ps + t[k].n_samples);
+            if (wire_host_ && b64) w.base64.assign(b64 + k * bs, t[k].n_chars);
+            w.continued = t[k].continued; w.started = t[k].started; w.ended = t[k].ended; w.in_speech = t[k].in_speech != 0;
+        }
+        return out;
+    }
+    af_session *handle() { return h_; }
+
+private:
+    af_session *h_ = nullptr;
+    size_t n_ = 0;
+    bool wire_host_ = true;
+};
+
 // vad.rs:8-54
 enum class VadLevel { Aggressive, Balanced, Relaxed };
 enum class VadState { Silence = 0, Speech = 1, Ending = 2 };

@@ -100,6 +100,11 @@ impl Pipeline {
     }
 }
 
+impl Pipeline {
+    /// the C handle, for the sessions of `stream.rs` built from this pipeline
+    pub(crate) fn handle(&self) -> *mut ffi::af_pipeline { self.h }
+}
+
 impl Drop for Pipeline {
     fn drop(&mut self) { unsafe { ffi::af_pipeline_destroy(self.h) } }
 }

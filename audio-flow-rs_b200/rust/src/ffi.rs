@@ -80,6 +80,46 @@ pub struct af_outputs {
 #[repr(C)] pub struct af_ring { _private: [u8; 0] }
 pub const AF_RING_EMPTY: c_int = -1;
 
+// ---- streaming sessions (audioflow_gpu.h, "streaming sessions", level metering, wire output) ----
+#[repr(C)] pub struct af_session { _p: [u8; 0] }
+
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct af_wire_config {
+    pub gate: u32,
+    pub pcm16: u32,
+    pub base64: u32,
+    pub mem: i32,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct af_wire_tick {
+    pub n_samples: u32,
+    pub n_chars: u32,
+    pub continued: u32,
+    pub started: u16,
+    pub ended: u16,
+    pub in_speech: u8,
+    pub pad: [u8; 3],
+}
+
+extern "C" {
+    pub fn af_session_create(p: *mut af_pipeline, n_streams: usize, sample_rate: u32, channels: u16, format: u16,
+                             max_tick_samples: u32, out: *mut *mut af_session) -> c_int;
+    pub fn af_session_destroy(s: *mut af_session);
+    pub fn af_session_push(s: *mut af_session, data: *const std::os::raw::c_void, in_stride: u64, n_samples: u32, mem: c_int,
+                           out: *const af_outputs, n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
+    pub fn af_session_push_rings(s: *mut af_session, rings: *const *mut af_ring, n_samples: u32, out: *const af_outputs,
+                                 n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
+    pub fn af_session_reset(s: *mut af_session) -> c_int;
+    pub fn af_session_enable_levels(s: *mut af_session, enable: c_int) -> c_int;
+    pub fn af_session_levels(s: *const af_session, level_db: *mut f32, peak: *mut f32, is_speech: *mut u8) -> c_int;
+    pub fn af_session_enable_wire(s: *mut af_session, cfg: *const af_wire_config) -> c_int;
+    pub fn af_session_wire(s: *const af_session, pcm16: *mut *const i16, pcm16_stride: *mut u64, base64: *mut *const c_char,
+                           base64_stride: *mut u64, ticks: *mut af_wire_tick, first_frame: *mut u64) -> c_int;
+}
+
 extern "C" {
     pub fn af_ring_create(capacity_samples: usize, out: *mut *mut af_ring) -> c_int;
     pub fn af_ring_destroy(r: *mut af_ring);

@@ -11,6 +11,7 @@
 //! Source only: the graft build image has no Rust toolchain (see INTEGRATION.md).
 mod ffi;
 pub mod batch;
+pub mod stream;
 
 use std::ptr;
 

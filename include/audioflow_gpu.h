@@ -351,6 +351,48 @@ AF_API int af_session_reset(af_session *s);
 AF_API int af_session_enable_levels(af_session *s, int enable);
 AF_API int af_session_levels(const af_session *s, float *level_db, float *peak, uint8_t *is_speech);
 
+/* ---- streaming wire output: what WebSocketClient::send_audio sends, per tick (websocket.rs:244-254) ----------------
+ * With the wire output enabled, every push (af_session_push, af_session_push_rings) leaves one payload per stream:
+ *   gate = 0: every 16 kHz sample the tick produced (the n_pcm samples af_session_push returns as f32);
+ *   gate = 1: only the speech (specs/0001-spec.md:466, scribe_client.rs:194-196; needs vad_enable and a VAD hop no
+ *             longer than its frame): for every VAD frame f completed in this tick that lies in a segment of
+ *             af_vad_segments -- a Speech frame, or the Ending frame that closes one -- the frame's hop, samples
+ *             [f*hop, (f+1)*hop) of the stream's 16 kHz signal, kept frames in order.  Concatenating the gated payloads
+ *             of all ticks gives af_vad_gate's PCM over the concatenated session PCM and states.  A frame completes
+ *             frame_len - hop samples after its hop ends, so the gated payload trails the newest samples by at least
+ *             that overlap (240 samples = 15 ms with the STFT frames, none with the 20 ms frames of
+ *             vad_frame_len = vad_hop = 320), plus the samples of a frame not yet complete.
+ * Encoding: PCM16 = (x.clamp(-1,1) * 32767) as i16, NaN -> 0 (websocket.rs:246-251); base64 = standard alphabet with '='
+ * padding over the little-endian bytes of THIS tick's payload alone (one send_audio call per tick), no terminator,
+ * af_pcm16_base64_len(n_samples) characters.  An empty payload has 0 samples and 0 characters.
+ * Per stream and tick an af_wire_tick (the event fields are 0 without the VAD):
+ *   started   segments whose first frame (a Speech frame whose predecessor, across ticks, is not Speech) is in the tick;
+ *   ended     segments closed by a frame of the tick: an Ending frame, or a Silence frame after a Speech frame;
+ *   in_speech the stream's latest completed frame is Speech (the tick's last frame; an earlier one if it completed none);
+ *   continued gated only: payload samples at the front that belong to the segment already open when the tick began
+ *             (the rest belongs to segments started in the tick); 0 ungated, where payloads are not frame-aligned.
+ * first_frame is the global index of the tick's first completed frame (the same for all streams).
+ * af_session_reset clears the carried segment state. */
+typedef struct af_wire_config {
+    uint32_t gate;            /* 0: every 16 kHz sample of the tick; 1: only the hops of its segment frames (needs the VAD) */
+    uint32_t pcm16;           /* produce the PCM16 samples */
+    uint32_t base64;          /* produce the base64 text of their little-endian bytes (no terminator) */
+    int32_t mem;              /* AF_MEM_HOST: session-owned pinned host rows; AF_MEM_DEVICE: device rows on the session's GPU */
+} af_wire_config;
+typedef struct af_wire_tick {
+    uint32_t n_samples, n_chars, continued;
+    uint16_t started, ended;
+    uint8_t in_speech, pad[3];
+} af_wire_tick;
+/* cfg NULL: off.  AF_ERR_INVALID for gate = 1 without the VAD (or with vad_hop > vad_frame_len), neither pcm16 nor
+ * base64, or a bad mem.  Allocates the rows: a tick's payload is bounded when the session is created. */
+AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg);
+/* The payloads of the last push: row k of pcm16 (int16 elements, stride in elements) and of base64 (bytes) holds stream
+ * k's payload; rows are NULL (stride 0) for an encoding that is off, and stay valid until the next push.  ticks: host
+ * array of n_streams (may be NULL).  AF_ERR_INVALID before the first push since af_session_enable_wire. */
+AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t *pcm16_stride, const char **base64,
+                           uint64_t *base64_stride, af_wire_tick *ticks, uint64_t *first_frame);
+
 /* ---- RingBuffer  (src-tauri/src/modules/audio/capture.rs:84-161): capture hand-off ------ */
 /* The cpal callback writes captured f32 samples, the processing task reads them.  Same semantics as the
  * reference: one slot stays free (capacity - 1 usable), a write drops what does not fit and returns the
