@@ -176,6 +176,12 @@ def load_library():
         "af_ring_read": (C.c_int, [vp, fp, sz, szp]), "af_ring_available": (sz, [vp]), "af_ring_clear": (None, [vp]),
         "af_session_push_rings": (C.c_int, [vp, C.POINTER(vp), C.c_uint32, C.POINTER(OutputsC),
                                             C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+        "af_session_push_streams": (C.c_int, [vp, vp, C.c_uint64, C.POINTER(C.c_uint32), u8p, C.c_int, C.POINTER(OutputsC),
+                                              C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+        "af_session_reset_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), sz]),
+        "af_session_push_rings_available": (C.c_int, [vp, C.POINTER(vp), C.c_uint32, u8p, C.POINTER(OutputsC),
+                                                      C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+        "af_session_wire_first_frames": (C.c_int, [vp, C.POINTER(C.c_uint64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -649,9 +655,39 @@ class ShardedBatch:
 # ---------------------------------------------------------------------------------------------
 # streaming sessions (BASELINE config 5)
 # ---------------------------------------------------------------------------------------------
+def stream_rows(xs, n_streams: int, channels: int, dtype):
+    """The rows of a ragged tick: xs[k] (1-D interleaved samples of stream k) at the start of row k of one [n_streams,
+    stride] array -> (array, uint32 counts).  ValueError before anything is pushed for a wrong stream count, a row that
+    is not 1-D, or a partial frame."""
+    if len(xs) != n_streams:
+        raise ValueError(f"{len(xs)} arrays for {n_streams} streams")
+    xs = [np.ascontiguousarray(x, dtype=dtype) for x in xs]
+    for k, x in enumerate(xs):
+        if x.ndim != 1:
+            raise ValueError(f"stream {k}: samples must be 1-D (interleaved), got shape {x.shape}")
+        if x.size % channels:
+            raise ValueError(f"stream {k}: {x.size} samples are not a whole number of {channels}-channel frames")
+    counts = np.array([x.size for x in xs], np.uint32)
+    buf = np.zeros((n_streams, max((int(counts.max()) + 3) // 4 * 4, 4)), dtype)
+    for k, x in enumerate(xs):
+        buf[k, :x.size] = x
+    return buf, counts
+
+
+def end_flags(end, n_streams: int):
+    """None, or one flag per stream as uint8 (ValueError for any other length)."""
+    if end is None:
+        return None
+    e = np.ascontiguousarray(end, dtype=bool).astype(np.uint8).reshape(-1)
+    if e.size != n_streams:
+        raise ValueError(f"{e.size} end flags for {n_streams} streams")
+    return e
+
+
 class Session:
     """n_streams lockstep streams with persistent device state (resampler position + residual input,
-    STFT overlap, VAD).  push() takes host arrays [n_streams, n_samples] and returns per-tick outputs."""
+    STFT overlap, VAD).  push() takes host arrays [n_streams, n_samples] and returns per-tick outputs.
+    push_streams() / push_rings_available() / reset_streams() give every stream its own timeline."""
 
     def __init__(self, pipe: Pipeline, n_streams: int, sample_rate: int, channels: int = 1, fmt: int = AF_FMT_F32,
                  max_tick_samples: int = 4096):
@@ -672,7 +708,7 @@ class Session:
     def reset(self):
         _check(load_library().af_session_reset(self._h))
 
-    def _tick(self, call) -> dict:
+    def _run(self, call):
         cfg = self.pipe.cfg
         M = max(cfg.n_mels, 1)
         pcm = np.zeros((self.S, (self.max_pcm + 3) // 4 * 4), np.float32)
@@ -685,13 +721,33 @@ class Session:
         u32p = C.POINTER(C.c_uint32)
         npcm, nf, nv = (np.zeros(self.S, np.uint32) for _ in range(3))
         _check(call(C.byref(o), npcm.ctypes.data_as(u32p), nf.ctypes.data_as(u32p), nv.ctypes.data_as(u32p)))
+        final = [dict(state=int(f.state), smoothed=float(f.smoothed_energy), speech_frames=int(f.speech_frames)) for f in fin]
+        return pcm, lm, vad, npcm, nf, nv, final, M
+
+    def _tick(self, call) -> dict:
+        """Lockstep form: [n_streams, n] arrays.  When the streams emitted different counts (their timelines have
+        diverged through push_streams / reset_streams), the per-stream form of push_streams instead: r["pcm"][k] etc. are
+        stream k's own outputs either way."""
+        pcm, lm, vad, npcm, nf, nv, final, M = self._run(call)
+        if (npcm != npcm[0]).any() or (nf != nf[0]).any() or (nv != nv[0]).any():
+            return self._per_stream(pcm, lm, vad, npcm, nf, nv, final, M)
         T = int(max(nf[0], nv[0]))
         return {"pcm": pcm[:, :npcm[0]].copy(), "logmel": lm[:, :int(nf[0]) * M].reshape(self.S, int(nf[0]), M).copy(),
-                "vad": vad[:, :int(nv[0])].copy(), "n_frames": T,
-                "vad_final": [dict(state=int(f.state), smoothed=float(f.smoothed_energy), speech_frames=int(f.speech_frames))
-                              for f in fin]}
+                "vad": vad[:, :int(nv[0])].copy(), "n_frames": T, "vad_final": final}
+
+    def _tick_streams(self, call) -> dict:
+        return self._per_stream(*self._run(call))
+
+    def _per_stream(self, pcm, lm, vad, npcm, nf, nv, final, M) -> dict:
+        """Per-stream lists: stream k's own pcm / logmel [n_feat[k], n_mels] / vad, the counts and vad_final."""
+        return {"pcm": [pcm[k, :npcm[k]].copy() for k in range(self.S)],
+                "logmel": [lm[k, :int(nf[k]) * M].reshape(int(nf[k]), M).copy() for k in range(self.S)],
+                "vad": [vad[k, :nv[k]].copy() for k in range(self.S)],
+                "n_pcm": npcm, "n_feat": nf, "n_vad": nv, "vad_final": final}
 
     def push(self, x: np.ndarray) -> dict:
+        """Every stream pushes x[k]; on a session whose streams have diverged the result may take the per-stream form
+        (see _tick)."""
         x = np.ascontiguousarray(x, dtype=np.int16 if self.fmt == AF_FMT_I16 else np.float32)
         assert x.ndim == 2 and x.shape[0] == self.S
         n = x.shape[1]
@@ -715,6 +771,32 @@ class Session:
         L = load_library()
         return self._tick(lambda o, a, b, c: L.af_session_push_rings(self._h, arr, n_samples, o, a, b, c))
 
+    def push_streams(self, xs, end=None) -> dict:
+        """One tick in which stream k pushes xs[k] (1-D interleaved samples, any whole number of frames, 0 included); end[k]
+        ends stream k after them (BatchResampler::flush), its next push starts afresh.  Returns per-stream lists."""
+        buf, counts = stream_rows(xs, self.S, self.channels, np.int16 if self.fmt == AF_FMT_I16 else np.float32)
+        e = end_flags(end, self.S)
+        L = load_library()
+        u32p = C.POINTER(C.c_uint32)
+        return self._tick_streams(lambda o, a, b, c: L.af_session_push_streams(
+            self._h, buf.ctypes.data, buf.shape[1], counts.ctypes.data_as(u32p),
+            e.ctypes.data_as(C.POINTER(C.c_uint8)) if e is not None else None, AF_MEM_HOST, o, a, b, c))
+
+    def reset_streams(self, ids):
+        """Streams `ids` start afresh at their next push, without a flush; the others are untouched."""
+        a = np.ascontiguousarray(ids, dtype=np.uint32).reshape(-1)
+        _check(load_library().af_session_reset_streams(self._h, a.ctypes.data_as(C.POINTER(C.c_uint32)), a.size))
+
+    def push_rings_available(self, rings, max_samples: int, end=None) -> dict:
+        """AudioCapturer::read_frame(max) for every stream: min(max_samples, available) whole frames from each ring."""
+        if len(rings) != self.S:
+            raise ValueError(f"{len(rings)} rings for {self.S} streams")
+        e = end_flags(end, self.S)
+        arr = (C.c_void_p * self.S)(*[r._h for r in rings])
+        L = load_library()
+        return self._tick_streams(lambda o, a, b, c: L.af_session_push_rings_available(
+            self._h, arr, max_samples, e.ctypes.data_as(C.POINTER(C.c_uint8)) if e is not None else None, o, a, b, c))
+
     def enable_wire(self, gate: bool, pcm16: bool = True, base64: bool = True, mem: int = AF_MEM_HOST):
         """Per-tick wire payloads (WebSocketClient::send_audio, websocket.rs:244-254); gate: speech frames only.
         gate=None switches the output off."""
@@ -728,7 +810,8 @@ class Session:
         self.wire_mem = mem
 
     def wire(self) -> dict:
-        """The payloads of the last push: {"first_frame", "streams": [per stream {pcm16: int16[n], base64: bytes, started,
+        """The payloads of the last push: {"first_frame", "first_frames" (uint64[n_streams]: each stream's first completed
+        frame in its own frame sequence), "streams": [per stream {pcm16: int16[n], base64: bytes, started,
         ended, in_speech, continued, n_samples, n_chars}]}.  With AF_MEM_DEVICE rows, pcm16 / base64 are None and the device
         rows are reported as "pcm16_ptr", "pcm16_stride" (elements), "base64_ptr", "base64_stride" (bytes)."""
         p, ps, b, bs, ff = C.c_void_p(), C.c_uint64(0), C.c_void_p(), C.c_uint64(0), C.c_uint64(0)
@@ -745,7 +828,9 @@ class Session:
             if host and b.value:
                 r["base64"] = C.string_at(b.value + k * bs.value, t.n_chars)
             streams.append(r)
-        out = {"first_frame": int(ff.value), "streams": streams}
+        ffs = np.zeros(self.S, np.uint64)
+        _check(load_library().af_session_wire_first_frames(self._h, ffs.ctypes.data_as(C.POINTER(C.c_uint64))))
+        out = {"first_frame": int(ff.value), "first_frames": ffs, "streams": streams}
         if not host:
             out.update(pcm16_ptr=p.value, pcm16_stride=int(ps.value), base64_ptr=b.value, base64_stride=int(bs.value))
         return out

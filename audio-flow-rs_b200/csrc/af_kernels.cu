@@ -939,16 +939,18 @@ __device__ __forceinline__ float session_resample_one(const SessionResample &J, 
     return interp_cubic(frac, y[0], y[1], y[2], y[3]);
 }
 
-__global__ void __launch_bounds__(256) af_session_tick_kernel(const SessionIngest I, const SessionResample R)
+// zero_history: the 16 retained frames are a fresh stream's zero history; pcm (or nullptr): the new samples also go there
+__device__ __forceinline__ void session_tick_row(const SessionIngest &I, const SessionResample &R, uint32_t s, bool zero_history,
+                                                 float *pcm)
 {
-    const uint32_t s = blockIdx.x;
     {
         const float *old = I.old_buf + (uint64_t)s * I.buf_stride;
         float *neu = I.new_buf + (uint64_t)s * I.buf_stride;
         const char *in = reinterpret_cast<const char *>(I.input) + (uint64_t)s * I.in_stride_bytes;
         const uint32_t total = I.keep + I.n_new_frames;
         for (uint32_t i = threadIdx.x; i < total; i += blockDim.x)
-            neu[i] = i < I.keep ? old[I.drop + i] : load_mono(in, I.n_samples, I.n_new_frames, I.channels, I.format, (int)(i - I.keep));
+            neu[i] = i < I.keep ? (zero_history ? 0.0f : old[I.drop + i])
+                                : load_mono(in, I.n_samples, I.n_new_frames, I.channels, I.format, (int)(i - I.keep));
     }
     __syncthreads();                                   // the row written above is read below by other threads of this CTA
     {
@@ -956,15 +958,57 @@ __global__ void __launch_bounds__(256) af_session_tick_kernel(const SessionInges
         const float *yold = R.y_old + (uint64_t)s * R.y_stride;
         float *ynew = R.y_new + (uint64_t)s * R.y_stride;
         const uint32_t total = R.y_keep + (uint32_t)(R.n_end - R.n_begin);
-        for (uint32_t i = threadIdx.x; i < total; i += blockDim.x)
-            ynew[i] = i < R.y_keep ? yold[R.y_drop + i] : session_resample_one(R, in, i - R.y_keep);
+        if (!pcm) {
+            for (uint32_t i = threadIdx.x; i < total; i += blockDim.x)
+                ynew[i] = i < R.y_keep ? yold[R.y_drop + i] : session_resample_one(R, in, i - R.y_keep);
+        } else {
+            for (uint32_t i = threadIdx.x; i < total; i += blockDim.x) {
+                if (i < R.y_keep) { ynew[i] = yold[R.y_drop + i]; continue; }
+                const float v = session_resample_one(R, in, i - R.y_keep);
+                ynew[i] = v;
+                pcm[i - R.y_keep] = v;
+            }
+        }
     }
+}
+
+__global__ void __launch_bounds__(256) af_session_tick_kernel(const SessionIngest I, const SessionResample R)
+{
+    session_tick_row(I, R, blockIdx.x, false, nullptr);
 }
 
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st)
 {
     if (n_streams == 0) return cudaSuccess;
     af_session_tick_kernel<<<n_streams, 256, 0, st>>>(I, R);
+    return cudaGetLastError();
+}
+
+// independent stream timelines: the same per CTA, with the stream's own lengths and positions from its StreamTick.  A
+// restart rewrites the zero history here and clears the stream's detector and wire segment state, so it costs no launch;
+// an end's zero padding is never materialised (n_valid_end stops at the data, the reads past it return 0).
+__global__ void __launch_bounds__(256) af_session_tick_streams_kernel(SessionIngest I, SessionResample R, const StreamTick *__restrict__ tab,
+                                                                      VadState *vad, uint8_t *wire_prev, float *pcm, uint64_t pcm_stride)
+{
+    const uint32_t s = blockIdx.x;
+    const StreamTick d = tab[s];
+    I.drop = d.in_drop; I.keep = d.in_keep; I.n_new_frames = d.n_new; I.n_samples = d.n_samples;
+    R.data_base = d.data_base; R.n_valid_end = d.n_valid_end; R.n_begin = d.n_begin; R.n_end = d.n_begin + d.n_y;
+    R.frac += d.frac_off; R.y_drop = d.y_drop; R.y_keep = d.y_keep;
+    const bool restart = (d.flags & TICK_RESTART) != 0;
+    if (restart && threadIdx.x == 0) {
+        VadState v; v.smoothed = 0.0f; v.state = 0; v.silence_frames = 0; v.speech_frames = 0;
+        vad[s] = v;
+        if (wire_prev) wire_prev[s] = 0;
+    }
+    session_tick_row(I, R, s, restart, pcm ? pcm + (uint64_t)s * pcm_stride : nullptr);
+}
+
+cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab, VadState *vad,
+                                        uint8_t *wire_prev, float *pcm, uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st)
+{
+    if (n_streams == 0) return cudaSuccess;
+    af_session_tick_streams_kernel<<<n_streams, 256, 0, st>>>(I, R, tab, vad, wire_prev, pcm, pcm_stride);
     return cudaGetLastError();
 }
 
@@ -988,11 +1032,13 @@ cudaError_t launch_session_setup(StreamDev *tab, TileDev *tiles, uint32_t n_stre
 
 // ---- level metering (events/mod.rs:41 AudioLevel{level, peak}): peak = max |y| over the tick's new 16 kHz samples ----
 // One warp per stream; max is order-independent, so the result is bit-exact against any reference order.
-__global__ void af_peak_kernel(const float *__restrict__ y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *__restrict__ peak)
+__global__ void af_peak_kernel(const float *__restrict__ y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *__restrict__ peak,
+                               const StreamTick *__restrict__ tab)
 {
     const uint32_t s = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (s >= n_streams) return;
     const float *row = y + (uint64_t)s * y_stride;
+    if (tab) { row += tab[s].y_keep; n = tab[s].n_y; }
     float m = 0.0f;
     for (uint32_t i = lane; i < n; i += 32) m = fmaxf(m, fabsf(row[i]));
 #pragma unroll
@@ -1000,10 +1046,11 @@ __global__ void af_peak_kernel(const float *__restrict__ y, uint64_t y_stride, u
     if (lane == 0) peak[s] = m;
 }
 
-cudaError_t launch_peak(const float *y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *peak, cudaStream_t st)
+cudaError_t launch_peak(const float *y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *peak, cudaStream_t st,
+                        const StreamTick *tab)
 {
     if (n_streams == 0) return cudaSuccess;
-    af_peak_kernel<<<(n_streams + 3) / 4, 128, 0, st>>>(y, y_stride, n, n_streams, peak);
+    af_peak_kernel<<<(n_streams + 3) / 4, 128, 0, st>>>(y, y_stride, n, n_streams, peak, tab);
     return cudaGetLastError();
 }
 
@@ -1068,9 +1115,9 @@ __global__ void af_pcm16_base64_kernel(const float *__restrict__ in, uint64_t n,
 // row (two samples per 32-bit store), the base64 row (one 3-byte group = 4 characters per 32-bit store) and the record.
 constexpr uint32_t WIRE_THREADS = 128;
 constexpr uint32_t VAD_SPEECH = 1, VAD_ENDING = 2;             // AF_VAD_SPEECH, AF_VAD_ENDING
-__device__ __forceinline__ float wire_sample(const WireJob &J, const float *row, const uint16_t *kept, uint32_t i)
+__device__ __forceinline__ float wire_sample(const WireJob &J, const float *row, const uint16_t *kept, uint32_t y_new, uint32_t i)
 {
-    return J.gate ? row[(uint32_t)kept[i / J.hop] * J.hop + i % J.hop] : row[J.y_new + i];
+    return J.gate ? row[(uint32_t)kept[i / J.hop] * J.hop + i % J.hop] : row[y_new + i];
 }
 __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const WireJob J)
 {
@@ -1080,7 +1127,10 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
     const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const float *row = J.y + (uint64_t)s * J.y_stride;
     const uint8_t *st = J.states ? J.states + (uint64_t)s * J.st_stride : nullptr;
-    const uint32_t T = st ? J.T : 0u;
+    uint32_t T = J.T, y_new = J.y_new, n_new = J.n_new;
+    bool end = false;                                            // the stream ends after this tick: an open segment closes
+    if (J.tab) { T = J.tab[s].T; y_new = J.tab[s].y_keep; n_new = J.tab[s].n_y; end = (J.tab[s].flags & TICK_END) != 0; }
+    if (!st) T = 0;
     const uint32_t prev = J.prev[s];
     if (t == 0) s_break = T;
     __syncthreads();
@@ -1104,12 +1154,12 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
         __syncthreads();                                         // s_warp is rewritten by the next round
     }
     const uint32_t brk = s_break;
-    const uint32_t n = J.gate ? kept * J.hop : J.n_new;
+    const uint32_t n = J.gate ? kept * J.hop : n_new;
     if (J.pcm16) {
         uint32_t *dst = reinterpret_cast<uint32_t *>(J.pcm16 + (uint64_t)s * J.pcm16_stride);
         for (uint32_t j = t; 2 * j < n; j += WIRE_THREADS) {
-            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, 2 * j));
-            const uint32_t b = 2 * j + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, 2 * j + 1)) : 0u;
+            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, y_new, 2 * j));
+            const uint32_t b = 2 * j + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, y_new, 2 * j + 1)) : 0u;
             dst[j] = a | (b << 16);
         }
     }
@@ -1118,8 +1168,8 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
         uint32_t *dst = reinterpret_cast<uint32_t *>(J.b64 + (uint64_t)s * J.b64_stride);
         for (uint32_t g = t; g < n_groups; g += WIRE_THREADS) {
             const uint32_t s0 = (3 * g) >> 1;
-            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, s0));
-            const uint32_t b = s0 + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, s0 + 1)) : 0u;
+            const uint32_t a = pcm16_of(wire_sample(J, row, s_kept, y_new, s0));
+            const uint32_t b = s0 + 1 < n ? pcm16_of(wire_sample(J, row, s_kept, y_new, s0 + 1)) : 0u;
             dst[g] = b64_quad(a, b, g, n_bytes);
         }
     }
@@ -1127,7 +1177,8 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
         // the segment open when the tick began runs on through its Speech frames and the Ending frame closing it
         uint32_t cont = 0;
         if (J.gate && prev == VAD_SPEECH) cont = brk < T ? brk + (st[brk] == VAD_ENDING ? 1u : 0u) : T;
-        const uint32_t last = T ? st[T - 1] : prev;
+        uint32_t last = T ? st[T - 1] : prev;
+        if (end && last == VAD_SPEECH) { ++ended; last = 0; }     // af_vad_segments closes a segment at the last frame
         WireTick r;
         r.n_samples = n; r.n_chars = J.b64 ? 4 * n_groups : 0u; r.continued = cont * J.hop;
         r.started = (uint16_t)started; r.ended = (uint16_t)ended; r.in_speech = last == VAD_SPEECH ? 1 : 0;

@@ -58,6 +58,20 @@ struct SessionResample {
     uint32_t y_drop, y_keep;
 };
 
+// one stream's part of a tick of independent stream timelines (af_session_push_streams), planned on the host; it
+// overrides the per-stream fields of SessionIngest / SessionResample / WireJob and the peak's range
+constexpr uint32_t TICK_RESTART = 1, TICK_END = 2;
+struct StreamTick {
+    uint32_t in_drop, in_keep;                                   // ingest: retained frames old[in_drop .. in_drop + in_keep)
+    uint32_t n_new, n_samples;                                   // this tick's frames / interleaved samples of the stream
+    long long data_base, n_valid_end;                            // resample (an end: n_valid_end at the real end of the data)
+    unsigned long long n_begin;
+    uint32_t n_y, frac_off;                                      // 16 kHz samples of the tick; RS_TABLE: fractions at frac[frac_off]
+    uint32_t y_drop, y_keep;                                     // carry: y_old[y_drop .. y_drop + y_keep); new samples at y_keep
+    uint32_t T, flags;                                           // frames completed; TICK_RESTART (history zeroed, detector and
+                                                                 // wire segment cleared first) | TICK_END
+};
+
 struct GateJob {             // VAD-gated compaction (all device pointers)
     const float *pcm; uint64_t pcm_stride;           // 16 kHz rows (or nullptr)
     const float *logmel; uint64_t logmel_stride;     // [frame][mel] rows (or nullptr)
@@ -88,12 +102,17 @@ struct WireJob {             // a session tick's wire payloads (all device point
     char *b64; uint64_t b64_stride;                  // (or nullptr; stride a multiple of 4)
     WireTick *ticks;
     uint32_t n_streams;
+    const StreamTick *tab;                           // ragged tick: per-stream y_new / n_new / T and the end flag (or nullptr)
 };
 cudaError_t launch_session_wire(const WireJob &job, cudaStream_t st);
 
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st);
+// the same with every stream planned by its own StreamTick; restarted streams clear vad[s] and (if non-null) wire_prev[s];
+// pcm (device, or nullptr) receives each stream's new samples at its row start
+cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab, VadState *vad,
+                                        uint8_t *wire_prev, float *pcm, uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st);
 cudaError_t launch_session_setup(StreamDev *tab, TileDev *tiles, uint32_t n_streams, uint32_t n, uint32_t n_frames, uint32_t n_vad,
                                  cudaStream_t st);
 // split: the batch holds tiles other than 48 kHz mono f32 -> 16 kHz; such batches (and quarter-staged ones) run the
@@ -102,7 +121,9 @@ cudaError_t launch_session_setup(StreamDev *tab, TileDev *tiles, uint32_t n_stre
 cudaError_t launch_fused(const FusedParams &P, int n_ctas, cudaStream_t st, bool split = false);
 cudaError_t launch_fused_split(const FusedParams &P, int n_ctas, cudaStream_t st);
 cudaError_t fused_pipe_stats_split(unsigned long long out[32]);
-cudaError_t launch_peak(const float *y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *peak, cudaStream_t st);
+// tab (or nullptr): stream s covers y[tab[s].y_keep, + tab[s].n_y) of its row instead of y[0, n)
+cudaError_t launch_peak(const float *y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *peak, cudaStream_t st,
+                        const StreamTick *tab = nullptr);
 
 cudaError_t launch_to_mono(const float *in, uint64_t n_samples, uint32_t channels, float *out, uint64_t n_frames,
                            cudaStream_t st);

@@ -1383,11 +1383,31 @@ struct af_session {
     WireTick *d_wire_ticks = nullptr;
     af_wire_tick *h_wire_ticks = nullptr;
     uint64_t wire_first_frame = 0;
+    // independent stream timelines (af_session_push_streams).  While `diverged`, ss[k] is stream k's bookkeeping and the
+    // shared scalars above are stale; otherwise every stream is at the shared state and a tick of equal counts takes the
+    // lockstep path.  The ping-pong buffers (in_cur, y_cur) flip for all streams on every tick either way.
+    struct StreamState {
+        RsRecurrence rec;
+        uint32_t in_len, in_drop, y_len, y_drop;
+        long long in_base;
+        uint64_t frames_emitted;
+        bool restart;                                          // start afresh at the next push (end / af_session_reset_streams)
+    };
+    std::vector<StreamState> ss, ss_next;
+    bool diverged = false;
+    StreamTick *h_tick = nullptr, *d_tick = nullptr;           // the tick's plan: [S] StreamTick, then [S] uint32 frame counts
+    float *d_pcm_stage = nullptr;                              // host-mode PCM rows of a ragged tick
+    std::vector<uint32_t> counts;                              // scratch: equal counts (af_session_push), ring reads
+    std::vector<uint64_t> first_frames, first_frames_next;     // per stream: first frame of the last push (ragged)
+    bool first_frames_ragged = false;
 };
 static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
               offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
 
 namespace {
+int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples, const uint8_t *end, int mem,
+                        const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
+
 void wire_free(af_session *s)
 {
     if (s->d_wire_pcm16) cudaFree(s->d_wire_pcm16);
@@ -1430,6 +1450,9 @@ AF_API void af_session_destroy(af_session *s)
     if (s->h_vad) cudaFreeHost(s->h_vad);
     wire_free(s);
     if (s->d_wire_prev) cudaFree(s->d_wire_prev);
+    if (s->d_tick) cudaFree(s->d_tick);
+    if (s->h_tick) cudaFreeHost(s->h_tick);
+    if (s->d_pcm_stage) cudaFree(s->d_pcm_stage);
     delete s;
 }
 
@@ -1441,6 +1464,7 @@ AF_API int af_session_reset(af_session *s)
     s->in_cur = 0; s->y_cur = 0; s->y_len = 0; s->frames_emitted = 0; s->in_drop = 0; s->y_drop = 0;
     s->in_len = 2 * RS_POLY;                       // rubato starts with 16 zero frames of history
     s->in_base = -2 * RS_POLY;
+    s->diverged = false;                           // every stream at the common start: lockstep again
     AF_CUDA(cudaMemset(s->in_buf[0], 0, s->S * s->in_stride * sizeof(float)));
     AF_CUDA(cudaMemset(s->d_vad, 0, s->S * sizeof(VadState)));
     if (s->d_wire_prev) AF_CUDA(cudaMemset(s->d_wire_prev, 0, s->S));   // no segment open
@@ -1526,6 +1550,8 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
     AF_CUDA(cudaMalloc(&s->d_energy, n_streams * s->energy_stride * sizeof(float)));
     s->frac_cap = max_new_y + 64;
     AF_CUDA(cudaMalloc(&s->d_frac, s->frac_cap * sizeof(float)));
+    s->ss.resize(n_streams); s->ss_next.resize(n_streams);
+    s->first_frames.assign(n_streams, 0); s->first_frames_next.assign(n_streams, 0);
     rc = af_session_reset(s.get());
     if (rc) return rc;
     *out = s.release();
@@ -1536,6 +1562,10 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
                            const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
 {
     if (!s || (!data && n_samples)) return fail(AF_ERR_INVALID, "null argument");
+    if (s->diverged) {                                           // streams on their own timelines: the same count for each
+        s->counts.assign(s->S, n_samples);
+        return af_session_push_streams(s, data, in_stride, s->counts.data(), nullptr, mem, o, n_pcm, n_feat, n_vad);
+    }
     if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
     if (n_samples % s->channels) return fail(AF_ERR_INVALID, "a tick must hold whole frames (n_samples %% channels == 0)");
     const uint32_t n_new = n_samples / s->channels;
@@ -1757,7 +1787,7 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
     AF_CUDA(cudaStreamSynchronize(st));
     restore.armed = false;
     s->levels_valid = s->levels;
-    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->frames_emitted; }
+    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->frames_emitted; s->first_frames_ragged = false; }
 
     // ---- 6. bookkeeping: the consumed chunks and the samples every future frame starts after are dropped by the next
     //         tick's ingest / resample kernels (in_drop, y_drop): no kernel and no second synchronisation here ----
@@ -1778,6 +1808,377 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
         if (n_feat) n_feat[k] = cfg.n_mels ? T : 0;
         if (n_vad) n_vad[k] = cfg.vad_enable ? T : 0;
     }
+    return AF_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// independent stream timelines: ragged ticks, end of stream (BatchResampler::flush), per-stream restart
+// ------------------------------------------------------------------------------------------
+namespace {
+using StreamState = af_session::StreamState;
+
+StreamState fresh_stream(const af_session *s)
+{
+    StreamState f{};
+    f.rec.init(s->rate, OUT_RATE);
+    f.in_len = 2 * RS_POLY;                                      // 16 zero frames of history, as af_session_reset
+    f.in_base = -2 * RS_POLY;
+    return f;
+}
+
+StreamState shared_stream(const af_session *s)
+{
+    StreamState c{};
+    c.rec = s->rec; c.in_len = s->in_len; c.in_drop = s->in_drop; c.y_len = s->y_len; c.y_drop = s->y_drop;
+    c.in_base = s->in_base; c.frames_emitted = s->frames_emitted; c.restart = false;
+    return c;
+}
+
+bool same_position(const StreamState &a, const StreamState &b)
+{
+    return !a.restart && !b.restart && a.rec.chunks == b.rec.chunks && a.rec.n_out == b.rec.n_out &&
+           a.rec.last_index == b.rec.last_index && a.in_len == b.in_len && a.in_drop == b.in_drop && a.y_len == b.y_len &&
+           a.y_drop == b.y_drop && a.in_base == b.in_base && a.frames_emitted == b.frames_emitted;
+}
+
+// RsRecurrence::step `chunks` times.  An exact recurrence (t = p / q, q a power of two) takes the closed form: the output
+// count of rs_exact_count and last_index = -4 + n_out * p / q - 128 * chunks, both exact (the step adds dyadic rationals
+// without rounding), so a thousand streams cost no per-output host loop.
+void rs_advance(RsRecurrence &r, uint32_t chunks, std::vector<float> *frac)
+{
+    if (!r.exact) {
+        for (uint32_t c = 0; c < chunks; ++c) r.step(frac);
+        return;
+    }
+    if (!chunks) return;
+    r.chunks += chunks;
+    r.n_out = rs_exact_count(r, r.chunks);
+    const long long num = (long long)r.n_out * (long long)r.p - (long long)RS_CHUNK * (long long)r.chunks * (long long)r.q;
+    r.last_index = -(double)(RS_POLY / 2) + (double)num / (double)r.q;
+}
+
+int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples, const uint8_t *end, int mem,
+                        const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
+{
+    AF_SCOPE(s->device);
+    const af_pipeline_config &cfg = s->pipe->cfg;
+    cudaStream_t st = cur_ctx().stream;
+    const size_t S = s->S;
+    const uint32_t bps = s->format == AF_FMT_I16 ? 2 : 4;
+    af_outputs none{};
+    if (!o) o = &none;
+
+    // ---- 0. buffers of the ragged path (allocated once; failures leave the session as it was) ----
+    const size_t tick_bytes = S * (sizeof(StreamTick) + sizeof(uint32_t));
+    if (!s->d_tick) {                                            // set together: a failed allocation leaves neither
+        StreamTick *d = nullptr, *h = nullptr;
+        cudaError_t e = cudaMalloc(&d, tick_bytes);
+        if (e == cudaSuccess) e = cudaHostAlloc((void **)&h, tick_bytes, cudaHostAllocDefault);
+        if (e != cudaSuccess) {
+            if (d) cudaFree(d);
+            return fail(AF_ERR_CUDA, "allocating the tick plan: %s", cudaGetErrorString(e));
+        }
+        s->d_tick = d; s->h_tick = h;
+    }
+    const bool table = s->rec.mode() == RS_TABLE;
+    if (table && s->frac_cap < S * s->max_new_y) {               // every stream's fractions, one slice after another
+        float *f = nullptr;
+        AF_CUDA(cudaMalloc(&f, S * s->max_new_y * sizeof(float)));
+        cudaFree(s->d_frac);
+        s->d_frac = f; s->frac_cap = S * s->max_new_y;
+    }
+
+    // ---- 1. plan every stream on copies of its state; the session changes only after the tick's synchronise ----
+    if (!s->diverged) {
+        const StreamState c = shared_stream(s);
+        for (size_t k = 0; k < S; ++k) s->ss[k] = c;
+    }
+    const StreamState fresh = fresh_stream(s);
+    StreamTick *tab = s->h_tick;
+    uint32_t *Ts = reinterpret_cast<uint32_t *>(tab + S);
+    uint32_t *d_T = reinterpret_cast<uint32_t *>(s->d_tick + S);
+    s->frac_host.clear();
+    uint32_t maxT = 0, max_ny = 0, max_n = 0;
+    for (size_t k = 0; k < S; ++k) {
+        const bool restart = s->ss[k].restart, fin = end && end[k];
+        StreamState c = restart ? fresh : s->ss[k];
+        const uint32_t n_new = n_samples[k] / s->channels;
+        const uint32_t residual = c.in_len - 2 * RS_POLY;
+        const uint32_t avail = residual + n_new;
+        const bool pass = c.rec.passthrough;
+        const uint32_t full = pass ? 0 : avail / RS_CHUNK;
+        // flush (resampler.rs:150-166): a residual is zero-padded to one more chunk.  The bound of max_new_y holds for it:
+        // ceil((127 + max_tick_frames) / 128) chunks <= the ceil((max_tick_frames + 128) / 128) it was sized for.
+        const uint32_t chunks = full + ((fin && !pass && avail % RS_CHUNK) ? 1 : 0);
+        const uint64_t n_begin = pass ? (uint64_t)(c.in_base + 2 * RS_POLY + residual) : c.rec.n_out;
+        const size_t frac_off = s->frac_host.size();
+        rs_advance(c.rec, chunks, table ? &s->frac_host : nullptr);
+        const uint64_t n_end = pass ? n_begin + n_new : c.rec.n_out;
+        const uint32_t n_y = (uint32_t)(n_end - n_begin);
+        if (c.y_len + n_y > s->y_stride) return fail(AF_ERR_CAPACITY, "internal: 16 kHz carry overflow (stream %zu)", k);
+        const uint32_t y_total = c.y_len + n_y;
+        uint32_t T = 0;
+        if (s->framing && y_total >= s->frame_len) T = 1 + (y_total - s->frame_len) / s->hop;
+        if (T && s->packed && T + 2 > s->pk_slots) return fail(AF_ERR_CAPACITY, "internal: %u frames do not fit %u frame slots", T, s->pk_slots);
+        StreamTick &d = tab[k];
+        d.in_drop = c.in_drop; d.in_keep = c.in_len; d.n_new = n_new; d.n_samples = n_samples[k];
+        d.data_base = c.in_base;
+        d.n_valid_end = pass ? c.in_base + (long long)(c.in_len + n_new)
+                             : c.in_base + 2 * RS_POLY + (long long)(fin ? avail : full * RS_CHUNK);
+        d.n_begin = n_begin; d.n_y = n_y; d.frac_off = (uint32_t)frac_off;
+        d.y_drop = c.y_drop; d.y_keep = c.y_len;
+        d.T = T; d.flags = (restart ? TICK_RESTART : 0u) | (fin ? TICK_END : 0u);
+        Ts[k] = T;
+        s->first_frames_next[k] = c.frames_emitted;
+        // the stream after the tick (as af_session_push's bookkeeping)
+        c.in_len += n_new;
+        if (!pass) {
+            const uint32_t consumed = full * RS_CHUNK;
+            c.in_drop = consumed; c.in_len -= consumed; c.in_base += consumed;
+        } else {
+            c.in_drop = c.in_len - 2 * RS_POLY; c.in_base += (long long)(c.in_len - 2 * RS_POLY); c.in_len = 2 * RS_POLY;
+        }
+        const uint32_t y_drop = s->framing ? std::min(T * s->hop, y_total) : y_total;
+        c.y_drop = y_drop; c.y_len = y_total - y_drop;
+        c.frames_emitted += T;
+        c.restart = fin;
+        s->ss_next[k] = c;
+        maxT = std::max(maxT, T); max_ny = std::max(max_ny, n_y); max_n = std::max(max_n, n_samples[k]);
+    }
+    if (s->frac_host.size() > s->frac_cap) return fail(AF_ERR_CAPACITY, "internal: fraction buffer overflow");
+    const bool want_pcm = cfg.write_pcm && o->pcm && max_ny;
+    const bool want_lm = maxT && cfg.n_mels && o->logmel;
+    const bool want_states = maxT && cfg.vad_enable && o->vad;
+    const bool need_states = want_states || (s->wire && maxT && cfg.vad_enable);
+    if (want_pcm && o->pcm_stride < max_ny) return fail(AF_ERR_CAPACITY, "pcm_stride %llu too small for %u samples", (unsigned long long)o->pcm_stride, max_ny);
+    if (want_lm && o->logmel_stride < (uint64_t)maxT * cfg.n_mels) return fail(AF_ERR_CAPACITY, "logmel_stride too small for %u frames", maxT);
+    if (want_states && o->vad_stride < maxT) return fail(AF_ERR_CAPACITY, "vad_stride too small for %u frames", maxT);
+    float *lm = nullptr; uint64_t lm_stride = 0;
+    uint8_t *states = nullptr; uint64_t st_stride = 0;
+    if (want_lm) {
+        if (mem == AF_MEM_HOST || s->packed) {
+            if (!s->d_lm) AF_CUDA(cudaMalloc(&s->d_lm, S * s->lm_stride * sizeof(float)));
+            lm = s->d_lm; lm_stride = s->lm_stride;
+        } else { lm = o->logmel; lm_stride = o->logmel_stride; }
+        if (lm_stride < (uint64_t)maxT * cfg.n_mels) return fail(AF_ERR_CAPACITY, "internal: log-mel staging too small for %u frames", maxT);
+    }
+    if (need_states) {
+        if (mem == AF_MEM_HOST || !want_states) {
+            if (!s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));
+            states = s->d_states; st_stride = s->st_stride;
+        } else { states = o->vad; st_stride = o->vad_stride; }
+        if (st_stride < maxT) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", maxT);
+    }
+    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)maxT * s->hop : max_ny;
+    if (s->wire && wire_n > s->wire_cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
+    float *pcm_dst = nullptr; uint64_t pcm_dst_stride = 0;
+    if (want_pcm) {
+        if (mem == AF_MEM_HOST) {
+            const uint64_t w = round_up(s->max_new_y, 4);
+            if (!s->d_pcm_stage) AF_CUDA(cudaMalloc(&s->d_pcm_stage, S * w * sizeof(float)));
+            pcm_dst = s->d_pcm_stage; pcm_dst_stride = w;
+        } else { pcm_dst = o->pcm; pcm_dst_stride = o->pcm_stride; }
+    }
+    const void *d_in = data;
+    uint64_t d_in_stride_bytes = in_stride * bps;
+    if (mem == AF_MEM_HOST && max_n) {
+        const size_t row = round_up((uint64_t)max_n * bps, 16);
+        if (s->in_stage_bytes < row * S) {
+            if (s->d_in_stage) cudaFree(s->d_in_stage);
+            s->d_in_stage = nullptr; s->in_stage_bytes = 0;
+            AF_CUDA(cudaMalloc(&s->d_in_stage, row * S));
+            s->in_stage_bytes = row * S;
+        }
+        d_in = s->d_in_stage; d_in_stride_bytes = row;
+    }
+
+    // From here on only CUDA failures can occur; the bookkeeping is committed after the synchronise (af_session_reset
+    // after an AF_ERR_CUDA: detector and wire state on the device may have advanced, the wire rows are refused).
+    if (s->wire) s->wire_valid = false;
+    // ---- 2. input (host rows: the last row is copied with its own count, the caller's buffer may end there), plan ----
+    if (mem == AF_MEM_HOST && max_n) {
+        if (S > 1)
+            AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)max_n * bps, S - 1,
+                                      cudaMemcpyHostToDevice, st));
+        if (n_samples[S - 1])
+            AF_CUDA(cudaMemcpyAsync(static_cast<char *>(s->d_in_stage) + (S - 1) * d_in_stride_bytes,
+                                    static_cast<const char *>(data) + (S - 1) * in_stride * bps, (size_t)n_samples[S - 1] * bps,
+                                    cudaMemcpyHostToDevice, st));
+    }
+    AF_CUDA(cudaMemcpyAsync(s->d_tick, s->h_tick, tick_bytes, cudaMemcpyHostToDevice, st));
+    if (!s->frac_host.empty())
+        AF_CUDA(cudaMemcpyAsync(s->d_frac, s->frac_host.data(), s->frac_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    const int in_next = s->in_cur ^ 1, y_next = s->y_cur ^ 1;
+    SessionIngest ing{};
+    ing.old_buf = s->in_buf[s->in_cur]; ing.new_buf = s->in_buf[in_next]; ing.buf_stride = s->in_stride;
+    ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.channels = s->channels; ing.format = s->format;
+    SessionResample rs{};
+    rs.in_buf = s->in_buf[in_next]; rs.in_stride = s->in_stride;
+    rs.p = s->rec.p; rs.q = s->rec.q; rs.mode = s->rec.mode(); rs.frac = s->d_frac;
+    rs.y_old = s->y_buf[s->y_cur]; rs.y_new = s->y_buf[y_next]; rs.y_stride = s->y_stride;
+    AF_CUDA(launch_session_tick_streams(ing, rs, s->d_tick, s->d_vad, s->d_wire_prev, pcm_dst, pcm_dst_stride, (uint32_t)S, st));
+    count_launch();
+    float *ycur = s->y_buf[y_next];
+
+    // ---- 3. PCM, levels ----
+    if (want_pcm && mem == AF_MEM_HOST)
+        AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), pcm_dst, pcm_dst_stride * sizeof(float),
+                                  (size_t)max_ny * sizeof(float), S, cudaMemcpyDeviceToHost, st));
+    if (s->levels) {
+        AF_CUDA(launch_peak(ycur, s->y_stride, 0, (uint32_t)S, s->d_peak, st, s->d_tick));
+        count_launch();
+    }
+
+    // ---- 4. frames: every frame slot of every row is computed by the packed launch (STFT frames with framing are always
+    //         packed), the energies of custom frames and the scan take each stream's count ----
+    if (maxT) {
+        if (s->packed) {
+            FusedParams P{};
+            P.streams = s->d_ptab[y_next]; P.tiles = s->d_ptiles[y_next]; P.n_tiles = s->pk_n;
+            const uint64_t vrows = s->pk_rows;
+            P.fft = cur_ctx().d_fft; P.mel = s->d_mel;
+            P.pcm = nullptr; P.pcm_stride = 0;
+            P.logmel = lm; P.logmel_stride = lm_stride * vrows;
+            P.energy = cfg.vad_enable ? s->d_energy : nullptr; P.energy_stride = s->energy_stride * vrows;
+            P.n_mels = lm ? cfg.n_mels : 0;
+            P.do_energy = cfg.vad_enable ? 1 : 0;
+            P.log_floor = cfg.log_floor;
+            P.log_scale = cfg.log10 ? 0.30102999566398120f : 0.69314718055994531f;
+            P.use_stage = kernel_variant() == "sync" ? 0u : 1u;
+            P.layout = fused_layout(P.do_energy != 0);
+            P.neg_zero = -0.0f;
+            if (P.n_mels || P.do_energy) {
+                AF_CUDA(launch_fused(P, (int)std::min<size_t>(P.n_tiles, (size_t)cur_ctx().sm_count), st));
+                count_launch(2);
+            }
+        } else {
+            EnergyJob ej{};
+            ej.y = ycur; ej.y_stride = s->y_stride; ej.n_frames = d_T; ej.n_frames_all = maxT;
+            ej.frame_len = s->frame_len; ej.hop = s->hop; ej.energy = s->d_energy; ej.energy_stride = s->energy_stride;
+            ej.n_streams = (uint32_t)S;
+            AF_CUDA(launch_frame_energy(ej, st));
+            count_launch();
+        }
+        if (cfg.vad_enable) {
+            ScanJob sj{};
+            sj.energy = s->d_energy; sj.energy_stride = s->energy_stride; sj.n_frames = d_T; sj.n_frames_all = maxT;
+            sj.states = states; sj.states_stride = st_stride; sj.state_io = s->d_vad;
+            sj.final_out = mem == AF_MEM_DEVICE ? reinterpret_cast<VadState *>(o->vad_final) : nullptr;
+            sj.prm = s->pipe->vad_prm; sj.n_streams = (uint32_t)S;
+            AF_CUDA(launch_vad_scan(sj, st));
+            count_launch();
+        }
+        if (mem == AF_MEM_DEVICE && lm && lm != o->logmel)
+            AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
+                                      (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToDevice, st));
+        if (mem == AF_MEM_HOST) {
+            if (lm) AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
+                                              (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
+            if (want_states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, maxT, S, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    // every stream's detector (a restarted one is fresh), whether or not a frame completed
+    if (cfg.vad_enable && o->vad_final && (mem == AF_MEM_HOST || !maxT))
+        AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad, S * sizeof(VadState),
+                                mem == AF_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+    // ---- 5. wire payloads ----
+    if (s->wire) {
+        const af_wire_config &wc = s->wire_cfg;
+        WireJob wj{};
+        wj.y = ycur; wj.y_stride = s->y_stride;
+        wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
+        wj.T = maxT; wj.hop = s->hop; wj.gate = wc.gate;                 // (T sizes the kept-frame list: the largest)
+        wj.prev = s->d_wire_prev;
+        wj.pcm16 = s->d_wire_pcm16; wj.pcm16_stride = s->wire_pcm16_stride;
+        wj.b64 = s->d_wire_b64; wj.b64_stride = s->wire_b64_stride;
+        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S; wj.tab = s->d_tick;
+        AF_CUDA(launch_session_wire(wj, st));
+        count_launch();
+        if (wc.mem == AF_MEM_HOST && wire_n) {
+            if (wc.pcm16)
+                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_pcm16, s->wire_pcm16_stride * sizeof(int16_t), s->d_wire_pcm16,
+                                          s->wire_pcm16_stride * sizeof(int16_t), wire_n * sizeof(int16_t), S, cudaMemcpyDeviceToHost, st));
+            if (wc.base64)
+                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_b64, s->wire_b64_stride, s->d_wire_b64, s->wire_b64_stride,
+                                          af_pcm16_base64_len(wire_n), S, cudaMemcpyDeviceToHost, st));
+        }
+        AF_CUDA(cudaMemcpyAsync(s->h_wire_ticks, s->d_wire_ticks, S * sizeof(af_wire_tick), cudaMemcpyDeviceToHost, st));
+    }
+    if (s->levels) {
+        AF_CUDA(cudaMemcpyAsync(s->h_peak, s->d_peak, S * sizeof(float), cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaMemcpyAsync(s->h_vad, s->d_vad, S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
+    }
+    AF_CUDA(cudaStreamSynchronize(st));
+
+    // ---- 6. commit; streams that all stand at the same position run in lockstep again ----
+    s->in_cur = in_next; s->y_cur = y_next;
+    s->ss.swap(s->ss_next);
+    s->first_frames.swap(s->first_frames_next);
+    s->levels_valid = s->levels;
+    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->first_frames[0]; s->first_frames_ragged = true; }
+    bool aligned = true;
+    for (size_t k = 0; k < S && aligned; ++k) aligned = same_position(s->ss[k], s->ss[0]);
+    s->diverged = !aligned;
+    if (aligned) {
+        const StreamState &c = s->ss[0];
+        s->rec = c.rec; s->in_len = c.in_len; s->in_drop = c.in_drop; s->y_len = c.y_len; s->y_drop = c.y_drop;
+        s->in_base = c.in_base; s->frames_emitted = c.frames_emitted;
+    }
+    for (size_t k = 0; k < S; ++k) {
+        if (n_pcm) n_pcm[k] = tab[k].n_y;
+        if (n_feat) n_feat[k] = cfg.n_mels ? tab[k].T : 0;
+        if (n_vad) n_vad[k] = cfg.vad_enable ? tab[k].T : 0;
+    }
+    return AF_OK;
+}
+}  // namespace
+
+extern "C" {
+
+AF_API int af_session_push_streams(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples,
+                                   const uint8_t *end, int mem, const af_outputs *out,
+                                   uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
+{
+    if (!s || !n_samples) return fail(AF_ERR_INVALID, "null argument");
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    bool equal = true, any_end = false;
+    for (size_t k = 0; k < s->S; ++k) {
+        const uint32_t n = n_samples[k];
+        if (n % s->channels) return fail(AF_ERR_INVALID, "stream %zu: a tick must hold whole frames (n_samples %% channels == 0)", k);
+        if (n / s->channels > s->max_tick_frames) return fail(AF_ERR_CAPACITY, "stream %zu: tick of %u frames exceeds max_tick_samples", k, n / s->channels);
+        if (in_stride < n) return fail(AF_ERR_INVALID, "stream %zu: in_stride smaller than n_samples", k);
+        if (n && !data) return fail(AF_ERR_INVALID, "null data");
+        equal = equal && n == n_samples[0];
+        any_end = any_end || (end && end[k]);
+    }
+    // every stream at the shared position and the same count: the lockstep tick (same launches and copies as always)
+    if (!s->diverged && equal && !any_end)
+        return af_session_push(s, data, in_stride, n_samples[0], mem, out, n_pcm, n_feat, n_vad);
+    return session_push_ragged(s, data, in_stride, n_samples, end, mem, out, n_pcm, n_feat, n_vad);
+}
+
+AF_API int af_session_reset_streams(af_session *s, const uint32_t *streams, size_t n)
+{
+    if (!s || (!streams && n)) return fail(AF_ERR_INVALID, "null argument");
+    for (size_t i = 0; i < n; ++i)
+        if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
+    if (!n) return AF_OK;
+    if (!s->diverged) {
+        const StreamState c = shared_stream(s);
+        for (size_t k = 0; k < s->S; ++k) s->ss[k] = c;
+        s->diverged = true;
+    }
+    for (size_t i = 0; i < n; ++i) s->ss[streams[i]].restart = true;   // applied by the stream's next tick kernel
+    return AF_OK;
+}
+
+AF_API int af_session_wire_first_frames(const af_session *s, uint64_t *first_frame)
+{
+    if (!s || !first_frame) return fail(AF_ERR_INVALID, "null argument");
+    if (!s->wire_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire");
+    for (size_t k = 0; k < s->S; ++k) first_frame[k] = s->first_frames_ragged ? s->first_frames[k] : s->wire_first_frame;
     return AF_OK;
 }
 
@@ -2004,6 +2405,36 @@ AF_API int af_session_push_rings(af_session *s, af_ring *const *rings, uint32_t 
         if (rc != AF_OK || got != n_samples) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
     }
     return af_session_push(s, s->ring_stage, stride, n_samples, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
+}
+
+// AudioCapturer::read_frame(max) for every stream: each ring gives what it holds, up to max_samples, in whole frames
+AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings, uint32_t max_samples, const uint8_t *end,
+                                           const af_outputs *out, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
+{
+    if (!s || !rings) return fail(AF_ERR_INVALID, "null argument");
+    if (s->format != AF_FMT_F32) return fail(AF_ERR_INVALID, "capture rings hold f32 samples; the session was created for i16");
+    if (max_samples / s->channels > s->max_tick_frames)
+        return fail(AF_ERR_CAPACITY, "max_samples %u exceeds the session's max_tick_samples", max_samples);
+    s->counts.resize(s->S);
+    for (size_t k = 0; k < s->S; ++k) {
+        if (!rings[k]) return fail(AF_ERR_INVALID, "ring %zu is null", k);
+        const size_t n = std::min<size_t>(max_samples, af_ring_available(rings[k]));
+        s->counts[k] = (uint32_t)(n - n % s->channels);
+    }
+    const uint64_t stride = round_up(std::max<uint32_t>(max_samples, 4), 4);
+    if (s->ring_stage_cap < stride * s->S) {
+        if (s->ring_stage) cudaFreeHost(s->ring_stage);
+        s->ring_stage = nullptr; s->ring_stage_cap = 0;
+        AF_CUDA(cudaHostAlloc((void **)&s->ring_stage, stride * s->S * sizeof(float), cudaHostAllocDefault));
+        s->ring_stage_cap = stride * s->S;
+    }
+    for (size_t k = 0; k < s->S; ++k) {
+        if (!s->counts[k]) continue;
+        size_t got = 0;
+        const int rc = af_ring_read(rings[k], s->ring_stage + k * stride, s->counts[k], &got);
+        if (rc != AF_OK || got != s->counts[k]) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
+    }
+    return af_session_push_streams(s, s->ring_stage, stride, s->counts.data(), end, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
 }
 
 }  // extern "C"

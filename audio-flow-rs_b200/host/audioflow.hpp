@@ -173,6 +173,32 @@ public:
     }
     void reset() { check(af_session_reset(h_)); }
 
+    // independent stream timelines: stream k pushes n_samples[k] samples from row k (rows in_stride apart); end[k] != 0
+    // (end may be empty) ends stream k after them (BatchResampler::flush); its next push starts afresh
+    TickCounts push_streams(const void *data, uint64_t in_stride, const std::vector<uint32_t> &n_samples,
+                            const std::vector<uint8_t> &end, int mem, const af_outputs *out = nullptr)
+    {
+        if (n_samples.size() != n_ || (!end.empty() && end.size() != n_)) throw std::invalid_argument("push_streams: one count and end flag per stream");
+        TickCounts c{std::vector<uint32_t>(n_), std::vector<uint32_t>(n_), std::vector<uint32_t>(n_)};
+        check(af_session_push_streams(h_, data, in_stride, n_samples.data(), end.empty() ? nullptr : end.data(), mem, out,
+                                      c.n_pcm.data(), c.n_feat.data(), c.n_vad.data()));
+        return c;
+    }
+    // AudioCapturer::read_frame(max) for every stream: what each ring holds, up to max_samples, in whole frames
+    TickCounts push_rings_available(std::vector<RingBuffer *> &rings, uint32_t max_samples, const std::vector<uint8_t> &end = {},
+                                    const af_outputs *out = nullptr)
+    {
+        if (rings.size() != n_ || (!end.empty() && end.size() != n_)) throw std::invalid_argument("push_rings_available: one ring and end flag per stream");
+        std::vector<af_ring *> hs;
+        for (RingBuffer *r : rings) hs.push_back(r->handle());
+        TickCounts c{std::vector<uint32_t>(n_), std::vector<uint32_t>(n_), std::vector<uint32_t>(n_)};
+        check(af_session_push_rings_available(h_, hs.data(), max_samples, end.empty() ? nullptr : end.data(), out,
+                                              c.n_pcm.data(), c.n_feat.data(), c.n_vad.data()));
+        return c;
+    }
+    // the listed streams start afresh at their next push, without a flush
+    void reset_streams(const std::vector<uint32_t> &streams) { check(af_session_reset_streams(h_, streams.data(), streams.size())); }
+
     void enable_levels(bool on = true) { check(af_session_enable_levels(h_, on ? 1 : 0)); }
     // AudioLevel{level, peak} / VolumeLevel{level, is_speech} of the last tick, per stream
     void levels(std::vector<float> *level_db, std::vector<float> *peak, std::vector<uint8_t> *is_speech) const
@@ -204,6 +230,13 @@ public:
             w.continued = t[k].continued; w.started = t[k].started; w.ended = t[k].ended; w.in_speech = t[k].in_speech != 0;
         }
         return out;
+    }
+    // per stream: the first frame completed by the last push, in the stream's own frame sequence since its last start
+    std::vector<uint64_t> wire_first_frames() const
+    {
+        std::vector<uint64_t> f(n_);
+        check(af_session_wire_first_frames(h_, f.data()));
+        return f;
     }
     af_session *handle() { return h_; }
 

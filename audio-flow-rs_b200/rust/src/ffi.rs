@@ -118,6 +118,13 @@ extern "C" {
     pub fn af_session_enable_wire(s: *mut af_session, cfg: *const af_wire_config) -> c_int;
     pub fn af_session_wire(s: *const af_session, pcm16: *mut *const i16, pcm16_stride: *mut u64, base64: *mut *const c_char,
                            base64_stride: *mut u64, ticks: *mut af_wire_tick, first_frame: *mut u64) -> c_int;
+    pub fn af_session_push_streams(s: *mut af_session, data: *const std::os::raw::c_void, in_stride: u64, n_samples: *const u32,
+                                   end: *const u8, mem: c_int, out: *const af_outputs,
+                                   n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
+    pub fn af_session_reset_streams(s: *mut af_session, streams: *const u32, n: usize) -> c_int;
+    pub fn af_session_push_rings_available(s: *mut af_session, rings: *const *mut af_ring, max_samples: u32, end: *const u8,
+                                           out: *const af_outputs, n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
+    pub fn af_session_wire_first_frames(s: *const af_session, first_frame: *mut u64) -> c_int;
 }
 
 extern "C" {

@@ -3,12 +3,16 @@
 //! (websocket.rs:244-254):
 //!
 //! ```ignore
-//! let mut s = Session::new(&pipeline, rings.len(), 48000, 960, Some(WireGate::Speech))?;
+//! let mut s = Session::new(&pipeline, rings.len(), 48000, 1920, Some(WireGate::Speech))?;
+//! let mut ends = vec![false; rings.len()];
 //! loop {
-//!     s.push_rings(&rings, 960)?;
+//!     // every stream takes what its capture callback delivered (up to 40 ms): a late callback stalls only its stream
+//!     s.push_rings_available(&rings, 1920, &ends)?;
 //!     for (k, p) in s.wire()?.into_iter().enumerate() {
 //!         if !p.audio_base_64.is_empty() { clients[k].send_audio(p.audio_base_64).await?; }
 //!     }
+//!     // ends[k] = caller k hung up (the next tick flushes it, its slot then serves a new caller);
+//!     // s.reset_streams(&[k]) drops a caller without a flush
 //! }
 //! ```
 //!
@@ -44,11 +48,11 @@ pub struct WirePayload {
     pub continued: u32,
 }
 
-/// Counts of one tick, the same for every stream.
+/// Counts of one stream in one tick (`push_rings` and `push_rings_available` return one per stream).
 #[derive(Debug, Clone, Copy, Default)]
 pub struct TickCounts { pub n_pcm: u32, pub n_feat: u32, pub n_vad: u32 }
 
-/// `af_session`: n lockstep 16 kHz streams of one (rate, mono f32) with their state on the GPU between ticks.
+/// `af_session`: n 16 kHz streams (lockstep, or each on its own timeline) of one (rate, mono f32) with their state on the GPU between ticks.
 pub struct Session { h: *mut ffi::af_session, n_streams: usize }
 unsafe impl Send for Session {}
 
@@ -67,15 +71,43 @@ impl Session {
     }
 
     /// `AudioCapturer::read_frame` (capture.rs:310-319) for every stream at once, pushed as one tick: takes exactly `n`
-    /// samples from each ring (one ring per stream), nothing unless every ring holds them.
-    pub fn push_rings(&mut self, rings: &[RingBuffer], n: u32) -> Result<TickCounts, AudioError> {
+    /// samples from each ring (one ring per stream), nothing unless every ring holds them.  Counts per stream (equal while
+    /// the streams are in lockstep).
+    pub fn push_rings(&mut self, rings: &[RingBuffer], n: u32) -> Result<Vec<TickCounts>, AudioError> {
         if rings.len() != self.n_streams {
             return Err(AudioError::ResamplingFailed(format!("{} rings for {} streams", rings.len(), self.n_streams)));
         }
         let hs: Vec<*mut ffi::af_ring> = rings.iter().map(|r| r.h).collect();
-        let mut c = TickCounts::default();
-        check(unsafe { ffi::af_session_push_rings(self.h, hs.as_ptr(), n, ptr::null(), &mut c.n_pcm, &mut c.n_feat, &mut c.n_vad) })?;
-        Ok(c)
+        let k = self.n_streams;
+        let (mut p, mut f, mut v) = (vec![0u32; k], vec![0u32; k], vec![0u32; k]);
+        check(unsafe {
+            ffi::af_session_push_rings(self.h, hs.as_ptr(), n, ptr::null(), p.as_mut_ptr(), f.as_mut_ptr(), v.as_mut_ptr())
+        })?;
+        Ok((0..k).map(|i| TickCounts { n_pcm: p[i], n_feat: f[i], n_vad: v[i] }).collect())
+    }
+
+    /// `AudioCapturer::read_frame(max)` for every stream: each ring gives `min(max, available)` samples and the streams
+    /// advance on their own timelines, so an empty ring stalls no other stream.  `ends[k]` (or an empty slice: none) ends
+    /// stream k after its samples (`BatchResampler::flush`); its next push starts a new stream.  Counts per stream.
+    pub fn push_rings_available(&mut self, rings: &[RingBuffer], max: u32, ends: &[bool]) -> Result<Vec<TickCounts>, AudioError> {
+        if rings.len() != self.n_streams || (!ends.is_empty() && ends.len() != self.n_streams) {
+            return Err(AudioError::ResamplingFailed(format!("{} rings and {} end flags for {} streams", rings.len(), ends.len(),
+                                                            self.n_streams)));
+        }
+        let hs: Vec<*mut ffi::af_ring> = rings.iter().map(|r| r.h).collect();
+        let e: Vec<u8> = ends.iter().map(|&b| b as u8).collect();
+        let n = self.n_streams;
+        let (mut p, mut f, mut v) = (vec![0u32; n], vec![0u32; n], vec![0u32; n]);
+        check(unsafe {
+            ffi::af_session_push_rings_available(self.h, hs.as_ptr(), max, if e.is_empty() { ptr::null() } else { e.as_ptr() },
+                                                 ptr::null(), p.as_mut_ptr(), f.as_mut_ptr(), v.as_mut_ptr())
+        })?;
+        Ok((0..n).map(|k| TickCounts { n_pcm: p[k], n_feat: f[k], n_vad: v[k] }).collect())
+    }
+
+    /// The listed streams start afresh at their next push, without a flush (the caller went away); the others continue.
+    pub fn reset_streams(&mut self, streams: &[u32]) -> Result<(), AudioError> {
+        check(unsafe { ffi::af_session_reset_streams(self.h, streams.as_ptr(), streams.len()) })
     }
 
     /// The payloads of the last tick, one per stream (valid until the next push; copied out here).

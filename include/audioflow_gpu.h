@@ -371,7 +371,8 @@ AF_API int af_session_levels(const af_session *s, float *level_db, float *peak, 
  *   in_speech the stream's latest completed frame is Speech (the tick's last frame; an earlier one if it completed none);
  *   continued gated only: payload samples at the front that belong to the segment already open when the tick began
  *             (the rest belongs to segments started in the tick); 0 ungated, where payloads are not frame-aligned.
- * first_frame is the global index of the tick's first completed frame (the same for all streams).
+ * first_frame is the global index of the tick's first completed frame (the same for all streams in lockstep; stream 0's
+ * once streams have their own timelines, see af_session_wire_first_frames).
  * af_session_reset clears the carried segment state. */
 typedef struct af_wire_config {
     uint32_t gate;            /* 0: every 16 kHz sample of the tick; 1: only the hops of its segment frames (needs the VAD) */
@@ -412,6 +413,41 @@ AF_API void af_ring_clear(af_ring *r);                                   /* capt
  * consumed unless every ring holds n_samples. */
 AF_API int af_session_push_rings(af_session *s, af_ring *const *rings, uint32_t n_samples, const af_outputs *out,
                                  uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
+
+/* ---- independent stream timelines: ragged ticks, end of stream, per-stream restart ----------------------------------
+ * Every stream of a session has its own timeline: stream k of a session behaves exactly like a one-stream session pushed
+ * the same ticks -- per tick the output of BatchResampler::process (resampler.rs:132-147) on that stream's samples, the
+ * frames they complete, the VAD over those frames, the wire payload and record of those frames, its levels.  af_session_push
+ * on a session whose streams have diverged is af_session_push_streams with all counts equal and no end; af_session_reset
+ * returns every stream to the common start.  All argument errors (a count above max_tick_samples: AF_ERR_CAPACITY; a
+ * partial frame, in_stride below a count, a stream index out of range, a null array: AF_ERR_INVALID; an output row too
+ * short for the largest count: AF_ERR_CAPACITY) are reported before any state changes.  After AF_ERR_CUDA, reset.
+ *
+ * One tick in which stream k pushes n_samples[k] interleaved samples (0 allowed; a whole number of frames; at most
+ * max_tick_samples) from the start of row k, rows in_stride samples apart (in_stride >= every n_samples[k]).
+ * end (may be NULL): end[k] != 0 ends stream k after this tick's samples -- BatchResampler::flush (resampler.rs:150-166):
+ * the residual input is zero-padded to one 128-frame chunk and resampled, every frame completed by it is emitted, the
+ * rest of the 16 kHz tail is dropped.  Its next push starts afresh, exactly like a stream of a newly created session.
+ * An end closes a wire segment that is still open (as af_vad_segments closes one at the last frame): that tick counts it
+ * in `ended` and reports in_speech = 0.
+ * Outputs go to row k's start; n_pcm[k] / n_feat[k] / n_vad[k] say how many each stream emitted (rows must hold the
+ * largest).  vad_final[k] of an ended stream is its detector after its last frame. */
+AF_API int af_session_push_streams(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples,
+                                   const uint8_t *end, int mem, const af_outputs *out,
+                                   uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
+/* Streams streams[0..n) start afresh at their next push without a flush: pending input, 16 kHz tail, detector and open
+ * wire segment are discarded (the caller went away).  Other streams are untouched.  A stream may be listed twice. */
+AF_API int af_session_reset_streams(af_session *s, const uint32_t *streams, size_t n);
+/* AudioCapturer::read_frame(max) (capture.rs:310-319, RingBuffer::read returns min(size, available)) for every stream:
+ * takes min(max_samples, available) samples from each ring, rounded down to whole frames (an empty ring pushes 0; a
+ * partial frame stays in the ring), and pushes them with af_session_push_streams.  Nothing is consumed when an argument
+ * is refused; max_samples above max_tick_samples is AF_ERR_CAPACITY. */
+AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings, uint32_t max_samples, const uint8_t *end,
+                                           const af_outputs *out, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
+/* Per stream (host array of n_streams): the index, in that stream's own frame sequence since its last start, of the
+ * first frame completed by the last push.  af_session_wire's first_frame is this value for stream 0.  AF_ERR_INVALID
+ * when af_session_wire would be. */
+AF_API int af_session_wire_first_frames(const af_session *s, uint64_t *first_frame);
 
 #ifdef __cplusplus
 }
