@@ -1012,24 +1012,6 @@ cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionRes
     return cudaGetLastError();
 }
 
-// every stream of a session has the same lengths: refresh the fused kernel's stream table in place
-__global__ void af_session_setup_kernel(StreamDev *tab, TileDev *tiles, uint32_t n_streams, uint32_t n, uint32_t n_frames,
-                                        uint32_t n_vad)
-{
-    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    tab[s].n_samples = n; tab[s].n_in = n; tab[s].n_out = n; tab[s].n_frames = n_frames; tab[s].n_vad_frames = n_vad;
-    plan_tile(tab[s], s, 0, &tiles[s]);               // the tick's single tile: positions and stage fills
-}
-
-cudaError_t launch_session_setup(StreamDev *tab, TileDev *tiles, uint32_t n_streams, uint32_t n, uint32_t n_frames, uint32_t n_vad,
-                                 cudaStream_t st)
-{
-    if (n_streams == 0) return cudaSuccess;
-    af_session_setup_kernel<<<(n_streams + 127) / 128, 128, 0, st>>>(tab, tiles, n_streams, n, n_frames, n_vad);
-    return cudaGetLastError();
-}
-
 // ---- level metering (events/mod.rs:41 AudioLevel{level, peak}): peak = max |y| over the tick's new 16 kHz samples ----
 // One warp per stream; max is order-independent, so the result is bit-exact against any reference order.
 __global__ void af_peak_kernel(const float *__restrict__ y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *__restrict__ peak,

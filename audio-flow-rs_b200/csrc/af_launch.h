@@ -113,8 +113,6 @@ cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R
 // pcm (device, or nullptr) receives each stream's new samples at its row start
 cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab, VadState *vad,
                                         uint8_t *wire_prev, float *pcm, uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st);
-cudaError_t launch_session_setup(StreamDev *tab, TileDev *tiles, uint32_t n_streams, uint32_t n, uint32_t n_frames, uint32_t n_vad,
-                                 cudaStream_t st);
 // split: the batch holds tiles other than 48 kHz mono f32 -> 16 kHz; such batches (and quarter-staged ones) run the
 // kernel of the second translation unit of af_fused.cu (AF_FUSED_SPLIT_TU), whose resampler role keeps the hot and the
 // general tiles in separate loops

@@ -1328,7 +1328,7 @@ AF_API size_t af_debug_resample_plan(uint32_t input_rate, uint32_t output_rate, 
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------
-// streaming sessions (BASELINE config 5): n_streams lockstep streams, state resident on the device
+// streaming sessions (BASELINE config 5): n_streams streams, state resident on the device
 // ------------------------------------------------------------------------------------------
 struct af_session {
     af_pipeline *pipe = nullptr;
@@ -1336,21 +1336,12 @@ struct af_session {
     MelTables *d_mel = nullptr;
     size_t S = 0;
     uint32_t rate = 0, channels = 1, format = 0, max_tick_frames = 0;
-    RsRecurrence rec;                 // shared by every stream (same number of frames pushed to all)
     // input history: last 16 frames + residual (< 128), ping-pong
     float *in_buf[2] = {nullptr, nullptr}; uint64_t in_stride = 0; int in_cur = 0;
-    uint32_t in_len = 0;              // frames currently held in in_buf[in_cur]
-    long long in_base = 0;            // global frame index of in_buf[in_cur][0]
     // 16 kHz carry (samples not yet covered by an emitted frame), ping-pong
     float *y_buf[2] = {nullptr, nullptr}; uint64_t y_stride = 0; int y_cur = 0;
-    uint32_t y_len = 0;
-    // frames / samples at the front of the current buffers that the NEXT tick's ingest / resample kernels skip: the
-    // compaction after a tick costs no kernel of its own
-    uint32_t in_drop = 0, y_drop = 0;
     uint32_t frame_len = WIN, hop = HOP;   // framing of the features / VAD
     bool framing = false;
-    StreamDev *d_tab[2] = {nullptr, nullptr};
-    TileDev *d_tiles = nullptr;
     // packed ticks (STFT frames): the rows of y_buf are a whole number of hops apart, so `pk_rows` consecutive streams
     // read as ONE virtual stream whose frame slot r * pk_slots + j is frame j of row r (the slots >= T straddle rows and
     // are ignored).  A tick of two frames per stream then fills the fused kernel's 32-frame steps instead of leaving
@@ -1366,7 +1357,6 @@ struct af_session {
     float *d_lm = nullptr; uint8_t *d_states = nullptr;       // host-mode staging of outputs
     uint64_t lm_stride = 0, st_stride = 0;
     std::vector<float> frac_host;
-    uint64_t frames_emitted = 0;
     float *ring_stage = nullptr; size_t ring_stage_cap = 0;   // pinned rows for af_session_push_rings
     // level metering (af_session_enable_levels): peak of the last tick per stream + the detector states, on the host
     bool levels = false, levels_valid = false;
@@ -1382,32 +1372,32 @@ struct af_session {
     uint64_t wire_cap = 0;                                    // payload samples a row holds
     WireTick *d_wire_ticks = nullptr;
     af_wire_tick *h_wire_ticks = nullptr;
-    uint64_t wire_first_frame = 0;
-    // independent stream timelines (af_session_push_streams).  While `diverged`, ss[k] is stream k's bookkeeping and the
-    // shared scalars above are stale; otherwise every stream is at the shared state and a tick of equal counts takes the
-    // lockstep path.  The ping-pong buffers (in_cur, y_cur) flip for all streams on every tick either way.
+    // the bookkeeping of one stream's timeline.  While !diverged, `shared` is the position of every stream and a tick of
+    // equal counts takes the lockstep tick kernel; while diverged, ss[k] is stream k's position (af_session_push_streams).
+    // The ping-pong buffers (in_cur, y_cur) flip for all streams on every tick either way.
     struct StreamState {
-        RsRecurrence rec;
-        uint32_t in_len, in_drop, y_len, y_drop;
-        long long in_base;
+        RsRecurrence rec;                                      // the stream's f64 chunk recurrence
+        uint32_t in_len;                                       // frames held in its row of in_buf[in_cur]
+        // frames / samples at the front of the current rows that the NEXT tick's ingest / resample skip: the compaction
+        // after a tick costs no kernel of its own
+        uint32_t in_drop, y_drop;
+        uint32_t y_len;                                        // 16 kHz carry held in its row of y_buf[y_cur]
+        long long in_base;                                     // global frame index of the row's first frame
         uint64_t frames_emitted;
         bool restart;                                          // start afresh at the next push (end / af_session_reset_streams)
     };
+    StreamState shared{};
     std::vector<StreamState> ss, ss_next;
     bool diverged = false;
     StreamTick *h_tick = nullptr, *d_tick = nullptr;           // the tick's plan: [S] StreamTick, then [S] uint32 frame counts
-    float *d_pcm_stage = nullptr;                              // host-mode PCM rows of a ragged tick
+    float *d_pcm_stage = nullptr;                              // host-mode PCM rows of a per-stream tick
     std::vector<uint32_t> counts;                              // scratch: equal counts (af_session_push), ring reads
-    std::vector<uint64_t> first_frames, first_frames_next;     // per stream: first frame of the last push (ragged)
-    bool first_frames_ragged = false;
+    std::vector<uint64_t> first_frames;                        // per stream: first frame completed by the last push
 };
 static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
               offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
 
 namespace {
-int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples, const uint8_t *end, int mem,
-                        const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
-
 void wire_free(af_session *s)
 {
     if (s->d_wire_pcm16) cudaFree(s->d_wire_pcm16);
@@ -1421,6 +1411,17 @@ void wire_free(af_session *s)
     s->wire_pcm16_stride = s->wire_b64_stride = s->wire_cap = 0;
     s->wire = s->wire_valid = false;
 }
+
+using StreamState = af_session::StreamState;
+
+StreamState fresh_stream(const af_session *s)
+{
+    StreamState f{};
+    f.rec.init(s->rate, OUT_RATE);
+    f.in_len = 2 * RS_POLY;                                      // rubato starts with 16 zero frames of history
+    f.in_base = -2 * RS_POLY;
+    return f;
+}
 }  // namespace
 
 extern "C" {
@@ -1433,11 +1434,9 @@ AF_API void af_session_destroy(af_session *s)
     for (int i = 0; i < 2; ++i) {
         if (s->in_buf[i]) cudaFree(s->in_buf[i]);
         if (s->y_buf[i]) cudaFree(s->y_buf[i]);
-        if (s->d_tab[i]) cudaFree(s->d_tab[i]);
         if (s->d_ptab[i]) cudaFree(s->d_ptab[i]);
         if (s->d_ptiles[i]) cudaFree(s->d_ptiles[i]);
     }
-    if (s->d_tiles) cudaFree(s->d_tiles);
     if (s->d_vad) cudaFree(s->d_vad);
     if (s->d_energy) cudaFree(s->d_energy);
     if (s->d_frac) cudaFree(s->d_frac);
@@ -1460,10 +1459,8 @@ AF_API int af_session_reset(af_session *s)
 {
     if (!s) return fail(AF_ERR_INVALID, "null session");
     AF_SCOPE(s->device);
-    s->rec.init(s->rate, OUT_RATE);
-    s->in_cur = 0; s->y_cur = 0; s->y_len = 0; s->frames_emitted = 0; s->in_drop = 0; s->y_drop = 0;
-    s->in_len = 2 * RS_POLY;                       // rubato starts with 16 zero frames of history
-    s->in_base = -2 * RS_POLY;
+    s->shared = fresh_stream(s);
+    s->in_cur = 0; s->y_cur = 0;
     s->diverged = false;                           // every stream at the common start: lockstep again
     AF_CUDA(cudaMemset(s->in_buf[0], 0, s->S * s->in_stride * sizeof(float)));
     AF_CUDA(cudaMemset(s->d_vad, 0, s->S * sizeof(VadState)));
@@ -1488,8 +1485,8 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
     if (p->cfg.n_mels && !(s->d_mel = pipe_mel(p))) return AF_ERR_CUDA;
     s->pipe = p; s->S = n_streams; s->rate = sample_rate; s->channels = channels; s->format = format;
     s->max_tick_frames = (max_tick_samples + channels - 1) / channels;
-    s->rec.init(sample_rate, OUT_RATE);
-    if (!s->rec.passthrough && s->rec.end_idx <= 0) return fail(AF_ERR_RESAMPLING_FAILED, "unsupported resampling ratio");
+    s->shared = fresh_stream(s.get());
+    if (!s->shared.rec.passthrough && s->shared.rec.end_idx <= 0) return fail(AF_ERR_RESAMPLING_FAILED, "unsupported resampling ratio");
     s->framing = cfg.n_mels != 0 || cfg.vad_enable;
     if (cfg.vad_enable && cfg.vad_frame_len != 0) { s->frame_len = cfg.vad_frame_len; s->hop = cfg.vad_hop; }
     s->in_stride = round_up(2 * RS_POLY + RS_CHUNK + s->max_tick_frames + 8, 4);
@@ -1513,16 +1510,6 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
         AF_CUDA(cudaMalloc(&s->in_buf[i], n_streams * s->in_stride * sizeof(float)));
         AF_CUDA(cudaMalloc(&s->y_buf[i], n_streams * s->y_stride * sizeof(float)));
         AF_CUDA(cudaMemset(s->y_buf[i], 0, n_streams * s->y_stride * sizeof(float)));
-        AF_CUDA(cudaMalloc(&s->d_tab[i], n_streams * sizeof(StreamDev)));
-        std::vector<StreamDev> tab(n_streams);
-        for (size_t k = 0; k < n_streams; ++k) {
-            StreamDev &d = tab[k];
-            memset(&d, 0, sizeof(d));
-            d.data = s->y_buf[i] + k * s->y_stride;
-            d.channels = 1; d.format = FMT_F32; d.p = 1; d.q = 1; d.mode = RS_PASSTHROUGH;
-            d.tile_begin = (uint32_t)k; d.n_tiles = 1; d.staged = 2;
-        }
-        AF_CUDA(cudaMemcpy(s->d_tab[i], tab.data(), n_streams * sizeof(StreamDev), cudaMemcpyHostToDevice));
         if (s->packed) {
             std::vector<StreamDev> ptab(s->pk_n);
             std::vector<TileDev> ptiles(s->pk_n);
@@ -1544,298 +1531,21 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
         }
     }
     if (s->y_stride > (uint64_t)TILE_SAMPLES) return fail(AF_ERR_INVALID, "max_tick_samples too large for a session (%u)", max_tick_samples);
-    AF_CUDA(cudaMalloc(&s->d_tiles, n_streams * sizeof(TileDev)));    // planned per tick by the session set-up kernel
-    AF_CUDA(cudaMemset(s->d_tiles, 0, n_streams * sizeof(TileDev)));
     AF_CUDA(cudaMalloc(&s->d_vad, n_streams * sizeof(VadState)));
     AF_CUDA(cudaMalloc(&s->d_energy, n_streams * s->energy_stride * sizeof(float)));
     s->frac_cap = max_new_y + 64;
     AF_CUDA(cudaMalloc(&s->d_frac, s->frac_cap * sizeof(float)));
     s->ss.resize(n_streams); s->ss_next.resize(n_streams);
-    s->first_frames.assign(n_streams, 0); s->first_frames_next.assign(n_streams, 0);
+    s->first_frames.assign(n_streams, 0);
     rc = af_session_reset(s.get());
     if (rc) return rc;
     *out = s.release();
     return AF_OK;
 }
 
-AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, uint32_t n_samples, int mem,
-                           const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
-{
-    if (!s || (!data && n_samples)) return fail(AF_ERR_INVALID, "null argument");
-    if (s->diverged) {                                           // streams on their own timelines: the same count for each
-        s->counts.assign(s->S, n_samples);
-        return af_session_push_streams(s, data, in_stride, s->counts.data(), nullptr, mem, o, n_pcm, n_feat, n_vad);
-    }
-    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
-    if (n_samples % s->channels) return fail(AF_ERR_INVALID, "a tick must hold whole frames (n_samples %% channels == 0)");
-    const uint32_t n_new = n_samples / s->channels;
-    if (n_new > s->max_tick_frames) return fail(AF_ERR_CAPACITY, "tick of %u frames exceeds max_tick_samples", n_new);
-    if (in_stride < n_samples) return fail(AF_ERR_INVALID, "in_stride smaller than n_samples");
-    AF_SCOPE(s->device);
-    const af_pipeline_config &cfg = s->pipe->cfg;
-    cudaStream_t st = cur_ctx().stream;
-    const size_t S = s->S;
-    const uint32_t bps = s->format == AF_FMT_I16 ? 2 : 4;
-    af_outputs none{};
-    if (!o) o = &none;
-
-    // ---- 0. plan the tick on COPIES of the session state and validate every caller-supplied size: a recoverable error
-    //         (a stride that is too small) must leave the session exactly as it was ----
-    // frames held: [history 16 | residual r | new n_new]; chunks formed from residual + new
-    const uint32_t residual = s->in_len - 2 * RS_POLY;
-    const uint32_t avail = residual + n_new;
-    const uint32_t chunks = s->rec.passthrough ? 0 : avail / RS_CHUNK;
-    RsRecurrence rec = s->rec;                                   // the shared f64 recurrence, advanced on a copy
-    const uint64_t n_begin = rec.passthrough ? (uint64_t)(s->in_base + 2 * RS_POLY + residual) : rec.n_out;
-    uint64_t n_end = n_begin;
-    s->frac_host.clear();                                        // (scratch, not state)
-    if (rec.passthrough) n_end = n_begin + n_new;
-    else {
-        for (uint32_t c = 0; c < chunks; ++c) rec.step(rec.exact ? nullptr : &s->frac_host);
-        n_end = rec.n_out;
-    }
-    const uint32_t n_y_new = (uint32_t)(n_end - n_begin);
-    if (s->y_len + n_y_new > s->y_stride) return fail(AF_ERR_CAPACITY, "internal: 16 kHz carry overflow");
-    if (s->frac_host.size() > s->frac_cap) return fail(AF_ERR_CAPACITY, "internal: fraction buffer overflow");
-    const uint32_t y_total = s->y_len + n_y_new;
-    uint32_t T = 0;
-    if (s->framing && y_total >= s->frame_len) T = 1 + (y_total - s->frame_len) / s->hop;
-    const bool want_pcm = cfg.write_pcm && o->pcm && n_y_new;
-    const bool want_lm = T && cfg.n_mels && o->logmel;
-    const bool want_states = T && cfg.vad_enable && o->vad;
-    // the wire output needs the tick's states for its events and its gate, whatever the caller asked for
-    const bool need_states = want_states || (s->wire && T && cfg.vad_enable);
-    if (want_pcm && o->pcm_stride < n_y_new) return fail(AF_ERR_CAPACITY, "pcm_stride %llu too small for %u samples", (unsigned long long)o->pcm_stride, n_y_new);
-    if (want_lm && o->logmel_stride < (uint64_t)T * cfg.n_mels) return fail(AF_ERR_CAPACITY, "logmel_stride too small for %u frames", T);
-    if (want_states && o->vad_stride < T) return fail(AF_ERR_CAPACITY, "vad_stride too small for %u frames", T);
-    if (T && s->packed && T + 2 > s->pk_slots) return fail(AF_ERR_CAPACITY, "internal: %u frames do not fit %u frame slots", T, s->pk_slots);
-    // internal staging buffers (allocation failures are reported before anything changes, too)
-    float *lm = nullptr; uint64_t lm_stride = 0;
-    uint8_t *states = nullptr; uint64_t st_stride = 0;
-    if (want_lm) {
-        if (mem == AF_MEM_HOST || s->packed) {                  // (packed ticks write every frame slot: internal buffer, then a strided copy)
-            if (!s->d_lm) AF_CUDA(cudaMalloc(&s->d_lm, S * s->lm_stride * sizeof(float)));
-            lm = s->d_lm; lm_stride = s->lm_stride;
-        } else { lm = o->logmel; lm_stride = o->logmel_stride; }
-        if (lm_stride < (uint64_t)T * cfg.n_mels) return fail(AF_ERR_CAPACITY, "internal: log-mel staging too small for %u frames", T);
-    }
-    if (need_states) {
-        if (mem == AF_MEM_HOST || !want_states) {
-            if (!s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));
-            states = s->d_states; st_stride = s->st_stride;
-        } else { states = o->vad; st_stride = o->vad_stride; }
-        if (st_stride < T) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", T);
-    }
-    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)T * s->hop : n_y_new;   // bound of this tick's payloads
-    if (s->wire && wire_n > s->wire_cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
-    const void *d_in = data;
-    uint64_t d_in_stride_bytes = in_stride * bps;
-    if (mem == AF_MEM_HOST && n_samples) {
-        const size_t row = round_up((uint64_t)n_samples * bps, 16);
-        if (s->in_stage_bytes < row * S) {
-            if (s->d_in_stage) cudaFree(s->d_in_stage);
-            s->d_in_stage = nullptr; s->in_stage_bytes = 0;
-            AF_CUDA(cudaMalloc(&s->d_in_stage, row * S));
-            s->in_stage_bytes = row * S;
-        }
-        d_in = s->d_in_stage; d_in_stride_bytes = row;
-    }
-
-    // From here on only CUDA failures can occur.  The bookkeeping is restored if one does (the ping-pong buffers keep
-    // the previous tick intact); the detector states and the wire output's carried segment state on the device may
-    // already have advanced -- af_session_reset after an AF_ERR_CUDA.  The wire rows may hold part of the failed tick,
-    // so af_session_wire refuses them until the next push.
-    struct Restore {
-        af_session *s; bool armed = true;
-        RsRecurrence rec; int in_cur, y_cur; uint32_t in_len, in_drop, y_len, y_drop; long long in_base; uint64_t frames_emitted;
-        explicit Restore(af_session *s_) : s(s_), rec(s_->rec), in_cur(s_->in_cur), y_cur(s_->y_cur), in_len(s_->in_len), in_drop(s_->in_drop),
-                                          y_len(s_->y_len), y_drop(s_->y_drop), in_base(s_->in_base), frames_emitted(s_->frames_emitted) {}
-        ~Restore()
-        {
-            if (!armed) return;
-            s->rec = rec; s->in_cur = in_cur; s->y_cur = y_cur; s->in_len = in_len; s->in_drop = in_drop; s->y_len = y_len;
-            s->y_drop = y_drop; s->in_base = in_base; s->frames_emitted = frames_emitted;
-            if (s->wire) s->wire_valid = false;
-        }
-    } restore(s);
-
-    const uint32_t y_new = s->y_len;                             // where the tick's new samples start in its 16 kHz rows
-    // ---- 1. input: host ticks are staged; then carry history + residual and append the downmixed frames ----
-    if (mem == AF_MEM_HOST && n_samples)
-        AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)n_samples * bps, S, cudaMemcpyHostToDevice, st));
-    SessionIngest ing{};
-    ing.old_buf = s->in_buf[s->in_cur]; ing.new_buf = s->in_buf[s->in_cur ^ 1]; ing.buf_stride = s->in_stride;
-    ing.drop = s->in_drop; ing.keep = s->in_len;                  // (the previous tick's consumed chunks are dropped here)
-    ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.n_samples = n_samples; ing.n_new_frames = n_new;
-    ing.channels = s->channels; ing.format = s->format;
-    s->in_cur ^= 1;                                              // (launched below, together with the resampling of the tick)
-    s->in_drop = 0;
-    s->in_len += n_new;
-
-    // ---- 2. resample the complete chunks (shared f64 recurrence on the host, fractions uploaded) ----
-    s->rec = rec;
-    if (!s->frac_host.empty())
-        AF_CUDA(cudaMemcpyAsync(s->d_frac, s->frac_host.data(), s->frac_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
-    SessionResample rs{};
-    rs.in_buf = s->in_buf[s->in_cur]; rs.in_stride = s->in_stride;
-    rs.data_base = s->in_base;
-    rs.n_valid_end = s->rec.passthrough ? s->in_base + (long long)s->in_len
-                                        : s->in_base + 2 * RS_POLY + (long long)((residual + n_new) / RS_CHUNK * RS_CHUNK);
-    rs.n_begin = n_begin; rs.n_end = n_end; rs.p = s->rec.p; rs.q = s->rec.q; rs.mode = s->rec.mode();
-    rs.frac = s->d_frac;
-    rs.y_old = s->y_buf[s->y_cur]; rs.y_new = s->y_buf[s->y_cur ^ 1]; rs.y_stride = s->y_stride;
-    rs.y_drop = s->y_drop; rs.y_keep = s->y_len;                  // (the samples the previous tick's frames consumed are dropped here)
-    AF_CUDA(launch_session_tick(ing, rs, (uint32_t)S, st));      // ingest + resample: one CTA per stream, one launch
-    count_launch();
-    s->y_cur ^= 1;
-    float *ycur = s->y_buf[s->y_cur];
-
-    // ---- 3. PCM of this tick ----
-    if (want_pcm)
-        AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), ycur + s->y_len, s->y_stride * sizeof(float),
-                                  (size_t)n_y_new * sizeof(float), S,
-                                  mem == AF_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
-
-    if (s->levels) {
-        AF_CUDA(launch_peak(ycur + s->y_len, s->y_stride, n_y_new, (uint32_t)S, s->d_peak, st));
-        count_launch();
-    }
-
-    // ---- 4. frames that became complete: features + VAD ----
-    const bool stft_frames = (s->frame_len == WIN && s->hop == HOP);
-    if (T) {
-        if (stft_frames) {
-            FusedParams P{};
-            uint64_t vrows = 1;                                 // real streams per stream of the launch
-            if (s->packed) {
-                P.streams = s->d_ptab[s->y_cur]; P.tiles = s->d_ptiles[s->y_cur]; P.n_tiles = s->pk_n;
-                vrows = s->pk_rows;
-            } else {
-                AF_CUDA(launch_session_setup(s->d_tab[s->y_cur], s->d_tiles, (uint32_t)S, y_total, T, cfg.vad_enable ? T : 0, st));
-                P.streams = s->d_tab[s->y_cur]; P.tiles = s->d_tiles; P.n_tiles = (uint32_t)S;
-            }
-            P.fft = cur_ctx().d_fft; P.mel = s->d_mel;
-            P.pcm = nullptr; P.pcm_stride = 0;
-            P.logmel = lm; P.logmel_stride = lm_stride * vrows;
-            P.energy = cfg.vad_enable ? s->d_energy : nullptr; P.energy_stride = s->energy_stride * vrows;
-            P.n_mels = lm ? cfg.n_mels : 0;
-            P.do_energy = cfg.vad_enable ? 1 : 0;
-            P.log_floor = cfg.log_floor;
-            P.log_scale = cfg.log10 ? 0.30102999566398120f : 0.69314718055994531f;
-            P.use_stage = kernel_variant() == "sync" ? 0u : 1u;
-            P.layout = fused_layout(P.do_energy != 0);
-            P.neg_zero = -0.0f;
-            if (P.n_mels || P.do_energy) {
-                AF_CUDA(launch_fused(P, (int)std::min<size_t>(P.n_tiles, (size_t)cur_ctx().sm_count), st));
-                count_launch(2);
-            }
-        } else {
-            EnergyJob ej{};
-            ej.y = ycur; ej.y_stride = s->y_stride; ej.n_frames = nullptr; ej.n_frames_all = T;
-            ej.frame_len = s->frame_len; ej.hop = s->hop; ej.energy = s->d_energy; ej.energy_stride = s->energy_stride;
-            ej.n_streams = (uint32_t)S;
-            AF_CUDA(launch_frame_energy(ej, st));
-            count_launch();
-        }
-        if (cfg.vad_enable) {
-            ScanJob sj{};
-            sj.energy = s->d_energy; sj.energy_stride = s->energy_stride; sj.n_frames = nullptr; sj.n_frames_all = T;
-            sj.states = states; sj.states_stride = st_stride; sj.state_io = s->d_vad;
-            sj.final_out = mem == AF_MEM_DEVICE ? reinterpret_cast<VadState *>(o->vad_final) : nullptr;
-            sj.prm = s->pipe->vad_prm; sj.n_streams = (uint32_t)S;
-            AF_CUDA(launch_vad_scan(sj, st));
-            count_launch();
-        }
-        if (mem == AF_MEM_DEVICE && lm && lm != o->logmel)
-            AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
-                                      (size_t)T * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToDevice, st));
-        if (mem == AF_MEM_HOST) {
-            if (lm) AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
-                                              (size_t)T * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
-            if (want_states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, T, S, cudaMemcpyDeviceToHost, st));
-            if (cfg.vad_enable && o->vad_final)
-                AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad, S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
-        }
-    }
-    // ---- 5. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
-    if (s->wire) {
-        const af_wire_config &wc = s->wire_cfg;
-        WireJob wj{};
-        wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = y_new; wj.n_new = n_y_new;
-        wj.states = (T && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
-        wj.T = T; wj.hop = s->hop; wj.gate = wc.gate;
-        wj.prev = s->d_wire_prev;
-        wj.pcm16 = s->d_wire_pcm16; wj.pcm16_stride = s->wire_pcm16_stride;
-        wj.b64 = s->d_wire_b64; wj.b64_stride = s->wire_b64_stride;
-        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S;
-        AF_CUDA(launch_session_wire(wj, st));
-        count_launch();
-        if (wc.mem == AF_MEM_HOST && wire_n) {
-            if (wc.pcm16)
-                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_pcm16, s->wire_pcm16_stride * sizeof(int16_t), s->d_wire_pcm16,
-                                          s->wire_pcm16_stride * sizeof(int16_t), wire_n * sizeof(int16_t), S, cudaMemcpyDeviceToHost, st));
-            if (wc.base64)
-                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_b64, s->wire_b64_stride, s->d_wire_b64, s->wire_b64_stride,
-                                          af_pcm16_base64_len(wire_n), S, cudaMemcpyDeviceToHost, st));
-        }
-        AF_CUDA(cudaMemcpyAsync(s->h_wire_ticks, s->d_wire_ticks, S * sizeof(af_wire_tick), cudaMemcpyDeviceToHost, st));
-    }
-    if (s->levels) {
-        AF_CUDA(cudaMemcpyAsync(s->h_peak, s->d_peak, S * sizeof(float), cudaMemcpyDeviceToHost, st));
-        AF_CUDA(cudaMemcpyAsync(s->h_vad, s->d_vad, S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
-    }
-    AF_CUDA(cudaStreamSynchronize(st));
-    restore.armed = false;
-    s->levels_valid = s->levels;
-    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->frames_emitted; s->first_frames_ragged = false; }
-
-    // ---- 6. bookkeeping: the consumed chunks and the samples every future frame starts after are dropped by the next
-    //         tick's ingest / resample kernels (in_drop, y_drop): no kernel and no second synchronisation here ----
-    if (!s->rec.passthrough) {
-        const uint32_t consumed = chunks * RS_CHUNK;              // keep [history 16 | new residual]
-        s->in_drop = consumed; s->in_len -= consumed; s->in_base += consumed;
-    } else {
-        // passthrough keeps nothing but the 16-frame history slot
-        s->in_drop = s->in_len - 2 * RS_POLY; s->in_base += (long long)(s->in_len - 2 * RS_POLY); s->in_len = 2 * RS_POLY;
-    }
-    uint32_t y_drop = s->framing ? T * s->hop : y_total;
-    if (y_drop > y_total) y_drop = y_total;
-    s->y_drop = y_drop;
-    s->y_len = y_total - y_drop;
-    s->frames_emitted += T;
-    for (size_t k = 0; k < S; ++k) {
-        if (n_pcm) n_pcm[k] = n_y_new;
-        if (n_feat) n_feat[k] = cfg.n_mels ? T : 0;
-        if (n_vad) n_vad[k] = cfg.vad_enable ? T : 0;
-    }
-    return AF_OK;
-}
-
 }  // extern "C"
 
-// ------------------------------------------------------------------------------------------
-// independent stream timelines: ragged ticks, end of stream (BatchResampler::flush), per-stream restart
-// ------------------------------------------------------------------------------------------
 namespace {
-using StreamState = af_session::StreamState;
-
-StreamState fresh_stream(const af_session *s)
-{
-    StreamState f{};
-    f.rec.init(s->rate, OUT_RATE);
-    f.in_len = 2 * RS_POLY;                                      // 16 zero frames of history, as af_session_reset
-    f.in_base = -2 * RS_POLY;
-    return f;
-}
-
-StreamState shared_stream(const af_session *s)
-{
-    StreamState c{};
-    c.rec = s->rec; c.in_len = s->in_len; c.in_drop = s->in_drop; c.y_len = s->y_len; c.y_drop = s->y_drop;
-    c.in_base = s->in_base; c.frames_emitted = s->frames_emitted; c.restart = false;
-    return c;
-}
-
 bool same_position(const StreamState &a, const StreamState &b)
 {
     return !a.restart && !b.restart && a.rec.chunks == b.rec.chunks && a.rec.n_out == b.rec.n_out &&
@@ -1859,8 +1569,73 @@ void rs_advance(RsRecurrence &r, uint32_t chunks, std::vector<float> *frac)
     r.last_index = -(double)(RS_POLY / 2) + (double)num / (double)r.q;
 }
 
-int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples, const uint8_t *end, int mem,
-                        const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
+// one stream's count in a tick: whole frames, at most max_tick_samples, within its input row
+int check_count(const af_session *s, uint32_t n, uint64_t in_stride)
+{
+    if (n % s->channels) return fail(AF_ERR_INVALID, "a tick of %u samples is not a whole number of frames", n);
+    if (n / s->channels > s->max_tick_frames) return fail(AF_ERR_CAPACITY, "tick of %u frames exceeds max_tick_samples", n / s->channels);
+    if (in_stride < n) return fail(AF_ERR_INVALID, "in_stride %llu smaller than a tick of %u samples", (unsigned long long)in_stride, n);
+    return AF_OK;
+}
+
+// Plans one stream's tick of n_samples from its state `now` (a fresh stream when it restarts): fills `d` and the state
+// after the tick, `next`, and appends the RS_TABLE fractions to s->frac_host at d.frac_off.  fin ends the stream after
+// the tick (BatchResampler::flush, resampler.rs:150-166).  Only internal capacity errors can occur; nothing changes.
+int plan_stream(af_session *s, const StreamState &now, uint32_t n_samples, bool fin, StreamTick &d, StreamState &next)
+{
+    StreamState c = now.restart ? fresh_stream(s) : now;
+    // frames held: [history 16 | residual r | new n_new]; chunks formed from residual + new
+    const uint32_t n_new = n_samples / s->channels;
+    const uint32_t residual = c.in_len - 2 * RS_POLY;
+    const uint32_t avail = residual + n_new;
+    const bool pass = c.rec.passthrough;
+    const uint32_t full = pass ? 0 : avail / RS_CHUNK;
+    // a flush zero-pads a residual to one more chunk.  The bound of max_new_y holds for it: ceil((127 + max_tick_frames)
+    // / 128) chunks <= the ceil((max_tick_frames + 128) / 128) it was sized for.
+    const uint32_t chunks = full + ((fin && !pass && avail % RS_CHUNK) ? 1 : 0);
+    const uint64_t n_begin = pass ? (uint64_t)(c.in_base + 2 * RS_POLY + residual) : c.rec.n_out;
+    const size_t frac_off = s->frac_host.size();
+    rs_advance(c.rec, chunks, c.rec.mode() == RS_TABLE ? &s->frac_host : nullptr);
+    const uint64_t n_end = pass ? n_begin + n_new : c.rec.n_out;
+    const uint32_t n_y = (uint32_t)(n_end - n_begin);
+    if (c.y_len + n_y > s->y_stride) return fail(AF_ERR_CAPACITY, "internal: 16 kHz carry overflow");
+    const uint32_t y_total = c.y_len + n_y;
+    uint32_t T = 0;
+    if (s->framing && y_total >= s->frame_len) T = 1 + (y_total - s->frame_len) / s->hop;
+    if (T && s->packed && T + 2 > s->pk_slots) return fail(AF_ERR_CAPACITY, "internal: %u frames do not fit %u frame slots", T, s->pk_slots);
+    d.in_drop = c.in_drop; d.in_keep = c.in_len; d.n_new = n_new; d.n_samples = n_samples;
+    d.data_base = c.in_base;
+    d.n_valid_end = pass ? c.in_base + (long long)(c.in_len + n_new)
+                         : c.in_base + 2 * RS_POLY + (long long)(fin ? avail : full * RS_CHUNK);
+    d.n_begin = n_begin; d.n_y = n_y; d.frac_off = (uint32_t)frac_off;
+    d.y_drop = c.y_drop; d.y_keep = c.y_len;
+    d.T = T; d.flags = (now.restart ? TICK_RESTART : 0u) | (fin ? TICK_END : 0u);
+    // the consumed chunks and the samples every future frame starts after are dropped by the next tick's ingest /
+    // resample (in_drop, y_drop): no kernel and no second synchronisation
+    c.in_len += n_new;
+    if (!pass) {
+        const uint32_t consumed = full * RS_CHUNK;              // keep [history 16 | new residual]
+        c.in_drop = consumed; c.in_len -= consumed; c.in_base += consumed;
+    } else {
+        // passthrough keeps nothing but the 16-frame history slot
+        c.in_drop = c.in_len - 2 * RS_POLY; c.in_base += (long long)(c.in_len - 2 * RS_POLY); c.in_len = 2 * RS_POLY;
+    }
+    const uint32_t y_drop = s->framing ? std::min(T * s->hop, y_total) : y_total;
+    c.y_drop = y_drop; c.y_len = y_total - y_drop;
+    c.frames_emitted += T;
+    c.restart = fin;
+    next = c;
+    return AF_OK;
+}
+
+// One tick.  per_stream: stream k pushes n_samples[k] from its own position ss[k] (end[k] != 0: its last tick), planned
+// into the uploaded table h_tick / d_tick that af_session_tick_streams_kernel reads.  Otherwise every stream pushes
+// n_samples[0] from `shared`, and af_session_tick_kernel takes that one plan as kernel parameters.  Everything after the
+// tick kernel is the same code for both.  Argument errors are reported before anything changes; the bookkeeping is
+// committed after the tick's synchronise, so an AF_ERR_CUDA leaves it as it was (reset after one: the detector and wire
+// state on the device may have advanced, and af_session_wire refuses the rows until the next push).
+int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples, const uint8_t *end,
+                 bool per_stream, int mem, const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
 {
     AF_SCOPE(s->device);
     const af_pipeline_config &cfg = s->pipe->cfg;
@@ -1870,95 +1645,56 @@ int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, con
     af_outputs none{};
     if (!o) o = &none;
 
-    // ---- 0. buffers of the ragged path (allocated once; failures leave the session as it was) ----
-    const size_t tick_bytes = S * (sizeof(StreamTick) + sizeof(uint32_t));
-    if (!s->d_tick) {                                            // set together: a failed allocation leaves neither
-        StreamTick *d = nullptr, *h = nullptr;
-        cudaError_t e = cudaMalloc(&d, tick_bytes);
-        if (e == cudaSuccess) e = cudaHostAlloc((void **)&h, tick_bytes, cudaHostAllocDefault);
-        if (e != cudaSuccess) {
-            if (d) cudaFree(d);
-            return fail(AF_ERR_CUDA, "allocating the tick plan: %s", cudaGetErrorString(e));
-        }
-        s->d_tick = d; s->h_tick = h;
-    }
-    const bool table = s->rec.mode() == RS_TABLE;
-    if (table && s->frac_cap < S * s->max_new_y) {               // every stream's fractions, one slice after another
-        float *f = nullptr;
-        AF_CUDA(cudaMalloc(&f, S * s->max_new_y * sizeof(float)));
-        cudaFree(s->d_frac);
-        s->d_frac = f; s->frac_cap = S * s->max_new_y;
-    }
-
-    // ---- 1. plan every stream on copies of its state; the session changes only after the tick's synchronise ----
-    if (!s->diverged) {
-        const StreamState c = shared_stream(s);
-        for (size_t k = 0; k < S; ++k) s->ss[k] = c;
-    }
-    const StreamState fresh = fresh_stream(s);
-    StreamTick *tab = s->h_tick;
-    uint32_t *Ts = reinterpret_cast<uint32_t *>(tab + S);
-    uint32_t *d_T = reinterpret_cast<uint32_t *>(s->d_tick + S);
-    s->frac_host.clear();
+    // ---- 0. plan every stream on copies of its state; validate every caller-supplied size ----
+    StreamTick one{};                   // the lockstep plan (all zero on a per-stream tick, whose kernels read the table)
+    StreamState shared_next{};
+    s->frac_host.clear();               // (scratch, not state)
     uint32_t maxT = 0, max_ny = 0, max_n = 0;
-    for (size_t k = 0; k < S; ++k) {
-        const bool restart = s->ss[k].restart, fin = end && end[k];
-        StreamState c = restart ? fresh : s->ss[k];
-        const uint32_t n_new = n_samples[k] / s->channels;
-        const uint32_t residual = c.in_len - 2 * RS_POLY;
-        const uint32_t avail = residual + n_new;
-        const bool pass = c.rec.passthrough;
-        const uint32_t full = pass ? 0 : avail / RS_CHUNK;
-        // flush (resampler.rs:150-166): a residual is zero-padded to one more chunk.  The bound of max_new_y holds for it:
-        // ceil((127 + max_tick_frames) / 128) chunks <= the ceil((max_tick_frames + 128) / 128) it was sized for.
-        const uint32_t chunks = full + ((fin && !pass && avail % RS_CHUNK) ? 1 : 0);
-        const uint64_t n_begin = pass ? (uint64_t)(c.in_base + 2 * RS_POLY + residual) : c.rec.n_out;
-        const size_t frac_off = s->frac_host.size();
-        rs_advance(c.rec, chunks, table ? &s->frac_host : nullptr);
-        const uint64_t n_end = pass ? n_begin + n_new : c.rec.n_out;
-        const uint32_t n_y = (uint32_t)(n_end - n_begin);
-        if (c.y_len + n_y > s->y_stride) return fail(AF_ERR_CAPACITY, "internal: 16 kHz carry overflow (stream %zu)", k);
-        const uint32_t y_total = c.y_len + n_y;
-        uint32_t T = 0;
-        if (s->framing && y_total >= s->frame_len) T = 1 + (y_total - s->frame_len) / s->hop;
-        if (T && s->packed && T + 2 > s->pk_slots) return fail(AF_ERR_CAPACITY, "internal: %u frames do not fit %u frame slots", T, s->pk_slots);
-        StreamTick &d = tab[k];
-        d.in_drop = c.in_drop; d.in_keep = c.in_len; d.n_new = n_new; d.n_samples = n_samples[k];
-        d.data_base = c.in_base;
-        d.n_valid_end = pass ? c.in_base + (long long)(c.in_len + n_new)
-                             : c.in_base + 2 * RS_POLY + (long long)(fin ? avail : full * RS_CHUNK);
-        d.n_begin = n_begin; d.n_y = n_y; d.frac_off = (uint32_t)frac_off;
-        d.y_drop = c.y_drop; d.y_keep = c.y_len;
-        d.T = T; d.flags = (restart ? TICK_RESTART : 0u) | (fin ? TICK_END : 0u);
-        Ts[k] = T;
-        s->first_frames_next[k] = c.frames_emitted;
-        // the stream after the tick (as af_session_push's bookkeeping)
-        c.in_len += n_new;
-        if (!pass) {
-            const uint32_t consumed = full * RS_CHUNK;
-            c.in_drop = consumed; c.in_len -= consumed; c.in_base += consumed;
-        } else {
-            c.in_drop = c.in_len - 2 * RS_POLY; c.in_base += (long long)(c.in_len - 2 * RS_POLY); c.in_len = 2 * RS_POLY;
+    const size_t tick_bytes = S * (sizeof(StreamTick) + sizeof(uint32_t));
+    if (!per_stream) {
+        const int rc = plan_stream(s, s->shared, n_samples[0], false, one, shared_next);
+        if (rc) return rc;
+        maxT = one.T; max_ny = one.n_y; max_n = n_samples[0];
+    } else {
+        if (!s->d_tick) {                                        // set together: a failed allocation leaves neither
+            StreamTick *d = nullptr, *h = nullptr;
+            cudaError_t e = cudaMalloc(&d, tick_bytes);
+            if (e == cudaSuccess) e = cudaHostAlloc((void **)&h, tick_bytes, cudaHostAllocDefault);
+            if (e != cudaSuccess) {
+                if (d) cudaFree(d);
+                return fail(AF_ERR_CUDA, "allocating the tick plan: %s", cudaGetErrorString(e));
+            }
+            s->d_tick = d; s->h_tick = h;
         }
-        const uint32_t y_drop = s->framing ? std::min(T * s->hop, y_total) : y_total;
-        c.y_drop = y_drop; c.y_len = y_total - y_drop;
-        c.frames_emitted += T;
-        c.restart = fin;
-        s->ss_next[k] = c;
-        maxT = std::max(maxT, T); max_ny = std::max(max_ny, n_y); max_n = std::max(max_n, n_samples[k]);
+        if (s->shared.rec.mode() == RS_TABLE && s->frac_cap < S * s->max_new_y) {   // every stream's fractions, one slice after another
+            float *f = nullptr;
+            AF_CUDA(cudaMalloc(&f, S * s->max_new_y * sizeof(float)));
+            cudaFree(s->d_frac);
+            s->d_frac = f; s->frac_cap = S * s->max_new_y;
+        }
+        if (!s->diverged) s->ss.assign(S, s->shared);
+        uint32_t *Ts = reinterpret_cast<uint32_t *>(s->h_tick + S);
+        for (size_t k = 0; k < S; ++k) {
+            const int rc = plan_stream(s, s->ss[k], n_samples[k], end && end[k], s->h_tick[k], s->ss_next[k]);
+            if (rc) return rc;
+            Ts[k] = s->h_tick[k].T;
+            maxT = std::max(maxT, Ts[k]); max_ny = std::max(max_ny, s->h_tick[k].n_y); max_n = std::max(max_n, n_samples[k]);
+        }
     }
     if (s->frac_host.size() > s->frac_cap) return fail(AF_ERR_CAPACITY, "internal: fraction buffer overflow");
     const bool want_pcm = cfg.write_pcm && o->pcm && max_ny;
     const bool want_lm = maxT && cfg.n_mels && o->logmel;
     const bool want_states = maxT && cfg.vad_enable && o->vad;
+    // the wire output needs the tick's states for its events and its gate, whatever the caller asked for
     const bool need_states = want_states || (s->wire && maxT && cfg.vad_enable);
     if (want_pcm && o->pcm_stride < max_ny) return fail(AF_ERR_CAPACITY, "pcm_stride %llu too small for %u samples", (unsigned long long)o->pcm_stride, max_ny);
     if (want_lm && o->logmel_stride < (uint64_t)maxT * cfg.n_mels) return fail(AF_ERR_CAPACITY, "logmel_stride too small for %u frames", maxT);
     if (want_states && o->vad_stride < maxT) return fail(AF_ERR_CAPACITY, "vad_stride too small for %u frames", maxT);
+    // internal staging buffers (allocation failures are reported before anything changes, too)
     float *lm = nullptr; uint64_t lm_stride = 0;
     uint8_t *states = nullptr; uint64_t st_stride = 0;
     if (want_lm) {
-        if (mem == AF_MEM_HOST || s->packed) {
+        if (mem == AF_MEM_HOST || s->packed) {                  // (packed ticks write every frame slot: internal buffer, then a strided copy)
             if (!s->d_lm) AF_CUDA(cudaMalloc(&s->d_lm, S * s->lm_stride * sizeof(float)));
             lm = s->d_lm; lm_stride = s->lm_stride;
         } else { lm = o->logmel; lm_stride = o->logmel_stride; }
@@ -1971,15 +1707,15 @@ int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, con
         } else { states = o->vad; st_stride = o->vad_stride; }
         if (st_stride < maxT) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", maxT);
     }
-    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)maxT * s->hop : max_ny;
+    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)maxT * s->hop : max_ny;   // bound of this tick's payloads
     if (s->wire && wire_n > s->wire_cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
-    float *pcm_dst = nullptr; uint64_t pcm_dst_stride = 0;
-    if (want_pcm) {
+    float *pcm_rows = nullptr; uint64_t pcm_rows_stride = 0;   // per-stream: the tick kernel writes each stream's PCM here
+    if (want_pcm && per_stream) {
         if (mem == AF_MEM_HOST) {
             const uint64_t w = round_up(s->max_new_y, 4);
             if (!s->d_pcm_stage) AF_CUDA(cudaMalloc(&s->d_pcm_stage, S * w * sizeof(float)));
-            pcm_dst = s->d_pcm_stage; pcm_dst_stride = w;
-        } else { pcm_dst = o->pcm; pcm_dst_stride = o->pcm_stride; }
+            pcm_rows = s->d_pcm_stage; pcm_rows_stride = w;
+        } else { pcm_rows = o->pcm; pcm_rows_stride = o->pcm_stride; }
     }
     const void *d_in = data;
     uint64_t d_in_stride_bytes = in_stride * bps;
@@ -1994,50 +1730,65 @@ int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, con
         d_in = s->d_in_stage; d_in_stride_bytes = row;
     }
 
-    // From here on only CUDA failures can occur; the bookkeeping is committed after the synchronise (af_session_reset
-    // after an AF_ERR_CUDA: detector and wire state on the device may have advanced, the wire rows are refused).
-    if (s->wire) s->wire_valid = false;
-    // ---- 2. input (host rows: the last row is copied with its own count, the caller's buffer may end there), plan ----
+    // From here on only CUDA failures can occur.
+    s->wire_valid = false;
+    // ---- 1. input: host rows are staged (the caller's buffer may end after the last row's own count: unless that is
+    //         the largest, the last row is copied on its own); then the plan and the tick kernel ----
     if (mem == AF_MEM_HOST && max_n) {
-        if (S > 1)
-            AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)max_n * bps, S - 1,
-                                      cudaMemcpyHostToDevice, st));
-        if (n_samples[S - 1])
+        const uint32_t n_last = per_stream ? n_samples[S - 1] : max_n;
+        const size_t rows = n_last == max_n ? S : S - 1;
+        AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)max_n * bps, rows,
+                                  cudaMemcpyHostToDevice, st));
+        if (rows < S && n_last)
             AF_CUDA(cudaMemcpyAsync(static_cast<char *>(s->d_in_stage) + (S - 1) * d_in_stride_bytes,
-                                    static_cast<const char *>(data) + (S - 1) * in_stride * bps, (size_t)n_samples[S - 1] * bps,
+                                    static_cast<const char *>(data) + (S - 1) * in_stride * bps, (size_t)n_last * bps,
                                     cudaMemcpyHostToDevice, st));
     }
-    AF_CUDA(cudaMemcpyAsync(s->d_tick, s->h_tick, tick_bytes, cudaMemcpyHostToDevice, st));
+    if (per_stream) AF_CUDA(cudaMemcpyAsync(s->d_tick, s->h_tick, tick_bytes, cudaMemcpyHostToDevice, st));
     if (!s->frac_host.empty())
         AF_CUDA(cudaMemcpyAsync(s->d_frac, s->frac_host.data(), s->frac_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     const int in_next = s->in_cur ^ 1, y_next = s->y_cur ^ 1;
+    const StreamTick *tab = per_stream ? s->d_tick : nullptr;
+    const uint32_t *d_T = per_stream ? reinterpret_cast<const uint32_t *>(s->d_tick + S) : nullptr;
     SessionIngest ing{};
     ing.old_buf = s->in_buf[s->in_cur]; ing.new_buf = s->in_buf[in_next]; ing.buf_stride = s->in_stride;
     ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.channels = s->channels; ing.format = s->format;
     SessionResample rs{};
     rs.in_buf = s->in_buf[in_next]; rs.in_stride = s->in_stride;
-    rs.p = s->rec.p; rs.q = s->rec.q; rs.mode = s->rec.mode(); rs.frac = s->d_frac;
+    rs.p = s->shared.rec.p; rs.q = s->shared.rec.q; rs.mode = s->shared.rec.mode(); rs.frac = s->d_frac;
     rs.y_old = s->y_buf[s->y_cur]; rs.y_new = s->y_buf[y_next]; rs.y_stride = s->y_stride;
-    AF_CUDA(launch_session_tick_streams(ing, rs, s->d_tick, s->d_vad, s->d_wire_prev, pcm_dst, pcm_dst_stride, (uint32_t)S, st));
+    if (per_stream) {
+        AF_CUDA(launch_session_tick_streams(ing, rs, tab, s->d_vad, s->d_wire_prev, pcm_rows, pcm_rows_stride, (uint32_t)S, st));
+    } else {                                                     // the fields the streams kernel takes from its descriptor
+        ing.drop = one.in_drop; ing.keep = one.in_keep; ing.n_samples = one.n_samples; ing.n_new_frames = one.n_new;
+        rs.data_base = one.data_base; rs.n_valid_end = one.n_valid_end; rs.n_begin = one.n_begin; rs.n_end = one.n_begin + one.n_y;
+        rs.y_drop = one.y_drop; rs.y_keep = one.y_keep;
+        AF_CUDA(launch_session_tick(ing, rs, (uint32_t)S, st));
+    }
     count_launch();
     float *ycur = s->y_buf[y_next];
 
-    // ---- 3. PCM, levels ----
-    if (want_pcm && mem == AF_MEM_HOST)
-        AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), pcm_dst, pcm_dst_stride * sizeof(float),
+    // ---- 2. PCM (lockstep: copied out of the 16 kHz rows; per-stream: written by the tick kernel), levels ----
+    if (want_pcm && !per_stream)
+        AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), ycur + one.y_keep, s->y_stride * sizeof(float),
+                                  (size_t)max_ny * sizeof(float), S,
+                                  mem == AF_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+    else if (want_pcm && mem == AF_MEM_HOST)
+        AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), pcm_rows, pcm_rows_stride * sizeof(float),
                                   (size_t)max_ny * sizeof(float), S, cudaMemcpyDeviceToHost, st));
     if (s->levels) {
-        AF_CUDA(launch_peak(ycur, s->y_stride, 0, (uint32_t)S, s->d_peak, st, s->d_tick));
+        AF_CUDA(launch_peak(ycur + one.y_keep, s->y_stride, one.n_y, (uint32_t)S, s->d_peak, st, tab));
         count_launch();
     }
 
-    // ---- 4. frames: every frame slot of every row is computed by the packed launch (STFT frames with framing are always
-    //         packed), the energies of custom frames and the scan take each stream's count ----
+    // ---- 3. frames that became complete: features + VAD.  STFT frames with framing are always packed: the packed
+    //         launch computes every frame slot of every row; the energies of custom frames and the scan take each
+    //         stream's count ----
     if (maxT) {
         if (s->packed) {
             FusedParams P{};
             P.streams = s->d_ptab[y_next]; P.tiles = s->d_ptiles[y_next]; P.n_tiles = s->pk_n;
-            const uint64_t vrows = s->pk_rows;
+            const uint64_t vrows = s->pk_rows;                  // real streams per stream of the launch
             P.fft = cur_ctx().d_fft; P.mel = s->d_mel;
             P.pcm = nullptr; P.pcm_stride = 0;
             P.logmel = lm; P.logmel_stride = lm_stride * vrows;
@@ -2079,21 +1830,21 @@ int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, con
             if (want_states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, maxT, S, cudaMemcpyDeviceToHost, st));
         }
     }
-    // every stream's detector (a restarted one is fresh), whether or not a frame completed
+    // every stream's detector (a restarted one is fresh), whether or not a frame completed; the scan wrote device rows
     if (cfg.vad_enable && o->vad_final && (mem == AF_MEM_HOST || !maxT))
         AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad, S * sizeof(VadState),
                                 mem == AF_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
-    // ---- 5. wire payloads ----
+    // ---- 4. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
     if (s->wire) {
         const af_wire_config &wc = s->wire_cfg;
         WireJob wj{};
-        wj.y = ycur; wj.y_stride = s->y_stride;
+        wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = one.y_keep; wj.n_new = one.n_y;
         wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
         wj.T = maxT; wj.hop = s->hop; wj.gate = wc.gate;                 // (T sizes the kept-frame list: the largest)
         wj.prev = s->d_wire_prev;
         wj.pcm16 = s->d_wire_pcm16; wj.pcm16_stride = s->wire_pcm16_stride;
         wj.b64 = s->d_wire_b64; wj.b64_stride = s->wire_b64_stride;
-        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S; wj.tab = s->d_tick;
+        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S; wj.tab = tab;
         AF_CUDA(launch_session_wire(wj, st));
         count_launch();
         if (wc.mem == AF_MEM_HOST && wire_n) {
@@ -2112,30 +1863,45 @@ int session_push_ragged(af_session *s, const void *data, uint64_t in_stride, con
     }
     AF_CUDA(cudaStreamSynchronize(st));
 
-    // ---- 6. commit; streams that all stand at the same position run in lockstep again ----
+    // ---- 5. commit; streams that all stand at the same position run in lockstep again ----
     s->in_cur = in_next; s->y_cur = y_next;
-    s->ss.swap(s->ss_next);
-    s->first_frames.swap(s->first_frames_next);
     s->levels_valid = s->levels;
-    if (s->wire) { s->wire_valid = true; s->wire_first_frame = s->first_frames[0]; s->first_frames_ragged = true; }
-    bool aligned = true;
-    for (size_t k = 0; k < S && aligned; ++k) aligned = same_position(s->ss[k], s->ss[0]);
-    s->diverged = !aligned;
-    if (aligned) {
-        const StreamState &c = s->ss[0];
-        s->rec = c.rec; s->in_len = c.in_len; s->in_drop = c.in_drop; s->y_len = c.y_len; s->y_drop = c.y_drop;
-        s->in_base = c.in_base; s->frames_emitted = c.frames_emitted;
+    s->wire_valid = s->wire;
+    if (!per_stream) {
+        s->shared = shared_next;
+    } else {
+        s->ss.swap(s->ss_next);
+        bool aligned = true;
+        for (size_t k = 0; k < S && aligned; ++k) aligned = same_position(s->ss[k], s->ss[0]);
+        s->diverged = !aligned;
+        if (aligned) s->shared = s->ss[0];
     }
     for (size_t k = 0; k < S; ++k) {
-        if (n_pcm) n_pcm[k] = tab[k].n_y;
-        if (n_feat) n_feat[k] = cfg.n_mels ? tab[k].T : 0;
-        if (n_vad) n_vad[k] = cfg.vad_enable ? tab[k].T : 0;
+        const StreamTick &d = per_stream ? s->h_tick[k] : one;
+        s->first_frames[k] = (per_stream ? s->ss[k] : s->shared).frames_emitted - d.T;
+        if (n_pcm) n_pcm[k] = d.n_y;
+        if (n_feat) n_feat[k] = cfg.n_mels ? d.T : 0;
+        if (n_vad) n_vad[k] = cfg.vad_enable ? d.T : 0;
     }
     return AF_OK;
 }
 }  // namespace
 
 extern "C" {
+
+AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, uint32_t n_samples, int mem,
+                           const af_outputs *o, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad)
+{
+    if (!s || (!data && n_samples)) return fail(AF_ERR_INVALID, "null argument");
+    if (s->diverged) {                                           // streams on their own timelines: the same count for each
+        s->counts.assign(s->S, n_samples);
+        return af_session_push_streams(s, data, in_stride, s->counts.data(), nullptr, mem, o, n_pcm, n_feat, n_vad);
+    }
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    const int rc = check_count(s, n_samples, in_stride);
+    if (rc) return rc;
+    return session_tick(s, data, in_stride, &n_samples, nullptr, false, mem, o, n_pcm, n_feat, n_vad);
+}
 
 AF_API int af_session_push_streams(af_session *s, const void *data, uint64_t in_stride, const uint32_t *n_samples,
                                    const uint8_t *end, int mem, const af_outputs *out,
@@ -2146,17 +1912,14 @@ AF_API int af_session_push_streams(af_session *s, const void *data, uint64_t in_
     bool equal = true, any_end = false;
     for (size_t k = 0; k < s->S; ++k) {
         const uint32_t n = n_samples[k];
-        if (n % s->channels) return fail(AF_ERR_INVALID, "stream %zu: a tick must hold whole frames (n_samples %% channels == 0)", k);
-        if (n / s->channels > s->max_tick_frames) return fail(AF_ERR_CAPACITY, "stream %zu: tick of %u frames exceeds max_tick_samples", k, n / s->channels);
-        if (in_stride < n) return fail(AF_ERR_INVALID, "stream %zu: in_stride smaller than n_samples", k);
+        const int rc = check_count(s, n, in_stride);
+        if (rc) return rc;
         if (n && !data) return fail(AF_ERR_INVALID, "null data");
         equal = equal && n == n_samples[0];
         any_end = any_end || (end && end[k]);
     }
     // every stream at the shared position and the same count: the lockstep tick (same launches and copies as always)
-    if (!s->diverged && equal && !any_end)
-        return af_session_push(s, data, in_stride, n_samples[0], mem, out, n_pcm, n_feat, n_vad);
-    return session_push_ragged(s, data, in_stride, n_samples, end, mem, out, n_pcm, n_feat, n_vad);
+    return session_tick(s, data, in_stride, n_samples, end, s->diverged || !equal || any_end, mem, out, n_pcm, n_feat, n_vad);
 }
 
 AF_API int af_session_reset_streams(af_session *s, const uint32_t *streams, size_t n)
@@ -2166,8 +1929,7 @@ AF_API int af_session_reset_streams(af_session *s, const uint32_t *streams, size
         if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
     if (!n) return AF_OK;
     if (!s->diverged) {
-        const StreamState c = shared_stream(s);
-        for (size_t k = 0; k < s->S; ++k) s->ss[k] = c;
+        s->ss.assign(s->S, s->shared);
         s->diverged = true;
     }
     for (size_t i = 0; i < n; ++i) s->ss[streams[i]].restart = true;   // applied by the stream's next tick kernel
@@ -2178,7 +1940,7 @@ AF_API int af_session_wire_first_frames(const af_session *s, uint64_t *first_fra
 {
     if (!s || !first_frame) return fail(AF_ERR_INVALID, "null argument");
     if (!s->wire_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire");
-    for (size_t k = 0; k < s->S; ++k) first_frame[k] = s->first_frames_ragged ? s->first_frames[k] : s->wire_first_frame;
+    std::copy(s->first_frames.begin(), s->first_frames.end(), first_frame);
     return AF_OK;
 }
 
@@ -2276,7 +2038,7 @@ AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t 
     if (base64) *base64 = host ? s->h_wire_b64 : s->d_wire_b64;
     if (base64_stride) *base64_stride = s->wire_b64_stride;
     if (ticks) memcpy(ticks, s->h_wire_ticks, s->S * sizeof(af_wire_tick));
-    if (first_frame) *first_frame = s->wire_first_frame;
+    if (first_frame) *first_frame = s->first_frames[0];
     return AF_OK;
 }
 
@@ -2379,6 +2141,26 @@ AF_API void af_ring_clear(af_ring *r)                                           
     memset(r->buf, 0, r->capacity * sizeof(float));
 }
 
+// Reads counts[k] samples (none for 0) from each ring into row k of the session's pinned staging rows, *stride samples
+// apart; a ring that yields fewer than it held a moment before fails the tick
+static int read_rings(af_session *s, af_ring *const *rings, const uint32_t *counts, uint32_t max_count, uint64_t *stride)
+{
+    *stride = round_up(std::max<uint32_t>(max_count, 4), 4);
+    if (s->ring_stage_cap < *stride * s->S) {
+        if (s->ring_stage) cudaFreeHost(s->ring_stage);
+        s->ring_stage = nullptr; s->ring_stage_cap = 0;
+        AF_CUDA(cudaHostAlloc((void **)&s->ring_stage, *stride * s->S * sizeof(float), cudaHostAllocDefault));
+        s->ring_stage_cap = *stride * s->S;
+    }
+    for (size_t k = 0; k < s->S; ++k) {
+        if (!counts[k]) continue;
+        size_t got = 0;
+        const int rc = af_ring_read(rings[k], s->ring_stage + k * *stride, counts[k], &got);
+        if (rc != AF_OK || got != counts[k]) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
+    }
+    return AF_OK;
+}
+
 // One session tick fed by the capture rings: takes exactly n_samples from each of the session's n_streams rings
 // (AudioCapturer::read_frame, capture.rs:310-319, for every stream at once) into the session's pinned staging rows
 // and pushes them.  Nothing is consumed unless every ring holds n_samples.
@@ -2392,18 +2174,10 @@ AF_API int af_session_push_rings(af_session *s, af_ring *const *rings, uint32_t 
         const size_t have = af_ring_available(rings[k]);
         if (have < n_samples) return fail(AF_ERR_INVALID, "ring %zu holds %zu samples, the tick needs %u", k, have, n_samples);
     }
-    const uint64_t stride = round_up(std::max<uint32_t>(n_samples, 4), 4);
-    if (s->ring_stage_cap < stride * s->S) {
-        if (s->ring_stage) cudaFreeHost(s->ring_stage);
-        s->ring_stage = nullptr; s->ring_stage_cap = 0;
-        AF_CUDA(cudaHostAlloc((void **)&s->ring_stage, stride * s->S * sizeof(float), cudaHostAllocDefault));
-        s->ring_stage_cap = stride * s->S;
-    }
-    for (size_t k = 0; k < s->S; ++k) {
-        size_t got = 0;
-        const int rc = af_ring_read(rings[k], s->ring_stage + k * stride, n_samples, &got);
-        if (rc != AF_OK || got != n_samples) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
-    }
+    s->counts.assign(s->S, n_samples);
+    uint64_t stride = 0;
+    const int rc = read_rings(s, rings, s->counts.data(), n_samples, &stride);
+    if (rc) return rc;
     return af_session_push(s, s->ring_stage, stride, n_samples, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
 }
 
@@ -2421,19 +2195,9 @@ AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings,
         const size_t n = std::min<size_t>(max_samples, af_ring_available(rings[k]));
         s->counts[k] = (uint32_t)(n - n % s->channels);
     }
-    const uint64_t stride = round_up(std::max<uint32_t>(max_samples, 4), 4);
-    if (s->ring_stage_cap < stride * s->S) {
-        if (s->ring_stage) cudaFreeHost(s->ring_stage);
-        s->ring_stage = nullptr; s->ring_stage_cap = 0;
-        AF_CUDA(cudaHostAlloc((void **)&s->ring_stage, stride * s->S * sizeof(float), cudaHostAllocDefault));
-        s->ring_stage_cap = stride * s->S;
-    }
-    for (size_t k = 0; k < s->S; ++k) {
-        if (!s->counts[k]) continue;
-        size_t got = 0;
-        const int rc = af_ring_read(rings[k], s->ring_stage + k * stride, s->counts[k], &got);
-        if (rc != AF_OK || got != s->counts[k]) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
-    }
+    uint64_t stride = 0;
+    const int rc = read_rings(s, rings, s->counts.data(), max_samples, &stride);
+    if (rc) return rc;
     return af_session_push_streams(s, s->ring_stage, stride, s->counts.data(), end, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
 }
 

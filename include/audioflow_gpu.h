@@ -336,7 +336,9 @@ AF_API void af_session_destroy(af_session *s);
 /* One tick: every stream pushes `n_samples` interleaved samples (device or host per `mem`,
  * rows `in_stride` samples apart).  Outputs produced by this tick are appended at the row
  * starts of `out`; counts (host arrays of n_streams, may be NULL) receive how many
- * PCM samples / feature frames / VAD frames each stream emitted. */
+ * PCM samples / feature frames / VAD frames each stream emitted.  With the VAD on, out->vad_final
+ * (if set) receives every stream's detector state after its last frame so far on every push of any
+ * kind, a push that completes no frame included. */
 AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, uint32_t n_samples, int mem,
                            const af_outputs *out, uint32_t *n_pcm, uint32_t *n_feat, uint32_t *n_vad);
 AF_API int af_session_reset(af_session *s);

@@ -22,12 +22,22 @@ def test_session_matches_reference_objects(af, orc, rate, tick, fmt, ch):
     lm = [[] for _ in range(S)]
     vad = [[] for _ in range(S)]
     per_tick_counts = []
+    dets = [orc.VoiceActivityDetector() for _ in range(S)]
+    carry = [np.zeros(0, np.float32) for _ in range(S)]
     for t in range(n_ticks):
         x = np.stack([xs[i][t * tick * ch:(t + 1) * tick * ch] for i in range(S)])
         r = ses.push(x)
         per_tick_counts.append(r["pcm"].shape[1])
         for i in range(S):
             pcm[i].append(r["pcm"][i]); lm[i].append(r["logmel"][i]); vad[i].append(r["vad"][i])
+            # vad_final after every tick, frameless ones included: the detector fed the frames completed so far
+            carry[i] = np.concatenate([carry[i], r["pcm"][i]])
+            while len(carry[i]) >= 400:
+                dets[i].detect(carry[i][:400])
+                carry[i] = carry[i][160:]
+            fin = r["vad_final"][i]
+            assert (fin["state"], fin["speech_frames"]) == (dets[i].state(), dets[i].speech_frame_count()), (t, i)
+            assert np.float32(fin["smoothed"]).view(np.uint32) == np.float32(dets[i].smoothed_energy()).view(np.uint32), (t, i)
     for i in range(S):
         xi = orc.i16_to_f32(xs[i]) if fmt == "i16" else xs[i]
         mono = orc.to_mono(xi, ch)

@@ -402,7 +402,24 @@ def test_errors_leave_the_session_untouched(af, orc):
     h = Harness(af, orc, S, 48000, ch, "f32", max_tick=960 * ch)
     L = af.load_library()
     u32p = C.POINTER(C.c_uint32)
+
+    def short_rows(push):
+        """Output rows too short for the largest stream's outputs: AF_ERR_CAPACITY, nothing changes."""
+        pcm, lm, vad = np.zeros((S, 1024), np.float32), np.zeros((S, 16 * 80), np.float32), np.zeros((S, 16), np.uint8)
+        for short in ("pcm", "logmel", "vad"):
+            o = af.OutputsC(pcm.ctypes.data, 8 if short == "pcm" else 1024, lm.ctypes.data, 10 if short == "logmel" else 16 * 80,
+                            vad.ctypes.data, 0 if short == "vad" else 16, None, 0, None)
+            rc = push(C.byref(o))
+            assert rc == af.AF_ERR_CAPACITY, (short, rc)
+
     for t in range(30):
+        if t == 0:
+            # the lockstep tick (every stream at the common position, equal counts): one tick so that the next completes
+            # frames, then its own checks
+            h.tick([960 * ch] * S)
+            buf = np.zeros((S, 960 * ch), np.float32)
+            short_rows(lambda o: L.af_session_push(h.ses._h, buf.ctypes.data, buf.shape[1], buf.shape[1], af.AF_MEM_HOST,
+                                                   o, None, None, None))
         if t % 5 == 2:
             buf = np.zeros((S, 2000 * ch), np.float32)
             for counts, stride, status in (([961 * ch, 2, 2], buf.shape[1], af.AF_ERR_CAPACITY),   # above max_tick_samples
@@ -418,15 +435,10 @@ def test_errors_leave_the_session_untouched(af, orc):
                 h.ses.reset_streams([1, S])                            # out of range: no stream is reset
             with pytest.raises(BufferError):
                 h.ses.push_streams([np.zeros(962 * ch, np.float32)] * S)
-            # output rows too short for the largest stream's outputs (the session has diverged: the ragged path checks)
+            # the session has diverged: the per-stream plan checks
             c = np.full(S, 960 * ch, np.uint32)
-            pcm, lm, vad = np.zeros((S, 1024), np.float32), np.zeros((S, 16 * 80), np.float32), np.zeros((S, 16), np.uint8)
-            for short in ("pcm", "logmel", "vad"):
-                o = af.OutputsC(pcm.ctypes.data, 8 if short == "pcm" else 1024, lm.ctypes.data, 10 if short == "logmel" else 16 * 80,
-                                vad.ctypes.data, 0 if short == "vad" else 16, None, 0, None)
-                rc = L.af_session_push_streams(h.ses._h, buf.ctypes.data, buf.shape[1], c.ctypes.data_as(u32p), None,
-                                               af.AF_MEM_HOST, C.byref(o), None, None, None)
-                assert rc == af.AF_ERR_CAPACITY, (short, rc)
+            short_rows(lambda o: L.af_session_push_streams(h.ses._h, buf.ctypes.data, buf.shape[1], c.ctypes.data_as(u32p), None,
+                                                           af.AF_MEM_HOST, o, None, None, None))
         end = [bool(rng.random() < 0.05) for _ in range(S)]
         r = h.tick(_ragged_counts(rng, S, 960, ch, t), end)
     h.finish(r)
