@@ -71,6 +71,10 @@ class OutputsC(C.Structure):
                 ("vad_final", C.c_void_p)]
 
 
+class StreamFormatC(C.Structure):
+    _fields_ = [("sample_rate", C.c_uint32), ("channels", C.c_uint16), ("pad", C.c_uint16), ("max_tick_samples", C.c_uint32)]
+
+
 class WireConfigC(C.Structure):
     _fields_ = [("gate", C.c_uint32), ("pcm16", C.c_uint32), ("base64", C.c_uint32), ("mem", C.c_int32)]
 
@@ -182,6 +186,9 @@ def load_library():
         "af_session_push_rings_available": (C.c_int, [vp, C.POINTER(vp), C.c_uint32, u8p, C.POINTER(OutputsC),
                                                       C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
         "af_session_wire_first_frames": (C.c_int, [vp, C.POINTER(C.c_uint64)]),
+        "af_session_create_formats": (C.c_int, [vp, sz, C.POINTER(StreamFormatC), sz, C.POINTER(C.c_uint32), C.c_uint16,
+                                                C.POINTER(vp)]),
+        "af_session_restart_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), sz]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -655,18 +662,19 @@ class ShardedBatch:
 # ---------------------------------------------------------------------------------------------
 # streaming sessions (BASELINE config 5)
 # ---------------------------------------------------------------------------------------------
-def stream_rows(xs, n_streams: int, channels: int, dtype):
+def stream_rows(xs, n_streams: int, channels, dtype):
     """The rows of a ragged tick: xs[k] (1-D interleaved samples of stream k) at the start of row k of one [n_streams,
-    stride] array -> (array, uint32 counts).  ValueError before anything is pushed for a wrong stream count, a row that
-    is not 1-D, or a partial frame."""
+    stride] array -> (array, uint32 counts).  channels: one count for all streams, or one per stream.  ValueError before
+    anything is pushed for a wrong stream count, a row that is not 1-D, or a partial frame."""
     if len(xs) != n_streams:
         raise ValueError(f"{len(xs)} arrays for {n_streams} streams")
+    ch = np.broadcast_to(np.asarray(channels, np.int64), (n_streams,))
     xs = [np.ascontiguousarray(x, dtype=dtype) for x in xs]
     for k, x in enumerate(xs):
         if x.ndim != 1:
             raise ValueError(f"stream {k}: samples must be 1-D (interleaved), got shape {x.shape}")
-        if x.size % channels:
-            raise ValueError(f"stream {k}: {x.size} samples are not a whole number of {channels}-channel frames")
+        if x.size % ch[k]:
+            raise ValueError(f"stream {k}: {x.size} samples are not a whole number of {ch[k]}-channel frames")
     counts = np.array([x.size for x in xs], np.uint32)
     buf = np.zeros((n_streams, max((int(counts.max()) + 3) // 4 * 4, 4)), dtype)
     for k, x in enumerate(xs):
@@ -687,18 +695,53 @@ def end_flags(end, n_streams: int):
 class Session:
     """n_streams lockstep streams with persistent device state (resampler position + residual input,
     STFT overlap, VAD).  push() takes host arrays [n_streams, n_samples] and returns per-tick outputs.
-    push_streams() / push_rings_available() / reset_streams() give every stream its own timeline."""
+    push_streams() / push_rings_available() / reset_streams() give every stream its own timeline.
+    Session.formats() builds a session whose streams each have their own capture format; restart_streams() moves a
+    stream to another one."""
 
     def __init__(self, pipe: Pipeline, n_streams: int, sample_rate: int, channels: int = 1, fmt: int = AF_FMT_F32,
                  max_tick_samples: int = 4096):
-        self.pipe, self.S, self.rate, self.channels, self.fmt = pipe, n_streams, sample_rate, channels, fmt
         h = C.c_void_p()
         _check(load_library().af_session_create(pipe._h, n_streams, sample_rate, channels, fmt, max_tick_samples, C.byref(h)))
-        self._h = h
-        max_frames = max_tick_samples // channels
-        self.max_pcm = load_library().af_resample_max_output(sample_rate, 16000, max_frames + 128) + 8
+        self._setup(pipe, h, [(sample_rate, channels, max_tick_samples)], np.zeros(n_streams, np.uint32), fmt)
+
+    @classmethod
+    def formats(cls, pipe: Pipeline, formats, stream_format, fmt: int = AF_FMT_F32) -> "Session":
+        """A session of len(stream_format) streams that admits `formats`, a list of (sample_rate, channels,
+        max_tick_samples); stream k starts in formats[stream_format[k]].  fmt (f32 / i16 samples) is the same for all."""
+        formats = [tuple(int(v) for v in f) for f in formats]
+        sf = np.ascontiguousarray(stream_format, dtype=np.uint32).reshape(-1)
+        if any(len(f) != 3 for f in formats):
+            raise ValueError("a format is (sample_rate, channels, max_tick_samples)")
+        arr = (StreamFormatC * max(len(formats), 1))(*[StreamFormatC(r, c, 0, m) for r, c, m in formats])
+        h = C.c_void_p()
+        _check(load_library().af_session_create_formats(pipe._h, sf.size, arr, len(formats),
+                                                        sf.ctypes.data_as(C.POINTER(C.c_uint32)), fmt, C.byref(h)))
+        self = cls.__new__(cls)
+        self._setup(pipe, h, formats, sf.copy(), fmt)
+        return self
+
+    def _setup(self, pipe, h, formats, stream_format, fmt):
+        self.pipe, self._h, self.S, self.fmt = pipe, h, stream_format.size, fmt
+        self.format_list = formats                      # (sample_rate, channels, max_tick_samples) per format
+        self.stream_format = stream_format              # each stream's current format (restart_streams changes it)
+        # a single-format session keeps its rate and channel count as attributes
+        self.rate, self.channels = formats[0][:2] if len(formats) == 1 else (None, None)
+        L = load_library()
+        self.max_pcm = max(L.af_resample_max_output(r, 16000, m // c + 128) + 8 for r, c, m in formats)
         self.max_T = self.max_pcm // 160 + 4
         self.wire_mem = None                            # where the wire rows live (enable_wire)
+
+    def stream_channels(self) -> np.ndarray:
+        """The channel count of every stream's current format."""
+        return np.array([self.format_list[f][1] for f in self.stream_format], np.int64)
+
+    def _check_frames(self, n: int):
+        ch = self.stream_channels()
+        bad = np.nonzero(n % ch)[0]
+        if bad.size:
+            k = int(bad[0])
+            raise ValueError(f"stream {k}: {n} samples are not a whole number of {ch[k]}-channel frames")
 
     def __del__(self):
         if getattr(self, "_h", None) and _lib is not None:
@@ -751,6 +794,7 @@ class Session:
         x = np.ascontiguousarray(x, dtype=np.int16 if self.fmt == AF_FMT_I16 else np.float32)
         assert x.ndim == 2 and x.shape[0] == self.S
         n = x.shape[1]
+        self._check_frames(n)
         L = load_library()
         return self._tick(lambda o, a, b, c: L.af_session_push(self._h, x.ctypes.data, n, n, AF_MEM_HOST, o, a, b, c))
 
@@ -767,6 +811,7 @@ class Session:
     def push_rings(self, rings, n_samples: int) -> dict:
         """One tick fed by the capture rings (AudioCapturer::read_frame for every stream, capture.rs:310-319)."""
         assert len(rings) == self.S
+        self._check_frames(n_samples)
         arr = (C.c_void_p * self.S)(*[r._h for r in rings])
         L = load_library()
         return self._tick(lambda o, a, b, c: L.af_session_push_rings(self._h, arr, n_samples, o, a, b, c))
@@ -774,7 +819,7 @@ class Session:
     def push_streams(self, xs, end=None) -> dict:
         """One tick in which stream k pushes xs[k] (1-D interleaved samples, any whole number of frames, 0 included); end[k]
         ends stream k after them (BatchResampler::flush), its next push starts afresh.  Returns per-stream lists."""
-        buf, counts = stream_rows(xs, self.S, self.channels, np.int16 if self.fmt == AF_FMT_I16 else np.float32)
+        buf, counts = stream_rows(xs, self.S, self.stream_channels(), np.int16 if self.fmt == AF_FMT_I16 else np.float32)
         e = end_flags(end, self.S)
         L = load_library()
         u32p = C.POINTER(C.c_uint32)
@@ -786,6 +831,21 @@ class Session:
         """Streams `ids` start afresh at their next push, without a flush; the others are untouched."""
         a = np.ascontiguousarray(ids, dtype=np.uint32).reshape(-1)
         _check(load_library().af_session_reset_streams(self._h, a.ctypes.data_as(C.POINTER(C.c_uint32)), a.size))
+
+    def restart_streams(self, ids, format_ids):
+        """Streams `ids` start afresh at their next push in formats[format_ids[i]] (reset_streams plus a new format)."""
+        a = np.ascontiguousarray(ids, dtype=np.int64).reshape(-1)
+        f = np.ascontiguousarray(format_ids, dtype=np.int64).reshape(-1)
+        if a.size != f.size:
+            raise ValueError(f"{a.size} streams and {f.size} formats")
+        if a.size and (a.min() < 0 or a.max() >= self.S):
+            raise ValueError(f"stream index out of range ({self.S} streams)")
+        if f.size and (f.min() < 0 or f.max() >= len(self.format_list)):
+            raise ValueError(f"format index out of range ({len(self.format_list)} formats)")
+        a32, f32 = a.astype(np.uint32), f.astype(np.uint32)
+        u32p = C.POINTER(C.c_uint32)
+        _check(load_library().af_session_restart_streams(self._h, a32.ctypes.data_as(u32p), f32.ctypes.data_as(u32p), a.size))
+        self.stream_format[a32] = f32
 
     def push_rings_available(self, rings, max_samples: int, end=None) -> dict:
         """AudioCapturer::read_frame(max) for every stream: min(max_samples, available) whole frames from each ring."""

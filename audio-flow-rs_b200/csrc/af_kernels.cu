@@ -986,15 +986,19 @@ cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R
 
 // independent stream timelines: the same per CTA, with the stream's own lengths and positions from its StreamTick.  A
 // restart rewrites the zero history here and clears the stream's detector and wire segment state, so it costs no launch;
-// an end's zero padding is never materialised (n_valid_end stops at the data, the reads past it return 0).
+// an end's zero padding is never materialised (n_valid_end stops at the data, the reads past it return 0).  Each stream
+// takes its channel count and resampling ratio from its format, so one launch serves streams of any mix of formats.
 __global__ void __launch_bounds__(256) af_session_tick_streams_kernel(SessionIngest I, SessionResample R, const StreamTick *__restrict__ tab,
-                                                                      VadState *vad, uint8_t *wire_prev, float *pcm, uint64_t pcm_stride)
+                                                                      const SessionFormat *__restrict__ fmts, VadState *vad,
+                                                                      uint8_t *wire_prev, float *pcm, uint64_t pcm_stride)
 {
     const uint32_t s = blockIdx.x;
     const StreamTick d = tab[s];
-    I.drop = d.in_drop; I.keep = d.in_keep; I.n_new_frames = d.n_new; I.n_samples = d.n_samples;
+    const SessionFormat f = fmts[d.flags >> TICK_FMT_SHIFT];
+    I.drop = d.in_drop; I.keep = d.in_keep; I.n_new_frames = d.n_new; I.n_samples = d.n_samples; I.channels = f.channels;
     R.data_base = d.data_base; R.n_valid_end = d.n_valid_end; R.n_begin = d.n_begin; R.n_end = d.n_begin + d.n_y;
     R.frac += d.frac_off; R.y_drop = d.y_drop; R.y_keep = d.y_keep;
+    R.p = f.p; R.q = f.q; R.mode = f.mode;
     const bool restart = (d.flags & TICK_RESTART) != 0;
     if (restart && threadIdx.x == 0) {
         VadState v; v.smoothed = 0.0f; v.state = 0; v.silence_frames = 0; v.speech_frames = 0;
@@ -1004,11 +1008,12 @@ __global__ void __launch_bounds__(256) af_session_tick_streams_kernel(SessionIng
     session_tick_row(I, R, s, restart, pcm ? pcm + (uint64_t)s * pcm_stride : nullptr);
 }
 
-cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab, VadState *vad,
-                                        uint8_t *wire_prev, float *pcm, uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st)
+cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab,
+                                        const SessionFormat *fmts, VadState *vad, uint8_t *wire_prev, float *pcm,
+                                        uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st)
 {
     if (n_streams == 0) return cudaSuccess;
-    af_session_tick_streams_kernel<<<n_streams, 256, 0, st>>>(I, R, tab, vad, wire_prev, pcm, pcm_stride);
+    af_session_tick_streams_kernel<<<n_streams, 256, 0, st>>>(I, R, tab, fmts, vad, wire_prev, pcm, pcm_stride);
     return cudaGetLastError();
 }
 

@@ -59,8 +59,13 @@ struct SessionResample {
 };
 
 // one stream's part of a tick of independent stream timelines (af_session_push_streams), planned on the host; it
-// overrides the per-stream fields of SessionIngest / SessionResample / WireJob and the peak's range
-constexpr uint32_t TICK_RESTART = 1, TICK_END = 2;
+// overrides the per-stream fields of SessionIngest / SessionResample / WireJob and the peak's range.  flags >>
+// TICK_FMT_SHIFT is the stream's index into the session's SessionFormat table (inside `flags`, so StreamTick keeps the
+// 64-byte layout the peak and wire kernels index)
+constexpr uint32_t TICK_RESTART = 1, TICK_END = 2, TICK_FMT_SHIFT = 16;
+struct SessionFormat {       // one capture format a session admits: load_mono's channels, session_resample_one's ratio
+    uint32_t channels, p, q, mode;
+};
 struct StreamTick {
     uint32_t in_drop, in_keep;                                   // ingest: retained frames old[in_drop .. in_drop + in_keep)
     uint32_t n_new, n_samples;                                   // this tick's frames / interleaved samples of the stream
@@ -109,10 +114,12 @@ cudaError_t launch_session_wire(const WireJob &job, cudaStream_t st);
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st);
-// the same with every stream planned by its own StreamTick; restarted streams clear vad[s] and (if non-null) wire_prev[s];
-// pcm (device, or nullptr) receives each stream's new samples at its row start
-cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab, VadState *vad,
-                                        uint8_t *wire_prev, float *pcm, uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st);
+// the same with every stream planned by its own StreamTick, in its own format fmts[tab[s].flags >> TICK_FMT_SHIFT];
+// restarted streams clear vad[s] and (if non-null) wire_prev[s]; pcm (device, or nullptr) receives each stream's new
+// samples at its row start
+cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionResample &R, const StreamTick *tab,
+                                        const SessionFormat *fmts, VadState *vad, uint8_t *wire_prev, float *pcm,
+                                        uint64_t pcm_stride, uint32_t n_streams, cudaStream_t st);
 // split: the batch holds tiles other than 48 kHz mono f32 -> 16 kHz; such batches (and quarter-staged ones) run the
 // kernel of the second translation unit of af_fused.cu (AF_FUSED_SPLIT_TU), whose resampler role keeps the hot and the
 // general tiles in separate loops

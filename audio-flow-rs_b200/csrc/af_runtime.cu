@@ -1335,7 +1335,14 @@ struct af_session {
     int device = -1;                  // the GPU that holds the session state
     MelTables *d_mel = nullptr;
     size_t S = 0;
-    uint32_t rate = 0, channels = 1, format = 0, max_tick_frames = 0;
+    // the capture formats the session admits (af_session_create: one); a stream's state names its format.  The buffers
+    // are sized for the largest bound over the formats: max_tick_frames, max_new_y (below) and max_ring_samples
+    struct Format { uint32_t rate, channels, max_tick_frames; };
+    std::vector<Format> fmts;
+    SessionFormat *d_fmts = nullptr;                           // their device table, read by af_session_tick_streams_kernel
+    bool any_table = false;                                    // some format resamples through a fraction table (RS_TABLE)
+    uint32_t format = 0, max_tick_frames = 0;
+    uint64_t max_ring_samples = 0;
     // input history: last 16 frames + residual (< 128), ping-pong
     float *in_buf[2] = {nullptr, nullptr}; uint64_t in_stride = 0; int in_cur = 0;
     // 16 kHz carry (samples not yet covered by an emitted frame), ping-pong
@@ -1385,10 +1392,12 @@ struct af_session {
         long long in_base;                                     // global frame index of the row's first frame
         uint64_t frames_emitted;
         bool restart;                                          // start afresh at the next push (end / af_session_reset_streams)
+        uint32_t fmt;                                          // index into fmts (of the next life while `restart`)
     };
     StreamState shared{};
     std::vector<StreamState> ss, ss_next;
     bool diverged = false;
+    std::vector<uint32_t> plan_slots;                          // scratch: open-addressing table of the tick's distinct plans
     StreamTick *h_tick = nullptr, *d_tick = nullptr;           // the tick's plan: [S] StreamTick, then [S] uint32 frame counts
     float *d_pcm_stage = nullptr;                              // host-mode PCM rows of a per-stream tick
     std::vector<uint32_t> counts;                              // scratch: equal counts (af_session_push), ring reads
@@ -1414,14 +1423,17 @@ void wire_free(af_session *s)
 
 using StreamState = af_session::StreamState;
 
-StreamState fresh_stream(const af_session *s)
+StreamState fresh_stream(const af_session *s, uint32_t fmt)
 {
     StreamState f{};
-    f.rec.init(s->rate, OUT_RATE);
+    f.rec.init(s->fmts[fmt].rate, OUT_RATE);
     f.in_len = 2 * RS_POLY;                                      // rubato starts with 16 zero frames of history
     f.in_base = -2 * RS_POLY;
+    f.fmt = fmt;
     return f;
 }
+
+uint32_t stream_fmt(const af_session *s, size_t k) { return s->diverged ? s->ss[k].fmt : s->shared.fmt; }
 }  // namespace
 
 extern "C" {
@@ -1452,6 +1464,7 @@ AF_API void af_session_destroy(af_session *s)
     if (s->d_tick) cudaFree(s->d_tick);
     if (s->h_tick) cudaFreeHost(s->h_tick);
     if (s->d_pcm_stage) cudaFree(s->d_pcm_stage);
+    if (s->d_fmts) cudaFree(s->d_fmts);
     delete s;
 }
 
@@ -1459,9 +1472,16 @@ AF_API int af_session_reset(af_session *s)
 {
     if (!s) return fail(AF_ERR_INVALID, "null session");
     AF_SCOPE(s->device);
-    s->shared = fresh_stream(s);
+    // every stream to the common start in its current format: lockstep again when they all share one
+    bool one = true;
+    for (size_t k = 1; k < s->S && one; ++k) one = stream_fmt(s, k) == stream_fmt(s, 0);
+    if (one) {
+        s->shared = fresh_stream(s, stream_fmt(s, 0));
+        s->diverged = false;
+    } else {
+        for (size_t k = 0; k < s->S; ++k) s->ss[k] = fresh_stream(s, s->ss[k].fmt);
+    }
     s->in_cur = 0; s->y_cur = 0;
-    s->diverged = false;                           // every stream at the common start: lockstep again
     AF_CUDA(cudaMemset(s->in_buf[0], 0, s->S * s->in_stride * sizeof(float)));
     AF_CUDA(cudaMemset(s->d_vad, 0, s->S * sizeof(VadState)));
     if (s->d_wire_prev) AF_CUDA(cudaMemset(s->d_wire_prev, 0, s->S));   // no segment open
@@ -1471,9 +1491,26 @@ AF_API int af_session_reset(af_session *s)
 AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_rate, uint16_t channels, uint16_t format,
                              uint32_t max_tick_samples, af_session **out)
 {
-    if (!p || !out || n_streams == 0) return fail(AF_ERR_INVALID, "bad argument");
-    if (channels == 0 || (format != AF_FMT_F32 && format != AF_FMT_I16) || sample_rate == 0 || max_tick_samples == 0)
-        return fail(AF_ERR_INVALID, "bad stream format");
+    const af_stream_format f{sample_rate, channels, 0, max_tick_samples};
+    return af_session_create_formats(p, n_streams, &f, 1, nullptr, format, out);
+}
+
+AF_API int af_session_create_formats(af_pipeline *p, size_t n_streams, const af_stream_format *formats, size_t n_formats,
+                                     const uint32_t *stream_format, uint16_t format, af_session **out)
+{
+    if (!p || !out || n_streams == 0 || (!formats && n_formats)) return fail(AF_ERR_INVALID, "bad argument");
+    if (n_formats == 0 || n_formats > (1u << (32 - TICK_FMT_SHIFT)))
+        return fail(AF_ERR_INVALID, "%zu formats (a session admits 1 to %u)", n_formats, 1u << (32 - TICK_FMT_SHIFT));
+    if (format != AF_FMT_F32 && format != AF_FMT_I16) return fail(AF_ERR_INVALID, "bad stream format");
+    for (size_t i = 0; i < n_formats; ++i) {
+        const af_stream_format &f = formats[i];
+        if (f.channels == 0 || f.sample_rate == 0 || f.max_tick_samples == 0 || f.pad != 0)
+            return fail(AF_ERR_INVALID, "bad stream format %zu", i);
+    }
+    if (stream_format)
+        for (size_t k = 0; k < n_streams; ++k)
+            if (stream_format[k] >= n_formats)
+                return fail(AF_ERR_INVALID, "stream %zu: format %u out of range (%zu formats)", k, stream_format[k], n_formats);
     int rc = require_ctx();
     if (rc) return rc;
     const af_pipeline_config &cfg = p->cfg;
@@ -1483,14 +1520,26 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
     std::unique_ptr<af_session, void (*)(af_session *)> s(new af_session, af_session_destroy);
     s->device = cur_device();
     if (p->cfg.n_mels && !(s->d_mel = pipe_mel(p))) return AF_ERR_CUDA;
-    s->pipe = p; s->S = n_streams; s->rate = sample_rate; s->channels = channels; s->format = format;
-    s->max_tick_frames = (max_tick_samples + channels - 1) / channels;
-    s->shared = fresh_stream(s.get());
-    if (!s->shared.rec.passthrough && s->shared.rec.end_idx <= 0) return fail(AF_ERR_RESAMPLING_FAILED, "unsupported resampling ratio");
+    s->pipe = p; s->S = n_streams; s->format = format;
+    std::vector<SessionFormat> dev(n_formats);
+    uint64_t max_new_y = 0;
+    for (size_t i = 0; i < n_formats; ++i) {
+        const af_stream_format &f = formats[i];
+        const uint32_t frames = (f.max_tick_samples + f.channels - 1) / f.channels;
+        RsRecurrence rec;
+        rec.init(f.sample_rate, OUT_RATE);
+        if (!rec.passthrough && rec.end_idx <= 0) return fail(AF_ERR_RESAMPLING_FAILED, "unsupported resampling ratio");
+        s->fmts.push_back({f.sample_rate, f.channels, frames});
+        dev[i] = {f.channels, rec.p, rec.q, rec.mode()};
+        s->any_table = s->any_table || rec.mode() == RS_TABLE;
+        s->max_tick_frames = std::max(s->max_tick_frames, frames);
+        // (a count of max_samples passes af_session_push_rings_available's check while max_samples / channels <= frames)
+        s->max_ring_samples = std::max<uint64_t>(s->max_ring_samples, (uint64_t)f.channels * (frames + 1) - 1);
+        max_new_y = std::max<uint64_t>(max_new_y, af_resample_max_output(f.sample_rate, OUT_RATE, frames + RS_CHUNK) + 8);
+    }
     s->framing = cfg.n_mels != 0 || cfg.vad_enable;
     if (cfg.vad_enable && cfg.vad_frame_len != 0) { s->frame_len = cfg.vad_frame_len; s->hop = cfg.vad_hop; }
     s->in_stride = round_up(2 * RS_POLY + RS_CHUNK + s->max_tick_frames + 8, 4);
-    const uint64_t max_new_y = af_resample_max_output(sample_rate, OUT_RATE, s->max_tick_frames + RS_CHUNK) + 8;
     s->max_new_y = max_new_y;
     s->y_stride = round_up(s->frame_len + s->hop + max_new_y + 8, 4);
     s->packed = s->framing && s->frame_len == WIN && s->hop == HOP;
@@ -1530,12 +1579,17 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
             AF_CUDA(cudaMemcpy(s->d_ptiles[i], ptiles.data(), s->pk_n * sizeof(TileDev), cudaMemcpyHostToDevice));
         }
     }
-    if (s->y_stride > (uint64_t)TILE_SAMPLES) return fail(AF_ERR_INVALID, "max_tick_samples too large for a session (%u)", max_tick_samples);
+    if (s->y_stride > (uint64_t)TILE_SAMPLES)
+        return fail(AF_ERR_INVALID, "max_tick_samples too large for a session (%u frames)", s->max_tick_frames);
     AF_CUDA(cudaMalloc(&s->d_vad, n_streams * sizeof(VadState)));
     AF_CUDA(cudaMalloc(&s->d_energy, n_streams * s->energy_stride * sizeof(float)));
     s->frac_cap = max_new_y + 64;
     AF_CUDA(cudaMalloc(&s->d_frac, s->frac_cap * sizeof(float)));
+    AF_CUDA(cudaMalloc(&s->d_fmts, n_formats * sizeof(SessionFormat)));
+    AF_CUDA(cudaMemcpy(s->d_fmts, dev.data(), n_formats * sizeof(SessionFormat), cudaMemcpyHostToDevice));
     s->ss.resize(n_streams); s->ss_next.resize(n_streams);
+    for (size_t k = 0; k < n_streams; ++k) s->ss[k].fmt = stream_format ? stream_format[k] : 0;
+    s->diverged = true;                            // (af_session_reset reads each stream's format from ss)
     s->first_frames.assign(n_streams, 0);
     rc = af_session_reset(s.get());
     if (rc) return rc;
@@ -1546,11 +1600,30 @@ AF_API int af_session_create(af_pipeline *p, size_t n_streams, uint32_t sample_r
 }  // extern "C"
 
 namespace {
-bool same_position(const StreamState &a, const StreamState &b)
+bool same_fields(const StreamState &a, const StreamState &b)
 {
-    return !a.restart && !b.restart && a.rec.chunks == b.rec.chunks && a.rec.n_out == b.rec.n_out &&
+    return a.fmt == b.fmt && a.rec.chunks == b.rec.chunks && a.rec.n_out == b.rec.n_out &&
            a.rec.last_index == b.rec.last_index && a.in_len == b.in_len && a.in_drop == b.in_drop && a.y_len == b.y_len &&
            a.y_drop == b.y_drop && a.in_base == b.in_base && a.frames_emitted == b.frames_emitted;
+}
+
+bool same_position(const StreamState &a, const StreamState &b) { return !a.restart && !b.restart && same_fields(a, b); }
+
+// A stream's plan (its StreamTick, fraction slice and next state) is a function of its format, its position (none while it
+// restarts: a fresh stream's), its count and its end flag; streams with equal keys share one plan.
+bool same_plan(const StreamState &a, uint32_t na, bool fa, const StreamState &b, uint32_t nb, bool fb)
+{
+    return na == nb && fa == fb && a.restart == b.restart && (a.restart ? a.fmt == b.fmt : same_fields(a, b));
+}
+
+uint64_t plan_hash(const StreamState &a, uint32_t n, bool fin)
+{
+    uint64_t h = ((uint64_t)a.fmt << 34) ^ ((uint64_t)n << 2) ^ (fin ? 1u : 0u) ^ (a.restart ? 2u : 0u);
+    if (!a.restart)
+        h ^= a.rec.chunks * 0x9E3779B97F4A7C15ull ^ (uint64_t)a.in_len << 40 ^ (uint64_t)a.y_len * 0xC2B2AE3D27D4EB4Full ^
+             (uint64_t)a.in_base * 0x165667B19E3779F9ull ^ a.frames_emitted;
+    h ^= h >> 33; h *= 0xFF51AFD7ED558CCDull; h ^= h >> 33;
+    return h;
 }
 
 // RsRecurrence::step `chunks` times.  An exact recurrence (t = p / q, q a power of two) takes the closed form: the output
@@ -1569,11 +1642,12 @@ void rs_advance(RsRecurrence &r, uint32_t chunks, std::vector<float> *frac)
     r.last_index = -(double)(RS_POLY / 2) + (double)num / (double)r.q;
 }
 
-// one stream's count in a tick: whole frames, at most max_tick_samples, within its input row
-int check_count(const af_session *s, uint32_t n, uint64_t in_stride)
+// one stream's count in a tick: whole frames of its format, at most its format's max_tick_samples, within its input row
+int check_count(const af_session *s, uint32_t fmt, uint32_t n, uint64_t in_stride)
 {
-    if (n % s->channels) return fail(AF_ERR_INVALID, "a tick of %u samples is not a whole number of frames", n);
-    if (n / s->channels > s->max_tick_frames) return fail(AF_ERR_CAPACITY, "tick of %u frames exceeds max_tick_samples", n / s->channels);
+    const af_session::Format &f = s->fmts[fmt];
+    if (n % f.channels) return fail(AF_ERR_INVALID, "a tick of %u samples is not a whole number of frames", n);
+    if (n / f.channels > f.max_tick_frames) return fail(AF_ERR_CAPACITY, "tick of %u frames exceeds max_tick_samples", n / f.channels);
     if (in_stride < n) return fail(AF_ERR_INVALID, "in_stride %llu smaller than a tick of %u samples", (unsigned long long)in_stride, n);
     return AF_OK;
 }
@@ -1583,9 +1657,9 @@ int check_count(const af_session *s, uint32_t n, uint64_t in_stride)
 // the tick (BatchResampler::flush, resampler.rs:150-166).  Only internal capacity errors can occur; nothing changes.
 int plan_stream(af_session *s, const StreamState &now, uint32_t n_samples, bool fin, StreamTick &d, StreamState &next)
 {
-    StreamState c = now.restart ? fresh_stream(s) : now;
+    StreamState c = now.restart ? fresh_stream(s, now.fmt) : now;
     // frames held: [history 16 | residual r | new n_new]; chunks formed from residual + new
-    const uint32_t n_new = n_samples / s->channels;
+    const uint32_t n_new = n_samples / s->fmts[c.fmt].channels;
     const uint32_t residual = c.in_len - 2 * RS_POLY;
     const uint32_t avail = residual + n_new;
     const bool pass = c.rec.passthrough;
@@ -1609,7 +1683,7 @@ int plan_stream(af_session *s, const StreamState &now, uint32_t n_samples, bool 
                          : c.in_base + 2 * RS_POLY + (long long)(fin ? avail : full * RS_CHUNK);
     d.n_begin = n_begin; d.n_y = n_y; d.frac_off = (uint32_t)frac_off;
     d.y_drop = c.y_drop; d.y_keep = c.y_len;
-    d.T = T; d.flags = (now.restart ? TICK_RESTART : 0u) | (fin ? TICK_END : 0u);
+    d.T = T; d.flags = (now.restart ? TICK_RESTART : 0u) | (fin ? TICK_END : 0u) | (c.fmt << TICK_FMT_SHIFT);
     // the consumed chunks and the samples every future frame starts after are dropped by the next tick's ingest /
     // resample (in_drop, y_drop): no kernel and no second synchronisation
     c.in_len += n_new;
@@ -1666,7 +1740,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
             }
             s->d_tick = d; s->h_tick = h;
         }
-        if (s->shared.rec.mode() == RS_TABLE && s->frac_cap < S * s->max_new_y) {   // every stream's fractions, one slice after another
+        if (s->any_table && s->frac_cap < S * s->max_new_y) {   // every distinct plan's fractions, one slice after another
             float *f = nullptr;
             AF_CUDA(cudaMalloc(&f, S * s->max_new_y * sizeof(float)));
             cudaFree(s->d_frac);
@@ -1674,9 +1748,22 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         }
         if (!s->diverged) s->ss.assign(S, s->shared);
         uint32_t *Ts = reinterpret_cast<uint32_t *>(s->h_tick + S);
+        size_t cap = 1;
+        while (cap < 2 * S) cap <<= 1;
+        s->plan_slots.assign(cap, UINT32_MAX);              // stream that planned each distinct key first
         for (size_t k = 0; k < S; ++k) {
-            const int rc = plan_stream(s, s->ss[k], n_samples[k], end && end[k], s->h_tick[k], s->ss_next[k]);
-            if (rc) return rc;
+            const bool fin = end && end[k];
+            size_t i = plan_hash(s->ss[k], n_samples[k], fin) & (cap - 1);
+            for (uint32_t j; (j = s->plan_slots[i]) != UINT32_MAX; i = (i + 1) & (cap - 1))
+                if (same_plan(s->ss[j], n_samples[j], end && end[j], s->ss[k], n_samples[k], fin)) break;
+            if (s->plan_slots[i] == UINT32_MAX) {
+                s->plan_slots[i] = (uint32_t)k;
+                const int rc = plan_stream(s, s->ss[k], n_samples[k], fin, s->h_tick[k], s->ss_next[k]);
+                if (rc) return rc;
+            } else {                                             // the same plan, and the same fraction slice
+                s->h_tick[k] = s->h_tick[s->plan_slots[i]];
+                s->ss_next[k] = s->ss_next[s->plan_slots[i]];
+            }
             Ts[k] = s->h_tick[k].T;
             maxT = std::max(maxT, Ts[k]); max_ny = std::max(max_ny, s->h_tick[k].n_y); max_n = std::max(max_n, n_samples[k]);
         }
@@ -1752,13 +1839,14 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     const uint32_t *d_T = per_stream ? reinterpret_cast<const uint32_t *>(s->d_tick + S) : nullptr;
     SessionIngest ing{};
     ing.old_buf = s->in_buf[s->in_cur]; ing.new_buf = s->in_buf[in_next]; ing.buf_stride = s->in_stride;
-    ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.channels = s->channels; ing.format = s->format;
+    ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.channels = s->fmts[s->shared.fmt].channels;
+    ing.format = s->format;
     SessionResample rs{};
     rs.in_buf = s->in_buf[in_next]; rs.in_stride = s->in_stride;
     rs.p = s->shared.rec.p; rs.q = s->shared.rec.q; rs.mode = s->shared.rec.mode(); rs.frac = s->d_frac;
     rs.y_old = s->y_buf[s->y_cur]; rs.y_new = s->y_buf[y_next]; rs.y_stride = s->y_stride;
     if (per_stream) {
-        AF_CUDA(launch_session_tick_streams(ing, rs, tab, s->d_vad, s->d_wire_prev, pcm_rows, pcm_rows_stride, (uint32_t)S, st));
+        AF_CUDA(launch_session_tick_streams(ing, rs, tab, s->d_fmts, s->d_vad, s->d_wire_prev, pcm_rows, pcm_rows_stride, (uint32_t)S, st));
     } else {                                                     // the fields the streams kernel takes from its descriptor
         ing.drop = one.in_drop; ing.keep = one.in_keep; ing.n_samples = one.n_samples; ing.n_new_frames = one.n_new;
         rs.data_base = one.data_base; rs.n_valid_end = one.n_valid_end; rs.n_begin = one.n_begin; rs.n_end = one.n_begin + one.n_y;
@@ -1898,7 +1986,7 @@ AF_API int af_session_push(af_session *s, const void *data, uint64_t in_stride, 
         return af_session_push_streams(s, data, in_stride, s->counts.data(), nullptr, mem, o, n_pcm, n_feat, n_vad);
     }
     if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
-    const int rc = check_count(s, n_samples, in_stride);
+    const int rc = check_count(s, s->shared.fmt, n_samples, in_stride);
     if (rc) return rc;
     return session_tick(s, data, in_stride, &n_samples, nullptr, false, mem, o, n_pcm, n_feat, n_vad);
 }
@@ -1912,7 +2000,7 @@ AF_API int af_session_push_streams(af_session *s, const void *data, uint64_t in_
     bool equal = true, any_end = false;
     for (size_t k = 0; k < s->S; ++k) {
         const uint32_t n = n_samples[k];
-        const int rc = check_count(s, n, in_stride);
+        const int rc = check_count(s, stream_fmt(s, k), n, in_stride);
         if (rc) return rc;
         if (n && !data) return fail(AF_ERR_INVALID, "null data");
         equal = equal && n == n_samples[0];
@@ -1933,6 +2021,19 @@ AF_API int af_session_reset_streams(af_session *s, const uint32_t *streams, size
         s->diverged = true;
     }
     for (size_t i = 0; i < n; ++i) s->ss[streams[i]].restart = true;   // applied by the stream's next tick kernel
+    return AF_OK;
+}
+
+AF_API int af_session_restart_streams(af_session *s, const uint32_t *streams, const uint32_t *format, size_t n)
+{
+    if (!s || ((!streams || !format) && n)) return fail(AF_ERR_INVALID, "null argument");
+    for (size_t i = 0; i < n; ++i) {
+        if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
+        if (format[i] >= s->fmts.size()) return fail(AF_ERR_INVALID, "format index %u out of range (%zu formats)", format[i], s->fmts.size());
+    }
+    const int rc = af_session_reset_streams(s, streams, n);
+    if (rc) return rc;
+    for (size_t i = 0; i < n; ++i) s->ss[streams[i]].fmt = format[i];   // the format of the next life
     return AF_OK;
 }
 
@@ -2174,6 +2275,10 @@ AF_API int af_session_push_rings(af_session *s, af_ring *const *rings, uint32_t 
         const size_t have = af_ring_available(rings[k]);
         if (have < n_samples) return fail(AF_ERR_INVALID, "ring %zu holds %zu samples, the tick needs %u", k, have, n_samples);
     }
+    for (size_t k = 0; k < s->S; ++k) {                          // the push's count checks, before any ring is read
+        const int rc = check_count(s, stream_fmt(s, k), n_samples, n_samples);
+        if (rc) return rc;
+    }
     s->counts.assign(s->S, n_samples);
     uint64_t stride = 0;
     const int rc = read_rings(s, rings, s->counts.data(), n_samples, &stride);
@@ -2187,13 +2292,14 @@ AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings,
 {
     if (!s || !rings) return fail(AF_ERR_INVALID, "null argument");
     if (s->format != AF_FMT_F32) return fail(AF_ERR_INVALID, "capture rings hold f32 samples; the session was created for i16");
-    if (max_samples / s->channels > s->max_tick_frames)
+    if (max_samples > s->max_ring_samples)
         return fail(AF_ERR_CAPACITY, "max_samples %u exceeds the session's max_tick_samples", max_samples);
     s->counts.resize(s->S);
     for (size_t k = 0; k < s->S; ++k) {
         if (!rings[k]) return fail(AF_ERR_INVALID, "ring %zu is null", k);
-        const size_t n = std::min<size_t>(max_samples, af_ring_available(rings[k]));
-        s->counts[k] = (uint32_t)(n - n % s->channels);
+        const af_session::Format &f = s->fmts[stream_fmt(s, k)];       // at most the stream's own bound, whole frames
+        const size_t n = std::min<size_t>({max_samples, (size_t)f.channels * f.max_tick_frames, af_ring_available(rings[k])});
+        s->counts[k] = (uint32_t)(n - n % f.channels);
     }
     uint64_t stride = 0;
     const int rc = read_rings(s, rings, s->counts.data(), max_samples, &stride);

@@ -154,6 +154,13 @@ public:
     {
         check(af_session_create(p, n_streams, sample_rate, channels, format, max_tick_samples, &h_));
     }
+    // a session of stream_format.size() streams that admits `formats`; stream k starts in formats[stream_format[k]]
+    Session(af_pipeline *p, const std::vector<af_stream_format> &formats, const std::vector<uint32_t> &stream_format,
+            uint16_t sample_format)
+        : n_(stream_format.size())
+    {
+        check(af_session_create_formats(p, n_, formats.data(), formats.size(), stream_format.data(), sample_format, &h_));
+    }
     Session(const Session &) = delete;
     ~Session() { if (h_) af_session_destroy(h_); }
 
@@ -198,6 +205,12 @@ public:
     }
     // the listed streams start afresh at their next push, without a flush
     void reset_streams(const std::vector<uint32_t> &streams) { check(af_session_reset_streams(h_, streams.data(), streams.size())); }
+    // the same, each stream starting in the session's format format[i]
+    void restart_streams(const std::vector<uint32_t> &streams, const std::vector<uint32_t> &format)
+    {
+        if (streams.size() != format.size()) throw std::invalid_argument("restart_streams: one format per stream");
+        check(af_session_restart_streams(h_, streams.data(), format.data(), streams.size()));
+    }
 
     void enable_levels(bool on = true) { check(af_session_enable_levels(h_, on ? 1 : 0)); }
     // AudioLevel{level, peak} / VolumeLevel{level, is_speech} of the last tick, per stream

@@ -104,6 +104,15 @@ pub struct af_wire_tick {
     pub pad: [u8; 3],
 }
 
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct af_stream_format {
+    pub sample_rate: u32,
+    pub channels: u16,
+    pub pad: u16,
+    pub max_tick_samples: u32,
+}
+
 extern "C" {
     pub fn af_session_create(p: *mut af_pipeline, n_streams: usize, sample_rate: u32, channels: u16, format: u16,
                              max_tick_samples: u32, out: *mut *mut af_session) -> c_int;
@@ -125,6 +134,9 @@ extern "C" {
     pub fn af_session_push_rings_available(s: *mut af_session, rings: *const *mut af_ring, max_samples: u32, end: *const u8,
                                            out: *const af_outputs, n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
     pub fn af_session_wire_first_frames(s: *const af_session, first_frame: *mut u64) -> c_int;
+    pub fn af_session_create_formats(p: *mut af_pipeline, n_streams: usize, formats: *const af_stream_format, n_formats: usize,
+                                     stream_format: *const u32, sample_format: u16, out: *mut *mut af_session) -> c_int;
+    pub fn af_session_restart_streams(s: *mut af_session, streams: *const u32, format: *const u32, n: usize) -> c_int;
 }
 
 extern "C" {

@@ -16,6 +16,16 @@
 //! }
 //! ```
 //!
+//! Callers whose capture devices differ share one session through `Session::with_formats`; a freed slot takes a caller
+//! with another device through `restart_streams`:
+//!
+//! ```ignore
+//! let formats = [StreamFormat::new(48000, 1, 960), StreamFormat::new(44100, 2, 1764)];
+//! let mut s = Session::with_formats(&pipeline, &formats, &device_format_of_each_caller, None)?;
+//! // caller k hung up; a 44.1 kHz stereo caller takes its slot
+//! s.restart_streams(&[k], &[1])?;
+//! ```
+//!
 //! Source only, like the rest of the crate (INTEGRATION.md).
 use crate::batch::Pipeline;
 use crate::ffi;
@@ -52,7 +62,17 @@ pub struct WirePayload {
 #[derive(Debug, Clone, Copy, Default)]
 pub struct TickCounts { pub n_pcm: u32, pub n_feat: u32, pub n_vad: u32 }
 
-/// `af_session`: n 16 kHz streams (lockstep, or each on its own timeline) of one (rate, mono f32) with their state on the GPU between ticks.
+/// One capture format of a session (`af_stream_format`): the device's rate and interleaved channel count, and the bound of
+/// one tick's samples for a stream in it.
+#[derive(Debug, Clone, Copy, PartialEq, Eq)]
+pub struct StreamFormat { pub sample_rate: u32, pub channels: u16, pub max_tick_samples: u32 }
+
+impl StreamFormat {
+    pub fn new(sample_rate: u32, channels: u16, max_tick_samples: u32) -> Self { Self { sample_rate, channels, max_tick_samples } }
+}
+
+/// `af_session`: n 16 kHz streams (lockstep, or each on its own timeline) of f32 capture, each in one of the session's
+/// formats (`new`: mono at one rate), with their state on the GPU between ticks.
 pub struct Session { h: *mut ffi::af_session, n_streams: usize }
 unsafe impl Send for Session {}
 
@@ -62,7 +82,25 @@ impl Session {
                wire: Option<WireGate>) -> Result<Self, AudioError> {
         let mut h = ptr::null_mut();
         check(unsafe { ffi::af_session_create(pipeline.handle(), n_streams, sample_rate, 1, ffi::AF_FMT_F32, max_tick_samples, &mut h) })?;
-        let s = Self { h, n_streams };
+        Self { h, n_streams }.with_wire(wire)
+    }
+
+    /// A session of `stream_format.len()` streams that admits `formats`; stream k starts in `formats[stream_format[k]]`.
+    pub fn with_formats(pipeline: &Pipeline, formats: &[StreamFormat], stream_format: &[u32],
+                        wire: Option<WireGate>) -> Result<Self, AudioError> {
+        let fs: Vec<ffi::af_stream_format> = formats.iter().map(|f| ffi::af_stream_format {
+            sample_rate: f.sample_rate, channels: f.channels, pad: 0, max_tick_samples: f.max_tick_samples,
+        }).collect();
+        let mut h = ptr::null_mut();
+        check(unsafe {
+            ffi::af_session_create_formats(pipeline.handle(), stream_format.len(), fs.as_ptr(), fs.len(), stream_format.as_ptr(),
+                                           ffi::AF_FMT_F32, &mut h)
+        })?;
+        Self { h, n_streams: stream_format.len() }.with_wire(wire)
+    }
+
+    fn with_wire(self, wire: Option<WireGate>) -> Result<Self, AudioError> {
+        let s = self;
         if let Some(g) = wire {
             let cfg = ffi::af_wire_config { gate: (g == WireGate::Speech) as u32, pcm16: 0, base64: 1, mem: ffi::AF_MEM_HOST };
             check(unsafe { ffi::af_session_enable_wire(s.h, &cfg) })?;
@@ -108,6 +146,14 @@ impl Session {
     /// The listed streams start afresh at their next push, without a flush (the caller went away); the others continue.
     pub fn reset_streams(&mut self, streams: &[u32]) -> Result<(), AudioError> {
         check(unsafe { ffi::af_session_reset_streams(self.h, streams.as_ptr(), streams.len()) })
+    }
+
+    /// `streams[i]` start afresh at their next push in the session's format `format[i]` (a new caller with another device).
+    pub fn restart_streams(&mut self, streams: &[u32], format: &[u32]) -> Result<(), AudioError> {
+        if streams.len() != format.len() {
+            return Err(AudioError::ResamplingFailed(format!("{} streams and {} formats", streams.len(), format.len())));
+        }
+        check(unsafe { ffi::af_session_restart_streams(self.h, streams.as_ptr(), format.as_ptr(), streams.len()) })
     }
 
     /// The payloads of the last tick, one per stream (valid until the next push; copied out here).

@@ -451,6 +451,42 @@ AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings,
  * when af_session_wire would be. */
 AF_API int af_session_wire_first_frames(const af_session *s, uint64_t *first_frame);
 
+/* ---- sessions of mixed capture formats: each stream with its own rate and channel count ----------------------------
+ * Capture devices differ (AudioFrame carries its own sample_rate and channels, capture.rs:30-42; every BatchResampler
+ * is built for its own device's rate, resampler.rs:115-166).  A session created with af_session_create_formats admits
+ * a list of formats; every stream is in one of them at a time and a restarted stream may take another.  Stream k
+ * behaves exactly like a one-stream af_session_create session of its current format pushed the same ticks: PCM,
+ * frames, VAD, vad_final, the wire payload and its record, the levels and af_session_wire_first_frames.  The output is
+ * 16 kHz for every format.  On every push, n_samples[k] must be a whole number of frames of stream k's channels
+ * (AF_ERR_INVALID) and at most its format's max_tick_samples (AF_ERR_CAPACITY); the other rules of af_session_push_streams
+ * hold, and all errors are reported before any state changes.  On such a session:
+ *   af_session_push                  is af_session_push_streams with all counts equal (the lockstep tick runs only
+ *                                    while every stream is in one format at one position);
+ *   af_session_push_rings            takes exactly n_samples from every ring, under the same count checks;
+ *   af_session_push_rings_available  refuses a max_samples above the largest bound over the formats (AF_ERR_CAPACITY);
+ *                                    stream k takes min(max_samples, its format's max_tick_samples, available), rounded
+ *                                    down to whole frames of its channels (a single-format session sees no change);
+ *   af_session_reset                 returns every stream to the common start in its current format. */
+typedef struct af_stream_format {
+    uint32_t sample_rate;        /* the stream's capture rate; output is always 16 kHz */
+    uint16_t channels;           /* interleaved channels */
+    uint16_t pad;                /* 0 */
+    uint32_t max_tick_samples;   /* bound of one tick's interleaved samples for a stream in this format */
+} af_stream_format;              /* 12 bytes */
+/* A session that admits the n_formats formats listed (1 to 65536).  Stream k starts in formats[stream_format[k]]
+ * (stream_format NULL: every stream in formats[0]).  sample_format (AF_FMT_F32 / AF_FMT_I16) is the same for the
+ * whole session, so in_stride keeps counting samples.  The buffers are sized for the largest bound over the
+ * admitted formats.  AF_ERR_INVALID for n_formats == 0, a zero rate, channel count or bound, a nonzero pad, a
+ * stream_format index out of range or a bound too large for a session; AF_ERR_RESAMPLING_FAILED for an unsupported
+ * ratio.  af_session_create(p, n, rate, channels, fmt, max, out) is this call with the one format
+ * {rate, channels, 0, max}. */
+AF_API int af_session_create_formats(af_pipeline *p, size_t n_streams, const af_stream_format *formats, size_t n_formats,
+                                     const uint32_t *stream_format, uint16_t sample_format, af_session **out);
+/* Streams streams[i] start afresh at their next push in formats[format[i]]: af_session_reset_streams plus a new
+ * format.  A stream that ended with a flush has nothing left to discard.  A stream or format index out of range is
+ * AF_ERR_INVALID, and nothing changes. */
+AF_API int af_session_restart_streams(af_session *s, const uint32_t *streams, const uint32_t *format, size_t n);
+
 #ifdef __cplusplus
 }
 #endif
