@@ -109,6 +109,7 @@ def load_library():
         "af_last_error": (sz, [C.c_char_p, sz]), "af_device_count": (C.c_int, [C.POINTER(C.c_int)]),
         "af_version": (C.c_char_p, []), "af_kernel_launch_count": (C.c_uint64, []),
         "af_debug_pipe_stats": (C.c_int, [C.POINTER(C.c_uint64)]),
+        "af_debug_live_allocations": (C.c_int, [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "af_host_alloc": (C.c_int, [C.POINTER(vp), sz]), "af_host_free": (C.c_int, [vp]),
         "af_to_mono": (C.c_int, [fp, sz, C.c_uint16, fp, sz, szp]),
         "af_resampler_create": (C.c_int, [C.c_uint32, C.c_uint32, C.POINTER(vp)]),
@@ -226,6 +227,13 @@ def init(device: int = -1):
 
 def kernel_launch_count() -> int:
     return int(load_library().af_kernel_launch_count())
+
+
+def live_allocations() -> tuple[int, int]:
+    """(device, pinned): the allocations the library holds right now (af_debug_live_allocations)."""
+    d, p = C.c_uint64(0), C.c_uint64(0)
+    _check(load_library().af_debug_live_allocations(C.byref(d), C.byref(p)))
+    return int(d.value), int(p.value)
 
 
 def set_kernel_variant(name: str):

@@ -8,6 +8,7 @@
 #include <memory>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/audioflow_gpu.h"
@@ -30,26 +31,82 @@ int fail(int code, const char *fmt, ...);
                                                    cudaGetErrorString(_e));                        \
     } while (0)
 
-struct DevBuf {                       // grow-only device buffer
-    void *p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t bytes)
+// Every device and pinned allocation of the library is owned by a Buf: move-only, freed when the owner is reset,
+// reassigned or destroyed.  g_live_allocs counts the live allocations of each kind (af_debug_live_allocations): the
+// one leak check that works on a GPU other processes share.
+enum class Mem { Device, Pinned };
+inline std::atomic<uint64_t> g_live_allocs[2]{};
+
+template <class T, Mem K>
+class Buf {
+  public:
+    Buf() = default;
+    Buf(Buf &&o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+    Buf &operator=(Buf &&o) noexcept
     {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want;
+        if (this != &o) {
+            reset();
+            std::swap(p_, o.p_);
+            std::swap(n_, o.n_);
+        }
+        return *this;
+    }
+    ~Buf() { reset(); }
+
+    T *get() const { return p_; }
+    size_t size() const { return n_; }             // elements
+
+    // n elements in place of what the owner held (host_flags: cudaHostAlloc's, pinned only); empty on failure
+    cudaError_t alloc(size_t n, unsigned host_flags = cudaHostAllocDefault)
+    {
+        reset();
+        void *p = nullptr;
+        const cudaError_t e = K == Mem::Device ? cudaMalloc(&p, n * sizeof(T)) : cudaHostAlloc(&p, n * sizeof(T), host_flags);
+        if (e != cudaSuccess) return e;
+        p_ = static_cast<T *>(p);
+        n_ = n;
+        if (p_) g_live_allocs[(int)K].fetch_add(1, std::memory_order_relaxed);
+        return cudaSuccess;
+    }
+    // at least n elements: reallocates only when n exceeds the size, and does not keep the contents
+    cudaError_t grow(size_t n) { return n <= n_ ? cudaSuccess : alloc(n); }
+
+    cudaError_t reset()
+    {
+        if (!p_) return cudaSuccess;
+        const cudaError_t e = K == Mem::Device ? cudaFree(p_) : cudaFreeHost(p_);
+        if (e == cudaSuccess) g_live_allocs[(int)K].fetch_sub(1, std::memory_order_relaxed);
+        p_ = nullptr;
+        n_ = 0;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+
+    // af_host_alloc hands an allocation to the caller and af_host_free takes it back: it stays counted meanwhile
+    T *release()
+    {
+        T *p = p_;
+        p_ = nullptr;
+        n_ = 0;
+        return p;
+    }
+    static Buf adopt(T *p)
+    {
+        Buf b;
+        b.p_ = p;
+        return b;
+    }
+
+  private:
+    T *p_ = nullptr;
+    size_t n_ = 0;
 };
 
+template <class T> using DevBuf = Buf<T, Mem::Device>;
+template <class T> using PinnedBuf = Buf<T, Mem::Pinned>;
+
 struct FracTable {                    // device copy of the f32 fractional offsets of one rate pair
-    float *d = nullptr;
+    DevBuf<float> d;
     size_t n = 0;
-    ~FracTable() { if (d) cudaFree(d); }
 };
 
 struct RatePlan {                     // batch-path plan of one (in, out) pair, grown on demand
@@ -60,7 +117,8 @@ struct RatePlan {                     // batch-path plan of one (in, out) pair, 
 };
 
 // One context per GPU the process uses.  A thread works on ONE device at a time: the one it selected with af_init /
-// af_init_multi, or the one the handle it passes was created on (DevScope).
+// af_init_multi, or the one the handle it passes was created on (DevScope).  The contexts live until the process ends
+// and are never destroyed: af_shutdown releases what they hold.
 struct Context {
     bool ready = false;
     int device = -1;
@@ -68,9 +126,9 @@ struct Context {
     cudaStream_t stream = nullptr;    // the stream the library enqueues on: its own (non-blocking) one, or the caller's (af_set_stream)
     cudaStream_t own = nullptr;
     cudaStream_t side = nullptr;      // second stream: the result gather runs here, off the compute stream
-    FftTables *d_fft = nullptr;
+    DevBuf<FftTables> d_fft;
     std::mutex mu;                    // guards the scratch buffers and the plan cache
-    DevBuf scratch_in, scratch_out, scratch_aux, scratch_jobs;
+    DevBuf<uint8_t> scratch_in, scratch_out, scratch_aux, scratch_jobs;
     std::map<uint64_t, RatePlan> plans;
 };
 

@@ -107,7 +107,7 @@ struct af_sharded_batch {
     std::vector<af_batch *> local;             // per local rank (index into g_comm.ranks)
     std::vector<int> ranks, devices;           // copies of the communicator's at creation
     uint64_t rows_max = 0, row_stride = 0;     // gather geometry: [n_ranks][rows_max][row_stride] bytes
-    std::vector<uint8_t *> gbuf[2];            // per local rank, double buffered
+    std::vector<DevBuf<uint8_t>> gbuf[2];      // per local rank, double buffered
     std::vector<cudaEvent_t> ev_compute[2], ev_gather_begin[2], ev_gather_end[2];
     std::vector<bool> gathered_once[2];
     uint64_t steps = 0;
@@ -242,7 +242,7 @@ AF_API void af_sharded_batch_destroy(af_sharded_batch *b)
         DevScope scope_(b->devices[li]);
         cudaDeviceSynchronize();
         for (int p = 0; p < 2; ++p) {
-            if (li < b->gbuf[p].size() && b->gbuf[p][li]) cudaFree(b->gbuf[p][li]);
+            if (li < b->gbuf[p].size()) b->gbuf[p][li].reset();
             if (li < b->ev_compute[p].size() && b->ev_compute[p][li]) cudaEventDestroy(b->ev_compute[p][li]);
             if (li < b->ev_gather_begin[p].size() && b->ev_gather_begin[p][li]) cudaEventDestroy(b->ev_gather_begin[p][li]);
             if (li < b->ev_gather_end[p].size() && b->ev_gather_end[p][li]) cudaEventDestroy(b->ev_gather_end[p][li]);
@@ -281,7 +281,7 @@ AF_API int af_sharded_batch_create(af_pipeline *p, const af_stream_desc *streams
     const size_t n_local = b->ranks.size();
     b->local.assign(n_local, nullptr);
     for (int q = 0; q < 2; ++q) {
-        b->gbuf[q].assign(n_local, nullptr);
+        b->gbuf[q].resize(n_local);
         b->ev_compute[q].assign(n_local, nullptr);
         b->ev_gather_begin[q].assign(n_local, nullptr);
         b->ev_gather_end[q].assign(n_local, nullptr);
@@ -298,8 +298,8 @@ AF_API int af_sharded_batch_create(af_pipeline *p, const af_stream_desc *streams
         if (cfg.vad_enable && mem == AF_MEM_DEVICE) {
             const size_t bytes = std::max<size_t>((size_t)b->n_ranks * b->rows_max * b->row_stride, 256);
             for (int q = 0; q < 2; ++q) {
-                AF_CUDA(cudaMalloc(&b->gbuf[q][li], bytes));
-                AF_CUDA(cudaMemset(b->gbuf[q][li], 0, bytes));
+                AF_CUDA(b->gbuf[q][li].alloc(bytes));
+                AF_CUDA(cudaMemset(b->gbuf[q][li].get(), 0, bytes));
                 AF_CUDA(cudaEventCreateWithFlags(&b->ev_compute[q][li], cudaEventDisableTiming));
                 AF_CUDA(cudaEventCreate(&b->ev_gather_begin[q][li]));
                 AF_CUDA(cudaEventCreate(&b->ev_gather_end[q][li]));
@@ -376,7 +376,7 @@ AF_API int af_sharded_batch_run(af_sharded_batch *b, const af_sharded_outputs *o
         if (do_gather) {
             // the gather that used this buffer two runs ago must have drained before the scan overwrites the slot
             if (b->gathered_once[par][li]) AF_CUDA(cudaStreamWaitEvent(st, b->ev_gather_end[par][li], 0));
-            int rc = batch_run_on(b->local[li], o, b->gbuf[par][li] + (size_t)r * slot_bytes, b->row_stride, st);
+            int rc = batch_run_on(b->local[li], o, b->gbuf[par][li].get() + (size_t)r * slot_bytes, b->row_stride, st);
             if (rc) return rc;
             AF_CUDA(cudaEventRecord(b->ev_compute[par][li], st));
         } else {
@@ -396,7 +396,7 @@ AF_API int af_sharded_batch_run(af_sharded_batch *b, const af_sharded_outputs *o
             for (size_t li = 0; li < n_local; ++li) {
                 const int r = b->ranks[li];
                 DevScope scope_(b->devices[li]);
-                ncclResult_t nr = g_nccl.AllGather(b->gbuf[par][li] + (size_t)r * slot_bytes, b->gbuf[par][li], slot_bytes, ncclUint8,
+                ncclResult_t nr = g_nccl.AllGather(b->gbuf[par][li].get() + (size_t)r * slot_bytes, b->gbuf[par][li].get(), slot_bytes, ncclUint8,
                                                    g_comm.comms[li], cur_ctx().side);
                 if (nr != ncclSuccess) { g_nccl.GroupEnd(); return fail(AF_ERR_CUDA, "ncclAllGather: %s", g_nccl.GetErrorString(nr)); }
             }
@@ -421,7 +421,7 @@ AF_API int af_sharded_batch_gathered(af_sharded_batch *b, int rank, const uint8_
     const int li = [&] { for (size_t i = 0; i < b->ranks.size(); ++i) if (b->ranks[i] == rank) return (int)i; return -1; }();
     if (li < 0) return fail(AF_ERR_INVALID, "rank %d is not owned by this process", rank);
     if (b->last_parity < 0) return fail(AF_ERR_INVALID, "no run with a gather yet");
-    if (states) *states = b->gbuf[b->last_parity][li];
+    if (states) *states = b->gbuf[b->last_parity][li].get();
     if (row_stride) *row_stride = b->row_stride;
     if (rows_per_rank) *rows_per_rank = b->rows_max;
     if (n_vad_frames) memcpy(n_vad_frames, b->n_vad.data(), b->n_vad.size() * sizeof(uint32_t));
@@ -439,7 +439,7 @@ AF_API int af_sharded_batch_gathered_host(af_sharded_batch *b, int rank, uint8_t
     if (stride < max_vad) return fail(AF_ERR_CAPACITY, "stride %llu < %llu frames", (unsigned long long)stride, (unsigned long long)max_vad);
     AF_SCOPE(b->devices[li]);
     cudaStream_t st = cur_ctx().side;                     // ordered after the gather
-    const uint8_t *g = b->gbuf[b->last_parity][li];
+    const uint8_t *g = b->gbuf[b->last_parity][li].get();
     const size_t width = (size_t)std::min<uint64_t>(stride, b->row_stride);
     for (int r = 0; r < b->n_ranks; ++r) {
         const size_t lo = b->first[r], cnt = b->first[r + 1] - lo;

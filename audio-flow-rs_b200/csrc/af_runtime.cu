@@ -18,7 +18,8 @@ namespace afrt {
 namespace {
 thread_local std::string g_err;
 std::atomic<uint64_t> g_launches{0};
-Context g_ctxs[MAX_DEV];
+// never destroyed: at process exit the statically linked cudart may be gone before a destructor could free anything
+Context *const g_ctxs = new Context[MAX_DEV];
 std::mutex g_init_mu;                 // serialises device initialisation / shutdown
 std::atomic<int> g_default_dev{-1};   // the first device initialised: what a thread without a selection of its own uses
 thread_local int t_dev = -1;          // the device this thread works on
@@ -74,8 +75,8 @@ int init_device(int device)
     AF_CUDA(cudaStreamCreateWithPriority(&c.side, cudaStreamNonBlocking, prio_lo));
     FftTables *h = new FftTables;
     build_fft_tables(h);
-    cudaError_t ce = cudaMalloc(&c.d_fft, sizeof(FftTables));
-    if (ce == cudaSuccess) ce = cudaMemcpy(c.d_fft, h, sizeof(FftTables), cudaMemcpyHostToDevice);
+    cudaError_t ce = c.d_fft.alloc(1);
+    if (ce == cudaSuccess) ce = cudaMemcpy(c.d_fft.get(), h, sizeof(FftTables), cudaMemcpyHostToDevice);
     delete h;
     AF_CUDA(ce);
     c.device = device;
@@ -127,6 +128,9 @@ int device_of_pointer(const void *p)
 
 namespace {
 
+// the context's scratch buffers grow with 25 % slack: a caller whose sizes creep up rarely reallocates
+cudaError_t reserve(DevBuf<uint8_t> &b, size_t bytes) { return bytes <= b.size() ? cudaSuccess : b.alloc(bytes + bytes / 4 + 256); }
+
 // warp-to-role layout of the fused kernel (warp_role, af_common.cuh): the V warp gets a lighter scheduler when it
 // has energy chains to run.  AF_LAYOUT=<n> overrides (experiments).
 uint32_t fused_layout(bool energies)
@@ -176,9 +180,9 @@ int plan_rate(uint32_t in_rate, uint32_t out_rate, uint64_t n_in, uint64_t *n_ou
                     if (rem == 0 && enc[n] >= 0.5f) enc[n] = -enc[n];
                 }
                 // (16 floats of slack: the kernel fetches whole quads)
-                AF_CUDA(cudaMalloc(&t->d, (t->n + 16) * sizeof(float)));
-                AF_CUDA(cudaMemset(t->d, 0, (t->n + 16) * sizeof(float)));
-                AF_CUDA(cudaMemcpy(t->d, enc.data(), t->n * sizeof(float), cudaMemcpyHostToDevice));
+                AF_CUDA(t->d.alloc(t->n + 16));
+                AF_CUDA(cudaMemset(t->d.get(), 0, (t->n + 16) * sizeof(float)));
+                AF_CUDA(cudaMemcpy(t->d.get(), enc.data(), t->n * sizeof(float), cudaMemcpyHostToDevice));
             }
             pl.dev = t;
         }
@@ -227,6 +231,13 @@ AF_API int af_debug_pipe_stats(uint64_t out[32])
     return AF_OK;
 }
 
+AF_API int af_debug_live_allocations(uint64_t *device, uint64_t *pinned)
+{
+    if (device) *device = g_live_allocs[(int)Mem::Device].load();
+    if (pinned) *pinned = g_live_allocs[(int)Mem::Pinned].load();
+    return AF_OK;
+}
+
 AF_API int af_init(int device)
 {
     // selects `device` for the calling thread (initialising it on first use); device < 0: keep the thread's / the
@@ -262,9 +273,8 @@ AF_API int af_shutdown(void)
         (void)cudaSetDevice(d);
         cudaDeviceSynchronize();
         c.plans.clear();
-        c.scratch_in.release(); c.scratch_out.release(); c.scratch_aux.release(); c.scratch_jobs.release();
-        if (c.d_fft) cudaFree(c.d_fft);
-        c.d_fft = nullptr;
+        c.scratch_in.reset(); c.scratch_out.reset(); c.scratch_aux.reset(); c.scratch_jobs.reset();
+        c.d_fft.reset();
         if (c.own) cudaStreamDestroy(c.own);
         if (c.side) cudaStreamDestroy(c.side);
         c.stream = nullptr; c.own = nullptr; c.side = nullptr;
@@ -282,13 +292,15 @@ AF_API int af_host_alloc(void **ptr, size_t bytes)
     if (!ptr) return fail(AF_ERR_INVALID, "null pointer");
     int rc = require_ctx();
     if (rc) return rc;
-    AF_CUDA(cudaHostAlloc(ptr, bytes ? bytes : 1, cudaHostAllocPortable));    // pinned for every device of the process
+    PinnedBuf<uint8_t> b;
+    AF_CUDA(b.alloc(bytes ? bytes : 1, cudaHostAllocPortable));    // pinned for every device of the process
+    *ptr = b.release();
     return AF_OK;
 }
 
 AF_API int af_host_free(void *ptr)
 {
-    if (ptr) AF_CUDA(cudaFreeHost(ptr));
+    AF_CUDA(PinnedBuf<uint8_t>::adopt(static_cast<uint8_t *>(ptr)).reset());
     return AF_OK;
 }
 
@@ -316,13 +328,13 @@ AF_API int af_to_mono(const float *samples, size_t n_samples, uint16_t channels,
     if (n_out) *n_out = frames;
     if (frames == 0) return AF_OK;
     std::lock_guard<std::mutex> lk(cur_ctx().mu);
-    AF_CUDA(cur_ctx().scratch_in.reserve(n_samples * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_out.reserve(frames * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_in, n_samples * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_out, frames * sizeof(float)));
     cudaStream_t st = cur_ctx().stream;
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, samples, n_samples * sizeof(float), cudaMemcpyHostToDevice, st));
-    AF_CUDA(launch_to_mono((const float *)cur_ctx().scratch_in.p, n_samples, channels, (float *)cur_ctx().scratch_out.p, frames, st));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), samples, n_samples * sizeof(float), cudaMemcpyHostToDevice, st));
+    AF_CUDA(launch_to_mono((const float *)cur_ctx().scratch_in.get(), n_samples, channels, (float *)cur_ctx().scratch_out.get(), frames, st));
     count_launch();
-    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.p, frames * sizeof(float), cudaMemcpyDeviceToHost, st));
+    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.get(), frames * sizeof(float), cudaMemcpyDeviceToHost, st));
     AF_CUDA(cudaStreamSynchronize(st));
     return AF_OK;
 }
@@ -363,25 +375,25 @@ static int resampler_run_chunks(af_resampler *r, const float *input, size_t n_ch
     cudaStream_t st = cur_ctx().stream;
     const size_t in_bytes = r->stage.size() * sizeof(float);
     const size_t frac_bytes = r->frac.size() * sizeof(float);
-    AF_CUDA(cur_ctx().scratch_in.reserve(in_bytes));
-    AF_CUDA(cur_ctx().scratch_aux.reserve(frac_bytes + 16));
-    AF_CUDA(cur_ctx().scratch_out.reserve(produced * sizeof(float) + 16));
-    AF_CUDA(cur_ctx().scratch_jobs.reserve(sizeof(ResampleJob)));
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, r->stage.data(), in_bytes, cudaMemcpyHostToDevice, st));
-    if (frac_bytes) AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_aux.p, r->frac.data(), frac_bytes, cudaMemcpyHostToDevice, st));
+    AF_CUDA(reserve(cur_ctx().scratch_in, in_bytes));
+    AF_CUDA(reserve(cur_ctx().scratch_aux, frac_bytes + 16));
+    AF_CUDA(reserve(cur_ctx().scratch_out, produced * sizeof(float) + 16));
+    AF_CUDA(reserve(cur_ctx().scratch_jobs, sizeof(ResampleJob)));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), r->stage.data(), in_bytes, cudaMemcpyHostToDevice, st));
+    if (frac_bytes) AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_aux.get(), r->frac.data(), frac_bytes, cudaMemcpyHostToDevice, st));
     ResampleJob job;
-    job.data = (const float *)cur_ctx().scratch_in.p;
+    job.data = (const float *)cur_ctx().scratch_in.get();
     job.data_base = (long long)(c0 * RS_CHUNK) - 2 * RS_POLY;
     job.n_valid_end = (long long)((c0 + n_chunks) * RS_CHUNK);
     job.n_begin = n_begin; job.n_end = n_end;
     job.p = r->rec.p; job.q = r->rec.q; job.mode = r->rec.mode();
-    job.frac = (const float *)cur_ctx().scratch_aux.p - n_begin;      // indexed by the global output index
-    job.out = (float *)cur_ctx().scratch_out.p;
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_jobs.p, &job, sizeof(job), cudaMemcpyHostToDevice, st));
+    job.frac = (const float *)cur_ctx().scratch_aux.get() - n_begin;      // indexed by the global output index
+    job.out = (float *)cur_ctx().scratch_out.get();
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_jobs.get(), &job, sizeof(job), cudaMemcpyHostToDevice, st));
     if (produced) {
-        AF_CUDA(launch_resample_jobs((const ResampleJob *)cur_ctx().scratch_jobs.p, 1, (uint32_t)produced, st));
+        AF_CUDA(launch_resample_jobs((const ResampleJob *)cur_ctx().scratch_jobs.get(), 1, (uint32_t)produced, st));
         count_launch();
-        AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.p, produced * sizeof(float), cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.get(), produced * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
     AF_CUDA(cudaStreamSynchronize(st));
     memcpy(r->hist, r->stage.data() + r->stage.size() - 2 * RS_POLY, sizeof(r->hist));
@@ -506,7 +518,7 @@ struct af_vad {
     af_vad_config cfg;
     VadParams prm;
     VadState host;                    // mirror of the device state after the last call
-    VadState *dev = nullptr;
+    DevBuf<VadState> dev;
 };
 
 static VadParams make_vad_params(const af_vad_config &c)
@@ -538,8 +550,8 @@ AF_API int af_vad_create(const af_vad_config *cfg, af_vad **out)
     if (cfg) v->cfg = *cfg; else af_vad_config_default(&v->cfg);
     v->prm = make_vad_params(v->cfg);
     memset(&v->host, 0, sizeof(v->host));
-    cudaError_t e = cudaMalloc(&v->dev, sizeof(VadState));
-    if (e == cudaSuccess) e = cudaMemset(v->dev, 0, sizeof(VadState));
+    cudaError_t e = v->dev.alloc(1);
+    if (e == cudaSuccess) e = cudaMemset(v->dev.get(), 0, sizeof(VadState));
     if (e != cudaSuccess) { delete v; AF_CUDA(e); }
     *out = v;
     return AF_OK;
@@ -548,7 +560,7 @@ AF_API int af_vad_create(const af_vad_config *cfg, af_vad **out)
 AF_API void af_vad_destroy(af_vad *v)
 {
     if (!v) return;
-    if (v->dev) { DevScope scope_(v->device); cudaFree(v->dev); }
+    DevScope scope_(v->device);
     delete v;
 }
 
@@ -565,22 +577,22 @@ AF_API int af_vad_detect_frames(af_vad *v, const float *samples, size_t n, uint3
     AF_SCOPE(v->device);
     std::lock_guard<std::mutex> lk(cur_ctx().mu);
     cudaStream_t st = cur_ctx().stream;
-    AF_CUDA(cur_ctx().scratch_in.reserve(n * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_aux.reserve(T * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_out.reserve(T));
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    AF_CUDA(reserve(cur_ctx().scratch_in, n * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_aux, T * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_out, T));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
     EnergyJob ej{};
-    ej.y = (const float *)cur_ctx().scratch_in.p; ej.y_stride = 0; ej.n_frames = nullptr; ej.n_frames_all = (uint32_t)T;
-    ej.frame_len = frame_len; ej.hop = hop; ej.energy = (float *)cur_ctx().scratch_aux.p; ej.energy_stride = 0; ej.n_streams = 1;
+    ej.y = (const float *)cur_ctx().scratch_in.get(); ej.y_stride = 0; ej.n_frames = nullptr; ej.n_frames_all = (uint32_t)T;
+    ej.frame_len = frame_len; ej.hop = hop; ej.energy = (float *)cur_ctx().scratch_aux.get(); ej.energy_stride = 0; ej.n_streams = 1;
     AF_CUDA(launch_frame_energy(ej, st));
     ScanJob sj{};
-    sj.energy = (const float *)cur_ctx().scratch_aux.p; sj.energy_stride = 0; sj.n_frames = nullptr; sj.n_frames_all = (uint32_t)T;
-    sj.states = (uint8_t *)cur_ctx().scratch_out.p; sj.states_stride = 0; sj.state_io = v->dev; sj.final_out = nullptr;
+    sj.energy = (const float *)cur_ctx().scratch_aux.get(); sj.energy_stride = 0; sj.n_frames = nullptr; sj.n_frames_all = (uint32_t)T;
+    sj.states = (uint8_t *)cur_ctx().scratch_out.get(); sj.states_stride = 0; sj.state_io = v->dev.get(); sj.final_out = nullptr;
     sj.prm = v->prm; sj.n_streams = 1;
     AF_CUDA(launch_vad_scan(sj, st));
     count_launch(2);
-    if (states) AF_CUDA(cudaMemcpyAsync(states, cur_ctx().scratch_out.p, T, cudaMemcpyDeviceToHost, st));
-    AF_CUDA(cudaMemcpyAsync(&v->host, v->dev, sizeof(VadState), cudaMemcpyDeviceToHost, st));
+    if (states) AF_CUDA(cudaMemcpyAsync(states, cur_ctx().scratch_out.get(), T, cudaMemcpyDeviceToHost, st));
+    AF_CUDA(cudaMemcpyAsync(&v->host, v->dev.get(), sizeof(VadState), cudaMemcpyDeviceToHost, st));
     AF_CUDA(cudaStreamSynchronize(st));
     return AF_OK;
 }
@@ -609,7 +621,7 @@ AF_API int af_vad_reset(af_vad *v)
     if (!v) return fail(AF_ERR_INVALID, "null detector");
     memset(&v->host, 0, sizeof(v->host));
     AF_SCOPE(v->device);
-    AF_CUDA(cudaMemset(v->dev, 0, sizeof(VadState)));
+    AF_CUDA(cudaMemset(v->dev.get(), 0, sizeof(VadState)));
     return AF_OK;
 }
 AF_API int af_vad_state(const af_vad *v) { return v ? v->host.state : 0; }
@@ -631,15 +643,15 @@ AF_API int af_vad_frame_energy(const float *frame, size_t n, float *energy)
     if (n == 0) { *energy = 0.0f; return AF_OK; }
     std::lock_guard<std::mutex> lk(cur_ctx().mu);
     cudaStream_t st = cur_ctx().stream;
-    AF_CUDA(cur_ctx().scratch_in.reserve(n * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_aux.reserve(sizeof(float)));
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, frame, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    AF_CUDA(reserve(cur_ctx().scratch_in, n * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_aux, sizeof(float)));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), frame, n * sizeof(float), cudaMemcpyHostToDevice, st));
     EnergyJob ej{};
-    ej.y = (const float *)cur_ctx().scratch_in.p; ej.n_frames_all = 1; ej.frame_len = (uint32_t)n; ej.hop = (uint32_t)n;
-    ej.energy = (float *)cur_ctx().scratch_aux.p; ej.n_streams = 1;
+    ej.y = (const float *)cur_ctx().scratch_in.get(); ej.n_frames_all = 1; ej.frame_len = (uint32_t)n; ej.hop = (uint32_t)n;
+    ej.energy = (float *)cur_ctx().scratch_aux.get(); ej.n_streams = 1;
     AF_CUDA(launch_frame_energy(ej, st));
     count_launch();
-    AF_CUDA(cudaMemcpyAsync(energy, cur_ctx().scratch_aux.p, sizeof(float), cudaMemcpyDeviceToHost, st));
+    AF_CUDA(cudaMemcpyAsync(energy, cur_ctx().scratch_aux.get(), sizeof(float), cudaMemcpyDeviceToHost, st));
     AF_CUDA(cudaStreamSynchronize(st));
     return AF_OK;
 }
@@ -652,12 +664,12 @@ AF_API int af_pcm16_encode(const float *samples, size_t n, int16_t *out)
     if (n == 0) return AF_OK;
     std::lock_guard<std::mutex> lk(cur_ctx().mu);
     cudaStream_t st = cur_ctx().stream;
-    AF_CUDA(cur_ctx().scratch_in.reserve(n * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_out.reserve(n * sizeof(int16_t)));
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
-    AF_CUDA(launch_pcm16((const float *)cur_ctx().scratch_in.p, n, (int16_t *)cur_ctx().scratch_out.p, st));
+    AF_CUDA(reserve(cur_ctx().scratch_in, n * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_out, n * sizeof(int16_t)));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    AF_CUDA(launch_pcm16((const float *)cur_ctx().scratch_in.get(), n, (int16_t *)cur_ctx().scratch_out.get(), st));
     count_launch();
-    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.p, n * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
+    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.get(), n * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
     AF_CUDA(cudaStreamSynchronize(st));
     return AF_OK;
 }
@@ -675,12 +687,12 @@ AF_API int af_pcm16_base64(const float *samples, size_t n, char *out, size_t out
     if (n == 0) return AF_OK;
     std::lock_guard<std::mutex> lk(cur_ctx().mu);
     cudaStream_t st = cur_ctx().stream;
-    AF_CUDA(cur_ctx().scratch_in.reserve(n * sizeof(float)));
-    AF_CUDA(cur_ctx().scratch_out.reserve(need));
-    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.p, samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
-    AF_CUDA(launch_pcm16_base64((const float *)cur_ctx().scratch_in.p, n, (char *)cur_ctx().scratch_out.p, st));
+    AF_CUDA(reserve(cur_ctx().scratch_in, n * sizeof(float)));
+    AF_CUDA(reserve(cur_ctx().scratch_out, need));
+    AF_CUDA(cudaMemcpyAsync(cur_ctx().scratch_in.get(), samples, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    AF_CUDA(launch_pcm16_base64((const float *)cur_ctx().scratch_in.get(), n, (char *)cur_ctx().scratch_out.get(), st));
     count_launch();
-    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.p, need, cudaMemcpyDeviceToHost, st));
+    AF_CUDA(cudaMemcpyAsync(out, cur_ctx().scratch_out.get(), need, cudaMemcpyDeviceToHost, st));
     AF_CUDA(cudaStreamSynchronize(st));
     if (n_out) *n_out = need;
     return AF_OK;
@@ -737,7 +749,7 @@ struct af_pipeline {
     af_pipeline_config cfg;
     VadParams vad_prm;
     MelTables h_mel;                              // built once on the host ...
-    MelTables *d_mel[MAX_DEV] = {};               // ... and copied to every device that runs the pipeline, on first use
+    DevBuf<MelTables> d_mel[MAX_DEV];             // ... and copied to every device that runs the pipeline, on first use
     std::mutex mu;
 };
 
@@ -748,16 +760,15 @@ MelTables *pipe_mel(af_pipeline *p)
     if (!p->cfg.n_mels) return nullptr;
     const int dev = cur_device();
     std::lock_guard<std::mutex> lk(p->mu);
-    if (!p->d_mel[dev]) {
-        cudaError_t e = cudaMalloc(&p->d_mel[dev], sizeof(MelTables));
-        if (e == cudaSuccess) e = cudaMemcpy(p->d_mel[dev], &p->h_mel, sizeof(MelTables), cudaMemcpyHostToDevice);
+    if (!p->d_mel[dev].get()) {
+        cudaError_t e = p->d_mel[dev].alloc(1);
+        if (e == cudaSuccess) e = cudaMemcpy(p->d_mel[dev].get(), &p->h_mel, sizeof(MelTables), cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {
-            if (p->d_mel[dev]) cudaFree(p->d_mel[dev]);
-            p->d_mel[dev] = nullptr;
+            p->d_mel[dev].reset();
             fail(AF_ERR_CUDA, "mel tables: %s", cudaGetErrorString(e));
         }
     }
-    return p->d_mel[dev];
+    return p->d_mel[dev].get();
 }
 }  // namespace
 
@@ -773,12 +784,12 @@ struct SubBatch {                     // a group of streams resident on the devi
     size_t first = 0, count = 0;      // range in af_batch::streams
     std::vector<StreamDev> h_streams;
     std::vector<TileDev> h_tiles;
-    StreamDev *d_streams = nullptr;
-    TileDev *d_tiles = nullptr;
-    uint32_t *d_nframes = nullptr, *d_nvad = nullptr;
+    DevBuf<StreamDev> d_streams;
+    DevBuf<TileDev> d_tiles;
+    DevBuf<uint32_t> d_nframes, d_nvad;
     std::vector<size_t> in_off;       // host mode: byte offset of each stream inside the slot input buffer
     size_t in_bytes = 0;
-    uint32_t *d_scan = nullptr;       // long streams: scratch of the many-CTA VAD scan (launch_vad_scan)
+    DevBuf<uint32_t> d_scan;          // long streams: scratch of the many-CTA VAD scan (launch_vad_scan)
     bool quarters = false;            // some stream stages its input in quarter steps (f32 stereo)
     bool split = false;               // some stream is not 48 kHz mono f32 -> 16 kHz (FusedParams::split)
     uint32_t per_p = 0, per_q = 0;    // p / q of the batch's RS_TABLE streams when the output period fits the kernel's position table
@@ -797,12 +808,12 @@ struct af_batch {
     uint64_t max_out = 0, max_frames = 0, max_vad = 0;
     uint64_t pcm_stride = 0, logmel_stride = 0, vad_stride = 0;
     // device scratch for outputs the caller did not ask for but the pipeline needs
-    float *d_energy = nullptr; uint64_t energy_stride = 0; size_t energy_rows = 0;
-    float *d_pcm_scratch = nullptr; size_t pcm_scratch_rows = 0;
+    DevBuf<float> d_energy; uint64_t energy_stride = 0;
+    DevBuf<float> d_pcm_scratch;
     // host mode slots
     struct Slot {
-        void *d_in = nullptr; float *d_pcm = nullptr; int16_t *d_pcm16 = nullptr; float *d_logmel = nullptr; uint8_t *d_vad = nullptr;
-        float *d_energy = nullptr; VadState *d_final = nullptr;
+        DevBuf<char> d_in; DevBuf<float> d_pcm; DevBuf<int16_t> d_pcm16; DevBuf<float> d_logmel; DevBuf<uint8_t> d_vad;
+        DevBuf<float> d_energy; DevBuf<VadState> d_final;
         cudaStream_t st = nullptr;
     };
     std::vector<Slot> slots;
@@ -829,7 +840,7 @@ int build_sub(af_batch *b, SubBatch &sb, const void *slot_in_base)
         d.n_in = hs.n_in; d.n_out = hs.n_out; d.n_frames = hs.n_frames; d.n_vad_frames = hs.n_vad_frames;
         d.channels = hs.desc.channels; d.format = hs.desc.format;
         d.p = hs.p; d.q = hs.q; d.mode = hs.mode;
-        d.frac = hs.table ? hs.table->d : nullptr;
+        d.frac = hs.table ? hs.table->d.get() : nullptr;
         {   // does the raw input of one step fit the shared-memory stage of the fused kernel?
             const uint64_t bps = hs.desc.format == AF_FMT_I16 ? 2 : 4;
             // (a step is staged in two fills of half a step each, or in four of a quarter: whichever fits a stage buffer)
@@ -855,17 +866,15 @@ int build_sub(af_batch *b, SubBatch &sb, const void *slot_in_base)
         }
         nf[i] = hs.n_frames; nv[i] = hs.n_vad_frames;
     }
-    if (!sb.d_streams) {
-        AF_CUDA(cudaMalloc(&sb.d_streams, sb.count * sizeof(StreamDev)));
-        AF_CUDA(cudaMalloc(&sb.d_tiles, (sb.h_tiles.size() + 1) * sizeof(TileDev)));
-        AF_CUDA(cudaMalloc(&sb.d_nframes, sb.count * sizeof(uint32_t)));
-        AF_CUDA(cudaMalloc(&sb.d_nvad, sb.count * sizeof(uint32_t)));
-    }
-    AF_CUDA(cudaMemcpy(sb.d_streams, sb.h_streams.data(), sb.count * sizeof(StreamDev), cudaMemcpyHostToDevice));
+    AF_CUDA(sb.d_streams.grow(sb.count));
+    AF_CUDA(sb.d_tiles.grow(sb.h_tiles.size() + 1));
+    AF_CUDA(sb.d_nframes.grow(sb.count));
+    AF_CUDA(sb.d_nvad.grow(sb.count));
+    AF_CUDA(cudaMemcpy(sb.d_streams.get(), sb.h_streams.data(), sb.count * sizeof(StreamDev), cudaMemcpyHostToDevice));
     if (!sb.h_tiles.empty())
-        AF_CUDA(cudaMemcpy(sb.d_tiles, sb.h_tiles.data(), sb.h_tiles.size() * sizeof(TileDev), cudaMemcpyHostToDevice));
-    AF_CUDA(cudaMemcpy(sb.d_nframes, nf.data(), sb.count * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    AF_CUDA(cudaMemcpy(sb.d_nvad, nv.data(), sb.count * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        AF_CUDA(cudaMemcpy(sb.d_tiles.get(), sb.h_tiles.data(), sb.h_tiles.size() * sizeof(TileDev), cudaMemcpyHostToDevice));
+    AF_CUDA(cudaMemcpy(sb.d_nframes.get(), nf.data(), sb.count * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    AF_CUDA(cudaMemcpy(sb.d_nvad.get(), nv.data(), sb.count * sizeof(uint32_t), cudaMemcpyHostToDevice));
     return AF_OK;
 }
 
@@ -879,8 +888,8 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
     const bool custom_vad = cfg.vad_enable && cfg.vad_frame_len != 0;
     if (!sb.h_tiles.empty()) {
         FusedParams P{};
-        P.streams = sb.d_streams; P.tiles = sb.d_tiles; P.n_tiles = (uint32_t)sb.h_tiles.size();
-        P.fft = cur_ctx().d_fft; P.mel = b->d_mel;
+        P.streams = sb.d_streams.get(); P.tiles = sb.d_tiles.get(); P.n_tiles = (uint32_t)sb.h_tiles.size();
+        P.fft = cur_ctx().d_fft.get(); P.mel = b->d_mel;
         P.pcm = pcm; P.pcm_stride = pcm_stride;
         P.logmel = cfg.n_mels ? logmel : nullptr; P.logmel_stride = logmel_stride;
         P.energy = stft_vad ? energy : nullptr; P.energy_stride = energy_stride;
@@ -899,7 +908,7 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
     }
     if (custom_vad) {
         EnergyJob ej{};
-        ej.y = pcm; ej.y_stride = pcm_stride; ej.n_frames = sb.d_nvad; ej.n_frames_all = (uint32_t)b->max_vad;
+        ej.y = pcm; ej.y_stride = pcm_stride; ej.n_frames = sb.d_nvad.get(); ej.n_frames_all = (uint32_t)b->max_vad;
         ej.frame_len = cfg.vad_frame_len; ej.hop = cfg.vad_hop; ej.energy = energy; ej.energy_stride = energy_stride;
         ej.n_streams = (uint32_t)sb.count;
         AF_CUDA(launch_frame_energy(ej, st));
@@ -907,12 +916,12 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
     }
     if (cfg.vad_enable) {
         ScanJob sj{};
-        sj.energy = energy; sj.energy_stride = energy_stride; sj.n_frames = sb.d_nvad; sj.n_frames_all = 0;
+        sj.energy = energy; sj.energy_stride = energy_stride; sj.n_frames = sb.d_nvad.get(); sj.n_frames_all = 0;
         sj.states = vad; sj.states_stride = vad_stride; sj.state_io = nullptr; sj.final_out = vad_final;
         sj.prm = b->pipe->vad_prm; sj.n_streams = (uint32_t)sb.count;
         if (b->max_vad > 16384 && b->max_vad < 0x40000000ull) {              // long streams: many CTAs per stream
-            if (!sb.d_scan) AF_CUDA(cudaMalloc(&sb.d_scan, sb.count * scan_scratch_words((uint32_t)b->max_vad) * sizeof(uint32_t)));
-            sj.max_frames = (uint32_t)b->max_vad; sj.scratch = sb.d_scan;
+            AF_CUDA(sb.d_scan.grow(sb.count * scan_scratch_words((uint32_t)b->max_vad)));
+            sj.max_frames = (uint32_t)b->max_vad; sj.scratch = sb.d_scan.get();
         }
         AF_CUDA(launch_vad_scan(sj, st));
         count_launch();
@@ -921,6 +930,9 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
 }
 
 uint64_t round_up(uint64_t v, uint64_t m) { return (v + m - 1) / m * m; }
+
+// n elements of T, but no fewer than 256 bytes
+template <class T> size_t min256(size_t n) { return std::max<size_t>(n, (256 + sizeof(T) - 1) / sizeof(T)); }
 
 }  // namespace
 
@@ -966,7 +978,7 @@ AF_API void af_pipeline_destroy(af_pipeline *p)
 {
     if (!p) return;
     for (int d = 0; d < MAX_DEV; ++d)
-        if (p->d_mel[d] && device_ctx(d)) { DevScope scope_(d); cudaFree(p->d_mel[d]); }
+        if (p->d_mel[d].get() && device_ctx(d)) { DevScope scope_(d); p->d_mel[d].reset(); }
     delete p;
 }
 
@@ -975,25 +987,8 @@ AF_API void af_batch_destroy(af_batch *b)
     if (!b) return;
     DevScope scope_(b->device);
     cudaDeviceSynchronize();
-    for (auto &sb : b->subs) {
-        if (sb.d_streams) cudaFree(sb.d_streams);
-        if (sb.d_tiles) cudaFree(sb.d_tiles);
-        if (sb.d_nframes) cudaFree(sb.d_nframes);
-        if (sb.d_nvad) cudaFree(sb.d_nvad);
-        if (sb.d_scan) cudaFree(sb.d_scan);
-    }
-    if (b->d_energy) cudaFree(b->d_energy);
-    if (b->d_pcm_scratch) cudaFree(b->d_pcm_scratch);
-    for (auto &s : b->slots) {
-        if (s.d_in) cudaFree(s.d_in);
-        if (s.d_pcm) cudaFree(s.d_pcm);
-        if (s.d_pcm16) cudaFree(s.d_pcm16);
-        if (s.d_logmel) cudaFree(s.d_logmel);
-        if (s.d_vad) cudaFree(s.d_vad);
-        if (s.d_energy) cudaFree(s.d_energy);
-        if (s.d_final) cudaFree(s.d_final);
+    for (auto &s : b->slots)
         if (s.st) cudaStreamDestroy(s.st);
-    }
     delete b;
 }
 
@@ -1093,18 +1088,18 @@ AF_API int af_batch_create(af_pipeline *p, const af_stream_desc *streams, size_t
         b->slots.resize(n_slots);
         for (auto &s : b->slots) {
             AF_CUDA(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking));
-            AF_CUDA(cudaMalloc(&s.d_in, std::max<size_t>(max_in, 256)));
-            AF_CUDA(cudaMalloc(&s.d_pcm, std::max<size_t>(max_rows * b->pcm_stride * sizeof(float), 256)));
-            if (cfg.pcm16) AF_CUDA(cudaMalloc(&s.d_pcm16, std::max<size_t>(max_rows * b->pcm_stride * sizeof(int16_t), 256)));
-            if (cfg.n_mels) AF_CUDA(cudaMalloc(&s.d_logmel, std::max<size_t>(max_rows * b->logmel_stride * sizeof(float), 256)));
+            AF_CUDA(s.d_in.alloc(min256<char>(max_in)));
+            AF_CUDA(s.d_pcm.alloc(min256<float>(max_rows * b->pcm_stride)));
+            if (cfg.pcm16) AF_CUDA(s.d_pcm16.alloc(min256<int16_t>(max_rows * b->pcm_stride)));
+            if (cfg.n_mels) AF_CUDA(s.d_logmel.alloc(min256<float>(max_rows * b->logmel_stride)));
             if (cfg.vad_enable) {
-                AF_CUDA(cudaMalloc(&s.d_vad, std::max<size_t>(max_rows * b->vad_stride, 256)));
-                AF_CUDA(cudaMalloc(&s.d_energy, std::max<size_t>(max_rows * b->energy_stride * sizeof(float), 256)));
-                AF_CUDA(cudaMalloc(&s.d_final, std::max<size_t>(max_rows * sizeof(VadState), 256)));
+                AF_CUDA(s.d_vad.alloc(min256<uint8_t>(max_rows * b->vad_stride)));
+                AF_CUDA(s.d_energy.alloc(min256<float>(max_rows * b->energy_stride)));
+                AF_CUDA(s.d_final.alloc(min256<VadState>(max_rows)));
             }
         }
         for (size_t g = 0; g < b->subs.size(); ++g) {
-            rc = build_sub(b.get(), b->subs[g], b->slots[g % n_slots].d_in);
+            rc = build_sub(b.get(), b->subs[g], b->slots[g % n_slots].d_in.get());
             if (rc) return rc;
         }
     }
@@ -1187,15 +1182,15 @@ int batch_run_on(af_batch *b, const af_outputs *o, uint8_t *vad, uint64_t vad_st
     const size_t S = b->streams.size();
     float *energy = o->energy; uint64_t energy_stride = o->energy_stride;
     if (cfg.vad_enable && !energy) {
-        if (!b->d_energy) AF_CUDA(cudaMalloc(&b->d_energy, std::max<size_t>(S * b->energy_stride * sizeof(float), 256)));
-        energy = b->d_energy; energy_stride = b->energy_stride;
+        AF_CUDA(b->d_energy.grow(min256<float>(S * b->energy_stride)));
+        energy = b->d_energy.get(); energy_stride = b->energy_stride;
     }
     float *pcm = cfg.write_pcm ? o->pcm : nullptr; uint64_t pcm_stride = o->pcm_stride;
     const bool wire16 = cfg.pcm16 && pcm;                        // PCM leaves as i16 wire samples: f32 rows stay internal
     if (wire16) pcm = nullptr;
     if ((wire16 || (cfg.vad_enable && cfg.vad_frame_len != 0)) && !pcm) {      // custom VAD frames read the PCM back
-        if (!b->d_pcm_scratch) AF_CUDA(cudaMalloc(&b->d_pcm_scratch, std::max<size_t>(S * b->pcm_stride * sizeof(float), 256)));
-        pcm = b->d_pcm_scratch; pcm_stride = b->pcm_stride;
+        AF_CUDA(b->d_pcm_scratch.grow(min256<float>(S * b->pcm_stride)));
+        pcm = b->d_pcm_scratch.get(); pcm_stride = b->pcm_stride;
     }
     int rc = run_sub(b, b->subs[0], pcm, pcm_stride, o->logmel, o->logmel_stride, vad, vad_stride, energy, energy_stride,
                      reinterpret_cast<VadState *>(o->vad_final), st);
@@ -1251,50 +1246,50 @@ AF_API int af_batch_run_host(af_batch *b, const af_outputs *o)
                 ++j;
             }
             if (bytes) {
-                cudaError_t ce = cudaMemcpyAsync((char *)sl.d_in + sb.in_off[i], d0.data, bytes, cudaMemcpyHostToDevice, st);
+                cudaError_t ce = cudaMemcpyAsync(sl.d_in.get() + sb.in_off[i], d0.data, bytes, cudaMemcpyHostToDevice, st);
                 if (ce == cudaErrorInvalidValue && j > i + 1) {
                     // rows that happen to be adjacent in host memory but belong to separate pinned allocations: CUDA refuses a
                     // copy that spans two of them.  Not sticky: copy this sub-batch stream by stream from now on.
                     (void)cudaGetLastError();
                     sb.no_merge = true;
                     j = i + 1;
-                    ce = bytes0 ? cudaMemcpyAsync((char *)sl.d_in + sb.in_off[i], d0.data, bytes0, cudaMemcpyHostToDevice, st) : cudaSuccess;
+                    ce = bytes0 ? cudaMemcpyAsync(sl.d_in.get() + sb.in_off[i], d0.data, bytes0, cudaMemcpyHostToDevice, st) : cudaSuccess;
                 }
                 AF_CUDA(ce);
             }
             i = j;
         }
         const bool need_pcm = (cfg.write_pcm && o->pcm) || (cfg.vad_enable && cfg.vad_frame_len != 0);
-        rc = run_sub(b, sb, need_pcm ? sl.d_pcm : nullptr, b->pcm_stride, sl.d_logmel, b->logmel_stride, sl.d_vad,
-                     b->vad_stride, sl.d_energy, b->energy_stride, sl.d_final, st);
+        rc = run_sub(b, sb, need_pcm ? sl.d_pcm.get() : nullptr, b->pcm_stride, sl.d_logmel.get(), b->logmel_stride, sl.d_vad.get(),
+                     b->vad_stride, sl.d_energy.get(), b->energy_stride, sl.d_final.get(), st);
         if (rc) return rc;
         const size_t r0 = sb.first;
         if (cfg.write_pcm && o->pcm && cfg.pcm16) {
-            AF_CUDA(launch_pcm16_rows(sl.d_pcm, b->pcm_stride, sl.d_pcm16, b->pcm_stride, (uint32_t)b->max_out, (uint32_t)sb.count, st));
+            AF_CUDA(launch_pcm16_rows(sl.d_pcm.get(), b->pcm_stride, sl.d_pcm16.get(), b->pcm_stride, (uint32_t)b->max_out, (uint32_t)sb.count, st));
             count_launch();
             int16_t *dst = reinterpret_cast<int16_t *>(o->pcm);
-            AF_CUDA(cudaMemcpy2DAsync(dst + r0 * o->pcm_stride, o->pcm_stride * sizeof(int16_t), sl.d_pcm16,
+            AF_CUDA(cudaMemcpy2DAsync(dst + r0 * o->pcm_stride, o->pcm_stride * sizeof(int16_t), sl.d_pcm16.get(),
                                       b->pcm_stride * sizeof(int16_t), b->max_out * sizeof(int16_t), sb.count,
                                       cudaMemcpyDeviceToHost, st));
         } else if (cfg.write_pcm && o->pcm)
-            AF_CUDA(cudaMemcpy2DAsync(o->pcm + r0 * o->pcm_stride, o->pcm_stride * sizeof(float), sl.d_pcm,
+            AF_CUDA(cudaMemcpy2DAsync(o->pcm + r0 * o->pcm_stride, o->pcm_stride * sizeof(float), sl.d_pcm.get(),
                                       b->pcm_stride * sizeof(float), b->max_out * sizeof(float), sb.count,
                                       cudaMemcpyDeviceToHost, st));
         if (cfg.n_mels && o->logmel && b->max_frames)
-            AF_CUDA(cudaMemcpy2DAsync(o->logmel + r0 * o->logmel_stride, o->logmel_stride * sizeof(float), sl.d_logmel,
+            AF_CUDA(cudaMemcpy2DAsync(o->logmel + r0 * o->logmel_stride, o->logmel_stride * sizeof(float), sl.d_logmel.get(),
                                       b->logmel_stride * sizeof(float), b->max_frames * cfg.n_mels * sizeof(float),
                                       sb.count, cudaMemcpyDeviceToHost, st));
         if (cfg.vad_enable && b->max_vad) {
             if (o->vad)
-                AF_CUDA(cudaMemcpy2DAsync(o->vad + r0 * o->vad_stride, o->vad_stride, sl.d_vad, b->vad_stride, b->max_vad,
+                AF_CUDA(cudaMemcpy2DAsync(o->vad + r0 * o->vad_stride, o->vad_stride, sl.d_vad.get(), b->vad_stride, b->max_vad,
                                           sb.count, cudaMemcpyDeviceToHost, st));
             if (o->energy)
-                AF_CUDA(cudaMemcpy2DAsync(o->energy + r0 * o->energy_stride, o->energy_stride * sizeof(float), sl.d_energy,
+                AF_CUDA(cudaMemcpy2DAsync(o->energy + r0 * o->energy_stride, o->energy_stride * sizeof(float), sl.d_energy.get(),
                                           b->energy_stride * sizeof(float), b->max_vad * sizeof(float), sb.count,
                                           cudaMemcpyDeviceToHost, st));
         }
         if (cfg.vad_enable && o->vad_final)
-            AF_CUDA(cudaMemcpyAsync(o->vad_final + r0, sl.d_final, sb.count * sizeof(VadState), cudaMemcpyDeviceToHost, st));
+            AF_CUDA(cudaMemcpyAsync(o->vad_final + r0, sl.d_final.get(), sb.count * sizeof(VadState), cudaMemcpyDeviceToHost, st));
     }
     for (auto &sl : b->slots) AF_CUDA(cudaStreamSynchronize(sl.st));
     return AF_OK;
@@ -1339,14 +1334,14 @@ struct af_session {
     // are sized for the largest bound over the formats: max_tick_frames, max_new_y (below) and max_ring_samples
     struct Format { uint32_t rate, channels, max_tick_frames; };
     std::vector<Format> fmts;
-    SessionFormat *d_fmts = nullptr;                           // their device table, read by af_session_tick_streams_kernel
+    DevBuf<SessionFormat> d_fmts;                              // their device table, read by af_session_tick_streams_kernel
     bool any_table = false;                                    // some format resamples through a fraction table (RS_TABLE)
     uint32_t format = 0, max_tick_frames = 0;
     uint64_t max_ring_samples = 0;
     // input history: last 16 frames + residual (< 128), ping-pong
-    float *in_buf[2] = {nullptr, nullptr}; uint64_t in_stride = 0; int in_cur = 0;
+    DevBuf<float> in_buf[2]; uint64_t in_stride = 0; int in_cur = 0;
     // 16 kHz carry (samples not yet covered by an emitted frame), ping-pong
-    float *y_buf[2] = {nullptr, nullptr}; uint64_t y_stride = 0; int y_cur = 0;
+    DevBuf<float> y_buf[2]; uint64_t y_stride = 0; int y_cur = 0;
     uint32_t frame_len = WIN, hop = HOP;   // framing of the features / VAD
     bool framing = false;
     // packed ticks (STFT frames): the rows of y_buf are a whole number of hops apart, so `pk_rows` consecutive streams
@@ -1355,30 +1350,37 @@ struct af_session {
     // 30 of 32 slots empty, and the tiles are planned once (the virtual streams never change length).
     bool packed = false;
     uint32_t pk_slots = 0, pk_rows = 0, pk_n = 0;          // frame slots per row, rows per virtual stream, virtual streams
-    StreamDev *d_ptab[2] = {nullptr, nullptr};
-    TileDev *d_ptiles[2] = {nullptr, nullptr};
-    VadState *d_vad = nullptr;
-    float *d_energy = nullptr; uint64_t energy_stride = 0;
-    float *d_frac = nullptr; size_t frac_cap = 0;
-    void *d_in_stage = nullptr; size_t in_stage_bytes = 0;    // host-mode staging of the tick input
-    float *d_lm = nullptr; uint8_t *d_states = nullptr;       // host-mode staging of outputs
+    DevBuf<StreamDev> d_ptab[2];
+    DevBuf<TileDev> d_ptiles[2];
+    DevBuf<VadState> d_vad;
+    DevBuf<float> d_energy; uint64_t energy_stride = 0;
+    DevBuf<float> d_frac;
+    DevBuf<char> d_in_stage;                                  // host-mode staging of the tick input
+    DevBuf<float> d_lm; DevBuf<uint8_t> d_states;             // host-mode staging of outputs
     uint64_t lm_stride = 0, st_stride = 0;
     std::vector<float> frac_host;
-    float *ring_stage = nullptr; size_t ring_stage_cap = 0;   // pinned rows for af_session_push_rings
+    PinnedBuf<float> ring_stage;                              // pinned rows for af_session_push_rings
     // level metering (af_session_enable_levels): peak of the last tick per stream + the detector states, on the host
+    struct Levels {
+        DevBuf<float> d_peak;
+        PinnedBuf<float> h_peak;
+        PinnedBuf<VadState> h_vad;
+    };
+    Levels lv;
     bool levels = false, levels_valid = false;
-    float *d_peak = nullptr, *h_peak = nullptr;
-    VadState *h_vad = nullptr;
     // wire output (af_session_enable_wire): device rows written by the wire kernel, pinned host copies for AF_MEM_HOST
+    struct Wire {
+        af_wire_config cfg{};
+        DevBuf<int16_t> d_pcm16; PinnedBuf<int16_t> h_pcm16; uint64_t pcm16_stride = 0;   // int16_t elements
+        DevBuf<char> d_b64; PinnedBuf<char> h_b64; uint64_t b64_stride = 0;               // bytes
+        uint64_t cap = 0;                                                                 // payload samples a row holds
+        DevBuf<WireTick> d_ticks;
+        PinnedBuf<af_wire_tick> h_ticks;
+    };
+    Wire wr;
     uint64_t max_new_y = 0;                                   // bound of the 16 kHz samples one tick produces
     bool wire = false, wire_valid = false;
-    af_wire_config wire_cfg{};
-    uint8_t *d_wire_prev = nullptr;                           // per stream: state of the latest completed frame
-    int16_t *d_wire_pcm16 = nullptr, *h_wire_pcm16 = nullptr; uint64_t wire_pcm16_stride = 0;   // int16_t elements
-    char *d_wire_b64 = nullptr, *h_wire_b64 = nullptr; uint64_t wire_b64_stride = 0;            // bytes
-    uint64_t wire_cap = 0;                                    // payload samples a row holds
-    WireTick *d_wire_ticks = nullptr;
-    af_wire_tick *h_wire_ticks = nullptr;
+    DevBuf<uint8_t> d_wire_prev;                              // per stream: state of the latest completed frame
     // the bookkeeping of one stream's timeline.  While !diverged, `shared` is the position of every stream and a tick of
     // equal counts takes the lockstep tick kernel; while diverged, ss[k] is stream k's position (af_session_push_streams).
     // The ping-pong buffers (in_cur, y_cur) flip for all streams on every tick either way.
@@ -1398,8 +1400,12 @@ struct af_session {
     std::vector<StreamState> ss, ss_next;
     bool diverged = false;
     std::vector<uint32_t> plan_slots;                          // scratch: open-addressing table of the tick's distinct plans
-    StreamTick *h_tick = nullptr, *d_tick = nullptr;           // the tick's plan: [S] StreamTick, then [S] uint32 frame counts
-    float *d_pcm_stage = nullptr;                              // host-mode PCM rows of a per-stream tick
+    struct TickPlan {                                          // the tick's plan: [S] StreamTick, then [S] uint32 frame counts
+        DevBuf<StreamTick> d;
+        PinnedBuf<StreamTick> h;
+    };
+    TickPlan tick;
+    DevBuf<float> d_pcm_stage;                                 // host-mode PCM rows of a per-stream tick
     std::vector<uint32_t> counts;                              // scratch: equal counts (af_session_push), ring reads
     std::vector<uint64_t> first_frames;                        // per stream: first frame completed by the last push
 };
@@ -1409,15 +1415,7 @@ static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, sta
 namespace {
 void wire_free(af_session *s)
 {
-    if (s->d_wire_pcm16) cudaFree(s->d_wire_pcm16);
-    if (s->h_wire_pcm16) cudaFreeHost(s->h_wire_pcm16);
-    if (s->d_wire_b64) cudaFree(s->d_wire_b64);
-    if (s->h_wire_b64) cudaFreeHost(s->h_wire_b64);
-    if (s->d_wire_ticks) cudaFree(s->d_wire_ticks);
-    if (s->h_wire_ticks) cudaFreeHost(s->h_wire_ticks);
-    s->d_wire_pcm16 = s->h_wire_pcm16 = nullptr; s->d_wire_b64 = s->h_wire_b64 = nullptr;
-    s->d_wire_ticks = nullptr; s->h_wire_ticks = nullptr;
-    s->wire_pcm16_stride = s->wire_b64_stride = s->wire_cap = 0;
+    s->wr = af_session::Wire{};
     s->wire = s->wire_valid = false;
 }
 
@@ -1443,28 +1441,6 @@ AF_API void af_session_destroy(af_session *s)
     if (!s) return;
     DevScope scope_(s->device);
     cudaDeviceSynchronize();
-    for (int i = 0; i < 2; ++i) {
-        if (s->in_buf[i]) cudaFree(s->in_buf[i]);
-        if (s->y_buf[i]) cudaFree(s->y_buf[i]);
-        if (s->d_ptab[i]) cudaFree(s->d_ptab[i]);
-        if (s->d_ptiles[i]) cudaFree(s->d_ptiles[i]);
-    }
-    if (s->d_vad) cudaFree(s->d_vad);
-    if (s->d_energy) cudaFree(s->d_energy);
-    if (s->d_frac) cudaFree(s->d_frac);
-    if (s->d_in_stage) cudaFree(s->d_in_stage);
-    if (s->d_lm) cudaFree(s->d_lm);
-    if (s->d_states) cudaFree(s->d_states);
-    if (s->ring_stage) cudaFreeHost(s->ring_stage);
-    if (s->d_peak) cudaFree(s->d_peak);
-    if (s->h_peak) cudaFreeHost(s->h_peak);
-    if (s->h_vad) cudaFreeHost(s->h_vad);
-    wire_free(s);
-    if (s->d_wire_prev) cudaFree(s->d_wire_prev);
-    if (s->d_tick) cudaFree(s->d_tick);
-    if (s->h_tick) cudaFreeHost(s->h_tick);
-    if (s->d_pcm_stage) cudaFree(s->d_pcm_stage);
-    if (s->d_fmts) cudaFree(s->d_fmts);
     delete s;
 }
 
@@ -1482,9 +1458,9 @@ AF_API int af_session_reset(af_session *s)
         for (size_t k = 0; k < s->S; ++k) s->ss[k] = fresh_stream(s, s->ss[k].fmt);
     }
     s->in_cur = 0; s->y_cur = 0;
-    AF_CUDA(cudaMemset(s->in_buf[0], 0, s->S * s->in_stride * sizeof(float)));
-    AF_CUDA(cudaMemset(s->d_vad, 0, s->S * sizeof(VadState)));
-    if (s->d_wire_prev) AF_CUDA(cudaMemset(s->d_wire_prev, 0, s->S));   // no segment open
+    AF_CUDA(cudaMemset(s->in_buf[0].get(), 0, s->S * s->in_stride * sizeof(float)));
+    AF_CUDA(cudaMemset(s->d_vad.get(), 0, s->S * sizeof(VadState)));
+    if (s->d_wire_prev.get()) AF_CUDA(cudaMemset(s->d_wire_prev.get(), 0, s->S));   // no segment open
     return AF_OK;
 }
 
@@ -1556,9 +1532,9 @@ AF_API int af_session_create_formats(af_pipeline *p, size_t n_streams, const af_
     }
     s->st_stride = round_up(max_frames, 16);
     for (int i = 0; i < 2; ++i) {
-        AF_CUDA(cudaMalloc(&s->in_buf[i], n_streams * s->in_stride * sizeof(float)));
-        AF_CUDA(cudaMalloc(&s->y_buf[i], n_streams * s->y_stride * sizeof(float)));
-        AF_CUDA(cudaMemset(s->y_buf[i], 0, n_streams * s->y_stride * sizeof(float)));
+        AF_CUDA(s->in_buf[i].alloc(n_streams * s->in_stride));
+        AF_CUDA(s->y_buf[i].alloc(n_streams * s->y_stride));
+        AF_CUDA(cudaMemset(s->y_buf[i].get(), 0, n_streams * s->y_stride * sizeof(float)));
         if (s->packed) {
             std::vector<StreamDev> ptab(s->pk_n);
             std::vector<TileDev> ptiles(s->pk_n);
@@ -1566,27 +1542,26 @@ AF_API int af_session_create_formats(af_pipeline *p, size_t n_streams, const af_
                 StreamDev &d = ptab[v];
                 memset(&d, 0, sizeof(d));
                 const uint64_t rows = std::min<uint64_t>(s->pk_rows, n_streams - (uint64_t)v * s->pk_rows);
-                d.data = s->y_buf[i] + (uint64_t)v * s->pk_rows * s->y_stride;
+                d.data = s->y_buf[i].get() + (uint64_t)v * s->pk_rows * s->y_stride;
                 d.n_samples = rows * s->y_stride; d.n_in = d.n_out = (uint32_t)d.n_samples;
                 d.n_frames = d.n_vad_frames = 1 + (d.n_out - WIN) / HOP;
                 d.channels = 1; d.format = FMT_F32; d.p = 1; d.q = 1; d.mode = RS_PASSTHROUGH;
                 d.tile_begin = v; d.n_tiles = 1; d.staged = 2;
                 plan_tile(d, v, 0, &ptiles[v]);
             }
-            AF_CUDA(cudaMalloc(&s->d_ptab[i], s->pk_n * sizeof(StreamDev)));
-            AF_CUDA(cudaMalloc(&s->d_ptiles[i], s->pk_n * sizeof(TileDev)));
-            AF_CUDA(cudaMemcpy(s->d_ptab[i], ptab.data(), s->pk_n * sizeof(StreamDev), cudaMemcpyHostToDevice));
-            AF_CUDA(cudaMemcpy(s->d_ptiles[i], ptiles.data(), s->pk_n * sizeof(TileDev), cudaMemcpyHostToDevice));
+            AF_CUDA(s->d_ptab[i].alloc(s->pk_n));
+            AF_CUDA(s->d_ptiles[i].alloc(s->pk_n));
+            AF_CUDA(cudaMemcpy(s->d_ptab[i].get(), ptab.data(), s->pk_n * sizeof(StreamDev), cudaMemcpyHostToDevice));
+            AF_CUDA(cudaMemcpy(s->d_ptiles[i].get(), ptiles.data(), s->pk_n * sizeof(TileDev), cudaMemcpyHostToDevice));
         }
     }
     if (s->y_stride > (uint64_t)TILE_SAMPLES)
         return fail(AF_ERR_INVALID, "max_tick_samples too large for a session (%u frames)", s->max_tick_frames);
-    AF_CUDA(cudaMalloc(&s->d_vad, n_streams * sizeof(VadState)));
-    AF_CUDA(cudaMalloc(&s->d_energy, n_streams * s->energy_stride * sizeof(float)));
-    s->frac_cap = max_new_y + 64;
-    AF_CUDA(cudaMalloc(&s->d_frac, s->frac_cap * sizeof(float)));
-    AF_CUDA(cudaMalloc(&s->d_fmts, n_formats * sizeof(SessionFormat)));
-    AF_CUDA(cudaMemcpy(s->d_fmts, dev.data(), n_formats * sizeof(SessionFormat), cudaMemcpyHostToDevice));
+    AF_CUDA(s->d_vad.alloc(n_streams));
+    AF_CUDA(s->d_energy.alloc(n_streams * s->energy_stride));
+    AF_CUDA(s->d_frac.alloc(max_new_y + 64));
+    AF_CUDA(s->d_fmts.alloc(n_formats));
+    AF_CUDA(cudaMemcpy(s->d_fmts.get(), dev.data(), n_formats * sizeof(SessionFormat), cudaMemcpyHostToDevice));
     s->ss.resize(n_streams); s->ss_next.resize(n_streams);
     for (size_t k = 0; k < n_streams; ++k) s->ss[k].fmt = stream_format ? stream_format[k] : 0;
     s->diverged = true;                            // (af_session_reset reads each stream's format from ss)
@@ -1725,29 +1700,24 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     s->frac_host.clear();               // (scratch, not state)
     uint32_t maxT = 0, max_ny = 0, max_n = 0;
     const size_t tick_bytes = S * (sizeof(StreamTick) + sizeof(uint32_t));
+    // the fractions of every distinct plan, one slice after another (a lockstep tick has one)
+    AF_CUDA(s->d_frac.grow(per_stream && s->any_table ? S * s->max_new_y : s->max_new_y + 64));
     if (!per_stream) {
         const int rc = plan_stream(s, s->shared, n_samples[0], false, one, shared_next);
         if (rc) return rc;
         maxT = one.T; max_ny = one.n_y; max_n = n_samples[0];
     } else {
-        if (!s->d_tick) {                                        // set together: a failed allocation leaves neither
-            StreamTick *d = nullptr, *h = nullptr;
-            cudaError_t e = cudaMalloc(&d, tick_bytes);
-            if (e == cudaSuccess) e = cudaHostAlloc((void **)&h, tick_bytes, cudaHostAllocDefault);
-            if (e != cudaSuccess) {
-                if (d) cudaFree(d);
-                return fail(AF_ERR_CUDA, "allocating the tick plan: %s", cudaGetErrorString(e));
-            }
-            s->d_tick = d; s->h_tick = h;
-        }
-        if (s->any_table && s->frac_cap < S * s->max_new_y) {   // every distinct plan's fractions, one slice after another
-            float *f = nullptr;
-            AF_CUDA(cudaMalloc(&f, S * s->max_new_y * sizeof(float)));
-            cudaFree(s->d_frac);
-            s->d_frac = f; s->frac_cap = S * s->max_new_y;
+        if (!s->tick.d.get()) {                                  // set together: a failed allocation leaves neither
+            af_session::TickPlan t;
+            const size_t n = (tick_bytes + sizeof(StreamTick) - 1) / sizeof(StreamTick);
+            cudaError_t e = t.d.alloc(n);
+            if (e == cudaSuccess) e = t.h.alloc(n);
+            if (e != cudaSuccess) return fail(AF_ERR_CUDA, "allocating the tick plan: %s", cudaGetErrorString(e));
+            s->tick = std::move(t);
         }
         if (!s->diverged) s->ss.assign(S, s->shared);
-        uint32_t *Ts = reinterpret_cast<uint32_t *>(s->h_tick + S);
+        StreamTick *h_tick = s->tick.h.get();
+        uint32_t *Ts = reinterpret_cast<uint32_t *>(h_tick + S);
         size_t cap = 1;
         while (cap < 2 * S) cap <<= 1;
         s->plan_slots.assign(cap, UINT32_MAX);              // stream that planned each distinct key first
@@ -1758,17 +1728,17 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
                 if (same_plan(s->ss[j], n_samples[j], end && end[j], s->ss[k], n_samples[k], fin)) break;
             if (s->plan_slots[i] == UINT32_MAX) {
                 s->plan_slots[i] = (uint32_t)k;
-                const int rc = plan_stream(s, s->ss[k], n_samples[k], fin, s->h_tick[k], s->ss_next[k]);
+                const int rc = plan_stream(s, s->ss[k], n_samples[k], fin, h_tick[k], s->ss_next[k]);
                 if (rc) return rc;
             } else {                                             // the same plan, and the same fraction slice
-                s->h_tick[k] = s->h_tick[s->plan_slots[i]];
+                h_tick[k] = h_tick[s->plan_slots[i]];
                 s->ss_next[k] = s->ss_next[s->plan_slots[i]];
             }
-            Ts[k] = s->h_tick[k].T;
-            maxT = std::max(maxT, Ts[k]); max_ny = std::max(max_ny, s->h_tick[k].n_y); max_n = std::max(max_n, n_samples[k]);
+            Ts[k] = h_tick[k].T;
+            maxT = std::max(maxT, Ts[k]); max_ny = std::max(max_ny, h_tick[k].n_y); max_n = std::max(max_n, n_samples[k]);
         }
     }
-    if (s->frac_host.size() > s->frac_cap) return fail(AF_ERR_CAPACITY, "internal: fraction buffer overflow");
+    if (s->frac_host.size() > s->d_frac.size()) return fail(AF_ERR_CAPACITY, "internal: fraction buffer overflow");
     const bool want_pcm = cfg.write_pcm && o->pcm && max_ny;
     const bool want_lm = maxT && cfg.n_mels && o->logmel;
     const bool want_states = maxT && cfg.vad_enable && o->vad;
@@ -1782,39 +1752,34 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     uint8_t *states = nullptr; uint64_t st_stride = 0;
     if (want_lm) {
         if (mem == AF_MEM_HOST || s->packed) {                  // (packed ticks write every frame slot: internal buffer, then a strided copy)
-            if (!s->d_lm) AF_CUDA(cudaMalloc(&s->d_lm, S * s->lm_stride * sizeof(float)));
-            lm = s->d_lm; lm_stride = s->lm_stride;
+            AF_CUDA(s->d_lm.grow(S * s->lm_stride));
+            lm = s->d_lm.get(); lm_stride = s->lm_stride;
         } else { lm = o->logmel; lm_stride = o->logmel_stride; }
         if (lm_stride < (uint64_t)maxT * cfg.n_mels) return fail(AF_ERR_CAPACITY, "internal: log-mel staging too small for %u frames", maxT);
     }
     if (need_states) {
         if (mem == AF_MEM_HOST || !want_states) {
-            if (!s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));
-            states = s->d_states; st_stride = s->st_stride;
+            AF_CUDA(s->d_states.grow(S * s->st_stride));
+            states = s->d_states.get(); st_stride = s->st_stride;
         } else { states = o->vad; st_stride = o->vad_stride; }
         if (st_stride < maxT) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", maxT);
     }
-    const uint64_t wire_n = s->wire_cfg.gate ? (uint64_t)maxT * s->hop : max_ny;   // bound of this tick's payloads
-    if (s->wire && wire_n > s->wire_cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
+    const uint64_t wire_n = s->wr.cfg.gate ? (uint64_t)maxT * s->hop : max_ny;   // bound of this tick's payloads
+    if (s->wire && wire_n > s->wr.cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
     float *pcm_rows = nullptr; uint64_t pcm_rows_stride = 0;   // per-stream: the tick kernel writes each stream's PCM here
     if (want_pcm && per_stream) {
         if (mem == AF_MEM_HOST) {
             const uint64_t w = round_up(s->max_new_y, 4);
-            if (!s->d_pcm_stage) AF_CUDA(cudaMalloc(&s->d_pcm_stage, S * w * sizeof(float)));
-            pcm_rows = s->d_pcm_stage; pcm_rows_stride = w;
+            AF_CUDA(s->d_pcm_stage.grow(S * w));
+            pcm_rows = s->d_pcm_stage.get(); pcm_rows_stride = w;
         } else { pcm_rows = o->pcm; pcm_rows_stride = o->pcm_stride; }
     }
     const void *d_in = data;
     uint64_t d_in_stride_bytes = in_stride * bps;
     if (mem == AF_MEM_HOST && max_n) {
         const size_t row = round_up((uint64_t)max_n * bps, 16);
-        if (s->in_stage_bytes < row * S) {
-            if (s->d_in_stage) cudaFree(s->d_in_stage);
-            s->d_in_stage = nullptr; s->in_stage_bytes = 0;
-            AF_CUDA(cudaMalloc(&s->d_in_stage, row * S));
-            s->in_stage_bytes = row * S;
-        }
-        d_in = s->d_in_stage; d_in_stride_bytes = row;
+        AF_CUDA(s->d_in_stage.grow(row * S));
+        d_in = s->d_in_stage.get(); d_in_stride_bytes = row;
     }
 
     // From here on only CUDA failures can occur.
@@ -1824,29 +1789,29 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     if (mem == AF_MEM_HOST && max_n) {
         const uint32_t n_last = per_stream ? n_samples[S - 1] : max_n;
         const size_t rows = n_last == max_n ? S : S - 1;
-        AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage, d_in_stride_bytes, data, in_stride * bps, (size_t)max_n * bps, rows,
+        AF_CUDA(cudaMemcpy2DAsync(s->d_in_stage.get(), d_in_stride_bytes, data, in_stride * bps, (size_t)max_n * bps, rows,
                                   cudaMemcpyHostToDevice, st));
         if (rows < S && n_last)
-            AF_CUDA(cudaMemcpyAsync(static_cast<char *>(s->d_in_stage) + (S - 1) * d_in_stride_bytes,
+            AF_CUDA(cudaMemcpyAsync(s->d_in_stage.get() + (S - 1) * d_in_stride_bytes,
                                     static_cast<const char *>(data) + (S - 1) * in_stride * bps, (size_t)n_last * bps,
                                     cudaMemcpyHostToDevice, st));
     }
-    if (per_stream) AF_CUDA(cudaMemcpyAsync(s->d_tick, s->h_tick, tick_bytes, cudaMemcpyHostToDevice, st));
+    if (per_stream) AF_CUDA(cudaMemcpyAsync(s->tick.d.get(), s->tick.h.get(), tick_bytes, cudaMemcpyHostToDevice, st));
     if (!s->frac_host.empty())
-        AF_CUDA(cudaMemcpyAsync(s->d_frac, s->frac_host.data(), s->frac_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+        AF_CUDA(cudaMemcpyAsync(s->d_frac.get(), s->frac_host.data(), s->frac_host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     const int in_next = s->in_cur ^ 1, y_next = s->y_cur ^ 1;
-    const StreamTick *tab = per_stream ? s->d_tick : nullptr;
-    const uint32_t *d_T = per_stream ? reinterpret_cast<const uint32_t *>(s->d_tick + S) : nullptr;
+    const StreamTick *tab = per_stream ? s->tick.d.get() : nullptr;
+    const uint32_t *d_T = per_stream ? reinterpret_cast<const uint32_t *>(tab + S) : nullptr;
     SessionIngest ing{};
-    ing.old_buf = s->in_buf[s->in_cur]; ing.new_buf = s->in_buf[in_next]; ing.buf_stride = s->in_stride;
+    ing.old_buf = s->in_buf[s->in_cur].get(); ing.new_buf = s->in_buf[in_next].get(); ing.buf_stride = s->in_stride;
     ing.input = d_in; ing.in_stride_bytes = d_in_stride_bytes; ing.channels = s->fmts[s->shared.fmt].channels;
     ing.format = s->format;
     SessionResample rs{};
-    rs.in_buf = s->in_buf[in_next]; rs.in_stride = s->in_stride;
-    rs.p = s->shared.rec.p; rs.q = s->shared.rec.q; rs.mode = s->shared.rec.mode(); rs.frac = s->d_frac;
-    rs.y_old = s->y_buf[s->y_cur]; rs.y_new = s->y_buf[y_next]; rs.y_stride = s->y_stride;
+    rs.in_buf = s->in_buf[in_next].get(); rs.in_stride = s->in_stride;
+    rs.p = s->shared.rec.p; rs.q = s->shared.rec.q; rs.mode = s->shared.rec.mode(); rs.frac = s->d_frac.get();
+    rs.y_old = s->y_buf[s->y_cur].get(); rs.y_new = s->y_buf[y_next].get(); rs.y_stride = s->y_stride;
     if (per_stream) {
-        AF_CUDA(launch_session_tick_streams(ing, rs, tab, s->d_fmts, s->d_vad, s->d_wire_prev, pcm_rows, pcm_rows_stride, (uint32_t)S, st));
+        AF_CUDA(launch_session_tick_streams(ing, rs, tab, s->d_fmts.get(), s->d_vad.get(), s->d_wire_prev.get(), pcm_rows, pcm_rows_stride, (uint32_t)S, st));
     } else {                                                     // the fields the streams kernel takes from its descriptor
         ing.drop = one.in_drop; ing.keep = one.in_keep; ing.n_samples = one.n_samples; ing.n_new_frames = one.n_new;
         rs.data_base = one.data_base; rs.n_valid_end = one.n_valid_end; rs.n_begin = one.n_begin; rs.n_end = one.n_begin + one.n_y;
@@ -1854,7 +1819,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         AF_CUDA(launch_session_tick(ing, rs, (uint32_t)S, st));
     }
     count_launch();
-    float *ycur = s->y_buf[y_next];
+    float *ycur = s->y_buf[y_next].get();
 
     // ---- 2. PCM (lockstep: copied out of the 16 kHz rows; per-stream: written by the tick kernel), levels ----
     if (want_pcm && !per_stream)
@@ -1865,7 +1830,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         AF_CUDA(cudaMemcpy2DAsync(o->pcm, o->pcm_stride * sizeof(float), pcm_rows, pcm_rows_stride * sizeof(float),
                                   (size_t)max_ny * sizeof(float), S, cudaMemcpyDeviceToHost, st));
     if (s->levels) {
-        AF_CUDA(launch_peak(ycur + one.y_keep, s->y_stride, one.n_y, (uint32_t)S, s->d_peak, st, tab));
+        AF_CUDA(launch_peak(ycur + one.y_keep, s->y_stride, one.n_y, (uint32_t)S, s->lv.d_peak.get(), st, tab));
         count_launch();
     }
 
@@ -1875,12 +1840,12 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     if (maxT) {
         if (s->packed) {
             FusedParams P{};
-            P.streams = s->d_ptab[y_next]; P.tiles = s->d_ptiles[y_next]; P.n_tiles = s->pk_n;
+            P.streams = s->d_ptab[y_next].get(); P.tiles = s->d_ptiles[y_next].get(); P.n_tiles = s->pk_n;
             const uint64_t vrows = s->pk_rows;                  // real streams per stream of the launch
-            P.fft = cur_ctx().d_fft; P.mel = s->d_mel;
+            P.fft = cur_ctx().d_fft.get(); P.mel = s->d_mel;
             P.pcm = nullptr; P.pcm_stride = 0;
             P.logmel = lm; P.logmel_stride = lm_stride * vrows;
-            P.energy = cfg.vad_enable ? s->d_energy : nullptr; P.energy_stride = s->energy_stride * vrows;
+            P.energy = cfg.vad_enable ? s->d_energy.get() : nullptr; P.energy_stride = s->energy_stride * vrows;
             P.n_mels = lm ? cfg.n_mels : 0;
             P.do_energy = cfg.vad_enable ? 1 : 0;
             P.log_floor = cfg.log_floor;
@@ -1895,15 +1860,15 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         } else {
             EnergyJob ej{};
             ej.y = ycur; ej.y_stride = s->y_stride; ej.n_frames = d_T; ej.n_frames_all = maxT;
-            ej.frame_len = s->frame_len; ej.hop = s->hop; ej.energy = s->d_energy; ej.energy_stride = s->energy_stride;
+            ej.frame_len = s->frame_len; ej.hop = s->hop; ej.energy = s->d_energy.get(); ej.energy_stride = s->energy_stride;
             ej.n_streams = (uint32_t)S;
             AF_CUDA(launch_frame_energy(ej, st));
             count_launch();
         }
         if (cfg.vad_enable) {
             ScanJob sj{};
-            sj.energy = s->d_energy; sj.energy_stride = s->energy_stride; sj.n_frames = d_T; sj.n_frames_all = maxT;
-            sj.states = states; sj.states_stride = st_stride; sj.state_io = s->d_vad;
+            sj.energy = s->d_energy.get(); sj.energy_stride = s->energy_stride; sj.n_frames = d_T; sj.n_frames_all = maxT;
+            sj.states = states; sj.states_stride = st_stride; sj.state_io = s->d_vad.get();
             sj.final_out = mem == AF_MEM_DEVICE ? reinterpret_cast<VadState *>(o->vad_final) : nullptr;
             sj.prm = s->pipe->vad_prm; sj.n_streams = (uint32_t)S;
             AF_CUDA(launch_vad_scan(sj, st));
@@ -1920,34 +1885,34 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     }
     // every stream's detector (a restarted one is fresh), whether or not a frame completed; the scan wrote device rows
     if (cfg.vad_enable && o->vad_final && (mem == AF_MEM_HOST || !maxT))
-        AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad, S * sizeof(VadState),
+        AF_CUDA(cudaMemcpyAsync(o->vad_final, s->d_vad.get(), S * sizeof(VadState),
                                 mem == AF_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
     // ---- 4. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
     if (s->wire) {
-        const af_wire_config &wc = s->wire_cfg;
+        const af_session::Wire &wr = s->wr;
         WireJob wj{};
         wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = one.y_keep; wj.n_new = one.n_y;
         wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
-        wj.T = maxT; wj.hop = s->hop; wj.gate = wc.gate;                 // (T sizes the kept-frame list: the largest)
-        wj.prev = s->d_wire_prev;
-        wj.pcm16 = s->d_wire_pcm16; wj.pcm16_stride = s->wire_pcm16_stride;
-        wj.b64 = s->d_wire_b64; wj.b64_stride = s->wire_b64_stride;
-        wj.ticks = s->d_wire_ticks; wj.n_streams = (uint32_t)S; wj.tab = tab;
+        wj.T = maxT; wj.hop = s->hop; wj.gate = wr.cfg.gate;              // (T sizes the kept-frame list: the largest)
+        wj.prev = s->d_wire_prev.get();
+        wj.pcm16 = wr.d_pcm16.get(); wj.pcm16_stride = wr.pcm16_stride;
+        wj.b64 = wr.d_b64.get(); wj.b64_stride = wr.b64_stride;
+        wj.ticks = wr.d_ticks.get(); wj.n_streams = (uint32_t)S; wj.tab = tab;
         AF_CUDA(launch_session_wire(wj, st));
         count_launch();
-        if (wc.mem == AF_MEM_HOST && wire_n) {
-            if (wc.pcm16)
-                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_pcm16, s->wire_pcm16_stride * sizeof(int16_t), s->d_wire_pcm16,
-                                          s->wire_pcm16_stride * sizeof(int16_t), wire_n * sizeof(int16_t), S, cudaMemcpyDeviceToHost, st));
-            if (wc.base64)
-                AF_CUDA(cudaMemcpy2DAsync(s->h_wire_b64, s->wire_b64_stride, s->d_wire_b64, s->wire_b64_stride,
+        if (wr.cfg.mem == AF_MEM_HOST && wire_n) {
+            if (wr.cfg.pcm16)
+                AF_CUDA(cudaMemcpy2DAsync(wr.h_pcm16.get(), wr.pcm16_stride * sizeof(int16_t), wr.d_pcm16.get(),
+                                          wr.pcm16_stride * sizeof(int16_t), wire_n * sizeof(int16_t), S, cudaMemcpyDeviceToHost, st));
+            if (wr.cfg.base64)
+                AF_CUDA(cudaMemcpy2DAsync(wr.h_b64.get(), wr.b64_stride, wr.d_b64.get(), wr.b64_stride,
                                           af_pcm16_base64_len(wire_n), S, cudaMemcpyDeviceToHost, st));
         }
-        AF_CUDA(cudaMemcpyAsync(s->h_wire_ticks, s->d_wire_ticks, S * sizeof(af_wire_tick), cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaMemcpyAsync(wr.h_ticks.get(), wr.d_ticks.get(), S * sizeof(af_wire_tick), cudaMemcpyDeviceToHost, st));
     }
     if (s->levels) {
-        AF_CUDA(cudaMemcpyAsync(s->h_peak, s->d_peak, S * sizeof(float), cudaMemcpyDeviceToHost, st));
-        AF_CUDA(cudaMemcpyAsync(s->h_vad, s->d_vad, S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaMemcpyAsync(s->lv.h_peak.get(), s->lv.d_peak.get(), S * sizeof(float), cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaMemcpyAsync(s->lv.h_vad.get(), s->d_vad.get(), S * sizeof(VadState), cudaMemcpyDeviceToHost, st));
     }
     AF_CUDA(cudaStreamSynchronize(st));
 
@@ -1965,7 +1930,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         if (aligned) s->shared = s->ss[0];
     }
     for (size_t k = 0; k < S; ++k) {
-        const StreamTick &d = per_stream ? s->h_tick[k] : one;
+        const StreamTick &d = per_stream ? s->tick.h.get()[k] : one;
         s->first_frames[k] = (per_stream ? s->ss[k] : s->shared).frames_emitted - d.T;
         if (n_pcm) n_pcm[k] = d.n_y;
         if (n_feat) n_feat[k] = cfg.n_mels ? d.T : 0;
@@ -2057,10 +2022,12 @@ AF_API int af_session_enable_levels(af_session *s, int enable)
 {
     if (!s) return fail(AF_ERR_INVALID, "null session");
     AF_SCOPE(s->device);
-    if (enable && !s->d_peak) {
-        AF_CUDA(cudaMalloc(&s->d_peak, s->S * sizeof(float)));
-        AF_CUDA(cudaHostAlloc((void **)&s->h_peak, s->S * sizeof(float), cudaHostAllocDefault));
-        AF_CUDA(cudaHostAlloc((void **)&s->h_vad, s->S * sizeof(VadState), cudaHostAllocDefault));
+    if (enable && !s->lv.d_peak.get()) {                 // all three buffers or none
+        af_session::Levels lv;
+        AF_CUDA(lv.d_peak.alloc(s->S));
+        AF_CUDA(lv.h_peak.alloc(s->S));
+        AF_CUDA(lv.h_vad.alloc(s->S));
+        s->lv = std::move(lv);
     }
     s->levels = enable != 0;
     s->levels_valid = false;
@@ -2073,11 +2040,12 @@ AF_API int af_session_levels(const af_session *s, float *level_db, float *peak, 
     if (!s->levels_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_levels");
     const bool vad = s->pipe->cfg.vad_enable != 0;
     for (size_t k = 0; k < s->S; ++k) {
-        if (peak) peak[k] = s->h_peak[k];
+        if (peak) peak[k] = s->lv.h_peak.get()[k];
         // VoiceActivityDetector::energy_db (vad.rs:192-194) through energy_to_dbfs (vad.rs:171-176), host libm
-        const float e = vad ? s->h_vad[k].smoothed : 0.0f;
+        const VadState &v = s->lv.h_vad.get()[k];
+        const float e = vad ? v.smoothed : 0.0f;
         if (level_db) level_db[k] = e <= 0.0f ? -INFINITY : 20.0f * log10f(e);
-        if (is_speech) is_speech[k] = (vad && s->h_vad[k].state == 1) ? 1 : 0;          // is_speaking, vad.rs:197-199
+        if (is_speech) is_speech[k] = (vad && v.state == 1) ? 1 : 0;          // is_speaking, vad.rs:197-199
     }
     return AF_OK;
 }
@@ -2102,27 +2070,30 @@ AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg)
     cudaDeviceSynchronize();
     wire_free(s);
     const size_t S = s->S;
+    af_session::Wire wr;                             // the session takes the rows once all of them are allocated
+    wr.cfg = *cfg;
     // ungated: the tick's new samples; gated: the hops of at most y_stride / hop + 2 frames
-    s->wire_cap = cfg->gate ? (s->y_stride / s->hop + 2) * s->hop : s->max_new_y;
+    wr.cap = cfg->gate ? (s->y_stride / s->hop + 2) * s->hop : s->max_new_y;
     if (cfg->pcm16) {
-        s->wire_pcm16_stride = round_up(s->wire_cap, 4);
-        AF_CUDA(cudaMalloc(&s->d_wire_pcm16, S * s->wire_pcm16_stride * sizeof(int16_t)));
-        if (cfg->mem == AF_MEM_HOST)
-            AF_CUDA(cudaHostAlloc((void **)&s->h_wire_pcm16, S * s->wire_pcm16_stride * sizeof(int16_t), cudaHostAllocDefault));
+        wr.pcm16_stride = round_up(wr.cap, 4);
+        AF_CUDA(wr.d_pcm16.alloc(S * wr.pcm16_stride));
+        if (cfg->mem == AF_MEM_HOST) AF_CUDA(wr.h_pcm16.alloc(S * wr.pcm16_stride));
     }
     if (cfg->base64) {
-        s->wire_b64_stride = round_up(af_pcm16_base64_len(s->wire_cap), 4);
-        AF_CUDA(cudaMalloc(&s->d_wire_b64, S * s->wire_b64_stride));
-        if (cfg->mem == AF_MEM_HOST) AF_CUDA(cudaHostAlloc((void **)&s->h_wire_b64, S * s->wire_b64_stride, cudaHostAllocDefault));
+        wr.b64_stride = round_up(af_pcm16_base64_len(wr.cap), 4);
+        AF_CUDA(wr.d_b64.alloc(S * wr.b64_stride));
+        if (cfg->mem == AF_MEM_HOST) AF_CUDA(wr.h_b64.alloc(S * wr.b64_stride));
     }
-    AF_CUDA(cudaMalloc(&s->d_wire_ticks, S * sizeof(WireTick)));
-    AF_CUDA(cudaHostAlloc((void **)&s->h_wire_ticks, S * sizeof(af_wire_tick), cudaHostAllocDefault));
-    if (!s->d_wire_prev) {                           // the carried segment state survives a re-enable, as the detector's does
-        AF_CUDA(cudaMalloc(&s->d_wire_prev, S));
-        AF_CUDA(cudaMemset(s->d_wire_prev, 0, S));
+    AF_CUDA(wr.d_ticks.alloc(S));
+    AF_CUDA(wr.h_ticks.alloc(S));
+    if (!s->d_wire_prev.get()) {                     // the carried segment state survives a re-enable, as the detector's does
+        DevBuf<uint8_t> prev;
+        AF_CUDA(prev.alloc(S));
+        AF_CUDA(cudaMemset(prev.get(), 0, S));
+        s->d_wire_prev = std::move(prev);
     }
-    if (pc.vad_enable && !s->d_states) AF_CUDA(cudaMalloc(&s->d_states, S * s->st_stride));   // the scan's states for the kernel
-    s->wire_cfg = *cfg;
+    if (pc.vad_enable) AF_CUDA(s->d_states.grow(S * s->st_stride));   // the scan's states for the kernel
+    s->wr = std::move(wr);
     s->wire = true;
     s->wire_valid = false;
     return AF_OK;
@@ -2133,12 +2104,13 @@ AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t 
 {
     if (!s) return fail(AF_ERR_INVALID, "null session");
     if (!s->wire_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire");
-    const bool host = s->wire_cfg.mem == AF_MEM_HOST;
-    if (pcm16) *pcm16 = host ? s->h_wire_pcm16 : s->d_wire_pcm16;
-    if (pcm16_stride) *pcm16_stride = s->wire_pcm16_stride;
-    if (base64) *base64 = host ? s->h_wire_b64 : s->d_wire_b64;
-    if (base64_stride) *base64_stride = s->wire_b64_stride;
-    if (ticks) memcpy(ticks, s->h_wire_ticks, s->S * sizeof(af_wire_tick));
+    const af_session::Wire &wr = s->wr;
+    const bool host = wr.cfg.mem == AF_MEM_HOST;
+    if (pcm16) *pcm16 = host ? wr.h_pcm16.get() : wr.d_pcm16.get();
+    if (pcm16_stride) *pcm16_stride = wr.pcm16_stride;
+    if (base64) *base64 = host ? wr.h_b64.get() : wr.d_b64.get();
+    if (base64_stride) *base64_stride = wr.b64_stride;
+    if (ticks) memcpy(ticks, wr.h_ticks.get(), s->S * sizeof(af_wire_tick));
     if (first_frame) *first_frame = s->first_frames[0];
     return AF_OK;
 }
@@ -2150,8 +2122,8 @@ AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t 
 // ------------------------------------------------------------------------------------------
 struct af_ring {
     float *buf = nullptr;
+    PinnedBuf<float> pinned;                        // owns buf when it is pinned (else buf is malloc'ed)
     size_t capacity = 0;
-    bool pinned = false;
     std::mutex mu;                                  // the reference locks its Vec for every call (capture.rs:103,124,159)
     std::atomic<size_t> write_pos{0}, read_pos{0};
 };
@@ -2176,7 +2148,7 @@ AF_API int af_ring_create(size_t capacity_samples, af_ring **out)
     r->capacity = capacity_samples;
     // pinned when a device is bound (the session copies straight out of it), plain memory otherwise: the ring is a
     // host container, not a compute path
-    if (cur_device() >= 0 && cur_ctx().ready && cudaHostAlloc((void **)&r->buf, capacity_samples * sizeof(float), cudaHostAllocPortable) == cudaSuccess) r->pinned = true;
+    if (cur_device() >= 0 && cur_ctx().ready && r->pinned.alloc(capacity_samples, cudaHostAllocPortable) == cudaSuccess) r->buf = r->pinned.get();
     else {
         cudaGetLastError();
         r->buf = static_cast<float *>(malloc(capacity_samples * sizeof(float)));
@@ -2190,7 +2162,7 @@ AF_API int af_ring_create(size_t capacity_samples, af_ring **out)
 AF_API void af_ring_destroy(af_ring *r)
 {
     if (!r) return;
-    if (r->pinned) cudaFreeHost(r->buf); else free(r->buf);
+    if (!r->pinned.get()) free(r->buf);
     delete r;
 }
 
@@ -2247,16 +2219,11 @@ AF_API void af_ring_clear(af_ring *r)                                           
 static int read_rings(af_session *s, af_ring *const *rings, const uint32_t *counts, uint32_t max_count, uint64_t *stride)
 {
     *stride = round_up(std::max<uint32_t>(max_count, 4), 4);
-    if (s->ring_stage_cap < *stride * s->S) {
-        if (s->ring_stage) cudaFreeHost(s->ring_stage);
-        s->ring_stage = nullptr; s->ring_stage_cap = 0;
-        AF_CUDA(cudaHostAlloc((void **)&s->ring_stage, *stride * s->S * sizeof(float), cudaHostAllocDefault));
-        s->ring_stage_cap = *stride * s->S;
-    }
+    AF_CUDA(s->ring_stage.grow(*stride * s->S));
     for (size_t k = 0; k < s->S; ++k) {
         if (!counts[k]) continue;
         size_t got = 0;
-        const int rc = af_ring_read(rings[k], s->ring_stage + k * *stride, counts[k], &got);
+        const int rc = af_ring_read(rings[k], s->ring_stage.get() + k * *stride, counts[k], &got);
         if (rc != AF_OK || got != counts[k]) return fail(AF_ERR_INVALID, "ring %zu changed under the tick (another reader?)", k);
     }
     return AF_OK;
@@ -2283,7 +2250,7 @@ AF_API int af_session_push_rings(af_session *s, af_ring *const *rings, uint32_t 
     uint64_t stride = 0;
     const int rc = read_rings(s, rings, s->counts.data(), n_samples, &stride);
     if (rc) return rc;
-    return af_session_push(s, s->ring_stage, stride, n_samples, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
+    return af_session_push(s, s->ring_stage.get(), stride, n_samples, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
 }
 
 // AudioCapturer::read_frame(max) for every stream: each ring gives what it holds, up to max_samples, in whole frames
@@ -2304,7 +2271,7 @@ AF_API int af_session_push_rings_available(af_session *s, af_ring *const *rings,
     uint64_t stride = 0;
     const int rc = read_rings(s, rings, s->counts.data(), max_samples, &stride);
     if (rc) return rc;
-    return af_session_push_streams(s, s->ring_stage, stride, s->counts.data(), end, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
+    return af_session_push_streams(s, s->ring_stage.get(), stride, s->counts.data(), end, AF_MEM_HOST, out, n_pcm, n_feat, n_vad);
 }
 
 }  // extern "C"

@@ -64,6 +64,10 @@ AF_API uint64_t af_kernel_launch_count(void);
  * call ([role][total, t0 .. t6], roles FFT / mel / VAD / resample).  All zero unless the library
  * was built with `make STATS=1`. */
 AF_API int af_debug_pipe_stats(uint64_t out[32]);
+/* Debugging aid: the device and the pinned host allocations the library holds right now, in every object it owns
+ * (sessions, batches, detectors, rings, af_host_alloc blocks) and in its per-device caches.  Either pointer may be
+ * NULL.  Unlike cudaMemGetInfo, this counts nothing of other processes on the same GPU: a leak check. */
+AF_API int af_debug_live_allocations(uint64_t *device, uint64_t *pinned);
 
 /* pinned host memory for the host-buffer entry points (optional but much faster) */
 AF_API int af_host_alloc(void **ptr, size_t bytes);
