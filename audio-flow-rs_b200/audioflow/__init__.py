@@ -190,6 +190,8 @@ def load_library():
         "af_session_create_formats": (C.c_int, [vp, sz, C.POINTER(StreamFormatC), sz, C.POINTER(C.c_uint32), C.c_uint16,
                                                 C.POINTER(vp)]),
         "af_session_restart_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), sz]),
+        "af_batch_set_vad_configs": (C.c_int, [vp, C.POINTER(_VadConfigC)]),
+        "af_session_set_vad_configs": (C.c_int, [vp, C.POINTER(C.c_uint32), C.POINTER(_VadConfigC), sz]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -376,6 +378,19 @@ class VadConfig:
                            self.min_speech_frames)
 
 
+def _vad_config_array(cfgs):
+    """A C array of the VadConfigs `cfgs` (ValueError for anything else, or a frame count outside uint64)."""
+    cfgs = list(cfgs)
+    for i, c in enumerate(cfgs):
+        if not isinstance(c, VadConfig):
+            raise ValueError(f"config {i} is not a VadConfig")
+        for name in ("silence_timeout_frames", "min_speech_frames"):
+            v = getattr(c, name)
+            if not isinstance(v, (int, np.integer)) or not 0 <= int(v) < 1 << 64:
+                raise ValueError(f"config {i}: {name} must be an integer in [0, 2^64)")
+    return (_VadConfigC * max(len(cfgs), 1))(*[c._c() for c in cfgs])
+
+
 class VoiceActivityDetector:
     def __init__(self, config: VadConfig | None = None):
         self.config = config if config is not None else VadConfig()
@@ -555,6 +570,19 @@ class Batch:
 
     def run_device(self, o: OutputsC, cuda_stream: int = 0):
         _check(load_library().af_batch_run(self._h, C.byref(o), cuda_stream or None))
+
+    def set_vad_configs(self, cfgs):
+        """One VadConfig per stream (VoiceActivityDetector::new(config) per caller) from the next run; None: the
+        pipeline's for every stream."""
+        if not self.pipe.cfg.vad_enable:
+            raise ValueError("the pipeline runs no VAD (vad_enable == 0)")
+        if cfgs is None:
+            _check(load_library().af_batch_set_vad_configs(self._h, None))
+            return
+        cfgs = list(cfgs)
+        if len(cfgs) != self.n:
+            raise ValueError(f"{len(cfgs)} configs for {self.n} streams")
+        _check(load_library().af_batch_set_vad_configs(self._h, _vad_config_array(cfgs)))
 
     def split(self, out: dict) -> list:
         res = []
@@ -854,6 +882,22 @@ class Session:
         u32p = C.POINTER(C.c_uint32)
         _check(load_library().af_session_restart_streams(self._h, a32.ctypes.data_as(u32p), f32.ctypes.data_as(u32p), a.size))
         self.stream_format[a32] = f32
+
+    def set_vad_configs(self, ids, cfgs):
+        """Stream ids[i] decides every frame completed from the next push on under cfgs[i] (the last entry wins for a
+        stream listed twice); the detector keeps its state.  The configuration stays with the slot across resets,
+        restarts and ends."""
+        if not self.pipe.cfg.vad_enable:
+            raise ValueError("the pipeline runs no VAD (vad_enable == 0)")
+        a = np.ascontiguousarray(ids, dtype=np.int64).reshape(-1)
+        cfgs = list(cfgs)
+        if a.size != len(cfgs):
+            raise ValueError(f"{a.size} streams and {len(cfgs)} configs")
+        if a.size and (a.min() < 0 or a.max() >= self.S):
+            raise ValueError(f"stream index out of range ({self.S} streams)")
+        arr = _vad_config_array(cfgs)
+        a32 = a.astype(np.uint32)
+        _check(load_library().af_session_set_vad_configs(self._h, a32.ctypes.data_as(C.POINTER(C.c_uint32)), arr, a.size))
 
     def push_rings_available(self, rings, max_samples: int, end=None) -> dict:
         """AudioCapturer::read_frame(max) for every stream: min(max_samples, available) whole frames from each ring."""

@@ -163,17 +163,19 @@ __device__ __forceinline__ void vad_machine_word(VadMachine &m, uint32_t bits, u
     }
 }
 
-__global__ void af_vad_scan_kernel(const ScanJob J)
+// flagged_only: the launch after the parallel kernel of a job with per-stream records takes only the streams flagged seq
+__global__ void af_vad_scan_kernel(const ScanJob J, uint32_t flagged_only)
 {
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= J.n_streams) return;
+    if (flagged_only && !J.recs[s].seq) return;
     const uint32_t T = J.n_frames ? J.n_frames[s] : J.n_frames_all;
     const float *e = J.energy + (uint64_t)s * J.energy_stride;
     uint8_t *out = J.states ? J.states + (uint64_t)s * J.states_stride : nullptr;
     VadState v;
     if (J.state_io) v = J.state_io[s];
     else { v.smoothed = 0.0f; v.state = 0; v.silence_frames = 0; v.speech_frames = 0; }
-    const VadParams prm = J.prm;
+    const VadParams prm = J.recs ? J.recs[s].prm : J.prm;
     // the fast path keeps the counters in 32 bits; fall back to the plain 64-bit step when they could overflow
     const bool small = v.silence_frames < 0x40000000ull && v.speech_frames < 0x40000000ull && T < 0x40000000u &&
                        prm.silence_timeout < 0x40000000ull && prm.min_speech < 0x80000000ull;
@@ -362,13 +364,17 @@ __global__ void __launch_bounds__(SCAN_THREADS) af_vad_scan_par_kernel(const Sca
     __shared__ float s_e[SCAN_E_FLOATS];                // energies of [b0 - lead, b0 + n), padded (epad)
     __shared__ int s_bad;
     const uint32_t s = blockIdx.x, tid = threadIdx.x;
+    if (J.recs) {                                        // (uniform over the CTA: before any barrier)
+        if (J.recs[s].seq) return;                       // the sequential kernel that follows takes this stream
+        warm = J.recs[s].warm;
+    }
     const uint32_t T = J.n_frames ? J.n_frames[s] : J.n_frames_all;
     const float *e = J.energy + (uint64_t)s * J.energy_stride;
     uint8_t *out = J.states ? J.states + (uint64_t)s * J.states_stride : nullptr;
     VadState v;
     if (J.state_io) v = J.state_io[s];
     else { v.smoothed = 0.0f; v.state = 0; v.silence_frames = 0; v.speech_frames = 0; }
-    const VadParams prm = J.prm;
+    const VadParams prm = J.recs ? J.recs[s].prm : J.prm;
     const float alpha = prm.alpha, beta = __fsub_rn(1.0f, prm.alpha), e_min = prm.e_min;
     const bool use_smoothed = alpha > 0.0f;
     const uint32_t timeout = (uint32_t)prm.silence_timeout, minsp = (uint32_t)prm.min_speech;
@@ -590,9 +596,13 @@ __global__ void __launch_bounds__(SCAN_THREADS) af_vad_long_a_kernel(const ScanJ
     const uint32_t T = J.n_frames ? J.n_frames[s] : J.n_frames_all;
     const uint32_t b0 = blk * SCAN_BLOCK;
     if (b0 >= T) return;
+    if (J.recs) {
+        if (J.recs[s].seq) return;
+        warm = J.recs[s].warm;
+    }
     const LongScanView V = long_scan_view(J.scratch, J.max_frames, s);
     const float *e = J.energy + (uint64_t)s * J.energy_stride;
-    const VadParams prm = J.prm;
+    const VadParams prm = J.recs ? J.recs[s].prm : J.prm;
     const float alpha = prm.alpha, beta = __fsub_rn(1.0f, prm.alpha), e_min = prm.e_min;
     const bool use_smoothed = alpha > 0.0f;
     const uint32_t timeout = (uint32_t)prm.silence_timeout, minsp = (uint32_t)prm.min_speech;
@@ -751,11 +761,11 @@ __global__ void __launch_bounds__(SCAN_THREADS) af_vad_long_a_kernel(const ScanJ
 __global__ void __launch_bounds__(32) af_vad_long_b_kernel(const ScanJob J)
 {
     const uint32_t s = blockIdx.x, lane = threadIdx.x;
-    if (s >= J.n_streams) return;
+    if (s >= J.n_streams || (J.recs && J.recs[s].seq)) return;
     const uint32_t T = J.n_frames ? J.n_frames[s] : J.n_frames_all;
     const LongScanView V = long_scan_view(J.scratch, J.max_frames, s);
     const float *e = J.energy + (uint64_t)s * J.energy_stride;
-    const VadParams prm = J.prm;
+    const VadParams prm = J.recs ? J.recs[s].prm : J.prm;
     const float alpha = prm.alpha, beta = __fsub_rn(1.0f, prm.alpha), e_min = prm.e_min;
     const bool use_smoothed = alpha > 0.0f;
     const uint32_t timeout = (uint32_t)prm.silence_timeout, minsp = (uint32_t)prm.min_speech;
@@ -841,11 +851,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) af_vad_long_c_kernel(const ScanJ
     const uint32_t blk = blockIdx.x, s = blockIdx.y;
     const uint32_t T = J.n_frames ? J.n_frames[s] : J.n_frames_all;
     const uint32_t b0 = blk * SCAN_BLOCK;
-    if (b0 >= T || !J.states) return;
+    if (b0 >= T || !J.states || (J.recs && J.recs[s].seq)) return;
     const LongScanView V = long_scan_view(J.scratch, J.max_frames, s);
     uint8_t *out = J.states + (uint64_t)s * J.states_stride;
     const bool aligned_out = (reinterpret_cast<uintptr_t>(out) & 15) == 0;
-    const uint32_t timeout = (uint32_t)J.prm.silence_timeout, minsp = (uint32_t)J.prm.min_speech;
+    const VadParams &prm = J.recs ? J.recs[s].prm : J.prm;
+    const uint32_t timeout = (uint32_t)prm.silence_timeout, minsp = (uint32_t)prm.min_speech;
     const uint32_t n = min(SCAN_BLOCK, T - b0), n_words = (n + 31) / 32;
     for (uint32_t w = threadIdx.x; w < n_words; w += SCAN_THREADS) {
         const uint32_t *en = V.entry + 3 * (size_t)((b0 >> 5) + w);
@@ -884,28 +895,69 @@ static uint32_t scan_warmup(float alpha)
     return ((uint32_t)std::ceil(w) + 31u) & ~31u;
 }
 
+// the parallel kernel keeps its counters in 32 bits and starts every stream from a fresh detector or from a state the
+// caller vouches for; streams resumed from a saved state may hold 64-bit counters -> sequential kernel
+static bool scan_small(const VadParams &prm)
+{
+    return prm.silence_timeout < 0x40000000ull && prm.min_speech < 0x40000000ull;
+}
+
+ScanRec scan_rec(const VadParams &prm)
+{
+    ScanRec r;
+    r.prm = prm;
+    r.warm = scan_warmup(prm.alpha);
+    r.seq = (r.warm == 0 || !scan_small(prm)) ? 1u : 0u;
+    return r;
+}
+
+// the parallel kernels over all streams of the job (with per-stream records, `warm` is each record's)
+static cudaError_t launch_scan_par(const ScanJob &job, uint32_t warm, cudaStream_t st)
+{
+    if (job.scratch && job.max_frames > 2u * SCAN_BLOCK && job.max_frames < 0x40000000u) {
+        // long streams: speculative block walks in parallel, a cheap sequential carry pass, parallel expansion
+        const dim3 grid(long_scan_blocks(job.max_frames), job.n_streams);
+        af_vad_long_a_kernel<<<grid, SCAN_THREADS, 0, st>>>(job, warm);
+        af_vad_long_b_kernel<<<job.n_streams, 32, 0, st>>>(job);
+        af_vad_long_c_kernel<<<grid, SCAN_THREADS, 0, st>>>(job);
+        return cudaGetLastError();
+    }
+    af_vad_scan_par_kernel<<<job.n_streams, SCAN_THREADS, 0, st>>>(job, warm);
+    return cudaGetLastError();
+}
+
+// with per-stream records: does some stream take the parallel kernels?
+static bool scan_recs_par(const ScanJob &job)
+{
+    return job.state_io == nullptr && job.n_frames_all < 0x40000000u && job.n_seq < job.n_streams;
+}
+
+uint32_t scan_launches(const ScanJob &job)
+{
+    return job.recs && scan_recs_par(job) && job.n_seq ? 2u : 1u;
+}
+
 cudaError_t launch_vad_scan(const ScanJob &job, cudaStream_t st)
 {
     if (job.n_streams == 0) return cudaSuccess;
-    const uint32_t warm = scan_warmup(job.prm.alpha);
-    // the parallel kernel keeps its counters in 32 bits and starts every stream from a fresh detector or from a
-    // state the caller vouches for; streams resumed from a saved state may hold 64-bit counters -> sequential kernel
-    const bool small = job.prm.silence_timeout < 0x40000000ull && job.prm.min_speech < 0x40000000ull &&
-                       job.n_frames_all < 0x40000000u;
-    if (warm != 0 && small && job.state_io == nullptr) {
-        if (job.scratch && job.max_frames > 2u * SCAN_BLOCK && job.max_frames < 0x40000000u) {
-            // long streams: speculative block walks in parallel, a cheap sequential carry pass, parallel expansion
-            const dim3 grid(long_scan_blocks(job.max_frames), job.n_streams);
-            af_vad_long_a_kernel<<<grid, SCAN_THREADS, 0, st>>>(job, warm);
-            af_vad_long_b_kernel<<<job.n_streams, 32, 0, st>>>(job);
-            af_vad_long_c_kernel<<<grid, SCAN_THREADS, 0, st>>>(job);
-            return cudaGetLastError();
+    const int threads = 32;                       // sequential kernel: one warp per CTA, spread the chains over the SMs
+    const uint32_t seq_ctas = (job.n_streams + threads - 1) / threads;
+    if (job.recs) {
+        // per-stream records: one stream that needs the sequential kernel leaves the others on the parallel ones.  The
+        // parallel (or long) kernel runs over all streams and the CTAs of flagged streams exit at once; the sequential
+        // kernel follows only when some stream is flagged, and its threads for the other streams exit
+        const bool par = scan_recs_par(job);
+        if (par) {
+            const cudaError_t e = launch_scan_par(job, 0, st);
+            if (e != cudaSuccess || job.n_seq == 0) return e;
         }
-        af_vad_scan_par_kernel<<<job.n_streams, SCAN_THREADS, 0, st>>>(job, warm);
+        af_vad_scan_kernel<<<seq_ctas, threads, 0, st>>>(job, par ? 1u : 0u);
         return cudaGetLastError();
     }
-    const int threads = 32;                       // one warp per CTA: spread the chains over the SMs
-    af_vad_scan_kernel<<<(job.n_streams + threads - 1) / threads, threads, 0, st>>>(job);
+    const uint32_t warm = scan_warmup(job.prm.alpha);
+    if (warm != 0 && scan_small(job.prm) && job.n_frames_all < 0x40000000u && job.state_io == nullptr)
+        return launch_scan_par(job, warm, st);
+    af_vad_scan_kernel<<<seq_ctas, threads, 0, st>>>(job, 0u);
     return cudaGetLastError();
 }
 

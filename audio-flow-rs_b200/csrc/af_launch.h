@@ -25,6 +25,13 @@ struct EnergyJob {           // generic frame energies over a device signal
     uint32_t n_streams;
 };
 
+struct ScanRec {             // one stream's detector configuration (ScanJob::recs), 32 bytes
+    VadParams prm;
+    uint32_t warm;           // EMA warm-up of the parallel kernels, scan_warmup(prm.alpha)
+    uint32_t seq;            // 1: the stream needs the sequential kernel (warm == 0, or counters beyond the 32-bit path)
+};
+ScanRec scan_rec(const VadParams &prm);
+
 struct ScanJob {             // EMA + threshold + state machine, one stream per thread
     const float *energy; uint64_t energy_stride;
     const uint32_t *n_frames; uint32_t n_frames_all;
@@ -38,8 +45,14 @@ struct ScanJob {             // EMA + threshold + state machine, one stream per 
     // scanned by many CTAs each (launch_vad_scan picks the path)
     uint32_t max_frames;
     uint32_t *scratch;
+    // per-stream configurations (optional, device): recs[s] replaces prm for stream s; n_seq of the records have seq set.
+    // The parallel (or long) kernel runs over every stream and the sequential kernel follows for the flagged ones only
+    const ScanRec *recs;
+    uint32_t n_seq;
 };
 size_t scan_scratch_words(uint32_t max_frames);
+// kernel launches launch_vad_scan enqueues for `job`, counting the three long-stream phases as one
+uint32_t scan_launches(const ScanJob &job);
 
 struct SessionIngest {
     const float *old_buf; float *new_buf; uint64_t buf_stride;   // mono f32 input history, ping-pong
@@ -134,7 +147,7 @@ cudaError_t launch_to_mono(const float *in, uint64_t n_samples, uint32_t channel
                            cudaStream_t st);
 cudaError_t launch_resample_jobs(const ResampleJob *jobs_dev, uint32_t n_jobs, uint32_t max_outputs, cudaStream_t st);
 cudaError_t launch_frame_energy(const EnergyJob &job, cudaStream_t st);
-cudaError_t launch_vad_scan(const ScanJob &job, cudaStream_t st);
+cudaError_t launch_vad_scan(const ScanJob &job, cudaStream_t st);   // (scan_launches above)
 cudaError_t launch_pcm16(const float *in, uint64_t n, int16_t *out, cudaStream_t st);
 cudaError_t launch_pcm16_base64(const float *in, uint64_t n, char *out, cudaStream_t st);   // 4 * ceil(2 n / 3) characters
 cudaError_t launch_pcm16_rows(const float *in, uint64_t in_stride, int16_t *out, uint64_t out_stride, uint32_t width, uint32_t rows,

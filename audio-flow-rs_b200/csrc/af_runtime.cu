@@ -4,6 +4,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 
 #include "af_internal.h"
 
@@ -531,6 +532,27 @@ static VadParams make_vad_params(const af_vad_config &c)
     return p;
 }
 
+// the scan records of n configurations: the e_min bisection (vad_energy_threshold) runs once per distinct threshold
+static void make_scan_recs(const af_vad_config *cfgs, size_t n, ScanRec *out)
+{
+    std::map<uint32_t, float> e_min;                  // threshold bits -> e_min
+    for (size_t i = 0; i < n; ++i) {
+        uint32_t bits;
+        memcpy(&bits, &cfgs[i].threshold_db, sizeof(bits));
+        auto it = e_min.find(bits);
+        if (it == e_min.end()) it = e_min.emplace(bits, vad_energy_threshold(cfgs[i].threshold_db)).first;
+        VadParams p;
+        p.alpha = cfgs[i].smoothing_factor;
+        p.e_min = it->second;
+        p.silence_timeout = cfgs[i].silence_timeout_frames;
+        p.min_speech = cfgs[i].min_speech_frames;
+        out[i] = scan_rec(p);
+    }
+}
+
+static bool same_rec(const ScanRec &a, const ScanRec &b) { return memcmp(&a, &b, sizeof(ScanRec)) == 0; }
+static_assert(sizeof(ScanRec) == 32, "ScanRec has no padding: same_rec compares bytes");
+
 AF_API void af_vad_config_default(af_vad_config *cfg)
 {
     if (!cfg) return;
@@ -790,6 +812,8 @@ struct SubBatch {                     // a group of streams resident on the devi
     std::vector<size_t> in_off;       // host mode: byte offset of each stream inside the slot input buffer
     size_t in_bytes = 0;
     DevBuf<uint32_t> d_scan;          // long streams: scratch of the many-CTA VAD scan (launch_vad_scan)
+    DevBuf<ScanRec> d_recs;           // its streams' VAD records (af_batch_set_vad_configs), or empty: the pipeline's
+    uint32_t n_seq = 0;               // records of d_recs flagged for the sequential scan kernel
     bool quarters = false;            // some stream stages its input in quarter steps (f32 stereo)
     bool split = false;               // some stream is not 48 kHz mono f32 -> 16 kHz (FusedParams::split)
     uint32_t per_p = 0, per_q = 0;    // p / q of the batch's RS_TABLE streams when the output period fits the kernel's position table
@@ -919,12 +943,13 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
         sj.energy = energy; sj.energy_stride = energy_stride; sj.n_frames = sb.d_nvad.get(); sj.n_frames_all = 0;
         sj.states = vad; sj.states_stride = vad_stride; sj.state_io = nullptr; sj.final_out = vad_final;
         sj.prm = b->pipe->vad_prm; sj.n_streams = (uint32_t)sb.count;
+        sj.recs = sb.d_recs.get(); sj.n_seq = sb.n_seq;
         if (b->max_vad > 16384 && b->max_vad < 0x40000000ull) {              // long streams: many CTAs per stream
             AF_CUDA(sb.d_scan.grow(sb.count * scan_scratch_words((uint32_t)b->max_vad)));
             sj.max_frames = (uint32_t)b->max_vad; sj.scratch = sb.d_scan.get();
         }
         AF_CUDA(launch_vad_scan(sj, st));
-        count_launch();
+        count_launch(scan_launches(sj));
     }
     return AF_OK;
 }
@@ -1295,6 +1320,41 @@ AF_API int af_batch_run_host(af_batch *b, const af_outputs *o)
     return AF_OK;
 }
 
+AF_API int af_batch_set_vad_configs(af_batch *b, const af_vad_config *cfgs)
+{
+    if (!b) return fail(AF_ERR_INVALID, "null batch");
+    if (!b->pipe->cfg.vad_enable) return fail(AF_ERR_INVALID, "the pipeline runs no VAD (vad_enable == 0)");
+    AF_SCOPE(b->device);
+    const size_t S = b->streams.size();
+    const ScanRec base = scan_rec(b->pipe->vad_prm);
+    std::vector<ScanRec> recs;
+    bool custom = false;                          // some stream differs from the pipeline: the scan takes the records
+    if (cfgs && S) {
+        recs.resize(S);
+        make_scan_recs(cfgs, S, recs.data());
+        for (size_t k = 0; k < S && !custom; ++k) custom = !same_rec(recs[k], base);
+    }
+    // every sub-batch's slice is allocated before anything changes
+    std::vector<DevBuf<ScanRec>> d(b->subs.size());
+    std::vector<uint32_t> n_seq(b->subs.size(), 0);
+    if (custom)
+        for (size_t g = 0; g < b->subs.size(); ++g) {
+            const SubBatch &sb = b->subs[g];
+            AF_CUDA(d[g].alloc(sb.count));
+            for (size_t i = 0; i < sb.count; ++i) n_seq[g] += recs[sb.first + i].seq;
+        }
+    AF_CUDA(cudaDeviceSynchronize());             // runs still in flight on the caller's streams read the old slices
+    if (custom)
+        for (size_t g = 0; g < b->subs.size(); ++g)
+            AF_CUDA(cudaMemcpy(d[g].get(), recs.data() + b->subs[g].first, b->subs[g].count * sizeof(ScanRec),
+                               cudaMemcpyHostToDevice));
+    for (size_t g = 0; g < b->subs.size(); ++g) {
+        b->subs[g].d_recs = std::move(d[g]);
+        b->subs[g].n_seq = n_seq[g];
+    }
+    return AF_OK;
+}
+
 AF_API int af_pipeline_run(af_pipeline *p, const af_stream_desc *streams, size_t n_streams, const af_outputs *out)
 {
     af_batch *b = nullptr;
@@ -1408,6 +1468,12 @@ struct af_session {
     DevBuf<float> d_pcm_stage;                                 // host-mode PCM rows of a per-stream tick
     std::vector<uint32_t> counts;                              // scratch: equal counts (af_session_push), ring reads
     std::vector<uint64_t> first_frames;                        // per stream: first frame completed by the last push
+    // per-stream detector configurations (af_session_set_vad_configs), allocated by the first call: host records, their
+    // device table, the range [recs_lo, recs_hi) set since the last upload, and how many records differ from the
+    // pipeline's (0: the scan takes the pipeline's configuration, as a session that never set one)
+    PinnedBuf<ScanRec> h_recs;
+    DevBuf<ScanRec> d_recs;
+    size_t recs_lo = 0, recs_hi = 0, n_custom_recs = 0;
 };
 static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
               offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
@@ -1871,6 +1937,13 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
             sj.states = states; sj.states_stride = st_stride; sj.state_io = s->d_vad.get();
             sj.final_out = mem == AF_MEM_DEVICE ? reinterpret_cast<VadState *>(o->vad_final) : nullptr;
             sj.prm = s->pipe->vad_prm; sj.n_streams = (uint32_t)S;
+            if (s->n_custom_recs) {                              // the records set since the last upload, in one copy
+                if (s->recs_lo < s->recs_hi)
+                    AF_CUDA(cudaMemcpyAsync(s->d_recs.get() + s->recs_lo, s->h_recs.get() + s->recs_lo,
+                                            (s->recs_hi - s->recs_lo) * sizeof(ScanRec), cudaMemcpyHostToDevice, st));
+                s->recs_lo = S; s->recs_hi = 0;
+                sj.recs = s->d_recs.get();
+            }
             AF_CUDA(launch_vad_scan(sj, st));
             count_launch();
         }
@@ -1999,6 +2072,39 @@ AF_API int af_session_restart_streams(af_session *s, const uint32_t *streams, co
     const int rc = af_session_reset_streams(s, streams, n);
     if (rc) return rc;
     for (size_t i = 0; i < n; ++i) s->ss[streams[i]].fmt = format[i];   // the format of the next life
+    return AF_OK;
+}
+
+AF_API int af_session_set_vad_configs(af_session *s, const uint32_t *streams, const af_vad_config *cfgs, size_t n)
+{
+    if (!s || ((!streams || !cfgs) && n)) return fail(AF_ERR_INVALID, "null argument");
+    if (!s->pipe->cfg.vad_enable) return fail(AF_ERR_INVALID, "the pipeline runs no VAD (vad_enable == 0)");
+    for (size_t i = 0; i < n; ++i)
+        if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
+    if (!n) return AF_OK;
+    AF_SCOPE(s->device);
+    const ScanRec base = scan_rec(s->pipe->vad_prm);
+    if (!s->h_recs.get()) {                                      // both tables or neither; the first upload takes all
+        PinnedBuf<ScanRec> h;
+        DevBuf<ScanRec> d;
+        AF_CUDA(h.alloc(s->S));
+        AF_CUDA(d.alloc(s->S));
+        std::fill(h.get(), h.get() + s->S, base);
+        s->h_recs = std::move(h);
+        s->d_recs = std::move(d);
+        s->recs_lo = 0; s->recs_hi = s->S;
+    }
+    std::vector<ScanRec> recs(n);
+    make_scan_recs(cfgs, n, recs.data());
+    ScanRec *h = s->h_recs.get();
+    for (size_t i = 0; i < n; ++i) {                             // in order: the last entry for a stream wins
+        const uint32_t k = streams[i];
+        s->n_custom_recs -= same_rec(h[k], base) ? 0 : 1;
+        h[k] = recs[i];
+        s->n_custom_recs += same_rec(h[k], base) ? 0 : 1;
+        s->recs_lo = std::min<size_t>(s->recs_lo, k);
+        s->recs_hi = std::max<size_t>(s->recs_hi, (size_t)k + 1);
+    }
     return AF_OK;
 }
 

@@ -211,6 +211,13 @@ public:
         if (streams.size() != format.size()) throw std::invalid_argument("restart_streams: one format per stream");
         check(af_session_restart_streams(h_, streams.data(), format.data(), streams.size()));
     }
+    // stream streams[i] decides its frames from the next push on under cfgs[i] (VoiceActivityDetector::new(config) per
+    // caller); the detector keeps its state and the configuration stays with the slot
+    void set_vad_configs(const std::vector<uint32_t> &streams, const std::vector<af_vad_config> &cfgs)
+    {
+        if (streams.size() != cfgs.size()) throw std::invalid_argument("set_vad_configs: one configuration per stream");
+        check(af_session_set_vad_configs(h_, streams.data(), cfgs.data(), streams.size()));
+    }
 
     void enable_levels(bool on = true) { check(af_session_enable_levels(h_, on ? 1 : 0)); }
     // AudioLevel{level, peak} / VolumeLevel{level, is_speech} of the last tick, per stream

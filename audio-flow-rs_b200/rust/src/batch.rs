@@ -40,12 +40,7 @@ impl Pipeline {
         match vad {
             Some(v) => {
                 cfg.vad_enable = 1;
-                cfg.vad = ffi::af_vad_config {
-                    threshold_db: v.threshold_db,
-                    smoothing_factor: v.smoothing_factor,
-                    silence_timeout_frames: v.silence_timeout_frames as u64,
-                    min_speech_frames: v.min_speech_frames as u64,
-                };
+                cfg.vad = vad_config_c(&v);
             }
             None => cfg.vad_enable = 0,
         }
@@ -63,6 +58,27 @@ impl Pipeline {
             let rc = ffi::af_batch_counts(b, no, nf, nv);
             if rc != ffi::AF_OK { return rc; }
             ffi::af_batch_strides(b, ps, ls, vs)
+        });
+        unsafe { ffi::af_batch_destroy(b) };
+        r
+    }
+
+    /// `process` with one `VadConfig` per frame (each caller's `VoiceActivityDetector::new(config)`, vad.rs:80-88); the
+    /// pipeline needs its detector on (`vad` not `None`).
+    pub fn process_with_vad_configs(&self, frames: &[AudioFrame], vad: &[VadConfig]) -> Result<Vec<StreamResult>, AudioError> {
+        if vad.len() != frames.len() {
+            return Err(AudioError::ResamplingFailed(format!("{} frames and {} configurations", frames.len(), vad.len())));
+        }
+        let descs = descs_of(frames);
+        let cfgs: Vec<ffi::af_vad_config> = vad.iter().map(vad_config_c).collect();
+        let mut b = ptr::null_mut();
+        check(unsafe { ffi::af_batch_create(self.h, descs.as_ptr(), descs.len(), ffi::AF_MEM_HOST, &mut b) })?;
+        let r = check(unsafe { ffi::af_batch_set_vad_configs(b, cfgs.as_ptr()) }).and_then(|_| {
+            self.run(frames.len(), |out| unsafe { ffi::af_batch_run_host(b, out) }, |no, nf, nv, ps, ls, vs| unsafe {
+                let rc = ffi::af_batch_counts(b, no, nf, nv);
+                if rc != ffi::AF_OK { return rc; }
+                ffi::af_batch_strides(b, ps, ls, vs)
+            })
         });
         unsafe { ffi::af_batch_destroy(b) };
         r
@@ -107,6 +123,15 @@ impl Pipeline {
 
 impl Drop for Pipeline {
     fn drop(&mut self) { unsafe { ffi::af_pipeline_destroy(self.h) } }
+}
+
+pub(crate) fn vad_config_c(v: &VadConfig) -> ffi::af_vad_config {
+    ffi::af_vad_config {
+        threshold_db: v.threshold_db,
+        smoothing_factor: v.smoothing_factor,
+        silence_timeout_frames: v.silence_timeout_frames as u64,
+        min_speech_frames: v.min_speech_frames as u64,
+    }
 }
 
 fn state_of(s: i32) -> VadState {

@@ -137,6 +137,7 @@ extern "C" {
     pub fn af_session_create_formats(p: *mut af_pipeline, n_streams: usize, formats: *const af_stream_format, n_formats: usize,
                                      stream_format: *const u32, sample_format: u16, out: *mut *mut af_session) -> c_int;
     pub fn af_session_restart_streams(s: *mut af_session, streams: *const u32, format: *const u32, n: usize) -> c_int;
+    pub fn af_session_set_vad_configs(s: *mut af_session, streams: *const u32, cfgs: *const af_vad_config, n: usize) -> c_int;
 }
 
 extern "C" {
@@ -162,6 +163,7 @@ extern "C" {
     pub fn af_batch_counts(b: *const af_batch, n_out: *mut u32, n_feat_frames: *mut u32, n_vad_frames: *mut u32) -> c_int;
     pub fn af_batch_strides(b: *const af_batch, pcm_stride: *mut u64, logmel_stride: *mut u64, vad_stride: *mut u64) -> c_int;
     pub fn af_batch_run_host(b: *mut af_batch, out: *const af_outputs) -> c_int;
+    pub fn af_batch_set_vad_configs(b: *mut af_batch, cfgs: *const af_vad_config) -> c_int;
 
     pub fn af_sharded_batch_create(p: *mut af_pipeline, streams: *const af_stream_desc, n_streams: usize, mem: c_int,
                                    out: *mut *mut af_sharded_batch) -> c_int;

@@ -29,7 +29,7 @@
 //! Source only, like the rest of the crate (INTEGRATION.md).
 use crate::batch::Pipeline;
 use crate::ffi;
-use crate::{AudioError, RingBuffer};
+use crate::{AudioError, RingBuffer, VadConfig};
 use std::ptr;
 
 fn check(rc: i32) -> Result<(), AudioError> {
@@ -154,6 +154,17 @@ impl Session {
             return Err(AudioError::ResamplingFailed(format!("{} streams and {} formats", streams.len(), format.len())));
         }
         check(unsafe { ffi::af_session_restart_streams(self.h, streams.as_ptr(), format.as_ptr(), streams.len()) })
+    }
+
+    /// Stream `streams[i]` decides every frame from the next push on under `cfgs[i]`: each caller's
+    /// `VoiceActivityDetector::new(config)` (vad.rs:80-88).  The detector keeps its state; the configuration stays with
+    /// the slot across resets, restarts and ends.
+    pub fn set_vad_configs(&mut self, streams: &[u32], cfgs: &[VadConfig]) -> Result<(), AudioError> {
+        if streams.len() != cfgs.len() {
+            return Err(AudioError::ResamplingFailed(format!("{} streams and {} configurations", streams.len(), cfgs.len())));
+        }
+        let c: Vec<ffi::af_vad_config> = cfgs.iter().map(crate::batch::vad_config_c).collect();
+        check(unsafe { ffi::af_session_set_vad_configs(self.h, streams.as_ptr(), c.as_ptr(), streams.len()) })
     }
 
     /// The payloads of the last tick, one per stream (valid until the next push; copied out here).

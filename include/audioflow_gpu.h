@@ -228,6 +228,16 @@ AF_API int af_batch_run(af_batch *b, const af_outputs *out, void *cuda_stream);
 /* Host-buffer run (the reference-facing call): copies the streams H2D (chunked, overlapped
  * with compute), runs the pipeline and copies the requested outputs back; blocking. */
 AF_API int af_batch_run_host(af_batch *b, const af_outputs *out);
+/* Per-stream VAD configurations (VoiceActivityDetector::new(config) per caller, vad.rs:21-43, 80-88).  A stream's
+ * configuration is the af_vad_config its frames are decided under; by default the pipeline's af_pipeline_config::vad.
+ * cfgs holds one configuration per stream (af_batch_n_streams); cfgs == NULL restores the pipeline's for every stream.
+ * The configurations apply from the next af_batch_run / af_batch_run_host.  Stream k's states, energies and vad_final
+ * are bit for bit those of a one-stream batch whose pipeline has vad = cfgs[k]; PCM and log-mel do not change.  Values
+ * are accepted exactly as af_vad_create accepts them (a NaN threshold never detects speech; a smoothing factor outside
+ * [0, 1] is scanned sequentially).  A stream whose configuration needs the sequential scan does not move the others off
+ * the parallel one: such a batch enqueues one more kernel.  AF_ERR_INVALID when the pipeline has vad_enable == 0.
+ * Sharded batches: af_sharded_batch_local(b, r) is an ordinary batch; give each local rank the slice of its streams. */
+AF_API int af_batch_set_vad_configs(af_batch *b, const af_vad_config *cfgs);
 /* One-shot convenience: create + run_host + destroy. */
 AF_API int af_pipeline_run(af_pipeline *p, const af_stream_desc *streams, size_t n_streams,
                            const af_outputs *out);
@@ -490,6 +500,22 @@ AF_API int af_session_create_formats(af_pipeline *p, size_t n_streams, const af_
  * format.  A stream that ended with a flush has nothing left to discard.  A stream or format index out of range is
  * AF_ERR_INVALID, and nothing changes. */
 AF_API int af_session_restart_streams(af_session *s, const uint32_t *streams, const uint32_t *format, size_t n);
+
+/* ---- per-stream VAD configurations: every caller's VoiceActivityDetector::new(config) (vad.rs:21-43, 80-88) ----------
+ * Stream streams[i] takes the configuration cfgs[i] (a stream listed twice takes its last entry); streams not listed keep
+ * theirs, by default the pipeline's af_pipeline_config::vad.  Every frame completed by the next push and later is decided
+ * under the new configuration; frames of earlier pushes are not revisited.  The detector keeps its state (smoothed
+ * energy, state, silence and speech counters): this is the reference detector with its `config` field replaced between
+ * two detect calls.  The reference has no such setter, so this is a definition (DESIGN.md section 10).
+ * The configuration belongs to the slot: it survives af_session_reset, af_session_reset_streams,
+ * af_session_restart_streams and an end.  A caller who takes over a slot sets it before or after the restart, before
+ * the first push, and gets a fresh detector with that configuration, exactly VoiceActivityDetector::new(config).
+ * Stream k behaves exactly like a one-stream session whose pipeline has its configuration, pushed the same ticks: states,
+ * vad_final, levels, the gated wire payload and its records, af_session_wire_first_frames.  A session whose streams all
+ * have the pipeline's configuration runs exactly as one that never called this.  Values are accepted as af_vad_create
+ * accepts them.  AF_ERR_INVALID, before anything changes, when the pipeline has vad_enable == 0, for a stream index out of
+ * range and for null arrays with n > 0. */
+AF_API int af_session_set_vad_configs(af_session *s, const uint32_t *streams, const af_vad_config *cfgs, size_t n);
 
 #ifdef __cplusplus
 }
