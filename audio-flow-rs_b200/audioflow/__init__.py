@@ -192,6 +192,9 @@ def load_library():
         "af_session_restart_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), sz]),
         "af_batch_set_vad_configs": (C.c_int, [vp, C.POINTER(_VadConfigC)]),
         "af_session_set_vad_configs": (C.c_int, [vp, C.POINTER(C.c_uint32), C.POINTER(_VadConfigC), sz]),
+        "af_session_stream_record_bytes": (sz, [vp]),
+        "af_session_export_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), sz, vp, C.c_int]),
+        "af_session_import_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), vp, sz, C.POINTER(C.c_uint32), C.c_int]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -728,6 +731,19 @@ def end_flags(end, n_streams: int):
     return e
 
 
+# a stream record begins with magic, version, bytes, frame_len, hop, flags, sample_rate, channels (uint32 each;
+# StreamRecord in af_runtime.cu): import_streams reads the rate and channels to name the format a record lands in
+_REC_RATE_END = 32
+
+
+def _device_records(t, n: int, rb: int) -> int:
+    """The device address of a contiguous CUDA uint8 array [n, rb] (ValueError for anything else)."""
+    ai = t.__cuda_array_interface__
+    if np.dtype(ai["typestr"]) != np.uint8 or tuple(ai["shape"]) != (n, rb) or ai.get("strides") not in (None, (rb, 1)):
+        raise ValueError(f"device records must be a contiguous uint8 array of shape ({n}, {rb})")
+    return int(ai["data"][0])
+
+
 class Session:
     """n_streams lockstep streams with persistent device state (resampler position + residual input,
     STFT overlap, VAD).  push() takes host arrays [n_streams, n_samples] and returns per-tick outputs.
@@ -898,6 +914,66 @@ class Session:
         arr = _vad_config_array(cfgs)
         a32 = a.astype(np.uint32)
         _check(load_library().af_session_set_vad_configs(self._h, a32.ctypes.data_as(C.POINTER(C.c_uint32)), arr, a.size))
+
+    def record_bytes(self) -> int:
+        """Bytes of one stream record of this session (export_streams / import_streams)."""
+        return int(load_library().af_session_stream_record_bytes(self._h))
+
+    def _ids(self, ids, what):
+        a = np.ascontiguousarray(ids, dtype=np.int64).reshape(-1)
+        if a.size and (a.min() < 0 or a.max() >= self.S):
+            raise ValueError(f"{what} index out of range ({self.S} streams)")
+        return a.astype(np.uint32)
+
+    def export_streams(self, ids, out=None):
+        """Stream records of streams `ids`: a uint8 array [len(ids), record_bytes] on the host, or, with `out` (a CUDA
+        uint8 tensor of that shape on the session's GPU, e.g. torch's), device records written into `out`.  The session
+        does not change."""
+        a = self._ids(ids, "stream")
+        rb = self.record_bytes()
+        if out is None:
+            rec, ptr, mem = np.zeros((a.size, rb), np.uint8), None, AF_MEM_HOST
+            ptr = rec.ctypes.data
+        else:
+            rec, ptr, mem = out, _device_records(out, a.size, rb), AF_MEM_DEVICE
+        _check(load_library().af_session_export_streams(self._h, a.ctypes.data_as(C.POINTER(C.c_uint32)), a.size, ptr, mem))
+        return rec
+
+    def import_streams(self, slots, records, format_ids=None):
+        """Slot slots[i] continues the stream of records[i] (export_streams' host array, or a CUDA uint8 tensor of device
+        records on the session's GPU); the slot's previous stream is discarded.  format_ids: per record an index into
+        this session's formats with the record's rate and channel count (None: the first such format).  The slots' VAD
+        configurations come with the records."""
+        a = self._ids(slots, "slot")
+        if np.unique(a).size != a.size:
+            raise ValueError("a slot is listed twice")
+        rb = self.record_bytes()
+        device = hasattr(records, "__cuda_array_interface__")
+        if device:
+            ptr, mem = _device_records(records, a.size, rb), AF_MEM_DEVICE
+            head = np.asarray(records[:, :_REC_RATE_END].cpu()) if a.size else np.zeros((0, _REC_RATE_END), np.uint8)
+        else:
+            records = np.asarray(records)
+            if records.dtype != np.uint8 or records.shape != (a.size, rb) or not records.flags.c_contiguous:
+                raise ValueError(f"records must be a contiguous uint8 array of shape ({a.size}, {rb})")
+            ptr, mem, head = records.ctypes.data, AF_MEM_HOST, records
+        if format_ids is None:
+            # the first admitted format with the record's rate and channel count (checked again by the library)
+            rc = head[:, _REC_RATE_END - 8:_REC_RATE_END].copy().view(np.uint32).reshape(-1, 2)
+            fmt = np.array([next((j for j, f in enumerate(self.format_list) if (f[0], f[1]) == (int(r), int(c))), -1)
+                            for r, c in rc], np.int64)
+            f_arg = None
+        else:
+            fmt = np.ascontiguousarray(format_ids, dtype=np.int64).reshape(-1)
+            if fmt.size != a.size:
+                raise ValueError(f"{a.size} slots and {fmt.size} formats")
+            if fmt.size and (fmt.min() < 0 or fmt.max() >= len(self.format_list)):
+                raise ValueError(f"format index out of range ({len(self.format_list)} formats)")
+            f_arg = fmt.astype(np.uint32)
+        u32p = C.POINTER(C.c_uint32)
+        _check(load_library().af_session_import_streams(self._h, a.ctypes.data_as(u32p), ptr, a.size,
+                                                        f_arg.ctypes.data_as(u32p) if f_arg is not None else None, mem))
+        self.stream_format[a] = fmt.astype(np.uint32)
 
     def push_rings_available(self, rings, max_samples: int, end=None) -> dict:
         """AudioCapturer::read_frame(max) for every stream: min(max_samples, available) whole frames from each ring."""

@@ -1069,6 +1069,59 @@ cudaError_t launch_session_tick_streams(const SessionIngest &I, const SessionRes
     return cudaGetLastError();
 }
 
+// ---- stream records: one CTA per listed stream gathers (pack) or scatters (unpack) its device state, so that moving a
+// whole session costs one launch each way.  The pack writes every byte of the record's device part (zeros past the
+// ranges), so two exports of the same state are byte-identical ----
+__global__ void __launch_bounds__(128) af_session_pack_kernel(const RecordJob J)
+{
+    const RecordMove m = J.tab[blockIdx.x];
+    uint8_t *r = J.rec + blockIdx.x * J.rec_bytes + J.dev_off;
+    float *dst = reinterpret_cast<float *>(r + sizeof(RecordDev));
+    const float *in = J.in_buf + (uint64_t)m.slot * J.in_stride + m.in_off;
+    const float *y = J.y_buf + (uint64_t)m.slot * J.y_stride + m.y_off;
+    for (uint32_t i = threadIdx.x; i < J.n_floats; i += blockDim.x) {
+        const uint32_t j = i - REC_IN_FRAMES;
+        dst[i] = i < REC_IN_FRAMES ? (i < m.in_len ? in[i] : 0.0f) : (j < m.y_len ? y[j] : 0.0f);
+    }
+    if (threadIdx.x == 0) {
+        RecordDev d;
+        d.vad = J.vad[m.slot];
+        d.wire = J.wire_prev ? J.wire_prev[m.slot] : 0;
+        for (int i = 0; i < 7; ++i) d.pad[i] = 0;
+        *reinterpret_cast<RecordDev *>(r) = d;
+    }
+}
+
+__global__ void __launch_bounds__(128) af_session_unpack_kernel(const RecordJob J)
+{
+    const RecordMove m = J.tab[blockIdx.x];
+    const uint8_t *r = J.rec + blockIdx.x * J.rec_bytes + J.dev_off;
+    const float *src = reinterpret_cast<const float *>(r + sizeof(RecordDev));
+    float *in = J.in_buf + (uint64_t)m.slot * J.in_stride;
+    float *y = J.y_buf + (uint64_t)m.slot * J.y_stride;
+    for (uint32_t i = threadIdx.x; i < m.in_len; i += blockDim.x) in[i] = src[i];
+    for (uint32_t i = threadIdx.x; i < m.y_len; i += blockDim.x) y[i] = src[REC_IN_FRAMES + i];
+    if (threadIdx.x == 0) {
+        const RecordDev d = *reinterpret_cast<const RecordDev *>(r);
+        J.vad[m.slot] = d.vad;
+        if (J.wire_prev) J.wire_prev[m.slot] = m.wire ? d.wire : 0;
+    }
+}
+
+cudaError_t launch_session_pack(const RecordJob &job, uint32_t n, cudaStream_t st)
+{
+    if (n == 0) return cudaSuccess;
+    af_session_pack_kernel<<<n, 128, 0, st>>>(job);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_session_unpack(const RecordJob &job, uint32_t n, cudaStream_t st)
+{
+    if (n == 0) return cudaSuccess;
+    af_session_unpack_kernel<<<n, 128, 0, st>>>(job);
+    return cudaGetLastError();
+}
+
 // ---- level metering (events/mod.rs:41 AudioLevel{level, peak}): peak = max |y| over the tick's new 16 kHz samples ----
 // One warp per stream; max is order-independent, so the result is bit-exact against any reference order.
 __global__ void af_peak_kernel(const float *__restrict__ y, uint64_t y_stride, uint32_t n, uint32_t n_streams, float *__restrict__ peak,

@@ -90,6 +90,32 @@ struct StreamTick {
                                                                  // wire segment cleared first) | TICK_END
 };
 
+// stream records (af_session_export_streams / af_session_import_streams): after the host-written header, a record holds
+// RecordDev and then REC_IN_FRAMES input frames (the history and residual, at most 2 * RS_POLY + RS_CHUNK - 1) and the
+// 16 kHz carry (fewer than frame_len samples), zero-padded to the record's end.  The pack / unpack kernels move this part
+constexpr uint32_t REC_IN_FRAMES = 2 * RS_POLY + RS_CHUNK - 1;
+struct RecordDev {           // 32 bytes
+    VadState vad;
+    uint8_t wire, pad[7];    // the stream's latest completed frame state (d_wire_prev)
+};
+struct RecordMove {          // one listed stream: its slot and the ranges of its current rows
+    uint32_t slot;
+    uint32_t in_off, in_len;                         // export: in_buf row [in_off, in_off + in_len); import writes from 0
+    uint32_t y_off, y_len;                           // the same for the y_buf row
+    uint32_t wire;                                   // import: 1 take the record's wire byte, 0 no segment open
+};
+struct RecordJob {
+    const RecordMove *tab;
+    uint8_t *rec; uint64_t rec_bytes; uint32_t dev_off;   // entry i's RecordDev is at rec + i * rec_bytes + dev_off
+    uint32_t n_floats;                               // floats after RecordDev up to the record's end
+    float *in_buf; uint64_t in_stride;               // the session's current rows (in_buf[in_cur], y_buf[y_cur])
+    float *y_buf; uint64_t y_stride;
+    VadState *vad;
+    uint8_t *wire_prev;                              // (or nullptr)
+};
+cudaError_t launch_session_pack(const RecordJob &job, uint32_t n, cudaStream_t st);
+cudaError_t launch_session_unpack(const RecordJob &job, uint32_t n, cudaStream_t st);
+
 struct GateJob {             // VAD-gated compaction (all device pointers)
     const float *pcm; uint64_t pcm_stride;           // 16 kHz rows (or nullptr)
     const float *logmel; uint64_t logmel_stride;     // [frame][mel] rows (or nullptr)

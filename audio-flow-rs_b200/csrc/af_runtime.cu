@@ -1474,6 +1474,16 @@ struct af_session {
     PinnedBuf<ScanRec> h_recs;
     DevBuf<ScanRec> d_recs;
     size_t recs_lo = 0, recs_hi = 0, n_custom_recs = 0;
+    std::vector<af_vad_config> vad_cfgs;                       // the configurations h_recs was made from (a record carries one)
+    // stream records (af_session_export_streams / af_session_import_streams), grown on demand: the per-stream move table,
+    // the headers of device records, and the staging rows of host records' device parts
+    struct Transfer {
+        PinnedBuf<RecordMove> h_moves;
+        DevBuf<RecordMove> d_moves;
+        PinnedBuf<uint8_t> h_hdr;
+        DevBuf<uint8_t> stage;
+    };
+    Transfer xfer;
 };
 static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
               offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
@@ -2011,6 +2021,41 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     }
     return AF_OK;
 }
+
+// The per-stream configuration tables, allocated once: every slot starts with the pipeline's (both tables or neither;
+// the first upload takes all)
+int alloc_vad_configs(af_session *s)
+{
+    if (s->h_recs.get()) return AF_OK;
+    PinnedBuf<ScanRec> h;
+    DevBuf<ScanRec> d;
+    AF_CUDA(h.alloc(s->S));
+    AF_CUDA(d.alloc(s->S));
+    std::fill(h.get(), h.get() + s->S, scan_rec(s->pipe->vad_prm));
+    s->h_recs = std::move(h);
+    s->d_recs = std::move(d);
+    s->vad_cfgs.assign(s->S, s->pipe->cfg.vad);
+    s->recs_lo = 0; s->recs_hi = s->S;
+    return AF_OK;
+}
+
+// Stream streams[i] takes cfgs[i], in order (the last entry for a stream wins); the tables exist
+void put_vad_configs(af_session *s, const uint32_t *streams, const af_vad_config *cfgs, size_t n)
+{
+    const ScanRec base = scan_rec(s->pipe->vad_prm);
+    std::vector<ScanRec> recs(n);
+    make_scan_recs(cfgs, n, recs.data());
+    ScanRec *h = s->h_recs.get();
+    for (size_t i = 0; i < n; ++i) {
+        const uint32_t k = streams[i];
+        s->n_custom_recs -= same_rec(h[k], base) ? 0 : 1;
+        h[k] = recs[i];
+        s->vad_cfgs[k] = cfgs[i];
+        s->n_custom_recs += same_rec(h[k], base) ? 0 : 1;
+        s->recs_lo = std::min<size_t>(s->recs_lo, k);
+        s->recs_hi = std::max<size_t>(s->recs_hi, (size_t)k + 1);
+    }
+}
 }  // namespace
 
 extern "C" {
@@ -2083,28 +2128,9 @@ AF_API int af_session_set_vad_configs(af_session *s, const uint32_t *streams, co
         if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
     if (!n) return AF_OK;
     AF_SCOPE(s->device);
-    const ScanRec base = scan_rec(s->pipe->vad_prm);
-    if (!s->h_recs.get()) {                                      // both tables or neither; the first upload takes all
-        PinnedBuf<ScanRec> h;
-        DevBuf<ScanRec> d;
-        AF_CUDA(h.alloc(s->S));
-        AF_CUDA(d.alloc(s->S));
-        std::fill(h.get(), h.get() + s->S, base);
-        s->h_recs = std::move(h);
-        s->d_recs = std::move(d);
-        s->recs_lo = 0; s->recs_hi = s->S;
-    }
-    std::vector<ScanRec> recs(n);
-    make_scan_recs(cfgs, n, recs.data());
-    ScanRec *h = s->h_recs.get();
-    for (size_t i = 0; i < n; ++i) {                             // in order: the last entry for a stream wins
-        const uint32_t k = streams[i];
-        s->n_custom_recs -= same_rec(h[k], base) ? 0 : 1;
-        h[k] = recs[i];
-        s->n_custom_recs += same_rec(h[k], base) ? 0 : 1;
-        s->recs_lo = std::min<size_t>(s->recs_lo, k);
-        s->recs_hi = std::max<size_t>(s->recs_hi, (size_t)k + 1);
-    }
+    const int rc = alloc_vad_configs(s);
+    if (rc) return rc;
+    put_vad_configs(s, streams, cfgs, n);
     return AF_OK;
 }
 
@@ -2113,6 +2139,242 @@ AF_API int af_session_wire_first_frames(const af_session *s, uint64_t *first_fra
     if (!s || !first_frame) return fail(AF_ERR_INVALID, "null argument");
     if (!s->wire_valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire");
     std::copy(s->first_frames.begin(), s->first_frames.end(), first_frame);
+    return AF_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// stream records: a live stream's complete state as bytes, continued by any compatible session on any GPU
+// ------------------------------------------------------------------------------------------
+namespace {
+constexpr uint32_t REC_MAGIC = 0x53524641u;               // "AFRS"
+constexpr uint32_t REC_VERSION = 1;                       // bump with any change of the layout or of what a field means
+constexpr uint32_t REC_FRAMING = 1, REC_VAD = 2, REC_RESTART = 4, REC_WIRE = 8;
+
+// The host-written head of a record; RecordDev and the two float ranges follow (af_launch.h).  The position is copied
+// field by field, never recomputed: on table-mode rates the f64 last_index drifts from the closed form, and every later
+// output's fraction depends on its exact bits.
+struct StreamRecord {
+    uint32_t magic, version, bytes;
+    uint32_t frame_len, hop, flags;                       // framing (REC_FRAMING, REC_VAD) and state (REC_RESTART, REC_WIRE)
+    uint32_t rate, channels;
+    uint64_t last_index;                                  // RsRecurrence::last_index, the f64 bit pattern
+    uint64_t chunks, n_out;                               // RsRecurrence::chunks, n_out
+    int64_t in_base;
+    uint64_t frames_emitted;
+    uint32_t in_len, y_len;                               // the two ranges (0, 0 for a pending restart)
+    af_vad_config vad;                                    // the stream's effective configuration
+    uint32_t pad[2];                                      // 0
+};
+static_assert(sizeof(StreamRecord) % 16 == 0 && sizeof(RecordDev) == 32, "record parts keep 16-byte alignment");
+
+uint32_t framing_flags(const af_session *s)
+{
+    return (s->framing ? REC_FRAMING : 0u) | (s->pipe->cfg.vad_enable ? REC_VAD : 0u);
+}
+
+size_t record_bytes(const af_session *s)
+{
+    return round_up(sizeof(StreamRecord) + sizeof(RecordDev) + sizeof(float) * (REC_IN_FRAMES + s->frame_len), 16);
+}
+
+// the move table in pinned memory, its device copy, and (n_hdr records) the pinned headers of device records
+int reserve_transfer(af_session *s, size_t n, size_t n_hdr)
+{
+    af_session::Transfer &x = s->xfer;
+    if (n > x.h_moves.size() || n > x.d_moves.size()) {
+        AF_CUDA(x.h_moves.alloc(n));
+        AF_CUDA(x.d_moves.alloc(n));
+    }
+    AF_CUDA(x.h_hdr.grow(n_hdr * sizeof(StreamRecord)));
+    return AF_OK;
+}
+
+RecordJob record_job(af_session *s, uint8_t *rec)
+{
+    RecordJob j{};
+    j.tab = s->xfer.d_moves.get();
+    j.rec = rec; j.rec_bytes = record_bytes(s); j.dev_off = sizeof(StreamRecord);
+    j.n_floats = (uint32_t)((j.rec_bytes - sizeof(StreamRecord) - sizeof(RecordDev)) / sizeof(float));
+    j.in_buf = s->in_buf[s->in_cur].get(); j.in_stride = s->in_stride;
+    j.y_buf = s->y_buf[s->y_cur].get(); j.y_stride = s->y_stride;
+    j.vad = s->d_vad.get();
+    j.wire_prev = s->d_wire_prev.get();
+    return j;
+}
+
+// A record's header against this session: AF_OK and the format it lands in, or AF_ERR_INVALID
+int check_record(const af_session *s, const StreamRecord &r, size_t i, const uint32_t *format, uint32_t *fmt)
+{
+    if (r.magic != REC_MAGIC || r.version != REC_VERSION)
+        return fail(AF_ERR_INVALID, "record %zu: not a stream record of this library build", i);
+    if (r.bytes != record_bytes(s)) return fail(AF_ERR_INVALID, "record %zu: %u bytes, this session's are %zu", i, r.bytes, record_bytes(s));
+    if ((r.flags & (REC_FRAMING | REC_VAD)) != framing_flags(s) || r.frame_len != s->frame_len || r.hop != s->hop)
+        return fail(AF_ERR_INVALID, "record %zu: framing %u/%u (flags %u) differs from this session's %u/%u (flags %u)", i,
+                    r.frame_len, r.hop, r.flags & (REC_FRAMING | REC_VAD), s->frame_len, s->hop, framing_flags(s));
+    if (r.in_len > REC_IN_FRAMES || (r.flags & REC_FRAMING ? r.y_len >= s->frame_len : r.y_len != 0))
+        return fail(AF_ERR_INVALID, "record %zu: corrupted ranges", i);
+    if (format) {
+        if (format[i] >= s->fmts.size()) return fail(AF_ERR_INVALID, "record %zu: format index %u out of range (%zu formats)", i, format[i], s->fmts.size());
+        const af_session::Format &f = s->fmts[format[i]];
+        if (f.rate != r.rate || f.channels != r.channels)
+            return fail(AF_ERR_INVALID, "record %zu: format %u is %u Hz x %u, the record's stream %u Hz x %u", i, format[i], f.rate,
+                        f.channels, r.rate, r.channels);
+        *fmt = format[i];
+        return AF_OK;
+    }
+    for (uint32_t k = 0; k < s->fmts.size(); ++k)
+        if (s->fmts[k].rate == r.rate && s->fmts[k].channels == r.channels) { *fmt = k; return AF_OK; }
+    return fail(AF_ERR_INVALID, "record %zu: no admitted format is %u Hz x %u", i, r.rate, r.channels);
+}
+}  // namespace
+
+extern "C" {
+
+AF_API size_t af_session_stream_record_bytes(const af_session *s) { return s ? record_bytes(s) : 0; }
+
+AF_API int af_session_export_streams(af_session *s, const uint32_t *streams, size_t n, void *records, int mem)
+{
+    if (!s || ((!streams || !records) && n)) return fail(AF_ERR_INVALID, "null argument");
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    for (size_t i = 0; i < n; ++i)
+        if (streams[i] >= s->S) return fail(AF_ERR_INVALID, "stream index %u out of range (%zu streams)", streams[i], s->S);
+    if (!n) return AF_OK;
+    if (mem == AF_MEM_DEVICE && device_of_pointer(records) != s->device)
+        return fail(AF_ERR_INVALID, "device records must live on the session's GPU %d", s->device);
+    AF_SCOPE(s->device);
+    cudaStream_t st = cur_ctx().stream;
+    const size_t rb = record_bytes(s);
+    int rc = reserve_transfer(s, n, mem == AF_MEM_DEVICE ? n : 0);
+    if (rc) return rc;
+    if (mem == AF_MEM_HOST) AF_CUDA(s->xfer.stage.grow(n * rb));
+    std::vector<StreamRecord> hdr(n);
+    RecordMove *mv = s->xfer.h_moves.get();
+    for (size_t i = 0; i < n; ++i) {
+        const uint32_t k = streams[i];
+        const StreamState &c = s->diverged ? s->ss[k] : s->shared;
+        StreamRecord &r = hdr[i];
+        memset(&r, 0, sizeof(r));
+        r.magic = REC_MAGIC; r.version = REC_VERSION; r.bytes = (uint32_t)rb;
+        r.frame_len = s->frame_len; r.hop = s->hop;
+        r.flags = framing_flags(s) | (c.restart ? REC_RESTART : 0u) | (s->wire && !c.restart ? REC_WIRE : 0u);
+        r.rate = s->fmts[c.fmt].rate; r.channels = s->fmts[c.fmt].channels;
+        r.vad = s->h_recs.get() ? s->vad_cfgs[k] : s->pipe->cfg.vad;
+        mv[i] = RecordMove{k, c.in_drop, 0, c.y_drop, 0, 0};
+        if (!c.restart) {                                        // a pending restart carries its format and configuration only
+            memcpy(&r.last_index, &c.rec.last_index, sizeof(double));
+            r.chunks = c.rec.chunks; r.n_out = c.rec.n_out;
+            r.in_base = c.in_base; r.frames_emitted = c.frames_emitted;
+            r.in_len = c.in_len; r.y_len = c.y_len;
+            mv[i].in_len = c.in_len; mv[i].y_len = c.y_len;
+        }
+    }
+    uint8_t *dst = mem == AF_MEM_HOST ? s->xfer.stage.get() : static_cast<uint8_t *>(records);
+    AF_CUDA(cudaMemcpyAsync(s->xfer.d_moves.get(), mv, n * sizeof(RecordMove), cudaMemcpyHostToDevice, st));
+    AF_CUDA(launch_session_pack(record_job(s, dst), (uint32_t)n, st));
+    count_launch();
+    const size_t H = sizeof(StreamRecord);
+    if (mem == AF_MEM_HOST) {
+        AF_CUDA(cudaMemcpy2DAsync(static_cast<uint8_t *>(records) + H, rb, dst + H, rb, rb - H, n, cudaMemcpyDeviceToHost, st));
+    } else {
+        memcpy(s->xfer.h_hdr.get(), hdr.data(), n * H);
+        AF_CUDA(cudaMemcpy2DAsync(records, rb, s->xfer.h_hdr.get(), H, H, n, cudaMemcpyHostToDevice, st));
+    }
+    AF_CUDA(cudaStreamSynchronize(st));
+    if (mem == AF_MEM_HOST)
+        for (size_t i = 0; i < n; ++i) memcpy(static_cast<uint8_t *>(records) + i * rb, &hdr[i], H);
+    return AF_OK;
+}
+
+AF_API int af_session_import_streams(af_session *s, const uint32_t *slots, const void *records, size_t n,
+                                     const uint32_t *format, int mem)
+{
+    if (!s || ((!slots || !records) && n)) return fail(AF_ERR_INVALID, "null argument");
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    std::vector<uint8_t> seen(s->S, 0);
+    for (size_t i = 0; i < n; ++i) {
+        if (slots[i] >= s->S) return fail(AF_ERR_INVALID, "slot %u out of range (%zu streams)", slots[i], s->S);
+        if (seen[slots[i]]++) return fail(AF_ERR_INVALID, "slot %u listed twice", slots[i]);
+    }
+    if (!n) return AF_OK;
+    if (mem == AF_MEM_DEVICE && device_of_pointer(records) != s->device)
+        return fail(AF_ERR_INVALID, "device records must live on the session's GPU %d", s->device);
+    AF_SCOPE(s->device);
+    cudaStream_t st = cur_ctx().stream;
+    const size_t rb = record_bytes(s), H = sizeof(StreamRecord);
+    int rc = reserve_transfer(s, n, mem == AF_MEM_DEVICE ? n : 0);
+    if (rc) return rc;
+    if (mem == AF_MEM_HOST) AF_CUDA(s->xfer.stage.grow(n * rb));
+    // ---- the headers: read where they are (device records: one strided copy), every one checked before anything changes ----
+    std::vector<StreamRecord> hdr(n);
+    if (mem == AF_MEM_HOST) {
+        for (size_t i = 0; i < n; ++i) memcpy(&hdr[i], static_cast<const uint8_t *>(records) + i * rb, H);
+    } else {
+        AF_CUDA(cudaMemcpy2DAsync(s->xfer.h_hdr.get(), H, records, rb, H, n, cudaMemcpyDeviceToHost, st));
+        AF_CUDA(cudaStreamSynchronize(st));
+        memcpy(hdr.data(), s->xfer.h_hdr.get(), n * H);
+    }
+    std::vector<uint32_t> fmt(n);
+    for (size_t i = 0; i < n; ++i) {
+        rc = check_record(s, hdr[i], i, format, &fmt[i]);
+        if (rc) return rc;
+    }
+    // the configurations that travel: the tables exist once a record brings one other than the pipeline's
+    if (s->pipe->cfg.vad_enable && !s->h_recs.get()) {
+        const ScanRec base = scan_rec(s->pipe->vad_prm);
+        std::vector<ScanRec> recs(n);
+        std::vector<af_vad_config> cfgs(n);
+        for (size_t i = 0; i < n; ++i) cfgs[i] = hdr[i].vad;
+        make_scan_recs(cfgs.data(), n, recs.data());
+        for (size_t i = 0; i < n && !s->h_recs.get(); ++i)
+            if (!same_rec(recs[i], base)) {
+                rc = alloc_vad_configs(s);
+                if (rc) return rc;
+            }
+    }
+    // ---- the device part: one launch scatters every record into the slots' current rows ----
+    RecordMove *mv = s->xfer.h_moves.get();
+    for (size_t i = 0; i < n; ++i)
+        mv[i] = RecordMove{slots[i], 0, hdr[i].in_len, 0, hdr[i].y_len, (hdr[i].flags & REC_WIRE) ? 1u : 0u};
+    s->wire_valid = s->levels_valid = false;                     // the last push's outputs no longer describe these slots
+    const uint8_t *src = static_cast<const uint8_t *>(records);
+    AF_CUDA(cudaMemcpyAsync(s->xfer.d_moves.get(), mv, n * sizeof(RecordMove), cudaMemcpyHostToDevice, st));
+    if (mem == AF_MEM_HOST) {
+        AF_CUDA(cudaMemcpy2DAsync(s->xfer.stage.get() + H, rb, src + H, rb, rb - H, n, cudaMemcpyHostToDevice, st));
+        src = s->xfer.stage.get();
+    }
+    AF_CUDA(launch_session_unpack(record_job(s, const_cast<uint8_t *>(src)), (uint32_t)n, st));
+    count_launch();
+    AF_CUDA(cudaStreamSynchronize(st));
+    // ---- commit: the slots' bookkeeping, their configurations; lockstep again when every stream stands at one position ----
+    if (!s->diverged) {
+        s->ss.assign(s->S, s->shared);
+        s->diverged = true;
+    }
+    for (size_t i = 0; i < n; ++i) {
+        const StreamRecord &r = hdr[i];
+        StreamState c = fresh_stream(s, fmt[i]);
+        if (r.flags & REC_RESTART) {
+            c.restart = true;                                    // the tick kernel clears history, detector and segment
+        } else {
+            memcpy(&c.rec.last_index, &r.last_index, sizeof(double));
+            c.rec.chunks = r.chunks; c.rec.n_out = r.n_out;
+            c.in_len = r.in_len; c.in_drop = 0;
+            c.y_len = r.y_len; c.y_drop = 0;
+            c.in_base = r.in_base; c.frames_emitted = r.frames_emitted;
+        }
+        s->ss[slots[i]] = c;
+    }
+    if (s->h_recs.get()) {
+        std::vector<af_vad_config> cfgs(n);
+        for (size_t i = 0; i < n; ++i) cfgs[i] = hdr[i].vad;
+        put_vad_configs(s, slots, cfgs.data(), n);
+    }
+    bool aligned = true;
+    for (size_t k = 0; k < s->S && aligned; ++k) aligned = same_position(s->ss[k], s->ss[0]);
+    s->diverged = !aligned;
+    if (aligned) s->shared = s->ss[0];
     return AF_OK;
 }
 

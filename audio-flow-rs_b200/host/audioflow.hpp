@@ -219,6 +219,24 @@ public:
         check(af_session_set_vad_configs(h_, streams.data(), cfgs.data(), streams.size()));
     }
 
+    // stream records: the complete state of the listed streams, record_bytes() each, back to back (host memory)
+    size_t record_bytes() const { return af_session_stream_record_bytes(h_); }
+    std::vector<uint8_t> export_streams(const std::vector<uint32_t> &streams)
+    {
+        std::vector<uint8_t> records(streams.size() * record_bytes());
+        check(af_session_export_streams(h_, streams.data(), streams.size(), records.data(), AF_MEM_HOST));
+        return records;
+    }
+    // slot slots[i] continues the stream of record i (format: empty, or per record an index into this session's formats)
+    void import_streams(const std::vector<uint32_t> &slots, const std::vector<uint8_t> &records,
+                        const std::vector<uint32_t> &format = {})
+    {
+        if (records.size() != slots.size() * record_bytes()) throw std::invalid_argument("import_streams: one record per slot");
+        if (!format.empty() && format.size() != slots.size()) throw std::invalid_argument("import_streams: one format per slot");
+        check(af_session_import_streams(h_, slots.data(), records.data(), slots.size(), format.empty() ? nullptr : format.data(),
+                                        AF_MEM_HOST));
+    }
+
     void enable_levels(bool on = true) { check(af_session_enable_levels(h_, on ? 1 : 0)); }
     // AudioLevel{level, peak} / VolumeLevel{level, is_speech} of the last tick, per stream
     void levels(std::vector<float> *level_db, std::vector<float> *peak, std::vector<uint8_t> *is_speech) const

@@ -138,6 +138,10 @@ extern "C" {
                                      stream_format: *const u32, sample_format: u16, out: *mut *mut af_session) -> c_int;
     pub fn af_session_restart_streams(s: *mut af_session, streams: *const u32, format: *const u32, n: usize) -> c_int;
     pub fn af_session_set_vad_configs(s: *mut af_session, streams: *const u32, cfgs: *const af_vad_config, n: usize) -> c_int;
+    pub fn af_session_stream_record_bytes(s: *const af_session) -> usize;
+    pub fn af_session_export_streams(s: *mut af_session, streams: *const u32, n: usize, records: *mut std::os::raw::c_void, mem: c_int) -> c_int;
+    pub fn af_session_import_streams(s: *mut af_session, slots: *const u32, records: *const std::os::raw::c_void, n: usize, format: *const u32,
+                                     mem: c_int) -> c_int;
 }
 
 extern "C" {

@@ -167,6 +167,34 @@ impl Session {
         check(unsafe { ffi::af_session_set_vad_configs(self.h, streams.as_ptr(), c.as_ptr(), streams.len()) })
     }
 
+    /// Bytes of one stream record of this session.
+    pub fn record_bytes(&self) -> usize {
+        unsafe { ffi::af_session_stream_record_bytes(self.h) }
+    }
+
+    /// The complete state of `streams[i]` as record i (`record_bytes()` each, back to back): what a `Send` resampler and
+    /// detector carry to another task.  The session does not change.
+    pub fn export_streams(&mut self, streams: &[u32]) -> Result<Vec<u8>, AudioError> {
+        let mut records = vec![0u8; streams.len() * self.record_bytes()];
+        check(unsafe {
+            ffi::af_session_export_streams(self.h, streams.as_ptr(), streams.len(), records.as_mut_ptr() as *mut std::os::raw::c_void, ffi::AF_MEM_HOST)
+        })?;
+        Ok(records)
+    }
+
+    /// Slot `slots[i]` continues the stream of record i, in `format[i]` (empty: the first format with the record's rate and
+    /// channel count).  The slot's previous stream is discarded; the caller's VAD configuration comes with the record.
+    pub fn import_streams(&mut self, slots: &[u32], records: &[u8], format: &[u32]) -> Result<(), AudioError> {
+        if records.len() != slots.len() * self.record_bytes() || (!format.is_empty() && format.len() != slots.len()) {
+            return Err(AudioError::ResamplingFailed(format!("{} slots, {} record bytes, {} formats", slots.len(), records.len(),
+                                                            format.len())));
+        }
+        let f = if format.is_empty() { ptr::null() } else { format.as_ptr() };
+        check(unsafe {
+            ffi::af_session_import_streams(self.h, slots.as_ptr(), records.as_ptr() as *const std::os::raw::c_void, slots.len(), f, ffi::AF_MEM_HOST)
+        })
+    }
+
     /// The payloads of the last tick, one per stream (valid until the next push; copied out here).
     pub fn wire(&self) -> Result<Vec<WirePayload>, AudioError> {
         let mut ticks = vec![ffi::af_wire_tick::default(); self.n_streams];

@@ -517,6 +517,51 @@ AF_API int af_session_restart_streams(af_session *s, const uint32_t *streams, co
  * range and for null arrays with n > 0. */
 AF_API int af_session_set_vad_configs(af_session *s, const uint32_t *streams, const af_vad_config *cfgs, size_t n);
 
+/* ---- stream records: a live stream leaves its slot and continues in another session, on any GPU ---------------------
+ * A stream record is a self-contained byte image of one stream, written by the library: resampler position, input
+ * history and residual, the 16 kHz carry of unfinished frames, the detector, the open wire segment and the stream's VAD
+ * configuration.  The layout is private; a record is an in-memory hand-off between sessions of the same library build (it
+ * carries a version, and a different one is refused), not a storage format.
+ * Definition: export stream j of session A after some push and import the record into slot k of session B.  From then on
+ * stream k of B behaves exactly like stream j of A would have when pushed the same ticks: PCM, frame counts, VAD states,
+ * vad_final, energies, log-mel (bitwise: the same kernels compute it), the wire payload and its af_wire_tick records
+ * (`continued` counts into a segment that was open before the move), the levels and af_session_wire_first_frames (which
+ * keeps counting in the stream's own frame sequence).  B may differ from A in everything else: number of streams, GPU,
+ * list of formats, max_tick_samples bounds, sample type (the state is mono f32), whether its streams have diverged, wire
+ * and levels settings, and its pipeline's default vad.
+ * Compatibility: B's framing must equal A's -- features or VAD on at all, vad_frame_len / vad_hop as the session uses them,
+ * and vad_enable -- and B must admit a format with the record's rate and channel count.  Everything downstream of the
+ * framing (n_mels, band edges, log settings, write_pcm) is B's.
+ * The VAD configuration travels with the caller: the record holds the stream's effective af_vad_config (its own, else A's
+ * pipeline's), and the import gives the slot that configuration exactly as af_session_set_vad_configs would (a slot whose
+ * configuration equals B's pipeline's does not count as custom).  This is the one exception to "the configuration belongs
+ * to the slot": a caller who takes over a slot by an import brings their own detector.
+ * Wire state: with A's wire output on, the record carries the state of the stream's latest completed frame; otherwise the
+ * import opens no segment, as af_session_enable_wire does.
+ * A stream exported after an end or af_session_reset_streams, or before its first push, is a pending restart in its
+ * format; imported, it starts afresh at its next push.
+ * After an import, af_session_wire, af_session_levels and af_session_wire_first_frames are AF_ERR_INVALID until the next
+ * push: the last push's outputs no longer describe the imported slots.
+ * The caller frees a moved stream's old slot with af_session_reset_streams; growing a full session is importing all of
+ * its streams into a larger one.  Device records cross GPUs by the caller's own copy (cudaMemcpyPeerAsync).
+ * Both calls block until the records (export) or the slots (import) are complete.  With mem == AF_MEM_DEVICE the records
+ * live on the session's GPU, and whatever produced them on other streams must have finished. */
+/* Bytes of one stream record of this session (a multiple of 16).  Fixed for a session: it depends only on its framing. */
+AF_API size_t af_session_stream_record_bytes(const af_session *s);
+/* Snapshot: record i (records + i * record_bytes) receives the complete state of stream streams[i] (a stream may be listed
+ * twice).  The session does not change.  mem: AF_MEM_HOST (any host memory) or AF_MEM_DEVICE (on the session's GPU).
+ * AF_ERR_INVALID, before anything is written, for a stream index out of range, null arrays with n > 0 and a bad mem. */
+AF_API int af_session_export_streams(af_session *s, const uint32_t *streams, size_t n, void *records, int mem);
+/* Slot slots[i] continues the stream of record i; the slot's previous stream is discarded, as by
+ * af_session_reset_streams.  format: NULL, or per record an index into B's formats with the record's rate and channel
+ * count (NULL: the first admitted format with them).  AF_ERR_INVALID, before anything changes, for a bad magic or version,
+ * a record size other than this session's, an incompatible framing or vad_enable, a rate and channel count no format
+ * admits, a slot out of range or listed twice, an explicit format index out of range or whose rate or channels differ
+ * from the record's, null arrays with n > 0 and a bad mem.  A session whose streams all stand at one position afterwards
+ * runs its next equal-count push as the lockstep tick. */
+AF_API int af_session_import_streams(af_session *s, const uint32_t *slots, const void *records, size_t n,
+                                     const uint32_t *format, int mem);
+
 #ifdef __cplusplus
 }
 #endif
