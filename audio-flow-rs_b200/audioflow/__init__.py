@@ -195,6 +195,8 @@ def load_library():
         "af_session_stream_record_bytes": (sz, [vp]),
         "af_session_export_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), sz, vp, C.c_int]),
         "af_session_import_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), vp, sz, C.POINTER(C.c_uint32), C.c_int]),
+        "af_session_enable_wire_features": (C.c_int, [vp, C.c_int, C.c_int]),
+        "af_session_wire_features": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -783,6 +785,8 @@ class Session:
         self.max_pcm = max(L.af_resample_max_output(r, 16000, m // c + 128) + 8 for r, c, m in formats)
         self.max_T = self.max_pcm // 160 + 4
         self.wire_mem = None                            # where the wire rows live (enable_wire)
+        self.wire_gate = False
+        self.features_mem = None                        # where the wire feature rows live (enable_wire_features)
 
     def stream_channels(self) -> np.ndarray:
         """The channel count of every stream's current format."""
@@ -991,11 +995,46 @@ class Session:
         L = load_library()
         if gate is None:
             _check(L.af_session_enable_wire(self._h, None))
-            self.wire_mem = None
+            self.wire_mem, self.wire_gate, self.features_mem = None, False, None
             return
         cfg = WireConfigC(int(gate), int(pcm16), int(base64), mem)
         _check(L.af_session_enable_wire(self._h, C.byref(cfg)))
-        self.wire_mem = mem
+        self.wire_mem, self.wire_gate = mem, bool(gate)
+        self.features_mem = None                        # every enable_wire call turns the features off
+
+    def enable_wire_features(self, on: bool = True, mem: int = AF_MEM_HOST):
+        """Beside the gated wire payload, the log-mel rows of its kept frames on every push (wire_features()).  Needs
+        enable_wire(gate=True), log-mel features and the VAD on the STFT frames; mem: AF_MEM_HOST or AF_MEM_DEVICE rows.
+        on=False switches them off.  ValueError before the library is called for anything else."""
+        if not on:
+            _check(load_library().af_session_enable_wire_features(self._h, 0, AF_MEM_HOST))
+            self.features_mem = None
+            return
+        cfg = self.pipe.cfg
+        if mem not in (AF_MEM_HOST, AF_MEM_DEVICE):
+            raise ValueError(f"bad memory kind {mem}")
+        if self.wire_mem is None or not self.wire_gate:
+            raise ValueError("wire features need the gated wire output: enable_wire(gate=True) first")
+        if not cfg.n_mels or not cfg.vad_enable:
+            raise ValueError("wire features need log-mel features (n_mels) and the VAD")
+        if cfg.vad_frame_len != 0 and (cfg.vad_frame_len, cfg.vad_hop) != (400, 160):
+            raise ValueError("wire features need the VAD on the STFT frames (vad_frame_len 0 or 400 / 160)")
+        _check(load_library().af_session_enable_wire_features(self._h, 1, mem))
+        self.features_mem = mem
+
+    def wire_features(self):
+        """The wire features of the last push: (rows, n_frames).  Host rows: a list of float32 [n_frames[k], n_mels]
+        arrays, one per stream.  Device rows: (pointer, stride in floats) of the session's [n_streams][stride] rows.
+        n_frames: uint32[n_streams]."""
+        p, st = C.c_void_p(), C.c_uint64(0)
+        n = np.zeros(self.S, np.uint32)
+        _check(load_library().af_session_wire_features(self._h, C.byref(p), C.byref(st), n.ctypes.data_as(C.POINTER(C.c_uint32))))
+        if self.features_mem != AF_MEM_HOST:
+            return (p.value, int(st.value)), n
+        M = self.pipe.cfg.n_mels
+        rows = [np.ctypeslib.as_array((C.c_float * (int(n[k]) * M)).from_address(p.value + 4 * k * st.value)).reshape(-1, M).copy()
+                if n[k] else np.zeros((0, M), np.float32) for k in range(self.S)]
+        return rows, n
 
     def wire(self) -> dict:
         """The payloads of the last push: {"first_frame", "first_frames" (uint64[n_streams]: each stream's first completed

@@ -1288,6 +1288,68 @@ cudaError_t launch_session_wire(const WireJob &J, cudaStream_t st)
     return cudaGetLastError();
 }
 
+// ---- session wire features: the log-mel rows of the frames the gated wire payload keeps ----
+// One CTA per stream (grid.x), launched before af_session_wire_kernel advances `prev`.  The kept frames are listed by the
+// wire kernel's rule (Speech, or Ending right after Speech, the frame before the tick's first being `prev`), written out
+// again here so that the wire kernel's code stays as it is; the tests check on every tick that the two agree.  Kept frame
+// i's log-mel row then goes to row i of the stream's output: 16-byte loads and stores when rows and strides allow
+// (J.vec), else one float per thread.
+__global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_logmel_kernel(const WireLogmelJob J)
+{
+    extern __shared__ uint16_t s_kept[];                         // the kept frames of the tick, in order
+    __shared__ uint32_t s_warp[WIRE_THREADS / 32];
+    const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const uint8_t *st = J.states ? J.states + (uint64_t)s * J.st_stride : nullptr;
+    uint32_t T = J.tab ? J.tab[s].T : J.T;
+    if (!st) T = 0;
+    const uint32_t prev = J.prev[s];
+    uint32_t kept = 0;
+    for (uint32_t base = 0; base < T; base += WIRE_THREADS) {   // (uniform trip count: every lane takes the ballots)
+        const uint32_t f = base + t;
+        const bool valid = f < T;
+        const uint32_t cur = valid ? st[f] : 0u, pre = valid ? (f ? st[f - 1] : prev) : 0u;
+        const bool keep = valid && (cur == VAD_SPEECH || (cur == VAD_ENDING && pre == VAD_SPEECH));
+        const uint32_t bal = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        __syncthreads();
+        uint32_t off = kept, all = 0;
+#pragma unroll
+        for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { off += w < warp ? s_warp[w] : 0u; all += s_warp[w]; }
+        if (keep) s_kept[off + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)f;
+        kept += all;
+        __syncthreads();                                         // s_warp is rewritten by the next round; s_kept is complete
+    }
+    const uint32_t M = J.n_mels;
+    const float *src = J.lm + (uint64_t)s * J.lm_stride;
+    float *dst = J.out + (uint64_t)s * J.out_stride;
+    if (J.vec) {
+        const uint32_t m4 = M / 4, n = kept * m4;
+        for (uint32_t i = t; i < n; i += WIRE_THREADS) {
+            const uint32_t r = i / m4, c = 4 * (i - r * m4);
+            const float4 v = *reinterpret_cast<const float4 *>(src + (uint64_t)s_kept[r] * M + c);
+            *reinterpret_cast<float4 *>(dst + (uint64_t)r * M + c) = v;
+        }
+    } else {
+        const uint32_t n = kept * M;
+        for (uint32_t i = t; i < n; i += WIRE_THREADS) {
+            const uint32_t r = i / M;
+            dst[i] = src[(uint64_t)s_kept[r] * M + (i - r * M)];
+        }
+    }
+    if (t == 0) J.n_frames[s] = kept;
+}
+
+cudaError_t launch_session_wire_logmel(const WireLogmelJob &J, cudaStream_t st)
+{
+    if (J.n_streams == 0) return cudaSuccess;
+    WireLogmelJob j = J;
+    j.vec = J.n_mels % 4 == 0 && J.lm_stride % 4 == 0 && J.out_stride % 4 == 0 &&
+            ((reinterpret_cast<uintptr_t>(J.lm) | reinterpret_cast<uintptr_t>(J.out)) & 15) == 0;
+    const size_t smem = J.states ? ((size_t)J.T * sizeof(uint16_t) + 3) & ~(size_t)3 : 0;
+    af_session_wire_logmel_kernel<<<J.n_streams, WIRE_THREADS, smem, st>>>(j);
+    return cudaGetLastError();
+}
+
 // the same over the rows of a batch: in [rows][in_stride] f32 -> out [rows][out_stride] i16, `width` samples per row
 // (four at a time: one 16-byte load, one 8-byte store; both strides are multiples of 4)
 __global__ void af_pcm16_rows_kernel(const float *__restrict__ in, uint64_t in_stride, int16_t *__restrict__ out, uint64_t out_stride,

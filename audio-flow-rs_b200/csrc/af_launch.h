@@ -150,6 +150,21 @@ struct WireJob {             // a session tick's wire payloads (all device point
 };
 cudaError_t launch_session_wire(const WireJob &job, cudaStream_t st);
 
+struct WireLogmelJob {       // a session tick's wire features: the log-mel rows of the gated wire's kept frames (device)
+    const float *lm; uint64_t lm_stride;             // the tick's log-mel: frame f of stream s at lm[s * lm_stride + f * n_mels]
+    uint32_t n_mels;
+    const uint8_t *states; uint64_t st_stride;       // VadState of the tick's T frames (nullptr: T == 0)
+    uint32_t T;                                      // frames of every stream (the largest on a ragged tick)
+    const uint8_t *prev;                             // per stream: state of the latest completed frame before the tick
+    float *out; uint64_t out_stride;                 // stream s's kept rows, back to back, at out[s * out_stride]
+    uint32_t *n_frames;                              // per stream: kept frames
+    uint32_t n_streams;
+    const StreamTick *tab;                           // ragged tick: per-stream T (or nullptr)
+    uint32_t vec;                                    // (set by the launch: 16-byte copies)
+};
+// Must run before launch_session_wire of the same tick, which advances prev
+cudaError_t launch_session_wire_logmel(const WireLogmelJob &job, cudaStream_t st);
+
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st);

@@ -1436,6 +1436,15 @@ struct af_session {
         uint64_t cap = 0;                                                                 // payload samples a row holds
         DevBuf<WireTick> d_ticks;
         PinnedBuf<af_wire_tick> h_ticks;
+        // wire features (af_session_enable_wire_features): the kept frames' log-mel rows and their counts; no rows: off.
+        // valid: a push has filled them since they were built
+        struct Features {
+            int mem = AF_MEM_HOST;
+            DevBuf<float> d_rows; PinnedBuf<float> h_rows; uint64_t stride = 0;          // floats
+            DevBuf<uint32_t> d_n; PinnedBuf<uint32_t> h_n;
+            bool valid = false;
+        };
+        Features feat;
     };
     Wire wr;
     uint64_t max_new_y = 0;                                   // bound of the 16 kHz samples one tick produces
@@ -1818,16 +1827,19 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     const bool want_pcm = cfg.write_pcm && o->pcm && max_ny;
     const bool want_lm = maxT && cfg.n_mels && o->logmel;
     const bool want_states = maxT && cfg.vad_enable && o->vad;
-    // the wire output needs the tick's states for its events and its gate, whatever the caller asked for
+    // the wire output needs the tick's states for its events and its gate, whatever the caller asked for; its features
+    // need the tick's log-mel the same way
     const bool need_states = want_states || (s->wire && maxT && cfg.vad_enable);
+    const bool feats = s->wire && s->wr.feat.d_rows.get();
+    const bool need_lm = want_lm || (feats && maxT);
     if (want_pcm && o->pcm_stride < max_ny) return fail(AF_ERR_CAPACITY, "pcm_stride %llu too small for %u samples", (unsigned long long)o->pcm_stride, max_ny);
     if (want_lm && o->logmel_stride < (uint64_t)maxT * cfg.n_mels) return fail(AF_ERR_CAPACITY, "logmel_stride too small for %u frames", maxT);
     if (want_states && o->vad_stride < maxT) return fail(AF_ERR_CAPACITY, "vad_stride too small for %u frames", maxT);
     // internal staging buffers (allocation failures are reported before anything changes, too)
     float *lm = nullptr; uint64_t lm_stride = 0;
     uint8_t *states = nullptr; uint64_t st_stride = 0;
-    if (want_lm) {
-        if (mem == AF_MEM_HOST || s->packed) {                  // (packed ticks write every frame slot: internal buffer, then a strided copy)
+    if (need_lm) {
+        if (mem == AF_MEM_HOST || s->packed || !want_lm) {      // (packed ticks write every frame slot: internal buffer, then a strided copy)
             AF_CUDA(s->d_lm.grow(S * s->lm_stride));
             lm = s->d_lm.get(); lm_stride = s->lm_stride;
         } else { lm = o->logmel; lm_stride = o->logmel_stride; }
@@ -1957,11 +1969,11 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
             AF_CUDA(launch_vad_scan(sj, st));
             count_launch();
         }
-        if (mem == AF_MEM_DEVICE && lm && lm != o->logmel)
+        if (mem == AF_MEM_DEVICE && want_lm && lm != o->logmel)
             AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
                                       (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToDevice, st));
         if (mem == AF_MEM_HOST) {
-            if (lm) AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
+            if (want_lm) AF_CUDA(cudaMemcpy2DAsync(o->logmel, o->logmel_stride * sizeof(float), lm, lm_stride * sizeof(float),
                                               (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
             if (want_states) AF_CUDA(cudaMemcpy2DAsync(o->vad, o->vad_stride, states, st_stride, maxT, S, cudaMemcpyDeviceToHost, st));
         }
@@ -1973,6 +1985,22 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     // ---- 4. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
     if (s->wire) {
         const af_session::Wire &wr = s->wr;
+        if (feats) {                                             // before the wire kernel, which advances d_wire_prev
+            const af_session::Wire::Features &wf = wr.feat;
+            WireLogmelJob fj{};
+            fj.lm = lm; fj.lm_stride = lm_stride; fj.n_mels = cfg.n_mels;
+            fj.states = maxT ? states : nullptr; fj.st_stride = st_stride; fj.T = maxT;
+            fj.prev = s->d_wire_prev.get();
+            fj.out = wf.d_rows.get(); fj.out_stride = wf.stride; fj.n_frames = wf.d_n.get();
+            fj.n_streams = (uint32_t)S; fj.tab = tab;
+            AF_CUDA(launch_session_wire_logmel(fj, st));
+            count_launch();
+            // (the rows hold the wire's bound of frames, and wire_n <= wr.cap above bounds maxT by it)
+            if (wf.mem == AF_MEM_HOST && maxT)
+                AF_CUDA(cudaMemcpy2DAsync(wf.h_rows.get(), wf.stride * sizeof(float), wf.d_rows.get(), wf.stride * sizeof(float),
+                                          (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
+            AF_CUDA(cudaMemcpyAsync(wf.h_n.get(), wf.d_n.get(), S * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        }
         WireJob wj{};
         wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = one.y_keep; wj.n_new = one.n_y;
         wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
@@ -2003,6 +2031,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     s->in_cur = in_next; s->y_cur = y_next;
     s->levels_valid = s->levels;
     s->wire_valid = s->wire;
+    if (feats) s->wr.feat.valid = true;
     if (!per_stream) {
         s->shared = shared_next;
     } else {
@@ -2480,6 +2509,48 @@ AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t 
     if (base64_stride) *base64_stride = wr.b64_stride;
     if (ticks) memcpy(ticks, wr.h_ticks.get(), s->S * sizeof(af_wire_tick));
     if (first_frame) *first_frame = s->first_frames[0];
+    return AF_OK;
+}
+
+// ---- wire features: the log-mel rows of the gated payload's frames, rows sized for the wire's bound of frames ----
+AF_API int af_session_enable_wire_features(af_session *s, int enable, int mem)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    AF_SCOPE(s->device);
+    if (!enable) {
+        cudaDeviceSynchronize();                     // (a failed tick may still be writing the rows)
+        s->wr.feat = af_session::Wire::Features{};
+        return AF_OK;
+    }
+    const af_pipeline_config &pc = s->pipe->cfg;
+    if (!s->wire || !s->wr.cfg.gate) return fail(AF_ERR_INVALID, "wire features need the gated wire output (af_session_enable_wire, gate = 1)");
+    if (!pc.n_mels || !pc.vad_enable) return fail(AF_ERR_INVALID, "wire features need log-mel features (n_mels) and the VAD");
+    if (s->frame_len != WIN || s->hop != HOP)
+        return fail(AF_ERR_INVALID, "wire features need the VAD on the STFT frames (vad_frame_len 0 or 400 / 160)");
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    const size_t S = s->S;
+    af_session::Wire::Features f;                    // the session takes the rows once all of them are allocated
+    f.mem = mem;
+    f.stride = round_up((s->y_stride / s->hop + 2) * pc.n_mels, 4);   // the frames whose hops the gated wire rows hold
+    AF_CUDA(f.d_rows.alloc(S * f.stride));
+    if (mem == AF_MEM_HOST) AF_CUDA(f.h_rows.alloc(S * f.stride));
+    AF_CUDA(f.d_n.alloc(S));
+    AF_CUDA(f.h_n.alloc(S));
+    // (the tick's log-mel staging is grown by the tick that first needs it, before anything changes: what is allocated
+    // here is exactly what disabling releases)
+    cudaDeviceSynchronize();                        // (the rows replaced may still be written)
+    s->wr.feat = std::move(f);
+    return AF_OK;
+}
+
+AF_API int af_session_wire_features(const af_session *s, const float **rows, uint64_t *stride, uint32_t *n_frames)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    const af_session::Wire::Features &f = s->wr.feat;
+    if (!s->wire_valid || !f.valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire_features");
+    if (rows) *rows = f.mem == AF_MEM_HOST ? f.h_rows.get() : f.d_rows.get();
+    if (stride) *stride = f.stride;
+    if (n_frames) memcpy(n_frames, f.h_n.get(), s->S * sizeof(uint32_t));
     return AF_OK;
 }
 

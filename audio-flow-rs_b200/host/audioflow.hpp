@@ -146,6 +146,12 @@ struct WirePayload {
     bool in_speech = false;
 };
 struct TickCounts { std::vector<uint32_t> n_pcm, n_feat, n_vad; };
+// the log-mel rows of the gated payload's frames (af_session_wire_features)
+struct WireFeatures {
+    const float *rows = nullptr;      // host or device rows, as enable_wire_features chose; valid until the next push
+    uint64_t stride = 0;              // floats from one stream's row to the next
+    std::vector<uint32_t> n_frames;   // per stream: its row holds n_frames[k] * n_mels floats
+};
 
 class Session {
 public:
@@ -268,6 +274,16 @@ public:
             w.continued = t[k].continued; w.started = t[k].started; w.ended = t[k].ended; w.in_speech = t[k].in_speech != 0;
         }
         return out;
+    }
+    // beside the gated payload, the log-mel rows of its frames (mem AF_MEM_HOST or AF_MEM_DEVICE rows); every
+    // enable_wire / disable_wire turns them off
+    void enable_wire_features(bool on = true, int mem = AF_MEM_HOST) { check(af_session_enable_wire_features(h_, on ? 1 : 0, mem)); }
+    WireFeatures wire_features() const
+    {
+        WireFeatures f;
+        f.n_frames.resize(n_);
+        check(af_session_wire_features(h_, &f.rows, &f.stride, f.n_frames.data()));
+        return f;
     }
     // per stream: the first frame completed by the last push, in the stream's own frame sequence since its last start
     std::vector<uint64_t> wire_first_frames() const

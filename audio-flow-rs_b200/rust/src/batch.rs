@@ -119,6 +119,7 @@ impl Pipeline {
 impl Pipeline {
     /// the C handle, for the sessions of `stream.rs` built from this pipeline
     pub(crate) fn handle(&self) -> *mut ffi::af_pipeline { self.h }
+    pub(crate) fn n_mels(&self) -> usize { self.cfg.n_mels as usize }
 }
 
 impl Drop for Pipeline {

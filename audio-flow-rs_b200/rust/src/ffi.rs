@@ -134,6 +134,8 @@ extern "C" {
     pub fn af_session_push_rings_available(s: *mut af_session, rings: *const *mut af_ring, max_samples: u32, end: *const u8,
                                            out: *const af_outputs, n_pcm: *mut u32, n_feat: *mut u32, n_vad: *mut u32) -> c_int;
     pub fn af_session_wire_first_frames(s: *const af_session, first_frame: *mut u64) -> c_int;
+    pub fn af_session_enable_wire_features(s: *mut af_session, enable: c_int, mem: c_int) -> c_int;
+    pub fn af_session_wire_features(s: *const af_session, rows: *mut *const f32, stride: *mut u64, n_frames: *mut u32) -> c_int;
     pub fn af_session_create_formats(p: *mut af_pipeline, n_streams: usize, formats: *const af_stream_format, n_formats: usize,
                                      stream_format: *const u32, sample_format: u16, out: *mut *mut af_session) -> c_int;
     pub fn af_session_restart_streams(s: *mut af_session, streams: *const u32, format: *const u32, n: usize) -> c_int;

@@ -16,6 +16,14 @@
 //! }
 //! ```
 //!
+//! A server that feeds an ASR model on the same GPU takes the log-mel rows of the same speech beside the payload:
+//!
+//! ```ignore
+//! s.enable_wire_features(true)?;
+//! // after every push: stream k's payload and the feature rows of exactly its frames
+//! for (k, (p, f)) in s.wire()?.into_iter().zip(s.wire_features()?).enumerate() { /* f.logmel: f.n_frames x n_mels */ }
+//! ```
+//!
 //! Callers whose capture devices differ share one session through `Session::with_formats`; a freed slot takes a caller
 //! with another device through `restart_streams`:
 //!
@@ -58,6 +66,15 @@ pub struct WirePayload {
     pub continued: u32,
 }
 
+/// One stream's wire features of one tick: the log-mel rows of the frames its gated payload keeps (`af_session_wire_features`).
+#[derive(Debug, Clone, Default)]
+pub struct WireFeatures {
+    /// `[frame][mel]` rows, `n_frames * n_mels` floats
+    pub logmel: Vec<f32>,
+    /// kept frames: `n_frames * 160` payload samples
+    pub n_frames: u32,
+}
+
 /// Counts of one stream in one tick (`push_rings` and `push_rings_available` return one per stream).
 #[derive(Debug, Clone, Copy, Default)]
 pub struct TickCounts { pub n_pcm: u32, pub n_feat: u32, pub n_vad: u32 }
@@ -73,7 +90,7 @@ impl StreamFormat {
 
 /// `af_session`: n 16 kHz streams (lockstep, or each on its own timeline) of f32 capture, each in one of the session's
 /// formats (`new`: mono at one rate), with their state on the GPU between ticks.
-pub struct Session { h: *mut ffi::af_session, n_streams: usize }
+pub struct Session { h: *mut ffi::af_session, n_streams: usize, n_mels: usize }
 unsafe impl Send for Session {}
 
 impl Session {
@@ -82,7 +99,7 @@ impl Session {
                wire: Option<WireGate>) -> Result<Self, AudioError> {
         let mut h = ptr::null_mut();
         check(unsafe { ffi::af_session_create(pipeline.handle(), n_streams, sample_rate, 1, ffi::AF_FMT_F32, max_tick_samples, &mut h) })?;
-        Self { h, n_streams }.with_wire(wire)
+        Self { h, n_streams, n_mels: pipeline.n_mels() }.with_wire(wire)
     }
 
     /// A session of `stream_format.len()` streams that admits `formats`; stream k starts in `formats[stream_format[k]]`.
@@ -96,7 +113,7 @@ impl Session {
             ffi::af_session_create_formats(pipeline.handle(), stream_format.len(), fs.as_ptr(), fs.len(), stream_format.as_ptr(),
                                            ffi::AF_FMT_F32, &mut h)
         })?;
-        Self { h, n_streams: stream_format.len() }.with_wire(wire)
+        Self { h, n_streams: stream_format.len(), n_mels: pipeline.n_mels() }.with_wire(wire)
     }
 
     fn with_wire(self, wire: Option<WireGate>) -> Result<Self, AudioError> {
@@ -211,6 +228,23 @@ impl Session {
                 in_speech: t.in_speech != 0,
                 continued: t.continued,
             }
+        }).collect())
+    }
+
+    /// Beside the gated payload (`WireGate::Speech`), the log-mel rows of its frames on every push, in pinned host rows.
+    /// Needs log-mel features and the VAD on the STFT frames.
+    pub fn enable_wire_features(&mut self, on: bool) -> Result<(), AudioError> {
+        check(unsafe { ffi::af_session_enable_wire_features(self.h, on as i32, ffi::AF_MEM_HOST) })
+    }
+
+    /// The feature rows of the last tick, one per stream beside `wire()`'s payloads (copied out here).
+    pub fn wire_features(&self) -> Result<Vec<WireFeatures>, AudioError> {
+        let mut n = vec![0u32; self.n_streams];
+        let (mut rows, mut stride) = (ptr::null(), 0u64);
+        check(unsafe { ffi::af_session_wire_features(self.h, &mut rows, &mut stride, n.as_mut_ptr()) })?;
+        Ok(n.iter().enumerate().map(|(k, &f)| WireFeatures {
+            logmel: unsafe { std::slice::from_raw_parts(rows.add(k * stride as usize), f as usize * self.n_mels) }.to_vec(),
+            n_frames: f,
         }).collect())
     }
 

@@ -409,6 +409,26 @@ AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg);
  * array of n_streams (may be NULL).  AF_ERR_INVALID before the first push since af_session_enable_wire. */
 AF_API int af_session_wire(const af_session *s, const int16_t **pcm16, uint64_t *pcm16_stride, const char **base64,
                            uint64_t *base64_stride, af_wire_tick *ticks, uint64_t *first_frame);
+/* ---- wire features: the speech-gated log-mel rows beside the gated PCM (SURVEY 8(f) f1 on a session) ----------------
+ * With the gated wire output on (gate = 1) and its features enabled, every push also leaves, per stream, the log-mel row
+ * of every frame the gated payload keeps in this tick -- a Speech frame in a segment, or the Ending frame that closes
+ * one -- in order, n_mels floats each, back to back.  For every stream k and tick: n_frames[k] * hop == the
+ * af_wire_tick's n_samples; the rows are, bit for bit, the kept frames' rows of the tick's log-mel (what out->logmel
+ * receives; the tick computes it whether or not out->logmel is set); the segment open when the tick began owns the first
+ * continued / hop rows; and concatenated over every tick since the stream's start they are af_vad_gate's log-mel over the
+ * concatenated session log-mel and states.  Log-mel row f belongs to VAD frame f, so the VAD must run on the STFT frames
+ * (vad_frame_len 0, or 400 / 160), as for af_vad_gate.  Everything the gated payload defines holds for the rows: ends
+ * close segments, af_session_reset_streams / af_session_restart_streams drop an open one, an imported stream continues
+ * its open segment, per-stream VAD configurations decide the frames.  A stream record carries nothing more.
+ * enable != 0: mem AF_MEM_HOST (session-owned pinned rows) or AF_MEM_DEVICE (rows on the session's GPU); the rows are
+ * sized here for the session's bound of frames per tick.  AF_ERR_INVALID, and nothing changes, when the wire output is
+ * off or ungated, for n_mels == 0 or vad_enable == 0, VAD frames other than the STFT frames, or a bad mem.  enable == 0:
+ * off.  Every af_session_enable_wire call (off, or a new configuration) turns the features off as well. */
+AF_API int af_session_enable_wire_features(af_session *s, int enable, int mem);
+/* The rows of the last push: row k (stride floats apart, a multiple of 4) holds stream k's n_frames[k] * n_mels floats,
+ * valid until the next push.  n_frames: host array of n_streams (may be NULL).  AF_ERR_INVALID whenever af_session_wire
+ * is (before the first push since enabling, after an import, after a failed push) and while the features are off. */
+AF_API int af_session_wire_features(const af_session *s, const float **rows, uint64_t *stride, uint32_t *n_frames);
 
 /* ---- RingBuffer  (src-tauri/src/modules/audio/capture.rs:84-161): capture hand-off ------ */
 /* The cpal callback writes captured f32 samples, the processing task reads them.  Same semantics as the
