@@ -641,7 +641,15 @@ __device__ __forceinline__ void resample_half_fast(const FusedSmem &sm, const Rs
         return;
     }
     const uint32_t a = rt.tile_rem + (tile_off + (uint32_t)i) * s.p;
-    if (q == 1) {
+    // An integer ratio whose f64 step is not exactly p (784 kHz, 1.488 MHz) is a TABLE rate with q == 1: its fractions are
+    // not zero and may flag the tap below, so it takes resample_part_rational.  Only the split unit meets such streams (the
+    // default one runs 48 kHz mono f32 alone), and the hot kernel keeps the code it had without the test.
+#ifdef AF_FUSED_SPLIT_TU
+    constexpr bool TABLE_Q1 = true;
+#else
+    constexpr bool TABLE_Q1 = false;
+#endif
+    if (q == 1 && (!TABLE_Q1 || mode == RS_EXACT)) {
         // integer step (48 kHz -> 16 kHz): frac == 0 exactly; the cubic returns y1 bit for bit whenever y1 != 0 and
         // the taps are finite with |x| < 2 -- checked per sample, everything else takes the polynomial
         int o = rt.tile_k + (int)a - 1 - f_lo;

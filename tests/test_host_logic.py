@@ -64,7 +64,11 @@ def test_output_len_tie_chunks_441(orc):
         assert audioflow.resample_output_len(44100, 16000, n) == exp
 
 
-@pytest.mark.parametrize("rate,mode", [(48000, 1), (44100, 2), (32000, 1), (22050, 2), (8000, 1), (24000, 1), (11025, 2)])
+# 49 kHz: q = 16, a power of two, but the f64 step is not exactly 49 / 16; 784 kHz and 1.488 MHz: integer ratios (q = 1)
+# whose f64 step is not exactly p either, so their fractions are not zero (at 1.488 MHz the recurrence sits just below
+# every integer position)
+@pytest.mark.parametrize("rate,mode", [(48000, 1), (44100, 2), (32000, 1), (22050, 2), (8000, 1), (24000, 1), (11025, 2),
+                                       (49000, 2), (784000, 2), (1488000, 2)])
 def test_resample_plan_fracs_match_oracle(orc, rate, mode):
     import audioflow
     L = audioflow.load_library()
