@@ -23,6 +23,7 @@ LIB_PATH = os.environ.get("AF_GPU_LIB") or os.path.join(os.path.dirname(_HERE), 
 AF_OK, AF_ERR_INVALID, AF_ERR_RESAMPLING_FAILED, AF_ERR_CUDA, AF_ERR_NO_DEVICE, AF_ERR_CAPACITY = range(6)
 AF_FMT_F32, AF_FMT_I16 = 0, 1
 AF_MEM_DEVICE, AF_MEM_HOST = 0, 1
+AF_WIRE_PREROLL_MAX = 100
 
 
 class AudioError(Exception):
@@ -197,6 +198,8 @@ def load_library():
         "af_session_import_streams": (C.c_int, [vp, C.POINTER(C.c_uint32), vp, sz, C.POINTER(C.c_uint32), C.c_int]),
         "af_session_enable_wire_features": (C.c_int, [vp, C.c_int, C.c_int]),
         "af_session_wire_features": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
+        "af_vad_segments_preroll": (C.c_int, [vp, C.c_uint32, vp, sz, C.c_uint32, vp]),
+        "af_session_set_wire_preroll": (C.c_int, [vp, C.c_uint32]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -787,6 +790,7 @@ class Session:
         self.wire_mem = None                            # where the wire rows live (enable_wire)
         self.wire_gate = False
         self.features_mem = None                        # where the wire feature rows live (enable_wire_features)
+        self.wire_preroll = 0                           # frames of pre-roll of the gated wire (set_wire_preroll)
 
     def stream_channels(self) -> np.ndarray:
         """The channel count of every stream's current format."""
@@ -995,12 +999,13 @@ class Session:
         L = load_library()
         if gate is None:
             _check(L.af_session_enable_wire(self._h, None))
-            self.wire_mem, self.wire_gate, self.features_mem = None, False, None
+            self.wire_mem, self.wire_gate, self.features_mem, self.wire_preroll = None, False, None, 0
             return
         cfg = WireConfigC(int(gate), int(pcm16), int(base64), mem)
         _check(L.af_session_enable_wire(self._h, C.byref(cfg)))
         self.wire_mem, self.wire_gate = mem, bool(gate)
         self.features_mem = None                        # every enable_wire call turns the features off
+        self.wire_preroll = 0                           # ... and sets the pre-roll back to 0
 
     def enable_wire_features(self, on: bool = True, mem: int = AF_MEM_HOST):
         """Beside the gated wire payload, the log-mel rows of its kept frames on every push (wire_features()).  Needs
@@ -1008,7 +1013,7 @@ class Session:
         on=False switches them off.  ValueError before the library is called for anything else."""
         if not on:
             _check(load_library().af_session_enable_wire_features(self._h, 0, AF_MEM_HOST))
-            self.features_mem = None
+            self.features_mem, self.wire_preroll = None, 0
             return
         cfg = self.pipe.cfg
         if mem not in (AF_MEM_HOST, AF_MEM_DEVICE):
@@ -1020,7 +1025,21 @@ class Session:
         if cfg.vad_frame_len != 0 and (cfg.vad_frame_len, cfg.vad_hop) != (400, 160):
             raise ValueError("wire features need the VAD on the STFT frames (vad_frame_len 0 or 400 / 160)")
         _check(load_library().af_session_enable_wire_features(self._h, 1, mem))
-        self.features_mem = mem
+        self.features_mem, self.wire_preroll = mem, 0
+
+    def set_wire_preroll(self, frames: int):
+        """Every speech segment of the gated payload (and of the wire features) reaches back up to `frames` frames
+        before its onset, never into the previous segment or before the stream's origin; the next push is every stream's
+        origin.  0 to AF_WIRE_PREROLL_MAX; 0 switches it off.  Needs enable_wire(gate=True); enable_wire and
+        enable_wire_features set it back to 0, so set it last.  ValueError before the library is called otherwise."""
+        if isinstance(frames, bool) or not isinstance(frames, (int, np.integer)):
+            raise ValueError(f"pre-roll frames must be an integer, not {frames!r}")
+        if not 0 <= frames <= AF_WIRE_PREROLL_MAX:
+            raise ValueError(f"pre-roll of {frames} frames (0 to {AF_WIRE_PREROLL_MAX})")
+        if self.wire_mem is None or not self.wire_gate:
+            raise ValueError("the pre-roll needs the gated wire output: enable_wire(gate=True) first")
+        _check(load_library().af_session_set_wire_preroll(self._h, int(frames)))
+        self.wire_preroll = int(frames)
 
     def wire_features(self):
         """The wire features of the last push: (rows, n_frames).  Host rows: a list of float32 [n_frames[k], n_mels]

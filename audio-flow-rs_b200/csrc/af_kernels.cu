@@ -1350,6 +1350,181 @@ cudaError_t launch_session_wire_logmel(const WireLogmelJob &J, cudaStream_t st)
     return cudaGetLastError();
 }
 
+// ---- session wire pre-roll: every segment the gated payload starts reaches back up to P frames ----
+// One CTA per stream (grid.x), launched after the scan instead of the features and wire kernels.  Frames are numbered
+// virtually: v < h is the v-th oldest of the h history frames (the frames after the stream's last kept frame, since its
+// origin, at most P), v >= h is the tick's frame v - h.  A kept frame's predecessor is kept unless it starts a segment, so
+// a frame is in the payload exactly when a kept frame of the tick lies within [v, v + P]: the kept frames themselves and
+// the pre-roll of every segment start, clamped at the previous kept frame and the origin by what the history holds.
+// (1) the kept bits and the events, by the wire kernel's rule; (2) the payload's frames, ballots and a block scan;
+// (3) PCM16, base64, log-mel rows and the record, pre-roll frames of earlier pushes read from the history; (4) after a
+// barrier, the tick's frames after its last kept frame (all of them if none is kept) go into the history.
+__device__ __forceinline__ bool any_kept(const uint32_t *bits, int32_t lo, int32_t hi)   // a kept frame in [lo, hi)?
+{
+    if (lo >= hi) return false;
+    const uint32_t w0 = (uint32_t)lo >> 5, w1 = (uint32_t)(hi - 1) >> 5;
+    for (uint32_t w = w0; w <= w1; ++w) {
+        uint32_t b = bits[w];
+        if (w == w0) b &= 0xffffffffu << (lo & 31);
+        if (w == w1) b &= 0xffffffffu >> (31 - ((hi - 1) & 31));
+        if (b) return true;
+    }
+    return false;
+}
+// payload sample i as PCM16: history frames were stored encoded, tick frames are encoded here (head: the ring slot of
+// the oldest history frame)
+__device__ __forceinline__ uint32_t preroll_sample(const WirePrerollJob &J, const float *row, const int16_t *hist,
+                                                   const uint16_t *list, uint32_t h, uint32_t head, uint32_t i)
+{
+    const uint32_t v = list[i / J.hop], j = i % J.hop;
+    if (v < h) return (uint32_t)(uint16_t)hist[((head + v) % J.P) * J.hop + j];
+    return pcm16_of(row[(v - h) * J.hop + j]);
+}
+__global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_preroll_kernel(const WirePrerollJob J)
+{
+    extern __shared__ uint32_t s_dyn[];
+    const uint32_t n_words = (J.T + 31) / 32;
+    uint32_t *s_bits = s_dyn;                                    // bit f % 32 of word f / 32: tick frame f is kept
+    uint16_t *s_list = reinterpret_cast<uint16_t *>(s_dyn + n_words);   // the payload's frames, virtual, in order
+    __shared__ uint32_t s_warp[WIRE_THREADS / 32];
+    __shared__ uint32_t s_break;                                 // first frame that is not Speech (T if none)
+    __shared__ int32_t s_last;                                   // last kept frame of the tick (-1 if none)
+    const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const float *row = J.y + (uint64_t)s * J.y_stride;
+    const uint8_t *st = J.states ? J.states + (uint64_t)s * J.st_stride : nullptr;
+    uint32_t T = J.T;
+    bool end = false, restart = false;
+    if (J.tab) { T = J.tab[s].T; end = (J.tab[s].flags & TICK_END) != 0; restart = (J.tab[s].flags & TICK_RESTART) != 0; }
+    if (!st) T = 0;
+    const uint32_t prev = J.prev[s], P = J.P, hop = J.hop;
+    const uint32_t h = restart ? 0u : J.hist_n[s], pos = J.hist_pos[s];
+    const uint32_t head = (pos + P - h) % P;
+    if (t == 0) { s_break = T; s_last = -1; }
+    __syncthreads();
+    uint32_t started = 0, ended = 0;
+    for (uint32_t base = 0; base < T; base += WIRE_THREADS) {   // (uniform trip count: every lane takes the ballots)
+        const uint32_t f = base + t;
+        const bool valid = f < T;
+        const uint32_t cur = valid ? st[f] : 0u, pre = valid ? (f ? st[f - 1] : prev) : 0u;
+        const bool sp = cur == VAD_SPEECH, psp = pre == VAD_SPEECH;
+        const bool keep = valid && (sp || (cur == VAD_ENDING && psp));
+        if (valid && !sp) atomicMin(&s_break, f);
+        if (keep) atomicMax(&s_last, (int32_t)f);
+        const uint32_t bal = __ballot_sync(0xffffffffu, keep);
+        const uint32_t w = (base >> 5) + warp;
+        if (lane == 0 && w < n_words) s_bits[w] = bal;
+        started += __syncthreads_count(valid && sp && !psp);    // (the barriers also publish s_bits, s_last, s_break)
+        ended += __syncthreads_count(valid && psp && !sp);
+    }
+    const uint32_t V = h + T;
+    uint32_t n_list = 0;
+    for (uint32_t base = 0; base < V; base += WIRE_THREADS) {
+        const uint32_t v = base + t;
+        const int32_t f = (int32_t)v - (int32_t)h;
+        const bool in = v < V && any_kept(s_bits, max(f, 0), min(f + (int32_t)P + 1, (int32_t)T));
+        const uint32_t bal = __ballot_sync(0xffffffffu, in);
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        __syncthreads();
+        uint32_t off = n_list, all = 0;
+#pragma unroll
+        for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { off += w < warp ? s_warp[w] : 0u; all += s_warp[w]; }
+        if (in) s_list[off + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)v;
+        n_list += all;
+        __syncthreads();                                         // s_warp is rewritten by the next round; s_list is complete
+    }
+    const int16_t *hist = J.hist_pcm + (uint64_t)s * P * hop;
+    const uint32_t n = n_list * hop;
+    if (J.pcm16) {
+        uint32_t *dst = reinterpret_cast<uint32_t *>(J.pcm16 + (uint64_t)s * J.pcm16_stride);
+        for (uint32_t j = t; 2 * j < n; j += WIRE_THREADS) {
+            const uint32_t a = preroll_sample(J, row, hist, s_list, h, head, 2 * j);
+            const uint32_t b = 2 * j + 1 < n ? preroll_sample(J, row, hist, s_list, h, head, 2 * j + 1) : 0u;
+            dst[j] = a | (b << 16);
+        }
+    }
+    const uint32_t n_bytes = 2 * n, n_groups = (n_bytes + 2) / 3;
+    if (J.b64) {
+        uint32_t *dst = reinterpret_cast<uint32_t *>(J.b64 + (uint64_t)s * J.b64_stride);
+        for (uint32_t g = t; g < n_groups; g += WIRE_THREADS) {
+            const uint32_t s0 = (3 * g) >> 1;
+            const uint32_t a = preroll_sample(J, row, hist, s_list, h, head, s0);
+            const uint32_t b = s0 + 1 < n ? preroll_sample(J, row, hist, s_list, h, head, s0 + 1) : 0u;
+            dst[g] = b64_quad(a, b, g, n_bytes);
+        }
+    }
+    const uint32_t M = J.n_mels;
+    if (J.lm_out) {
+        const float *src = J.lm + (uint64_t)s * J.lm_stride, *hl = J.hist_lm + (uint64_t)s * P * M;
+        float *dst = J.lm_out + (uint64_t)s * J.lm_out_stride;
+        for (uint32_t i = t; i < n_list * M; i += WIRE_THREADS) {
+            const uint32_t r = i / M, c = i - r * M, v = s_list[r];
+            dst[i] = v < h ? hl[((head + v) % P) * M + c] : src[(uint64_t)(v - h) * M + c];
+        }
+    }
+    if (t == 0) {
+        // the wire kernel's record; only n_samples and n_chars count the pre-roll
+        uint32_t cont = 0;
+        if (prev == VAD_SPEECH) cont = s_break < T ? s_break + (st[s_break] == VAD_ENDING ? 1u : 0u) : T;
+        uint32_t last = T ? st[T - 1] : prev;
+        if (end && last == VAD_SPEECH) { ++ended; last = 0; }
+        WireTick r;
+        r.n_samples = n; r.n_chars = J.b64 ? 4 * n_groups : 0u; r.continued = cont * hop;
+        r.started = (uint16_t)started; r.ended = (uint16_t)ended; r.in_speech = last == VAD_SPEECH ? 1 : 0;
+        r.pad[0] = r.pad[1] = r.pad[2] = 0;
+        J.ticks[s] = r;
+        J.prev[s] = (uint8_t)last;
+        if (J.lm_out) J.n_frames[s] = n_list;
+    }
+    __syncthreads();                                             // every history read above is done
+    const int32_t lk = s_last;
+    const uint32_t n_app = T - (uint32_t)(lk + 1), skip = n_app > P ? n_app - P : 0u;
+    if (!end) {                                                  // (an end empties the history: the next push is an origin)
+        int16_t *hp = J.hist_pcm + (uint64_t)s * P * hop;
+        for (uint32_t i = t; i < (n_app - skip) * hop; i += WIRE_THREADS) {
+            const uint32_t j = skip + i / hop, k = i % hop;
+            hp[((pos + j) % P) * hop + k] = (int16_t)pcm16_of(row[(uint64_t)(lk + 1 + j) * hop + k]);
+        }
+        if (J.lm_out) {
+            const float *src = J.lm + (uint64_t)s * J.lm_stride;
+            float *hl = J.hist_lm + (uint64_t)s * P * M;
+            for (uint32_t i = t; i < (n_app - skip) * M; i += WIRE_THREADS) {
+                const uint32_t j = skip + i / M, c = i % M;
+                hl[((pos + j) % P) * M + c] = src[(uint64_t)(lk + 1 + j) * M + c];
+            }
+        }
+    }
+    if (t == 0) {
+        J.hist_n[s] = end ? 0u : min(P, (lk >= 0 ? 0u : h) + n_app);
+        J.hist_pos[s] = (pos + n_app) % P;
+    }
+}
+
+cudaError_t launch_session_wire_preroll(const WirePrerollJob &J, cudaStream_t st)
+{
+    if (J.n_streams == 0) return cudaSuccess;
+    const size_t smem = (size_t)(J.T + 31) / 32 * sizeof(uint32_t) + (((size_t)(J.T + J.P) * sizeof(uint16_t) + 3) & ~(size_t)3);
+    if (J.T + J.P > 0xffffu) return cudaErrorInvalidValue;      // (frame indices are 16-bit, as in the wire kernel)
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(af_session_wire_preroll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    af_session_wire_preroll_kernel<<<J.n_streams, WIRE_THREADS, smem, st>>>(J);
+    return cudaGetLastError();
+}
+
+__global__ void af_session_preroll_clear_kernel(const RecordMove *__restrict__ tab, uint32_t n, uint32_t *__restrict__ hist_n)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) hist_n[tab[i].slot] = 0;
+}
+
+cudaError_t launch_session_preroll_clear(const RecordMove *tab, uint32_t n, uint32_t *hist_n, cudaStream_t st)
+{
+    if (n == 0) return cudaSuccess;
+    af_session_preroll_clear_kernel<<<(n + 255) / 256, 256, 0, st>>>(tab, n, hist_n);
+    return cudaGetLastError();
+}
+
 // the same over the rows of a batch: in [rows][in_stride] f32 -> out [rows][out_stride] i16, `width` samples per row
 // (four at a time: one 16-byte load, one 8-byte store; both strides are multiples of 4)
 __global__ void af_pcm16_rows_kernel(const float *__restrict__ in, uint64_t in_stride, int16_t *__restrict__ out, uint64_t out_stride,
@@ -1488,6 +1663,29 @@ cudaError_t launch_vad_segments(const uint8_t *states, uint64_t stride, const ui
 {
     if (n_streams == 0) return cudaSuccess;
     af_vad_segments_kernel<<<n_streams, SEG_THREADS, 0, st>>>(states, stride, n_frames, n_streams, seg, seg_cap, n_seg);
+    return cudaGetLastError();
+}
+
+// ---- segment pre-roll: one thread per segment slot.  A thread rewrites its segment's start and reads only the end of
+// the one before, so the update in place has no hazard ----
+__global__ void af_vad_segments_preroll_kernel(uint32_t *__restrict__ seg, uint32_t seg_cap, const uint32_t *__restrict__ n_seg,
+                                               uint32_t n_streams, uint32_t P)
+{
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)n_streams * seg_cap) return;
+    const uint32_t s = (uint32_t)(i / seg_cap), k = (uint32_t)(i - (uint64_t)s * seg_cap);
+    if (k >= n_seg[s]) return;
+    uint32_t *sg = seg + 2 * i;
+    const uint32_t start = sg[0], lo = k ? sg[-1] : 0u;         // the previous segment's end (exclusive), or frame 0
+    sg[0] = max(start > P ? start - P : 0u, min(lo, start));
+}
+
+cudaError_t launch_vad_segments_preroll(uint32_t *seg, uint32_t seg_cap, const uint32_t *n_seg, uint32_t n_streams, uint32_t P,
+                                        cudaStream_t st)
+{
+    const uint64_t n = (uint64_t)n_streams * seg_cap;
+    if (n == 0 || P == 0) return cudaSuccess;
+    af_vad_segments_preroll_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(seg, seg_cap, n_seg, n_streams, P);
     return cudaGetLastError();
 }
 

@@ -165,6 +165,30 @@ struct WireLogmelJob {       // a session tick's wire features: the log-mel rows
 // Must run before launch_session_wire of the same tick, which advances prev
 cudaError_t launch_session_wire_logmel(const WireLogmelJob &job, cudaStream_t st);
 
+struct WirePrerollJob {      // a session tick's gated wire payloads with P frames of pre-roll (all device pointers)
+    const float *y; uint64_t y_stride;               // 16 kHz rows: frame f of the tick starts at y[f * hop]
+    const uint8_t *states; uint64_t st_stride;       // VadState of the tick's T frames (nullptr: T == 0)
+    uint32_t T, hop, P;                              // T: the largest frame count of the tick; P >= 1
+    uint8_t *prev;                                   // per stream: state of the latest completed frame, carried across ticks
+    int16_t *pcm16; uint64_t pcm16_stride;           // (or nullptr)
+    char *b64; uint64_t b64_stride;                  // (or nullptr; stride a multiple of 4)
+    WireTick *ticks;
+    const float *lm; uint64_t lm_stride; uint32_t n_mels;   // wire features: the tick's log-mel (lm_out nullptr: off)
+    float *lm_out; uint64_t lm_out_stride;           // stream s's payload rows, back to back, at lm_out[s * lm_out_stride]
+    uint32_t *n_frames;                              // per stream: payload frames (features on)
+    // per stream: a ring of P frames -- their PCM16 hops at hist_pcm[s * P * hop], their log-mel rows (features on) at
+    // hist_lm[s * P * n_mels] -- holding the hist_n[s] latest frames after the last payload frame, hist_pos[s] the slot
+    // the next frame goes to
+    int16_t *hist_pcm; float *hist_lm;
+    uint32_t *hist_n, *hist_pos;
+    uint32_t n_streams;
+    const StreamTick *tab;                           // ragged tick: per-stream y_new / T, the end and restart flags (or nullptr)
+};
+// Runs instead of launch_session_wire_logmel and launch_session_wire when the pre-roll is on
+cudaError_t launch_session_wire_preroll(const WirePrerollJob &job, cudaStream_t st);
+// an import: the history of every listed slot becomes empty (one launch for all of them)
+cudaError_t launch_session_preroll_clear(const RecordMove *tab, uint32_t n, uint32_t *hist_n, cudaStream_t st);
+
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);
 cudaError_t launch_session_tick(const SessionIngest &I, const SessionResample &R, uint32_t n_streams, cudaStream_t st);
@@ -195,5 +219,9 @@ cudaError_t launch_pcm16_rows(const float *in, uint64_t in_stride, int16_t *out,
                               cudaStream_t st);
 cudaError_t launch_vad_segments(const uint8_t *states, uint64_t stride, const uint32_t *n_frames, uint32_t n_streams,
                                 uint32_t *seg, uint32_t seg_cap, uint32_t *n_seg, cudaStream_t st);
+// in place on launch_vad_segments' output: every segment starts up to P frames earlier, never before the previous
+// segment's end or frame 0
+cudaError_t launch_vad_segments_preroll(uint32_t *seg, uint32_t seg_cap, const uint32_t *n_seg, uint32_t n_streams, uint32_t P,
+                                        cudaStream_t st);
 
 }  // namespace af

@@ -735,6 +735,22 @@ AF_API int af_vad_segments(const uint8_t *states, uint64_t vad_stride, const uin
     return AF_OK;
 }
 
+AF_API int af_vad_segments_preroll(uint32_t *seg, uint32_t seg_cap, const uint32_t *n_seg, size_t n_streams,
+                                   uint32_t preroll_frames, void *cuda_stream)
+{
+    if (!seg || !n_seg) return fail(AF_ERR_INVALID, "null argument");
+    if (preroll_frames == 0) return AF_OK;                       // the segments as they are
+    int rc = require_ctx();
+    if (rc) return rc;
+    const int owner = device_of_pointer(seg);
+    AF_SCOPE(owner >= 0 && device_ctx(owner) ? owner : cur_device());
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : cur_ctx().stream;
+    AF_CUDA(launch_vad_segments_preroll(seg, seg_cap, n_seg, (uint32_t)n_streams, preroll_frames, st));
+    if ((uint64_t)n_streams * seg_cap) count_launch();
+    if (!cuda_stream) AF_CUDA(cudaStreamSynchronize(st));
+    return AF_OK;
+}
+
 AF_API int af_vad_gate(const float *pcm, uint64_t pcm_stride, const float *logmel, uint64_t logmel_stride, uint32_t n_mels,
                        const uint32_t *n_out, uint32_t hop, const uint32_t *seg, uint32_t seg_cap, const uint32_t *n_seg,
                        size_t n_streams, const af_gate_outputs *out, void *cuda_stream)
@@ -1445,6 +1461,15 @@ struct af_session {
             bool valid = false;
         };
         Features feat;
+        // pre-roll (af_session_set_wire_preroll): P frames; per stream a ring of the PCM16 hops (and, with features, the
+        // log-mel rows) of up to P frames after its last payload frame, its count of valid frames and its next slot.
+        // frames == 0: off, nothing allocated
+        struct Preroll {
+            uint32_t frames = 0;
+            DevBuf<int16_t> d_pcm; DevBuf<float> d_lm;
+            DevBuf<uint32_t> d_n, d_pos;
+        };
+        Preroll pre;
     };
     Wire wr;
     uint64_t max_new_y = 0;                                   // bound of the 16 kHz samples one tick produces
@@ -1546,6 +1571,7 @@ AF_API int af_session_reset(af_session *s)
     AF_CUDA(cudaMemset(s->in_buf[0].get(), 0, s->S * s->in_stride * sizeof(float)));
     AF_CUDA(cudaMemset(s->d_vad.get(), 0, s->S * sizeof(VadState)));
     if (s->d_wire_prev.get()) AF_CUDA(cudaMemset(s->d_wire_prev.get(), 0, s->S));   // no segment open
+    if (s->wr.pre.frames) AF_CUDA(cudaMemset(s->wr.pre.d_n.get(), 0, s->S * sizeof(uint32_t)));   // no pre-roll history
     return AF_OK;
 }
 
@@ -1852,7 +1878,9 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
         } else { states = o->vad; st_stride = o->vad_stride; }
         if (st_stride < maxT) return fail(AF_ERR_CAPACITY, "internal: state staging too small for %u frames", maxT);
     }
-    const uint64_t wire_n = s->wr.cfg.gate ? (uint64_t)maxT * s->hop : max_ny;   // bound of this tick's payloads
+    // bound of this tick's payloads: gated, the tick's frames and, once one completed, the pre-roll of earlier pushes
+    const uint32_t pre = s->wire ? s->wr.pre.frames : 0;
+    const uint64_t wire_n = s->wr.cfg.gate ? (uint64_t)(maxT ? maxT + pre : 0) * s->hop : max_ny;
     if (s->wire && wire_n > s->wr.cap) return fail(AF_ERR_CAPACITY, "internal: %llu wire samples exceed the rows", (unsigned long long)wire_n);
     float *pcm_rows = nullptr; uint64_t pcm_rows_stride = 0;   // per-stream: the tick kernel writes each stream's PCM here
     if (want_pcm && per_stream) {
@@ -1985,7 +2013,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     // ---- 4. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
     if (s->wire) {
         const af_session::Wire &wr = s->wr;
-        if (feats) {                                             // before the wire kernel, which advances d_wire_prev
+        if (feats && !pre) {                                     // before the wire kernel, which advances d_wire_prev
             const af_session::Wire::Features &wf = wr.feat;
             WireLogmelJob fj{};
             fj.lm = lm; fj.lm_stride = lm_stride; fj.n_mels = cfg.n_mels;
@@ -2001,16 +2029,43 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
                                           (size_t)maxT * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
             AF_CUDA(cudaMemcpyAsync(wf.h_n.get(), wf.d_n.get(), S * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         }
-        WireJob wj{};
-        wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = one.y_keep; wj.n_new = one.n_y;
-        wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
-        wj.T = maxT; wj.hop = s->hop; wj.gate = wr.cfg.gate;              // (T sizes the kept-frame list: the largest)
-        wj.prev = s->d_wire_prev.get();
-        wj.pcm16 = wr.d_pcm16.get(); wj.pcm16_stride = wr.pcm16_stride;
-        wj.b64 = wr.d_b64.get(); wj.b64_stride = wr.b64_stride;
-        wj.ticks = wr.d_ticks.get(); wj.n_streams = (uint32_t)S; wj.tab = tab;
-        AF_CUDA(launch_session_wire(wj, st));
-        count_launch();
+        if (pre) {                                               // one launch: payloads, features, records, history
+            const af_session::Wire::Features &wf = wr.feat;
+            WirePrerollJob pj{};
+            pj.y = ycur; pj.y_stride = s->y_stride;
+            pj.states = maxT ? states : nullptr; pj.st_stride = st_stride;
+            pj.T = maxT; pj.hop = s->hop; pj.P = pre;
+            pj.prev = s->d_wire_prev.get();
+            pj.pcm16 = wr.d_pcm16.get(); pj.pcm16_stride = wr.pcm16_stride;
+            pj.b64 = wr.d_b64.get(); pj.b64_stride = wr.b64_stride;
+            pj.ticks = wr.d_ticks.get();
+            if (feats) {
+                pj.lm = lm; pj.lm_stride = lm_stride; pj.n_mels = cfg.n_mels;
+                pj.lm_out = wf.d_rows.get(); pj.lm_out_stride = wf.stride; pj.n_frames = wf.d_n.get();
+                pj.hist_lm = wr.pre.d_lm.get();
+            }
+            pj.hist_pcm = wr.pre.d_pcm.get(); pj.hist_n = wr.pre.d_n.get(); pj.hist_pos = wr.pre.d_pos.get();
+            pj.n_streams = (uint32_t)S; pj.tab = tab;
+            AF_CUDA(launch_session_wire_preroll(pj, st));
+            count_launch();
+            if (feats) {
+                if (wf.mem == AF_MEM_HOST && wire_n)
+                    AF_CUDA(cudaMemcpy2DAsync(wf.h_rows.get(), wf.stride * sizeof(float), wf.d_rows.get(), wf.stride * sizeof(float),
+                                              (size_t)(wire_n / s->hop) * cfg.n_mels * sizeof(float), S, cudaMemcpyDeviceToHost, st));
+                AF_CUDA(cudaMemcpyAsync(wf.h_n.get(), wf.d_n.get(), S * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            }
+        } else {
+            WireJob wj{};
+            wj.y = ycur; wj.y_stride = s->y_stride; wj.y_new = one.y_keep; wj.n_new = one.n_y;
+            wj.states = (maxT && cfg.vad_enable) ? states : nullptr; wj.st_stride = st_stride;
+            wj.T = maxT; wj.hop = s->hop; wj.gate = wr.cfg.gate;          // (T sizes the kept-frame list: the largest)
+            wj.prev = s->d_wire_prev.get();
+            wj.pcm16 = wr.d_pcm16.get(); wj.pcm16_stride = wr.pcm16_stride;
+            wj.b64 = wr.d_b64.get(); wj.b64_stride = wr.b64_stride;
+            wj.ticks = wr.d_ticks.get(); wj.n_streams = (uint32_t)S; wj.tab = tab;
+            AF_CUDA(launch_session_wire(wj, st));
+            count_launch();
+        }
         if (wr.cfg.mem == AF_MEM_HOST && wire_n) {
             if (wr.cfg.pcm16)
                 AF_CUDA(cudaMemcpy2DAsync(wr.h_pcm16.get(), wr.pcm16_stride * sizeof(int16_t), wr.d_pcm16.get(),
@@ -2375,6 +2430,10 @@ AF_API int af_session_import_streams(af_session *s, const uint32_t *slots, const
     }
     AF_CUDA(launch_session_unpack(record_job(s, const_cast<uint8_t *>(src)), (uint32_t)n, st));
     count_launch();
+    if (s->wr.pre.frames) {                                      // a record carries no history: the import is an origin
+        AF_CUDA(launch_session_preroll_clear(s->xfer.d_moves.get(), (uint32_t)n, s->wr.pre.d_n.get(), st));
+        count_launch();
+    }
     AF_CUDA(cudaStreamSynchronize(st));
     // ---- commit: the slots' bookkeeping, their configurations; lockstep again when every stream stands at one position ----
     if (!s->diverged) {
@@ -2447,6 +2506,58 @@ AF_API int af_session_levels(const af_session *s, float *level_db, float *peak, 
     return AF_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// The payload rows of w.cfg for a tick's payload and `pre` frames of pre-roll, into w: the session's rows stay as they
+// are until the caller moves these in.  Ungated: the tick's new samples; gated: the hops of at most y_stride / hop + 2
+// frames, plus the pre-roll's
+int wire_rows(const af_session *s, uint32_t pre, af_session::Wire &w)
+{
+    const size_t S = s->S;
+    w.cap = w.cfg.gate ? (s->y_stride / s->hop + 2 + pre) * s->hop : s->max_new_y;
+    if (w.cfg.pcm16) {
+        w.pcm16_stride = round_up(w.cap, 4);
+        AF_CUDA(w.d_pcm16.alloc(S * w.pcm16_stride));
+        if (w.cfg.mem == AF_MEM_HOST) AF_CUDA(w.h_pcm16.alloc(S * w.pcm16_stride));
+    }
+    if (w.cfg.base64) {
+        w.b64_stride = round_up(af_pcm16_base64_len(w.cap), 4);
+        AF_CUDA(w.d_b64.alloc(S * w.b64_stride));
+        if (w.cfg.mem == AF_MEM_HOST) AF_CUDA(w.h_b64.alloc(S * w.b64_stride));
+    }
+    return AF_OK;
+}
+
+// The feature rows in `mem` for the frames of wire_rows(s, pre, .), into f
+int feature_rows(const af_session *s, int mem, uint32_t pre, af_session::Wire::Features &f)
+{
+    const size_t S = s->S;
+    f.mem = mem;
+    f.stride = round_up((s->y_stride / s->hop + 2 + pre) * s->pipe->cfg.n_mels, 4);
+    AF_CUDA(f.d_rows.alloc(S * f.stride));
+    if (mem == AF_MEM_HOST) AF_CUDA(f.h_rows.alloc(S * f.stride));
+    AF_CUDA(f.d_n.alloc(S));
+    AF_CUDA(f.h_n.alloc(S));
+    return AF_OK;
+}
+
+// The session takes w's payload rows and the pre-roll state `p` (once the device no longer writes the old ones); the
+// last push's rows are gone with them
+void take_wire_rows(af_session *s, af_session::Wire &w, af_session::Wire::Preroll &&p)
+{
+    af_session::Wire &wr = s->wr;
+    wr.cap = w.cap;
+    wr.d_pcm16 = std::move(w.d_pcm16); wr.h_pcm16 = std::move(w.h_pcm16); wr.pcm16_stride = w.pcm16_stride;
+    wr.d_b64 = std::move(w.d_b64); wr.h_b64 = std::move(w.h_b64); wr.b64_stride = w.b64_stride;
+    wr.pre = std::move(p);
+    s->wire_valid = false;
+    wr.feat.valid = false;
+}
+}  // namespace
+
+extern "C" {
+
 // ---- streaming wire output (websocket.rs:244-254 per tick): rows sized for the largest payload a tick can produce ----
 AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg)
 {
@@ -2469,18 +2580,8 @@ AF_API int af_session_enable_wire(af_session *s, const af_wire_config *cfg)
     const size_t S = s->S;
     af_session::Wire wr;                             // the session takes the rows once all of them are allocated
     wr.cfg = *cfg;
-    // ungated: the tick's new samples; gated: the hops of at most y_stride / hop + 2 frames
-    wr.cap = cfg->gate ? (s->y_stride / s->hop + 2) * s->hop : s->max_new_y;
-    if (cfg->pcm16) {
-        wr.pcm16_stride = round_up(wr.cap, 4);
-        AF_CUDA(wr.d_pcm16.alloc(S * wr.pcm16_stride));
-        if (cfg->mem == AF_MEM_HOST) AF_CUDA(wr.h_pcm16.alloc(S * wr.pcm16_stride));
-    }
-    if (cfg->base64) {
-        wr.b64_stride = round_up(af_pcm16_base64_len(wr.cap), 4);
-        AF_CUDA(wr.d_b64.alloc(S * wr.b64_stride));
-        if (cfg->mem == AF_MEM_HOST) AF_CUDA(wr.h_b64.alloc(S * wr.b64_stride));
-    }
+    int rc = wire_rows(s, 0, wr);
+    if (rc) return rc;
     AF_CUDA(wr.d_ticks.alloc(S));
     AF_CUDA(wr.h_ticks.alloc(S));
     if (!s->d_wire_prev.get()) {                     // the carried segment state survives a re-enable, as the detector's does
@@ -2517,8 +2618,15 @@ AF_API int af_session_enable_wire_features(af_session *s, int enable, int mem)
 {
     if (!s) return fail(AF_ERR_INVALID, "null session");
     AF_SCOPE(s->device);
+    af_session::Wire rows;                           // the pre-roll goes back to 0: the payload rows without it
+    rows.cfg = s->wr.cfg;
     if (!enable) {
+        if (s->wr.pre.frames) {
+            const int rc = wire_rows(s, 0, rows);
+            if (rc) return rc;
+        }
         cudaDeviceSynchronize();                     // (a failed tick may still be writing the rows)
+        if (s->wr.pre.frames) take_wire_rows(s, rows, af_session::Wire::Preroll{});
         s->wr.feat = af_session::Wire::Features{};
         return AF_OK;
     }
@@ -2528,18 +2636,47 @@ AF_API int af_session_enable_wire_features(af_session *s, int enable, int mem)
     if (s->frame_len != WIN || s->hop != HOP)
         return fail(AF_ERR_INVALID, "wire features need the VAD on the STFT frames (vad_frame_len 0 or 400 / 160)");
     if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
-    const size_t S = s->S;
     af_session::Wire::Features f;                    // the session takes the rows once all of them are allocated
-    f.mem = mem;
-    f.stride = round_up((s->y_stride / s->hop + 2) * pc.n_mels, 4);   // the frames whose hops the gated wire rows hold
-    AF_CUDA(f.d_rows.alloc(S * f.stride));
-    if (mem == AF_MEM_HOST) AF_CUDA(f.h_rows.alloc(S * f.stride));
-    AF_CUDA(f.d_n.alloc(S));
-    AF_CUDA(f.h_n.alloc(S));
+    int rc = feature_rows(s, mem, 0, f);             // the frames whose hops the gated wire rows hold
+    if (rc) return rc;
+    if (s->wr.pre.frames && (rc = wire_rows(s, 0, rows))) return rc;
     // (the tick's log-mel staging is grown by the tick that first needs it, before anything changes: what is allocated
     // here is exactly what disabling releases)
     cudaDeviceSynchronize();                        // (the rows replaced may still be written)
+    if (s->wr.pre.frames) take_wire_rows(s, rows, af_session::Wire::Preroll{});
     s->wr.feat = std::move(f);
+    return AF_OK;
+}
+
+// ---- wire pre-roll: every segment of the gated payload reaches back up to P frames (af_session_set_wire_preroll) ----
+AF_API int af_session_set_wire_preroll(af_session *s, uint32_t frames)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    if (!s->wire || !s->wr.cfg.gate) return fail(AF_ERR_INVALID, "the pre-roll needs the gated wire output (af_session_enable_wire, gate = 1)");
+    if (frames > AF_WIRE_PREROLL_MAX) return fail(AF_ERR_INVALID, "pre-roll of %u frames (at most %u)", frames, AF_WIRE_PREROLL_MAX);
+    AF_SCOPE(s->device);
+    const size_t S = s->S;
+    const af_session::Wire::Features &cur = s->wr.feat;
+    // everything is allocated before anything changes: payload rows and feature rows that hold the pre-roll, the history
+    af_session::Wire rows;
+    rows.cfg = s->wr.cfg;
+    int rc = wire_rows(s, frames, rows);
+    if (rc) return rc;
+    af_session::Wire::Features f;
+    if (cur.d_rows.get() && (rc = feature_rows(s, cur.mem, frames, f))) return rc;
+    af_session::Wire::Preroll p;
+    p.frames = frames;
+    if (frames) {
+        AF_CUDA(p.d_pcm.alloc(S * frames * s->hop));
+        if (cur.d_rows.get()) AF_CUDA(p.d_lm.alloc(S * frames * s->pipe->cfg.n_mels));
+        AF_CUDA(p.d_n.alloc(S));
+        AF_CUDA(p.d_pos.alloc(S));
+        AF_CUDA(cudaMemset(p.d_n.get(), 0, S * sizeof(uint32_t)));   // every stream's origin is the next push
+        AF_CUDA(cudaMemset(p.d_pos.get(), 0, S * sizeof(uint32_t)));
+    }
+    cudaDeviceSynchronize();                         // (the rows replaced may still be written)
+    take_wire_rows(s, rows, std::move(p));
+    if (cur.d_rows.get()) s->wr.feat = std::move(f);
     return AF_OK;
 }
 

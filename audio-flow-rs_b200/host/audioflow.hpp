@@ -285,6 +285,9 @@ public:
         check(af_session_wire_features(h_, &f.rows, &f.stride, f.n_frames.data()));
         return f;
     }
+    // every segment of the gated payload (and its features) reaches back up to `frames` frames before its onset
+    // (0 .. AF_WIRE_PREROLL_MAX, 0: off); enable_wire / enable_wire_features set it back to 0, so set it last
+    void set_wire_preroll(uint32_t frames) { check(af_session_set_wire_preroll(h_, frames)); }
     // per stream: the first frame completed by the last push, in the stream's own frame sequence since its last start
     std::vector<uint64_t> wire_first_frames() const
     {

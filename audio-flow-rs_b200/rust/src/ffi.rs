@@ -23,6 +23,7 @@ pub const AF_FMT_F32: u16 = 0;
 pub const AF_FMT_I16: u16 = 1;
 pub const AF_MEM_DEVICE: c_int = 0;
 pub const AF_MEM_HOST: c_int = 1;
+pub const AF_WIRE_PREROLL_MAX: u32 = 100;
 
 // ---- the batched fast path (audioflow_gpu.h, "Batched fast path") ----
 #[repr(C)] pub struct af_pipeline { _p: [u8; 0] }
@@ -136,6 +137,10 @@ extern "C" {
     pub fn af_session_wire_first_frames(s: *const af_session, first_frame: *mut u64) -> c_int;
     pub fn af_session_enable_wire_features(s: *mut af_session, enable: c_int, mem: c_int) -> c_int;
     pub fn af_session_wire_features(s: *const af_session, rows: *mut *const f32, stride: *mut u64, n_frames: *mut u32) -> c_int;
+    pub fn af_session_set_wire_preroll(s: *mut af_session, frames: u32) -> c_int;
+    /// device pointers: af_vad_segments' output, rewritten in place
+    pub fn af_vad_segments_preroll(seg: *mut u32, seg_cap: u32, n_seg: *const u32, n_streams: usize, preroll_frames: u32,
+                                   cuda_stream: *mut std::os::raw::c_void) -> c_int;
     pub fn af_session_create_formats(p: *mut af_pipeline, n_streams: usize, formats: *const af_stream_format, n_formats: usize,
                                      stream_format: *const u32, sample_format: u16, out: *mut *mut af_session) -> c_int;
     pub fn af_session_restart_streams(s: *mut af_session, streams: *const u32, format: *const u32, n: usize) -> c_int;

@@ -24,6 +24,12 @@
 //! for (k, (p, f)) in s.wire()?.into_iter().zip(s.wire_features()?).enumerate() { /* f.logmel: f.n_frames x n_mels */ }
 //! ```
 //!
+//! A pre-roll keeps the frames just before every detected onset, which the detector reports a few frames late:
+//!
+//! ```ignore
+//! s.set_wire_preroll(15)?;   // 150 ms before every segment start (after enable_wire_features, which resets it)
+//! ```
+//!
 //! Callers whose capture devices differ share one session through `Session::with_formats`; a freed slot takes a caller
 //! with another device through `restart_streams`:
 //!
@@ -246,6 +252,13 @@ impl Session {
             logmel: unsafe { std::slice::from_raw_parts(rows.add(k * stride as usize), f as usize * self.n_mels) }.to_vec(),
             n_frames: f,
         }).collect())
+    }
+
+    /// Every speech segment of the gated payload (and of its features) reaches back up to `frames` frames before its
+    /// onset (0 ..= `AF_WIRE_PREROLL_MAX`, 0: off), never into the previous segment or before the stream's origin.
+    /// `enable_wire_features` sets it back to 0: set it last.
+    pub fn set_wire_preroll(&mut self, frames: u32) -> Result<(), AudioError> {
+        check(unsafe { ffi::af_session_set_wire_preroll(self.h, frames) })
     }
 
     /// `AudioLevel` / `VolumeLevel` payloads of the last tick: (level_db, peak, is_speech) per stream.

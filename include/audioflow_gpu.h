@@ -254,6 +254,13 @@ AF_API int af_set_kernel_variant(const char *name);
 AF_API int af_vad_segments(const uint8_t *states, uint64_t vad_stride, const uint32_t *n_frames,
                            size_t n_streams, uint32_t *seg, uint32_t seg_cap, uint32_t *n_seg,
                            void *cuda_stream);
+/* Pre-roll, in place on af_vad_segments' output (device pointers; the first min(n_seg, seg_cap)
+ * segments of each stream): segment k [start, end) becomes [max(start - P, end of segment k - 1,
+ * 0), end), the first segment's predecessor ending at 0.  The segments stay disjoint and in
+ * order, and af_vad_gate then keeps the P frames before every onset (fewer where the previous
+ * segment or the stream's start is closer).  Any P; P = 0 leaves seg untouched. */
+AF_API int af_vad_segments_preroll(uint32_t *seg, uint32_t seg_cap, const uint32_t *n_seg, size_t n_streams,
+                                   uint32_t preroll_frames, void *cuda_stream);
 
 /* ---- VAD-gated output (SURVEY 8(f) f1, second half) ------------------------------------- */
 /* What the reference's spec wants in front of the wire (specs/0001-spec.md:466: drop the silent stretches before
@@ -429,6 +436,30 @@ AF_API int af_session_enable_wire_features(af_session *s, int enable, int mem);
  * valid until the next push.  n_frames: host array of n_streams (may be NULL).  AF_ERR_INVALID whenever af_session_wire
  * is (before the first push since enabling, after an import, after a failed push) and while the features are off. */
 AF_API int af_session_wire_features(const af_session *s, const float **rows, uint64_t *stride, uint32_t *n_frames);
+/* ---- wire pre-roll: every speech segment of the gated payload reaches back P frames ------------------------------------
+ * The detector says Speech a few frames after an onset (the smoothed energy has to cross the threshold), and a quiet
+ * lead-in below the threshold never does; a gated payload that starts at the detected frame clips the first phoneme.
+ * With a pre-roll of P frames, a segment start g (a kept frame that is Speech after a frame that is not, across ticks)
+ * also brings in its pre-roll frames [max(g - P, k + 1, o), g): k is the last kept frame before g (-1 if none), so the
+ * pre-roll never reaches into the previous segment or repeats a frame; o is the stream's origin, the first frame after
+ * its start (creation, af_session_reset, af_session_reset_streams, af_session_restart_streams, the push after an end),
+ * after an import into its slot, or after the latest af_session_set_wire_preroll call.  A tick's gated payload then
+ * holds, in frame order, every kept frame completed in the tick and every pre-roll frame of a segment started in it,
+ * whichever push completed that frame.  Per stream and tick: n_frames * hop == n_samples; the PCM16 and base64 rows
+ * encode those frames' hops (the base64 this tick's bytes alone); the wire features, when on, are the log-mel rows of
+ * the same frames; concatenated since the origin, the payloads are af_vad_gate's output over the stream's PCM, log-mel
+ * and states since the origin with the segments of af_vad_segments_preroll.  started, ended, in_speech and continued
+ * are those without the pre-roll: the pre-roll belongs to its new segment, after the continued samples, and only
+ * n_samples and n_chars grow.  The history of up to P frames stays on the session's GPU; a stream record does not carry
+ * it (the record's layout depends on the framing alone), so an import starts a new origin.
+ * frames: 0 to AF_WIRE_PREROLL_MAX.  Grows the wire rows by frames * hop samples and the feature rows by
+ * frames * n_mels floats, allocates the history for `frames`, and makes the next push every stream's origin; the last
+ * push's rows are released (af_session_wire refuses until the next push).  frames = 0 frees the history: the session
+ * then runs as one that never set a pre-roll.  AF_ERR_INVALID, and nothing changes, when the gated wire output is off or
+ * for frames > AF_WIRE_PREROLL_MAX.  Every af_session_enable_wire and af_session_enable_wire_features call sets the
+ * pre-roll back to 0: set it last. */
+#define AF_WIRE_PREROLL_MAX 100
+AF_API int af_session_set_wire_preroll(af_session *s, uint32_t frames);
 
 /* ---- RingBuffer  (src-tauri/src/modules/audio/capture.rs:84-161): capture hand-off ------ */
 /* The cpal callback writes captured f32 samples, the processing task reads them.  Same semantics as the
