@@ -24,6 +24,7 @@ AF_OK, AF_ERR_INVALID, AF_ERR_RESAMPLING_FAILED, AF_ERR_CUDA, AF_ERR_NO_DEVICE, 
 AF_FMT_F32, AF_FMT_I16 = 0, 1
 AF_MEM_DEVICE, AF_MEM_HOST = 0, 1
 AF_WIRE_PREROLL_MAX = 100
+AF_WIRE_SEG_CONTINUED, AF_WIRE_SEG_CLOSED = 1, 2
 
 
 class AudioError(Exception):
@@ -83,6 +84,16 @@ class WireConfigC(C.Structure):
 class WireTickC(C.Structure):
     _fields_ = [("n_samples", C.c_uint32), ("n_chars", C.c_uint32), ("continued", C.c_uint32), ("started", C.c_uint16),
                 ("ended", C.c_uint16), ("in_speech", C.c_uint8), ("pad", C.c_uint8 * 3)]
+
+
+class WireSegmentC(C.Structure):
+    _fields_ = [("frame", C.c_int32), ("offset", C.c_uint32), ("n_frames", C.c_uint32), ("preroll", C.c_uint16),
+                ("flags", C.c_uint8), ("pad", C.c_uint8)]
+
+
+# af_wire_segment as a numpy structured type (Session.wire_segments)
+WIRE_SEGMENT_DTYPE = np.dtype([("frame", "<i4"), ("offset", "<u4"), ("n_frames", "<u4"), ("preroll", "<u2"), ("flags", "u1"),
+                               ("pad", "u1")])
 
 
 AF_MAX_GPUS = 16
@@ -200,6 +211,8 @@ def load_library():
         "af_session_wire_features": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
         "af_vad_segments_preroll": (C.c_int, [vp, C.c_uint32, vp, sz, C.c_uint32, vp]),
         "af_session_set_wire_preroll": (C.c_int, [vp, C.c_uint32]),
+        "af_session_enable_wire_segments": (C.c_int, [vp, C.c_int, C.c_int]),
+        "af_session_wire_segments": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -791,6 +804,7 @@ class Session:
         self.wire_gate = False
         self.features_mem = None                        # where the wire feature rows live (enable_wire_features)
         self.wire_preroll = 0                           # frames of pre-roll of the gated wire (set_wire_preroll)
+        self.segments_mem = None                        # where the wire segment table lives (enable_wire_segments)
 
     def stream_channels(self) -> np.ndarray:
         """The channel count of every stream's current format."""
@@ -999,13 +1013,14 @@ class Session:
         L = load_library()
         if gate is None:
             _check(L.af_session_enable_wire(self._h, None))
-            self.wire_mem, self.wire_gate, self.features_mem, self.wire_preroll = None, False, None, 0
+            self.wire_mem, self.wire_gate, self.features_mem, self.wire_preroll, self.segments_mem = None, False, None, 0, None
             return
         cfg = WireConfigC(int(gate), int(pcm16), int(base64), mem)
         _check(L.af_session_enable_wire(self._h, C.byref(cfg)))
         self.wire_mem, self.wire_gate = mem, bool(gate)
         self.features_mem = None                        # every enable_wire call turns the features off
         self.wire_preroll = 0                           # ... and sets the pre-roll back to 0
+        self.segments_mem = None                        # ... and turns the segment table off
 
     def enable_wire_features(self, on: bool = True, mem: int = AF_MEM_HOST):
         """Beside the gated wire payload, the log-mel rows of its kept frames on every push (wire_features()).  Needs
@@ -1040,6 +1055,36 @@ class Session:
             raise ValueError("the pre-roll needs the gated wire output: enable_wire(gate=True) first")
         _check(load_library().af_session_set_wire_preroll(self._h, int(frames)))
         self.wire_preroll = int(frames)
+
+    def enable_wire_segments(self, on: bool = True, mem: int = AF_MEM_HOST):
+        """Beside the gated wire payload, its segment table on every push (wire_segments()): where each utterance's
+        piece starts in the payload, how many frames it has, its frame in the stream and its pre-roll.  Needs
+        enable_wire(gate=True); mem: AF_MEM_HOST or AF_MEM_DEVICE rows.  Leaves the features and the pre-roll as they are.
+        on=False switches it off.  ValueError before the library is called for anything else."""
+        if not on:
+            _check(load_library().af_session_enable_wire_segments(self._h, 0, AF_MEM_HOST))
+            self.segments_mem = None
+            return
+        if mem not in (AF_MEM_HOST, AF_MEM_DEVICE):
+            raise ValueError(f"bad memory kind {mem}")
+        if self.wire_mem is None or not self.wire_gate:
+            raise ValueError("wire segments need the gated wire output: enable_wire(gate=True) first")
+        _check(load_library().af_session_enable_wire_segments(self._h, 1, mem))
+        self.segments_mem = mem
+
+    def wire_segments(self):
+        """The segment table of the last push: (rows, n_segs).  Host rows: a list of WIRE_SEGMENT_DTYPE arrays of
+        n_segs[k] pieces, one per stream.  Device rows: (pointer, stride in entries) of the session's [n_streams][stride]
+        af_wire_segment rows.  n_segs: uint32[n_streams]."""
+        p, st = C.c_void_p(), C.c_uint64(0)
+        n = np.zeros(self.S, np.uint32)
+        _check(load_library().af_session_wire_segments(self._h, C.byref(p), C.byref(st), n.ctypes.data_as(C.POINTER(C.c_uint32))))
+        if self.segments_mem != AF_MEM_HOST:
+            return (p.value, int(st.value)), n
+        esz = WIRE_SEGMENT_DTYPE.itemsize
+        rows = [np.frombuffer((C.c_uint8 * (int(n[k]) * esz)).from_address(p.value + esz * k * st.value), WIRE_SEGMENT_DTYPE).copy()
+                if n[k] else np.zeros(0, WIRE_SEGMENT_DTYPE) for k in range(self.S)]
+        return rows, n
 
     def wire_features(self):
         """The wire features of the last push: (rows, n_frames).  Host rows: a list of float32 [n_frames[k], n_mels]

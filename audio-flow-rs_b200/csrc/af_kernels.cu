@@ -1205,16 +1205,32 @@ __global__ void af_pcm16_base64_kernel(const float *__restrict__ in, uint64_t n,
 // with a small custom hop), counting segment starts / closes on the way; payload sample i is then sample
 // kept[i / hop] * hop + i % hop of the tick's 16 kHz row.  Ungated, sample i is the tick's new sample i.  Then the PCM16
 // row (two samples per 32-bit store), the base64 row (one 3-byte group = 4 characters per 32-bit store) and the record.
+// With the segment table on (J.segs), the same rounds list the segment starts with one more ballot: a start's piece begins
+// at its position in the kept list, after the piece of the segment open when the tick began (the lead piece, listed first,
+// 0 frames when that segment closes on the tick's first frame or by an end without a frame).  A last pass turns the offsets
+// into frame counts and marks every piece CLOSED but an open last one.
 constexpr uint32_t WIRE_THREADS = 128;
 constexpr uint32_t VAD_SPEECH = 1, VAD_ENDING = 2;             // AF_VAD_SPEECH, AF_VAD_ENDING
 __device__ __forceinline__ float wire_sample(const WireJob &J, const float *row, const uint16_t *kept, uint32_t y_new, uint32_t i)
 {
     return J.gate ? row[(uint32_t)kept[i / J.hop] * J.hop + i % J.hop] : row[y_new + i];
 }
+// the pieces' frame counts from their offsets (kept: the payload's frames), CLOSED on all but an open last one, the count
+__device__ __forceinline__ void wire_segments_close(WireSegment *segs, uint32_t *n_segs, uint32_t np, uint32_t kept,
+                                                    bool open)
+{
+    for (uint32_t i = threadIdx.x; i < np; i += WIRE_THREADS) {
+        const uint32_t next = i + 1 < np ? segs[i + 1].offset : kept;
+        segs[i].n_frames = next - segs[i].offset;
+        if (i + 1 < np || !open) segs[i].flags |= WIRE_SEG_CLOSED;
+    }
+    if (threadIdx.x == 0) *n_segs = np;
+}
 __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const WireJob J)
 {
     extern __shared__ uint16_t s_kept[];                         // gated: the kept frames of the tick, in order
     __shared__ uint32_t s_warp[WIRE_THREADS / 32];
+    __shared__ uint32_t s_wseg[WIRE_THREADS / 32];              // table on: segment starts per warp of the round
     __shared__ uint32_t s_break;                                 // first frame that is not Speech (T if none)
     const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const float *row = J.y + (uint64_t)s * J.y_stride;
@@ -1224,7 +1240,12 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
     if (J.tab) { T = J.tab[s].T; y_new = J.tab[s].y_keep; n_new = J.tab[s].n_y; end = (J.tab[s].flags & TICK_END) != 0; }
     if (!st) T = 0;
     const uint32_t prev = J.prev[s];
-    if (t == 0) s_break = T;
+    WireSegment *segs = J.segs ? J.segs + (uint64_t)s * J.seg_stride : nullptr;
+    const uint32_t lead = segs && prev == VAD_SPEECH && (T || end) ? 1u : 0u;   // the open segment's piece comes first
+    if (t == 0) {
+        s_break = T;
+        if (lead) { WireSegment g{}; g.flags = WIRE_SEG_CONTINUED; segs[0] = g; }
+    }
     __syncthreads();
     uint32_t kept = 0, started = 0, ended = 0;
     for (uint32_t base = 0; base < T; base += WIRE_THREADS) {   // (uniform trip count: every lane takes the ballots)
@@ -1233,17 +1254,34 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
         const uint32_t cur = valid ? st[f] : 0u, pre = valid ? (f ? st[f - 1] : prev) : 0u;
         const bool sp = cur == VAD_SPEECH, psp = pre == VAD_SPEECH;
         const bool keep = valid && (sp || (cur == VAD_ENDING && psp));
+        const bool start = valid && sp && !psp;
         if (valid && !sp) atomicMin(&s_break, f);
         const uint32_t bal = __ballot_sync(0xffffffffu, keep);
+        uint32_t sbal = 0;
+        if (segs) { sbal = __ballot_sync(0xffffffffu, start); if (lane == 0) s_wseg[warp] = __popc(sbal); }
         if (lane == 0) s_warp[warp] = __popc(bal);
-        started += __syncthreads_count(valid && sp && !psp);    // (the barrier also publishes s_warp)
+        const uint32_t started0 = started;
+        started += __syncthreads_count(start);                   // (the barrier also publishes s_warp, s_wseg)
         ended += __syncthreads_count(valid && psp && !sp);
         uint32_t off = kept, all = 0;
 #pragma unroll
         for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { off += w < warp ? s_warp[w] : 0u; all += s_warp[w]; }
-        if (J.gate && keep) s_kept[off + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)f;
+        off += __popc(bal & ((1u << lane) - 1u));
+        if (J.gate && keep) s_kept[off] = (uint16_t)f;
+        if (segs && start) {                                     // a start is kept: its piece begins at its payload frame
+            uint32_t i = lead + started0 + __popc(sbal & ((1u << lane) - 1u));
+#pragma unroll
+            for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) i += w < warp ? s_wseg[w] : 0u;
+            WireSegment g{};
+            g.frame = (int32_t)f; g.offset = off;
+            segs[i] = g;
+        }
         kept += all;
         __syncthreads();                                         // s_warp is rewritten by the next round
+    }
+    if (segs) {
+        const bool open = (T ? st[T - 1] : prev) == VAD_SPEECH && !end;
+        wire_segments_close(segs, J.n_segs + s, lead + started, kept, open);
     }
     const uint32_t brk = s_break;
     const uint32_t n = J.gate ? kept * J.hop : n_new;
@@ -1280,9 +1318,17 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_kernel(const Wir
     }
 }
 
+// a tick of T frames has at most ceil(T / 2) segment starts (a start follows a frame that is not Speech) and one piece of
+// the segment open before it
+__host__ __forceinline__ bool wire_segments_fit(const WireSegment *segs, uint64_t stride, uint32_t T)
+{
+    return !segs || stride >= (uint64_t)(T + 1) / 2 + 1;
+}
+
 cudaError_t launch_session_wire(const WireJob &J, cudaStream_t st)
 {
     if (J.n_streams == 0) return cudaSuccess;
+    if (!wire_segments_fit(J.segs, J.seg_stride, J.states ? J.T : 0)) return cudaErrorInvalidValue;
     const size_t smem = J.gate && J.states ? ((size_t)J.T * sizeof(uint16_t) + 3) & ~(size_t)3 : 0;
     af_session_wire_kernel<<<J.n_streams, WIRE_THREADS, smem, st>>>(J);
     return cudaGetLastError();
@@ -1359,6 +1405,9 @@ cudaError_t launch_session_wire_logmel(const WireLogmelJob &J, cudaStream_t st)
 // (1) the kept bits and the events, by the wire kernel's rule; (2) the payload's frames, ballots and a block scan;
 // (3) PCM16, base64, log-mel rows and the record, pre-roll frames of earlier pushes read from the history; (4) after a
 // barrier, the tick's frames after its last kept frame (all of them if none is kept) go into the history.
+// Table on (J.segs): in (2) a payload frame begins a piece when it is a pre-roll frame or a segment start and the payload
+// frame before it, if any, is not adjacent or is kept: everything between a kept frame and the next start belongs to the
+// start's pre-roll.  The lead piece (the segment open when the tick began) comes first, as in the wire kernel.
 __device__ __forceinline__ bool any_kept(const uint32_t *bits, int32_t lo, int32_t hi)   // a kept frame in [lo, hi)?
 {
     if (lo >= hi) return false;
@@ -1370,6 +1419,16 @@ __device__ __forceinline__ bool any_kept(const uint32_t *bits, int32_t lo, int32
         if (b) return true;
     }
     return false;
+}
+// first kept frame in [lo, hi), or hi
+__device__ __forceinline__ int32_t first_kept(const uint32_t *bits, int32_t lo, int32_t hi)
+{
+    while (lo < hi) {
+        const uint32_t b = bits[lo >> 5] & (0xffffffffu << (lo & 31));
+        if (b) return min((lo & ~31) + __ffs(b) - 1, hi);
+        lo = (lo & ~31) + 32;
+    }
+    return hi;
 }
 // payload sample i as PCM16: history frames were stored encoded, tick frames are encoded here (head: the ring slot of
 // the oldest history frame)
@@ -1387,6 +1446,7 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_preroll_kernel(c
     uint32_t *s_bits = s_dyn;                                    // bit f % 32 of word f / 32: tick frame f is kept
     uint16_t *s_list = reinterpret_cast<uint16_t *>(s_dyn + n_words);   // the payload's frames, virtual, in order
     __shared__ uint32_t s_warp[WIRE_THREADS / 32];
+    __shared__ uint32_t s_wseg[WIRE_THREADS / 32];              // table on: pieces begun per warp of the round
     __shared__ uint32_t s_break;                                 // first frame that is not Speech (T if none)
     __shared__ int32_t s_last;                                   // last kept frame of the tick (-1 if none)
     const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
@@ -1399,7 +1459,12 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_preroll_kernel(c
     const uint32_t prev = J.prev[s], P = J.P, hop = J.hop;
     const uint32_t h = restart ? 0u : J.hist_n[s], pos = J.hist_pos[s];
     const uint32_t head = (pos + P - h) % P;
-    if (t == 0) { s_break = T; s_last = -1; }
+    WireSegment *segs = J.segs ? J.segs + (uint64_t)s * J.seg_stride : nullptr;
+    const uint32_t lead = segs && prev == VAD_SPEECH && (T || end) ? 1u : 0u;   // the open segment's piece comes first
+    if (t == 0) {
+        s_break = T; s_last = -1;
+        if (lead) { WireSegment g{}; g.flags = WIRE_SEG_CONTINUED; segs[0] = g; }
+    }
     __syncthreads();
     uint32_t started = 0, ended = 0;
     for (uint32_t base = 0; base < T; base += WIRE_THREADS) {   // (uniform trip count: every lane takes the ballots)
@@ -1417,20 +1482,50 @@ __global__ void __launch_bounds__(WIRE_THREADS) af_session_wire_preroll_kernel(c
         ended += __syncthreads_count(valid && psp && !sp);
     }
     const uint32_t V = h + T;
-    uint32_t n_list = 0;
+    uint32_t n_list = 0, n_pieces = lead;
     for (uint32_t base = 0; base < V; base += WIRE_THREADS) {
         const uint32_t v = base + t;
         const int32_t f = (int32_t)v - (int32_t)h;
         const bool in = v < V && any_kept(s_bits, max(f, 0), min(f + (int32_t)P + 1, (int32_t)T));
         const uint32_t bal = __ballot_sync(0xffffffffu, in);
         if (lane == 0) s_warp[warp] = __popc(bal);
+        bool begins = false, kept_v = false;
+        uint32_t pbal = 0;
+        if (segs) {
+            if (in) {                                            // (then f < T)
+                kept_v = f >= 0 && ((s_bits[f >> 5] >> (f & 31)) & 1u);
+                const bool start = kept_v && st[f] == VAD_SPEECH && (f ? st[f - 1] : prev) != VAD_SPEECH;
+                const bool kept_p = f >= 1 && ((s_bits[(f - 1) >> 5] >> ((f - 1) & 31)) & 1u);
+                begins = (start || !kept_v) &&
+                         (v == 0 || kept_p || !any_kept(s_bits, max(f - 1, 0), min(f + (int32_t)P, (int32_t)T)));
+            }
+            pbal = __ballot_sync(0xffffffffu, begins);
+            if (lane == 0) s_wseg[warp] = __popc(pbal);
+        }
         __syncthreads();
         uint32_t off = n_list, all = 0;
 #pragma unroll
         for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { off += w < warp ? s_warp[w] : 0u; all += s_warp[w]; }
-        if (in) s_list[off + __popc(bal & ((1u << lane) - 1u))] = (uint16_t)v;
+        off += __popc(bal & ((1u << lane) - 1u));
+        if (in) s_list[off] = (uint16_t)v;
+        if (segs) {
+            uint32_t i = n_pieces + __popc(pbal & ((1u << lane) - 1u)), pieces = 0;
+#pragma unroll
+            for (uint32_t w = 0; w < WIRE_THREADS / 32; ++w) { i += w < warp ? s_wseg[w] : 0u; pieces += s_wseg[w]; }
+            if (begins) {                                        // a pre-roll frame's onset is the first kept frame after it
+                WireSegment g{};
+                g.frame = f; g.offset = off;
+                g.preroll = kept_v ? 0 : (uint16_t)(first_kept(s_bits, max(f, 0), min(f + (int32_t)P + 1, (int32_t)T)) - f);
+                segs[i] = g;
+            }
+            n_pieces += pieces;
+        }
         n_list += all;
         __syncthreads();                                         // s_warp is rewritten by the next round; s_list is complete
+    }
+    if (segs) {
+        const bool open = (T ? st[T - 1] : prev) == VAD_SPEECH && !end;
+        wire_segments_close(segs, J.n_segs + s, n_pieces, n_list, open);
     }
     const int16_t *hist = J.hist_pcm + (uint64_t)s * P * hop;
     const uint32_t n = n_list * hop;
@@ -1504,6 +1599,7 @@ cudaError_t launch_session_wire_preroll(const WirePrerollJob &J, cudaStream_t st
     if (J.n_streams == 0) return cudaSuccess;
     const size_t smem = (size_t)(J.T + 31) / 32 * sizeof(uint32_t) + (((size_t)(J.T + J.P) * sizeof(uint16_t) + 3) & ~(size_t)3);
     if (J.T + J.P > 0xffffu) return cudaErrorInvalidValue;      // (frame indices are 16-bit, as in the wire kernel)
+    if (!wire_segments_fit(J.segs, J.seg_stride, J.states ? J.T : 0)) return cudaErrorInvalidValue;
     if (smem > 48 * 1024) {
         const cudaError_t e = cudaFuncSetAttribute(af_session_wire_preroll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;

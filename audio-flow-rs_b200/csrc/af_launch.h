@@ -136,6 +136,14 @@ struct WireTick {            // af_wire_tick (static_assert'ed in af_runtime.cu)
     uint8_t in_speech, pad[3];
 };
 
+struct WireSegment {         // af_wire_segment (static_assert'ed in af_runtime.cu)
+    int32_t frame;
+    uint32_t offset, n_frames;
+    uint16_t preroll;
+    uint8_t flags, pad;
+};
+constexpr uint8_t WIRE_SEG_CONTINUED = 1, WIRE_SEG_CLOSED = 2;
+
 struct WireJob {             // a session tick's wire payloads (all device pointers)
     const float *y; uint64_t y_stride;               // 16 kHz rows: frame f of the tick starts at y[f * hop]
     uint32_t y_new, n_new;                           // the tick's new samples are y[y_new, y_new + n_new)
@@ -147,6 +155,9 @@ struct WireJob {             // a session tick's wire payloads (all device point
     WireTick *ticks;
     uint32_t n_streams;
     const StreamTick *tab;                           // ragged tick: per-stream y_new / n_new / T and the end flag (or nullptr)
+    // gated: stream s's pieces at segs[s * seg_stride], their count at n_segs[s] (segs nullptr: off; seg_stride >=
+    // ceil(T / 2) + 1)
+    WireSegment *segs; uint64_t seg_stride; uint32_t *n_segs;
 };
 cudaError_t launch_session_wire(const WireJob &job, cudaStream_t st);
 
@@ -183,6 +194,7 @@ struct WirePrerollJob {      // a session tick's gated wire payloads with P fram
     uint32_t *hist_n, *hist_pos;
     uint32_t n_streams;
     const StreamTick *tab;                           // ragged tick: per-stream y_new / T, the end and restart flags (or nullptr)
+    WireSegment *segs; uint64_t seg_stride; uint32_t *n_segs;   // as in WireJob
 };
 // Runs instead of launch_session_wire_logmel and launch_session_wire when the pre-roll is on
 cudaError_t launch_session_wire_preroll(const WirePrerollJob &job, cudaStream_t st);

@@ -1470,6 +1470,15 @@ struct af_session {
             DevBuf<uint32_t> d_n, d_pos;
         };
         Preroll pre;
+        // segment table (af_session_enable_wire_segments): per stream the pieces of the gated payload and their count;
+        // no rows: off.  valid: a push has filled them since they were built
+        struct Segments {
+            int mem = AF_MEM_HOST;
+            DevBuf<WireSegment> d_rows; PinnedBuf<af_wire_segment> h_rows; uint64_t stride = 0;   // entries
+            DevBuf<uint32_t> d_n; PinnedBuf<uint32_t> h_n;
+            bool valid = false;
+        };
+        Segments seg;
     };
     Wire wr;
     uint64_t max_new_y = 0;                                   // bound of the 16 kHz samples one tick produces
@@ -1521,6 +1530,11 @@ struct af_session {
 };
 static_assert(sizeof(WireTick) == sizeof(af_wire_tick) && offsetof(WireTick, started) == offsetof(af_wire_tick, started) &&
               offsetof(WireTick, in_speech) == offsetof(af_wire_tick, in_speech), "WireTick mirrors af_wire_tick");
+static_assert(sizeof(af_wire_segment) == 16 && sizeof(WireSegment) == sizeof(af_wire_segment) &&
+              offsetof(WireSegment, offset) == offsetof(af_wire_segment, offset) &&
+              offsetof(WireSegment, n_frames) == offsetof(af_wire_segment, n_frames) &&
+              offsetof(WireSegment, preroll) == offsetof(af_wire_segment, preroll) &&
+              offsetof(WireSegment, flags) == offsetof(af_wire_segment, flags), "WireSegment mirrors af_wire_segment");
 
 namespace {
 void wire_free(af_session *s)
@@ -2013,6 +2027,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     // ---- 4. wire payloads: one launch for all streams after the scan; host rows receive only what bounds the payloads ----
     if (s->wire) {
         const af_session::Wire &wr = s->wr;
+        const af_session::Wire::Segments &ws = wr.seg;
         if (feats && !pre) {                                     // before the wire kernel, which advances d_wire_prev
             const af_session::Wire::Features &wf = wr.feat;
             WireLogmelJob fj{};
@@ -2046,6 +2061,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
             }
             pj.hist_pcm = wr.pre.d_pcm.get(); pj.hist_n = wr.pre.d_n.get(); pj.hist_pos = wr.pre.d_pos.get();
             pj.n_streams = (uint32_t)S; pj.tab = tab;
+            pj.segs = ws.d_rows.get(); pj.seg_stride = ws.stride; pj.n_segs = ws.d_n.get();
             AF_CUDA(launch_session_wire_preroll(pj, st));
             count_launch();
             if (feats) {
@@ -2063,8 +2079,16 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
             wj.pcm16 = wr.d_pcm16.get(); wj.pcm16_stride = wr.pcm16_stride;
             wj.b64 = wr.d_b64.get(); wj.b64_stride = wr.b64_stride;
             wj.ticks = wr.d_ticks.get(); wj.n_streams = (uint32_t)S; wj.tab = tab;
+            wj.segs = ws.d_rows.get(); wj.seg_stride = ws.stride; wj.n_segs = ws.d_n.get();
             AF_CUDA(launch_session_wire(wj, st));
             count_launch();
+        }
+        if (ws.d_rows.get()) {                                   // (a tick of T frames has at most ceil(T / 2) + 1 pieces)
+            if (ws.mem == AF_MEM_HOST)
+                AF_CUDA(cudaMemcpy2DAsync(ws.h_rows.get(), ws.stride * sizeof(WireSegment), ws.d_rows.get(),
+                                          ws.stride * sizeof(WireSegment), ((maxT + 1) / 2 + 1) * sizeof(WireSegment), S,
+                                          cudaMemcpyDeviceToHost, st));
+            AF_CUDA(cudaMemcpyAsync(ws.h_n.get(), ws.d_n.get(), S * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         }
         if (wr.cfg.mem == AF_MEM_HOST && wire_n) {
             if (wr.cfg.pcm16)
@@ -2087,6 +2111,7 @@ int session_tick(af_session *s, const void *data, uint64_t in_stride, const uint
     s->levels_valid = s->levels;
     s->wire_valid = s->wire;
     if (feats) s->wr.feat.valid = true;
+    if (s->wire && s->wr.seg.d_rows.get()) s->wr.seg.valid = true;
     if (!per_stream) {
         s->shared = shared_next;
     } else {
@@ -2677,6 +2702,45 @@ AF_API int af_session_set_wire_preroll(af_session *s, uint32_t frames)
     cudaDeviceSynchronize();                         // (the rows replaced may still be written)
     take_wire_rows(s, rows, std::move(p));
     if (cur.d_rows.get()) s->wr.feat = std::move(f);
+    return AF_OK;
+}
+
+// ---- wire segments: the pieces of every segment in the gated payload, rows sized for the wire's bound of frames ----
+AF_API int af_session_enable_wire_segments(af_session *s, int enable, int mem)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    AF_SCOPE(s->device);
+    if (!enable) {
+        cudaDeviceSynchronize();                     // (a failed tick may still be writing the rows)
+        s->wr.seg = af_session::Wire::Segments{};
+        return AF_OK;
+    }
+    if (!s->wire || !s->wr.cfg.gate) return fail(AF_ERR_INVALID, "wire segments need the gated wire output (af_session_enable_wire, gate = 1)");
+    if (mem != AF_MEM_DEVICE && mem != AF_MEM_HOST) return fail(AF_ERR_INVALID, "bad memory kind %d", mem);
+    const size_t S = s->S;
+    af_session::Wire::Segments g;                    // the session takes the rows once all of them are allocated
+    g.mem = mem;
+    // the frames of the payload rows without the pre-roll (T_max, as wire_rows), and at most ceil(T_max / 2) + 1 pieces:
+    // the pre-roll adds frames to pieces, never pieces
+    const uint64_t T_max = s->y_stride / s->hop + 2;
+    g.stride = (T_max + 1) / 2 + 1;
+    AF_CUDA(g.d_rows.alloc(S * g.stride));
+    if (mem == AF_MEM_HOST) AF_CUDA(g.h_rows.alloc(S * g.stride));
+    AF_CUDA(g.d_n.alloc(S));
+    AF_CUDA(g.h_n.alloc(S));
+    cudaDeviceSynchronize();                        // (the rows replaced may still be written)
+    s->wr.seg = std::move(g);
+    return AF_OK;
+}
+
+AF_API int af_session_wire_segments(const af_session *s, const af_wire_segment **rows, uint64_t *stride, uint32_t *n_segs)
+{
+    if (!s) return fail(AF_ERR_INVALID, "null session");
+    const af_session::Wire::Segments &g = s->wr.seg;
+    if (!s->wire_valid || !g.valid) return fail(AF_ERR_INVALID, "no tick has been pushed since af_session_enable_wire_segments");
+    if (rows) *rows = g.mem == AF_MEM_HOST ? g.h_rows.get() : reinterpret_cast<const af_wire_segment *>(g.d_rows.get());
+    if (stride) *stride = g.stride;
+    if (n_segs) memcpy(n_segs, g.h_n.get(), s->S * sizeof(uint32_t));
     return AF_OK;
 }
 

@@ -152,6 +152,12 @@ struct WireFeatures {
     uint64_t stride = 0;              // floats from one stream's row to the next
     std::vector<uint32_t> n_frames;   // per stream: its row holds n_frames[k] * n_mels floats
 };
+// where each segment's piece lies in the gated payload (af_session_wire_segments)
+struct WireSegments {
+    const af_wire_segment *rows = nullptr;   // host or device rows, as enable_wire_segments chose; valid until the next push
+    uint64_t stride = 0;                     // entries from one stream's row to the next
+    std::vector<uint32_t> n_segs;            // per stream: its row holds n_segs[k] pieces
+};
 
 class Session {
 public:
@@ -288,6 +294,16 @@ public:
     // every segment of the gated payload (and its features) reaches back up to `frames` frames before its onset
     // (0 .. AF_WIRE_PREROLL_MAX, 0: off); enable_wire / enable_wire_features set it back to 0, so set it last
     void set_wire_preroll(uint32_t frames) { check(af_session_set_wire_preroll(h_, frames)); }
+    // beside the gated payload, its segment table (mem AF_MEM_HOST or AF_MEM_DEVICE rows); leaves the features and the
+    // pre-roll as they are; every enable_wire / disable_wire turns it off
+    void enable_wire_segments(bool on = true, int mem = AF_MEM_HOST) { check(af_session_enable_wire_segments(h_, on ? 1 : 0, mem)); }
+    WireSegments wire_segments() const
+    {
+        WireSegments g;
+        g.n_segs.resize(n_);
+        check(af_session_wire_segments(h_, &g.rows, &g.stride, g.n_segs.data()));
+        return g;
+    }
     // per stream: the first frame completed by the last push, in the stream's own frame sequence since its last start
     std::vector<uint64_t> wire_first_frames() const
     {

@@ -24,6 +24,8 @@ pub const AF_FMT_I16: u16 = 1;
 pub const AF_MEM_DEVICE: c_int = 0;
 pub const AF_MEM_HOST: c_int = 1;
 pub const AF_WIRE_PREROLL_MAX: u32 = 100;
+pub const AF_WIRE_SEG_CONTINUED: u8 = 1;
+pub const AF_WIRE_SEG_CLOSED: u8 = 2;
 
 // ---- the batched fast path (audioflow_gpu.h, "Batched fast path") ----
 #[repr(C)] pub struct af_pipeline { _p: [u8; 0] }
@@ -94,6 +96,17 @@ pub struct af_wire_config {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Default, Debug, PartialEq, Eq)]
+pub struct af_wire_segment {
+    pub frame: i32,
+    pub offset: u32,
+    pub n_frames: u32,
+    pub preroll: u16,
+    pub flags: u8,
+    pub pad: u8,
+}
+
+#[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct af_wire_tick {
     pub n_samples: u32,
@@ -138,6 +151,9 @@ extern "C" {
     pub fn af_session_enable_wire_features(s: *mut af_session, enable: c_int, mem: c_int) -> c_int;
     pub fn af_session_wire_features(s: *const af_session, rows: *mut *const f32, stride: *mut u64, n_frames: *mut u32) -> c_int;
     pub fn af_session_set_wire_preroll(s: *mut af_session, frames: u32) -> c_int;
+    pub fn af_session_enable_wire_segments(s: *mut af_session, enable: c_int, mem: c_int) -> c_int;
+    pub fn af_session_wire_segments(s: *const af_session, rows: *mut *const af_wire_segment, stride: *mut u64,
+                                    n_segs: *mut u32) -> c_int;
     /// device pointers: af_vad_segments' output, rewritten in place
     pub fn af_vad_segments_preroll(seg: *mut u32, seg_cap: u32, n_seg: *const u32, n_streams: usize, preroll_frames: u32,
                                    cuda_stream: *mut std::os::raw::c_void) -> c_int;

@@ -30,6 +30,15 @@
 //! s.set_wire_preroll(15)?;   // 150 ms before every segment start (after enable_wire_features, which resets it)
 //! ```
 //!
+//! A coarse tick can hold several utterances; the segment table cuts the payload into them and timestamps each:
+//!
+//! ```ignore
+//! s.enable_wire_segments(true)?;
+//! for (k, (p, segs)) in s.wire()?.into_iter().zip(s.wire_segments()?).enumerate() {
+//!     for g in segs { /* samples [g.offset, g.offset + g.n_frames) * 160; onset: tick's first frame + g.frame + g.preroll */ }
+//! }
+//! ```
+//!
 //! Callers whose capture devices differ share one session through `Session::with_formats`; a freed slot takes a caller
 //! with another device through `restart_streams`:
 //!
@@ -79,6 +88,22 @@ pub struct WireFeatures {
     pub logmel: Vec<f32>,
     /// kept frames: `n_frames * 160` payload samples
     pub n_frames: u32,
+}
+
+/// One piece of a segment in one stream's gated payload of one tick (`af_wire_segment`): `offset` and `n_frames` in
+/// payload frames, `frame` relative to the tick's first completed frame, `flags` of `AF_WIRE_SEG_CONTINUED` /
+/// `AF_WIRE_SEG_CLOSED`.
+#[derive(Debug, Clone, Copy, Default, PartialEq, Eq)]
+pub struct WireSegment {
+    /// the piece's first payload frame, relative to the tick's first completed frame (negative: pre-roll of earlier pushes)
+    pub frame: i32,
+    /// payload frame where the piece starts (sample `offset * 160`, feature row `offset`)
+    pub offset: u32,
+    /// payload frames of the piece (0 only for a segment that closes without a frame in the tick)
+    pub n_frames: u32,
+    /// pre-roll frames at the piece's front: the detected onset is `frame + preroll`
+    pub preroll: u16,
+    pub flags: u8,
 }
 
 /// Counts of one stream in one tick (`push_rings` and `push_rings_available` return one per stream).
@@ -259,6 +284,24 @@ impl Session {
     /// `enable_wire_features` sets it back to 0: set it last.
     pub fn set_wire_preroll(&mut self, frames: u32) -> Result<(), AudioError> {
         check(unsafe { ffi::af_session_set_wire_preroll(self.h, frames) })
+    }
+
+    /// Beside the gated payload (`WireGate::Speech`), its segment table on every push, in pinned host rows. Leaves the
+    /// features and the pre-roll as they are.
+    pub fn enable_wire_segments(&mut self, on: bool) -> Result<(), AudioError> {
+        check(unsafe { ffi::af_session_enable_wire_segments(self.h, on as i32, ffi::AF_MEM_HOST) })
+    }
+
+    /// The pieces of the last tick, one list per stream beside `wire()`'s payloads (copied out here).
+    pub fn wire_segments(&self) -> Result<Vec<Vec<WireSegment>>, AudioError> {
+        let mut n = vec![0u32; self.n_streams];
+        let (mut rows, mut stride) = (ptr::null(), 0u64);
+        check(unsafe { ffi::af_session_wire_segments(self.h, &mut rows, &mut stride, n.as_mut_ptr()) })?;
+        Ok(n.iter().enumerate().map(|(k, &c)| {
+            let r = unsafe { std::slice::from_raw_parts(rows.add(k * stride as usize), c as usize) };
+            r.iter().map(|g| WireSegment { frame: g.frame, offset: g.offset, n_frames: g.n_frames, preroll: g.preroll, flags: g.flags })
+                .collect()
+        }).collect())
     }
 
     /// `AudioLevel` / `VolumeLevel` payloads of the last tick: (level_db, peak, is_speech) per stream.

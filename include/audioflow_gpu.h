@@ -460,6 +460,50 @@ AF_API int af_session_wire_features(const af_session *s, const float **rows, uin
  * pre-roll back to 0: set it last. */
 #define AF_WIRE_PREROLL_MAX 100
 AF_API int af_session_set_wire_preroll(af_session *s, uint32_t frames);
+/* ---- wire segments: where each utterance lies in a tick's gated payload -------------------------------------------------
+ * A coarse or ragged tick (1 s ticks, af_session_push_rings_available after a stall) can hold several utterances back to
+ * back, and with a pre-roll a payload reaches back into earlier pushes; the counts of af_wire_tick cannot cut it apart
+ * or timestamp it.  With the gated wire on and its segment table enabled, every push also leaves a list of pieces per
+ * stream.  A piece is the part of one segment that lies in this tick's payload; segments are those of af_vad_segments,
+ * pre-rolled as af_session_set_wire_preroll defines.  Pieces are listed in payload order.  Per stream and tick:
+ *   - pieces tile the payload: the first starts at offset 0, offset[i + 1] == offset[i] + n_frames[i], and
+ *     sum(n_frames) * hop == n_samples;
+ *   - pieces without AF_WIRE_SEG_CONTINUED number `started`, pieces with AF_WIRE_SEG_CLOSED number `ended`; a CONTINUED
+ *     piece comes first, and its n_frames * hop == continued;
+ *   - every piece but the last is CLOSED; the last lacks CLOSED exactly when in_speech is 1.  A tick that completes no
+ *     frame and closes nothing has no pieces, even while a segment is open;
+ *   - closing-only piece: a segment open when the tick began that closes with no payload frame in the tick (the tick's
+ *     first frame is Silence after Speech, or an end comes with no completed frame) is one piece with
+ *     CONTINUED | CLOSED and n_frames = 0, frame = 0.  No other piece has 0 frames;
+ *   - a reset or restart drops an open segment (the next tick has no CONTINUED piece); after an import, a segment open
+ *     in the record continues with a CONTINUED piece; under a pre-roll an import is an origin, as for the payload.
+ * Concatenated since the stream's origin, each CONTINUED piece joined to the open segment and frames made global as
+ * first_frames[k] + frame (af_session_wire_first_frames), the pieces are exactly af_vad_segments (+
+ * af_vad_segments_preroll with the session's P) over the stream's concatenated states, and their cumulative payload
+ * offsets are af_vad_gate's seg_offset.  The table counts VAD frames, so it needs no STFT frames (20 ms VAD frames
+ * work).  Payload sample offset * hop and wire-feature row `offset` are the piece's first. */
+#define AF_WIRE_SEG_CONTINUED 1   /* belongs to the segment open when the tick began */
+#define AF_WIRE_SEG_CLOSED 2      /* the segment closes in this tick: its Ending frame, a Silence frame after Speech, or the end */
+typedef struct af_wire_segment {
+    int32_t frame;            /* the piece's first payload frame, relative to the tick's first completed frame
+                                 (af_session_wire_first_frames[k]); negative when a pre-roll reaches into earlier pushes */
+    uint32_t offset;          /* payload frame index where the piece starts: sample offset * hop, wire-feature row offset */
+    uint32_t n_frames;        /* payload frames of the piece (0 only for the closing-only piece) */
+    uint16_t preroll;         /* pre-roll frames at the piece's front: the detected onset is frame + preroll (0 if CONTINUED) */
+    uint8_t flags;            /* AF_WIRE_SEG_CONTINUED | AF_WIRE_SEG_CLOSED */
+    uint8_t pad;              /* 0 */
+} af_wire_segment;            /* 16 bytes */
+/* enable != 0: mem AF_MEM_HOST (session-owned pinned rows) or AF_MEM_DEVICE (rows on the session's GPU), sized for the
+ * session's bound of frames per tick T: a tick has at most started + 1 pieces and started <= ceil(T / 2), so a row holds
+ * ceil(T / 2) + 1 entries.  enable == 0: off, the rows are freed.  AF_ERR_INVALID, and nothing changes, when the wire
+ * output is off or ungated, or for a bad mem.  Neither the features nor the pre-roll change: unlike the other enable
+ * calls this one does NOT set the pre-roll back to 0 (a row's size does not depend on it).  Every af_session_enable_wire
+ * call turns the table off. */
+AF_API int af_session_enable_wire_segments(af_session *s, int enable, int mem);
+/* The table of the last push: row k (stride entries apart) holds stream k's n_segs[k] pieces, valid until the next
+ * push.  n_segs: host array of n_streams (may be NULL).  AF_ERR_INVALID whenever af_session_wire is (before the first
+ * push since enabling, after an import, after a failed push) and while the table is off. */
+AF_API int af_session_wire_segments(const af_session *s, const af_wire_segment **rows, uint64_t *stride, uint32_t *n_segs);
 
 /* ---- RingBuffer  (src-tauri/src/modules/audio/capture.rs:84-161): capture hand-off ------ */
 /* The cpal callback writes captured f32 samples, the processing task reads them.  Same semantics as the
