@@ -213,6 +213,9 @@ def load_library():
         "af_session_set_wire_preroll": (C.c_int, [vp, C.c_uint32]),
         "af_session_enable_wire_segments": (C.c_int, [vp, C.c_int, C.c_int]),
         "af_session_wire_segments": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
+        "af_batch_set_resampler": (C.c_int, [vp, C.c_uint32]),
+        "af_debug_polyphase_filter": (sz, [C.c_uint32, C.c_uint32, C.POINTER(C.c_float), sz, C.POINTER(C.c_uint32),
+                                           C.POINTER(C.c_uint32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -242,6 +245,28 @@ def _check(rc: int):
     if rc == AF_ERR_CAPACITY:
         raise BufferError(msg)
     raise ValueError(msg)
+
+
+RESAMPLERS = {"cubic": 0, "polyphase": 1}      # AF_RESAMPLE_CUBIC, AF_RESAMPLE_POLYPHASE
+
+
+def _resampler_code(name: str) -> int:
+    if name not in RESAMPLERS:
+        raise ValueError(f"unknown resampler {name!r}: one of {sorted(RESAMPLERS)}")
+    return RESAMPLERS[name]
+
+
+def debug_polyphase_filter(rate: int, out_rate: int = 16000):
+    """(h, p, q): the f32 taps of the polyphase filter for rate -> out_rate (scipy.signal.resample_poly's default
+    filter for f32 input) and the reduced ratio rate / out_rate = p / q.  ValueError when max(p, q) > 65536."""
+    L = load_library()
+    p, q = C.c_uint32(0), C.c_uint32(0)
+    n = L.af_debug_polyphase_filter(rate, out_rate, None, 0, C.byref(p), C.byref(q))
+    if n == 0:
+        raise ValueError(f"{rate} Hz -> {out_rate} Hz: ratio {p.value}/{q.value} is outside the polyphase filter's bound")
+    h = np.empty(n, np.float32)
+    L.af_debug_polyphase_filter(rate, out_rate, h.ctypes.data_as(C.POINTER(C.c_float)), n, None, None)
+    return h, int(p.value), int(q.value)
 
 
 def init(device: int = -1):
@@ -605,6 +630,12 @@ class Batch:
             raise ValueError(f"{len(cfgs)} configs for {self.n} streams")
         _check(load_library().af_batch_set_vad_configs(self._h, _vad_config_array(cfgs)))
 
+    def set_resampler(self, name: str):
+        """"cubic" (the reference's rubato cubic, the default) or "polyphase" (anti-aliased, scipy's resample_poly
+        filter) from the next run; counts and strides stay as they are."""
+        code = _resampler_code(name)
+        _check(load_library().af_batch_set_resampler(self._h, code))
+
     def split(self, out: dict) -> list:
         res = []
         M = self.pipe.cfg.n_mels
@@ -681,6 +712,14 @@ class ShardedBatch:
         if not h:
             return None
         return Batch(self.pipe, None, self.mem, _handle=h, _n=self.shard(rank)[1])
+
+    def set_resampler(self, name: str):
+        """Batch.set_resampler on every rank this process runs."""
+        code = _resampler_code(name)
+        for r in range(self.n_ranks):
+            b = self.local(r)
+            if b is not None:
+                _check(load_library().af_batch_set_resampler(b._h, code))
 
     def run(self, outs: ShardedOutputsC, gather: bool = True, wait: bool = True):
         _check(load_library().af_sharded_batch_run(self._h, C.byref(outs), int(gather), 0 if wait else 1))

@@ -1,5 +1,7 @@
 // af_launch.h -- host-callable launch wrappers implemented in the .cu files.
 #pragma once
+#include <vector>
+
 #include "af_common.cuh"
 
 namespace af {
@@ -200,6 +202,43 @@ struct WirePrerollJob {      // a session tick's gated wire payloads with P fram
 cudaError_t launch_session_wire_preroll(const WirePrerollJob &job, cudaStream_t st);
 // an import: the history of every listed slot becomes empty (one launch for all of them)
 cudaError_t launch_session_preroll_clear(const RecordMove *tab, uint32_t n, uint32_t *hist_n, cudaStream_t st);
+
+// Polyphase resampling of batches (af_polyphase.cu): ratios p / q = in_rate / out_rate (reduced) with max(p, q) <=
+// POLY_MAX_RATIO; L = 10 max(p, q), 2L + 1 taps.  polyphase_ratio is false outside the bound; polyphase_filter writes
+// the taps of resample_poly(x, q, p) for f32 input
+constexpr int POLY_MAX_RATIO = 65536;
+constexpr int FIR_THREADS = 256;
+constexpr int FIR_HOT_R = 7;                          // 48 kHz: consecutive outputs per thread
+constexpr int FIR_HOT_TILE = FIR_THREADS * FIR_HOT_R; // 48 kHz: outputs per tile
+constexpr int FIR_HOT_TAPS = 61;                      // 48 kHz: 2L + 1
+constexpr int FIR_TILE_MAX = 4096;                    // other ratios: outputs per tile, fewer when the stage would not fit
+constexpr int FIR_STAGE_MAX = 12288;                  // other ratios: staged input samples per tile
+constexpr int FIR_TAPS_SMEM = 9216;                   // other ratios: tap tables up to this length are staged per tile
+bool polyphase_ratio(uint32_t in_rate, uint32_t out_rate, uint32_t *p, uint32_t *q);
+void polyphase_filter(uint32_t p, uint32_t q, std::vector<float> *h);
+
+struct FirStream {           // one stream of a FIR launch (device)
+    const void *data;        // interleaved input (f32 / i16)
+    uint64_t n_samples;
+    uint32_t n_in, n_out;    // mono frames; 16 kHz outputs (the cubic path's count)
+    uint32_t channels, format;
+    uint32_t p, q, L;
+    uint32_t tile_out;       // outputs per tile (fir_tile_outputs)
+    const float *h;          // 2L + 1 taps
+    float *y;                // its 16 kHz row (16-byte aligned)
+    uint32_t taps_smem;      // 1: the taps are staged in shared memory
+    uint32_t pad_;
+};
+struct FirJob {              // one launch: every tile of a sub-batch
+    const FirStream *streams;
+    const uint2 *tiles;      // (stream, tile index within the stream)
+    uint32_t n_tiles;
+    uint32_t smem_floats;    // dynamic shared memory: the largest fir_smem_floats of the launch's streams
+    float h3[FIR_HOT_TAPS];  // the 48 kHz taps (p = 3, q = 1), read as constant operands
+};
+uint32_t fir_tile_outputs(uint32_t p, uint32_t q);
+size_t fir_smem_floats(uint32_t p, uint32_t q, bool taps_smem);
+cudaError_t launch_polyphase_fir(const FirJob &job, cudaStream_t st);
 
 size_t fused_smem_bytes();
 cudaError_t fused_pipe_stats(unsigned long long out[32]);

@@ -836,6 +836,18 @@ struct SubBatch {                     // a group of streams resident on the devi
     bool no_merge = false;            // host mode: a merged copy was refused (rows adjacent in memory but separately allocated)
 };
 
+// af_batch_set_resampler(AF_RESAMPLE_POLYPHASE): the FIR writes each sub-batch's 16 kHz rows into a scratch block and
+// the fused kernel runs over them as 16 kHz mono f32 streams (counts, frames and strides are the batch's own)
+struct Polyphase {
+    std::vector<HostStream> rows;             // stream i as the fused kernel sees it: 16 kHz mono f32, n_in = n_out
+    std::map<uint32_t, DevBuf<float>> taps;   // one tap table per input rate of the batch
+    std::vector<DevBuf<float>> d_rows;        // the rows: one block (device batches) or one per slot (host batches)
+    std::vector<SubBatch> subs;               // the fused plan of each sub-batch over its rows
+    std::vector<FirJob> jobs;                 // the FIR launch of each sub-batch
+    std::vector<DevBuf<FirStream>> d_fir;
+    std::vector<DevBuf<uint2>> d_tiles;
+};
+
 }  // namespace
 
 struct af_batch {
@@ -858,13 +870,14 @@ struct af_batch {
     };
     std::vector<Slot> slots;
     size_t slot_rows = 0;
+    std::unique_ptr<Polyphase> poly;  // polyphase resampling (af_batch_set_resampler), or null: the cubic path
 };
 
 namespace {
 
-int build_sub(af_batch *b, SubBatch &sb, const void *slot_in_base)
+int build_sub(const std::vector<HostStream> &streams, SubBatch &sb, const void *slot_in_base)
 {
-    // (re)build the device tables of a sub-batch; slot_in_base != null (host mode) rebases the inputs
+    // (re)build the device tables of a sub-batch; slot_in_base != null (host mode, polyphase rows) rebases the inputs
     sb.h_streams.resize(sb.count);
     sb.h_tiles.clear();
     sb.quarters = false;
@@ -872,7 +885,7 @@ int build_sub(af_batch *b, SubBatch &sb, const void *slot_in_base)
     sb.split = false;
     std::vector<uint32_t> nf(sb.count), nv(sb.count);
     for (size_t i = 0; i < sb.count; ++i) {
-        const HostStream &hs = b->streams[sb.first + i];
+        const HostStream &hs = streams[sb.first + i];
         StreamDev &d = sb.h_streams[i];
         memset(&d, 0, sizeof(d));
         d.data = slot_in_base ? (const void *)((const char *)slot_in_base + sb.in_off[i]) : hs.desc.data;
@@ -918,17 +931,23 @@ int build_sub(af_batch *b, SubBatch &sb, const void *slot_in_base)
     return AF_OK;
 }
 
-// enqueue the kernels of one sub-batch on `st`; all pointers are device pointers of rows [0, sb.count)
-int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *logmel, uint64_t logmel_stride,
+// enqueue the kernels of sub-batch g on `st`; all pointers are device pointers of rows [0, sb.count)
+int run_sub(af_batch *b, size_t g, float *pcm, uint64_t pcm_stride, float *logmel, uint64_t logmel_stride,
             uint8_t *vad, uint64_t vad_stride, float *energy, uint64_t energy_stride, VadState *vad_final,
             cudaStream_t st)
 {
     const af_pipeline_config &cfg = b->pipe->cfg;
     const bool stft_vad = cfg.vad_enable && cfg.vad_frame_len == 0;
     const bool custom_vad = cfg.vad_enable && cfg.vad_frame_len != 0;
-    if (!sb.h_tiles.empty()) {
+    SubBatch &sb = b->subs[g];
+    const SubBatch &fp = b->poly ? b->poly->subs[g] : sb;     // what the fused kernel reads: the FIR's rows or the input
+    if (b->poly && b->poly->jobs[g].n_tiles) {
+        AF_CUDA(launch_polyphase_fir(b->poly->jobs[g], st));
+        count_launch();
+    }
+    if (!fp.h_tiles.empty()) {
         FusedParams P{};
-        P.streams = sb.d_streams.get(); P.tiles = sb.d_tiles.get(); P.n_tiles = (uint32_t)sb.h_tiles.size();
+        P.streams = fp.d_streams.get(); P.tiles = fp.d_tiles.get(); P.n_tiles = (uint32_t)fp.h_tiles.size();
         P.fft = cur_ctx().d_fft.get(); P.mel = b->d_mel;
         P.pcm = pcm; P.pcm_stride = pcm_stride;
         P.logmel = cfg.n_mels ? logmel : nullptr; P.logmel_stride = logmel_stride;
@@ -939,11 +958,11 @@ int run_sub(af_batch *b, SubBatch &sb, float *pcm, uint64_t pcm_stride, float *l
         P.log_scale = cfg.log10 ? 0.30102999566398120f : 0.69314718055994531f;   // log10(2) : ln(2)
         P.use_stage = kernel_variant() == "sync" ? 0u : 1u;
         P.layout = fused_layout(stft_vad);
-        P.quarters = sb.quarters ? 1u : 0u;
+        P.quarters = fp.quarters ? 1u : 0u;
         P.neg_zero = -0.0f;
-        P.per_p = sb.per_p; P.per_q = sb.per_q;
-        const int n_ctas = (int)std::min<size_t>(sb.h_tiles.size(), (size_t)cur_ctx().sm_count);   // one persistent CTA per SM
-        AF_CUDA(launch_fused(P, n_ctas, st, sb.split));
+        P.per_p = fp.per_p; P.per_q = fp.per_q;
+        const int n_ctas = (int)std::min<size_t>(fp.h_tiles.size(), (size_t)cur_ctx().sm_count);   // one persistent CTA per SM
+        AF_CUDA(launch_fused(P, n_ctas, st, fp.split));
         count_launch();
     }
     if (custom_vad) {
@@ -1098,7 +1117,7 @@ AF_API int af_batch_create(af_pipeline *p, const af_stream_desc *streams, size_t
     if (mem == AF_MEM_DEVICE) {
         b->subs.resize(1);
         b->subs[0].first = 0; b->subs[0].count = n_streams;
-        if (n_streams) { rc = build_sub(b.get(), b->subs[0], nullptr); if (rc) return rc; }
+        if (n_streams) { rc = build_sub(b->streams, b->subs[0], nullptr); if (rc) return rc; }
     } else {
         // host mode: groups of streams of ~32 MB input (measured: 96 MB 29.4 ms, 32 MB 28.3 ms per cfg2 batch against a
         // PCIe ceiling of 28.1 ms on the box), cycled through 3 slots so that the H2D copy of
@@ -1140,7 +1159,7 @@ AF_API int af_batch_create(af_pipeline *p, const af_stream_desc *streams, size_t
             }
         }
         for (size_t g = 0; g < b->subs.size(); ++g) {
-            rc = build_sub(b.get(), b->subs[g], b->slots[g % n_slots].d_in.get());
+            rc = build_sub(b->streams, b->subs[g], b->slots[g % n_slots].d_in.get());
             if (rc) return rc;
         }
     }
@@ -1233,7 +1252,7 @@ int batch_run_on(af_batch *b, const af_outputs *o, uint8_t *vad, uint64_t vad_st
         AF_CUDA(b->d_pcm_scratch.grow(min256<float>(S * b->pcm_stride)));
         pcm = b->d_pcm_scratch.get(); pcm_stride = b->pcm_stride;
     }
-    int rc = run_sub(b, b->subs[0], pcm, pcm_stride, o->logmel, o->logmel_stride, vad, vad_stride, energy, energy_stride,
+    int rc = run_sub(b, 0, pcm, pcm_stride, o->logmel, o->logmel_stride, vad, vad_stride, energy, energy_stride,
                      reinterpret_cast<VadState *>(o->vad_final), st);
     if (rc) return rc;
     if (wire16) {                                                // websocket.rs:246-251 on the rows, 2 bytes per sample out
@@ -1301,7 +1320,7 @@ AF_API int af_batch_run_host(af_batch *b, const af_outputs *o)
             i = j;
         }
         const bool need_pcm = (cfg.write_pcm && o->pcm) || (cfg.vad_enable && cfg.vad_frame_len != 0);
-        rc = run_sub(b, sb, need_pcm ? sl.d_pcm.get() : nullptr, b->pcm_stride, sl.d_logmel.get(), b->logmel_stride, sl.d_vad.get(),
+        rc = run_sub(b, g, need_pcm ? sl.d_pcm.get() : nullptr, b->pcm_stride, sl.d_logmel.get(), b->logmel_stride, sl.d_vad.get(),
                      b->vad_stride, sl.d_energy.get(), b->energy_stride, sl.d_final.get(), st);
         if (rc) return rc;
         const size_t r0 = sb.first;
@@ -1369,6 +1388,110 @@ AF_API int af_batch_set_vad_configs(af_batch *b, const af_vad_config *cfgs)
         b->subs[g].n_seq = n_seq[g];
     }
     return AF_OK;
+}
+
+AF_API int af_batch_set_resampler(af_batch *b, uint32_t filter)
+{
+    if (!b) return fail(AF_ERR_INVALID, "null batch");
+    if (filter != AF_RESAMPLE_CUBIC && filter != AF_RESAMPLE_POLYPHASE) return fail(AF_ERR_INVALID, "unknown resampling filter %u", filter);
+    const size_t S = b->streams.size();
+    for (size_t i = 0; i < S && filter == AF_RESAMPLE_POLYPHASE; ++i) {
+        uint32_t p, q;
+        if (!polyphase_ratio(b->streams[i].desc.sample_rate, OUT_RATE, &p, &q))
+            return fail(AF_ERR_RESAMPLING_FAILED, "stream %zu: %u Hz -> %d Hz reduces to %u / %u; the polyphase filter takes max(p, q) <= %d",
+                        i, b->streams[i].desc.sample_rate, OUT_RATE, p, q, POLY_MAX_RATIO);
+    }
+    AF_SCOPE(b->device);
+    if (filter == AF_RESAMPLE_CUBIC) {
+        if (b->poly) {
+            AF_CUDA(cudaDeviceSynchronize());     // runs still in flight read the rows
+            b->poly.reset();
+        }
+        return AF_OK;
+    }
+    // everything is built before anything changes
+    auto ph = std::make_unique<Polyphase>();
+    std::map<uint32_t, std::vector<float>> h_taps;
+    for (const HostStream &hs : b->streams) {
+        const uint32_t rate = hs.desc.sample_rate;
+        if (h_taps.count(rate)) continue;
+        uint32_t p, q;
+        polyphase_ratio(rate, OUT_RATE, &p, &q);
+        polyphase_filter(p, q, &h_taps[rate]);
+        const std::vector<float> &h = h_taps[rate];
+        AF_CUDA(ph->taps[rate].alloc(h.size()));
+        AF_CUDA(cudaMemcpy(ph->taps[rate].get(), h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
+    }
+    ph->rows.resize(S);
+    for (size_t i = 0; i < S; ++i) {
+        const HostStream &hs = b->streams[i];
+        HostStream &r = ph->rows[i];
+        r = hs;
+        r.desc.data = nullptr; r.desc.n_samples = hs.n_out; r.desc.sample_rate = OUT_RATE;
+        r.desc.channels = 1; r.desc.format = AF_FMT_F32;
+        r.n_in = hs.n_out; r.mode = RS_PASSTHROUGH; r.p = r.q = 1; r.table.reset();
+    }
+    const size_t n_blocks = b->mem == AF_MEM_DEVICE ? 1 : b->slots.size();
+    const size_t block_rows = b->mem == AF_MEM_DEVICE ? S : b->slot_rows;
+    ph->d_rows.resize(n_blocks);
+    for (auto &d : ph->d_rows) AF_CUDA(d.alloc(min256<float>(block_rows * b->pcm_stride)));
+    const size_t G = b->subs.size();
+    ph->subs.resize(G); ph->jobs.resize(G); ph->d_fir.resize(G); ph->d_tiles.resize(G);
+    for (size_t g = 0; g < G; ++g) {
+        const SubBatch &sb = b->subs[g];
+        float *rows = ph->d_rows[g % n_blocks].get();
+        const char *in_base = b->mem == AF_MEM_DEVICE ? nullptr : b->slots[g % b->slots.size()].d_in.get();
+        SubBatch &fp = ph->subs[g];
+        fp.first = sb.first; fp.count = sb.count;
+        std::vector<FirStream> fs(sb.count);
+        std::vector<uint2> tiles;
+        FirJob &J = ph->jobs[g];
+        J = FirJob{};
+        for (size_t i = 0; i < sb.count; ++i) {
+            const HostStream &hs = b->streams[sb.first + i];
+            FirStream &f = fs[i];
+            memset(&f, 0, sizeof(f));
+            f.data = in_base ? (const void *)(in_base + sb.in_off[i]) : hs.desc.data;
+            f.n_samples = hs.desc.n_samples; f.n_in = hs.n_in; f.n_out = hs.n_out;
+            f.channels = hs.desc.channels; f.format = hs.desc.format;
+            polyphase_ratio(hs.desc.sample_rate, OUT_RATE, &f.p, &f.q);
+            f.L = 10 * std::max(f.p, f.q);
+            f.tile_out = fir_tile_outputs(f.p, f.q);
+            f.h = ph->taps[hs.desc.sample_rate].get();
+            f.y = rows + i * b->pcm_stride;
+            f.taps_smem = 2 * f.L + 1 <= (uint32_t)FIR_TAPS_SMEM ? 1u : 0u;
+            if (f.p == 3 && f.q == 1) memcpy(J.h3, h_taps[hs.desc.sample_rate].data(), sizeof(J.h3));
+            const uint32_t n_tiles = (hs.n_out + f.tile_out - 1) / f.tile_out;
+            for (uint32_t t = 0; t < n_tiles; ++t) tiles.push_back(make_uint2((uint32_t)i, t));
+            if (n_tiles) J.smem_floats = std::max<uint32_t>(J.smem_floats, (uint32_t)fir_smem_floats(f.p, f.q, f.taps_smem));
+            fp.in_off.push_back(i * b->pcm_stride * sizeof(float));
+        }
+        AF_CUDA(ph->d_fir[g].alloc(std::max<size_t>(sb.count, 1)));
+        AF_CUDA(ph->d_tiles[g].alloc(std::max<size_t>(tiles.size(), 1)));
+        if (sb.count) AF_CUDA(cudaMemcpy(ph->d_fir[g].get(), fs.data(), sb.count * sizeof(FirStream), cudaMemcpyHostToDevice));
+        if (!tiles.empty()) AF_CUDA(cudaMemcpy(ph->d_tiles[g].get(), tiles.data(), tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice));
+        J.streams = ph->d_fir[g].get(); J.tiles = ph->d_tiles[g].get(); J.n_tiles = (uint32_t)tiles.size();
+        if (sb.count) {
+            int rc = build_sub(ph->rows, fp, rows);
+            if (rc) return rc;
+        }
+    }
+    AF_CUDA(cudaDeviceSynchronize());             // runs still in flight read the previous rows
+    b->poly = std::move(ph);
+    return AF_OK;
+}
+
+AF_API size_t af_debug_polyphase_filter(uint32_t input_rate, uint32_t output_rate, float *h, size_t cap, uint32_t *p, uint32_t *q)
+{
+    uint32_t p_ = 0, q_ = 0;
+    const bool ok = polyphase_ratio(input_rate, output_rate, &p_, &q_);
+    if (p) *p = p_;
+    if (q) *q = q_;
+    if (!ok) return 0;
+    std::vector<float> t;
+    polyphase_filter(p_, q_, &t);
+    for (size_t i = 0; i < t.size() && i < cap && h; ++i) h[i] = t[i];
+    return t.size();
 }
 
 AF_API int af_pipeline_run(af_pipeline *p, const af_stream_desc *streams, size_t n_streams, const af_outputs *out)

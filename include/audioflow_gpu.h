@@ -238,6 +238,24 @@ AF_API int af_batch_run_host(af_batch *b, const af_outputs *out);
  * the parallel one: such a batch enqueues one more kernel.  AF_ERR_INVALID when the pipeline has vad_enable == 0.
  * Sharded batches: af_sharded_batch_local(b, r) is an ordinary batch; give each local rank the slice of its streams. */
 AF_API int af_batch_set_vad_configs(af_batch *b, const af_vad_config *cfgs);
+/* Resampling filter of a batch.  AF_RESAMPLE_CUBIC (the default) is the reference's rubato FastFixedIn cubic, which has
+ * no anti-alias filter: everything between 8 kHz and the input's Nyquist folds into the 0-8 kHz band.
+ * AF_RESAMPLE_POLYPHASE is scipy.signal.resample_poly(m, q, p)'s default filter on the downmix m, for R / 16000 = p / q
+ * reduced and L = 10 max(p, q): h = firwin(2L + 1, 1 / max(p, q), window=('kaiser', 5.0)) in f64, cast to f32, times
+ * (float)q; y[n] = sum_k m[k] h[n p + L - k q] over ascending k (m = 0 outside the stream) as a chain of fmaf from
+ * +0.0f; 16 kHz streams are copied.  Passband within 0.02 dB to 6 kHz, at most -56.8 dB from 10 kHz up (for every rate
+ * above 16 kHz), -6 dB at 8 kHz.  Counts and strides do not change (n_out stays the cubic path's), and everything
+ * downstream (PCM rows, pcm16, log-mel, energies, VAD) is what the batch computes for 16 kHz mono f32 streams holding
+ * y[0 .. n_out).  Every stream's rate must reduce to max(p, q) <= 65536 (every common capture rate does), else
+ * AF_ERR_RESAMPLING_FAILED naming the first stream that does not; AF_ERR_INVALID for a null batch or an unknown
+ * filter.  On an error nothing changes.  The filter applies from the next af_batch_run / af_batch_run_host.
+ * AF_RESAMPLE_CUBIC frees what the polyphase filter allocated (a 16 kHz row block, tap tables and tile tables).
+ * Sharded batches: set it on af_sharded_batch_local(b, r) for each local rank. */
+enum { AF_RESAMPLE_CUBIC = 0, AF_RESAMPLE_POLYPHASE = 1 };
+AF_API int af_batch_set_resampler(af_batch *b, uint32_t filter);
+/* The polyphase taps for input_rate -> output_rate (host only, no GPU needed): returns 2L + 1 and writes the first cap
+ * taps to h and the reduced ratio to *p, *q (any may be NULL); 0 when max(p, q) > 65536. */
+AF_API size_t af_debug_polyphase_filter(uint32_t input_rate, uint32_t output_rate, float *h, size_t cap, uint32_t *p, uint32_t *q);
 /* One-shot convenience: create + run_host + destroy. */
 AF_API int af_pipeline_run(af_pipeline *p, const af_stream_desc *streams, size_t n_streams,
                            const af_outputs *out);
