@@ -178,6 +178,7 @@ def load_library():
         "af_sharded_batch_run_host": (C.c_int, [vp, C.POINTER(OutputsC)]),
         "af_debug_vad_energy_threshold": (C.c_float, [C.c_float]),
         "af_debug_resample_plan": (sz, [C.c_uint32, C.c_uint32, sz, fp, sz, C.POINTER(C.c_int)]),
+        "af_debug_tile_order": (C.c_uint64, [C.POINTER(C.c_uint32), sz, C.c_uint32, C.POINTER(C.c_uint32)]),
         "af_session_create": (C.c_int, [vp, sz, C.c_uint32, C.c_uint16, C.c_uint16, C.c_uint32, C.POINTER(vp)]),
         "af_session_destroy": (None, [vp]),
         "af_session_push": (C.c_int, [vp, vp, C.c_uint64, C.c_uint32, C.c_int, C.POINTER(OutputsC),

@@ -153,7 +153,7 @@ struct StreamDev {
     uint32_t p, q;           // input step per output = p / q (reduced)
     uint32_t mode;           // RS_*
     const float *frac;       // RS_TABLE: f32 fractional offsets by output index
-    uint32_t tile_begin;     // first global tile of this stream
+    uint32_t tile_begin;     // first tile of this stream in planning order (batches launch them in balance_tile_order)
     uint32_t n_tiles;
     uint32_t staged;         // parts per step when the input is staged through shared memory (2 or 4); 0: it does not fit
                              // (taps come from global memory; the step still runs as two parts)

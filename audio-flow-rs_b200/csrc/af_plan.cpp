@@ -6,6 +6,7 @@
 #include <cstring>
 #include <limits>
 #include <numeric>
+#include <queue>
 
 namespace af {
 
@@ -173,6 +174,41 @@ float vad_energy_threshold(float threshold_db)
         if (speech(bits_to_f32(mid))) hi = mid; else lo = mid;
     }
     return bits_to_f32(hi);
+}
+
+uint64_t tile_order_max_steps(const std::vector<uint32_t> &steps, const std::vector<uint32_t> &order, uint32_t n_ctas)
+{
+    if (n_ctas == 0) return 0;
+    std::vector<uint64_t> load(n_ctas, 0);
+    for (size_t i = 0; i < order.size(); ++i) load[i % n_ctas] += steps[order[i]];
+    return *std::max_element(load.begin(), load.end());
+}
+
+std::vector<uint32_t> balance_tile_order(const std::vector<uint32_t> &steps, uint32_t n_ctas)
+{
+    const size_t n = steps.size();
+    std::vector<uint32_t> order(n);
+    std::iota(order.begin(), order.end(), 0u);
+    if (n_ctas == 0 || n <= n_ctas) return order;          // one tile per CTA at most: nothing to balance
+    // CTA c walks a fixed number of positions (ceil or floor of n / n_ctas).  Longest tile first, each to the least
+    // loaded CTA that still has a free position; ties go to the lower CTA index.
+    std::vector<uint32_t> by_len(order);
+    std::stable_sort(by_len.begin(), by_len.end(), [&](uint32_t a, uint32_t b) { return steps[a] > steps[b]; });
+    std::vector<uint64_t> load(n_ctas, 0);
+    std::vector<uint32_t> used(n_ctas, 0);
+    std::vector<uint32_t> balanced(n);
+    using Key = std::pair<uint64_t, uint32_t>;               // (load, CTA)
+    std::priority_queue<Key, std::vector<Key>, std::greater<Key>> open;
+    for (uint32_t c = 0; c < n_ctas; ++c) open.push({0, c});
+    for (const uint32_t t : by_len) {
+        const uint32_t c = open.top().second;
+        open.pop();
+        balanced[c + (size_t)used[c] * n_ctas] = t;
+        load[c] += steps[t];
+        if (c + (size_t)(++used[c]) * n_ctas < n) open.push({load[c], c});
+    }
+    if (tile_order_max_steps(steps, balanced, n_ctas) < tile_order_max_steps(steps, order, n_ctas)) order.swap(balanced);
+    return order;
 }
 
 }  // namespace af

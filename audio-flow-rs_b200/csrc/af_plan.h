@@ -35,5 +35,12 @@ void build_fft_tables(FftTables *t);
 bool build_mel_tables(uint32_t n_mels, float f_min, float f_max, MelTables *t);
 // smallest f32 e with 20*log10f(e) > threshold_db under the host libm; NaN if none
 float vad_energy_threshold(float threshold_db);
+// Launch order of the tiles of one fused launch over n_ctas CTAs, CTA c running the tiles at positions c, c + n_ctas,
+// c + 2 n_ctas, ...: order[i] is the tile (index into steps) placed at position i, chosen so that the CTAs' step counts
+// are as even as the fixed number of positions each CTA walks allows.  Never more steps on the busiest CTA than the
+// identity order gives.
+std::vector<uint32_t> balance_tile_order(const std::vector<uint32_t> &steps, uint32_t n_ctas);
+// steps on the busiest CTA when the tiles run in that order
+uint64_t tile_order_max_steps(const std::vector<uint32_t> &steps, const std::vector<uint32_t> &order, uint32_t n_ctas);
 
 }  // namespace af

@@ -919,6 +919,16 @@ int build_sub(const std::vector<HostStream> &streams, SubBatch &sb, const void *
         }
         nf[i] = hs.n_frames; nv[i] = hs.n_vad_frames;
     }
+    {   // a stream's last tile is often short: lay the tiles out so that every CTA of the launch (run_sub) gets a near-equal
+        // share of the steps -- the kernel ends with its busiest CTA
+        std::vector<uint32_t> steps(sb.h_tiles.size());
+        for (size_t t = 0; t < steps.size(); ++t) steps[t] = sb.h_tiles[t].n_steps;
+        const std::vector<uint32_t> order = balance_tile_order(steps, (uint32_t)std::min<size_t>(steps.size(), (size_t)cur_ctx().sm_count));
+        std::vector<TileDev> planned;
+        planned.swap(sb.h_tiles);
+        sb.h_tiles.reserve(planned.size());
+        for (const uint32_t t : order) sb.h_tiles.push_back(planned[t]);
+    }
     AF_CUDA(sb.d_streams.grow(sb.count));
     AF_CUDA(sb.d_tiles.grow(sb.h_tiles.size() + 1));
     AF_CUDA(sb.d_nframes.grow(sb.count));
@@ -1517,6 +1527,14 @@ AF_API size_t af_debug_resample_plan(uint32_t input_rate, uint32_t output_rate, 
     for (size_t c = 0; c < n_chunks; ++c) r.step(&f);
     for (size_t i = 0; i < f.size() && i < cap; ++i) frac[i] = f[i];
     return f.size();
+}
+
+AF_API uint64_t af_debug_tile_order(const uint32_t *steps, size_t n, uint32_t n_ctas, uint32_t *order)
+{
+    const std::vector<uint32_t> st(steps, steps + n);
+    const std::vector<uint32_t> o = balance_tile_order(st, n_ctas);
+    std::copy(o.begin(), o.end(), order);
+    return tile_order_max_steps(st, o, n_ctas);
 }
 
 }  // extern "C"

@@ -364,6 +364,9 @@ AF_API float af_debug_vad_energy_threshold(float threshold_db);
  * an (input_rate -> output_rate) stream; returns the number of outputs (may exceed cap). */
 AF_API size_t af_debug_resample_plan(uint32_t input_rate, uint32_t output_rate, size_t n_chunks, float *frac,
                                      size_t cap, int *mode);
+/* the order in which a batch launches its tiles over n_ctas CTAs (CTA c runs positions c, c + n_ctas, ...), given
+ * each tile's step count: order[i] = tile placed at position i (n entries).  Returns the step count of the busiest CTA. */
+AF_API uint64_t af_debug_tile_order(const uint32_t *steps, size_t n, uint32_t n_ctas, uint32_t *order);
 
 /* ---- streaming sessions (persistent per-stream state; BASELINE config 5) ---------------- */
 typedef struct af_session af_session;
